@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — AV-HuBERT-Large encoder 6 s-clips/sec on N B200s (BASELINE.json metric), one JSON line.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 A "step" is one pass of the hot path (AVHubertModel.extract_finetune, audio+video) over one batch of
@@ -263,7 +263,14 @@ def main():
     ap.add_argument("--config5-steps", type=int, default=5,
                     help="timed fine-tuning steps of BASELINE config 5 (forward + backward + gradient all-reduce; 0 = skip)")
     ap.add_argument("--profile-json", default=None, help="write the per-kernel-class breakdown here")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the features the last timed step returned (rank 0) as DIR/features.npy, float32, so that "
+                         "two builds can be compared output for output (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -377,6 +384,11 @@ def main():
     ms = e0.elapsed_time(e1)
     clocks_timed = sampler.summary(t_region0, t_region1)
     checksum = float(y.float().abs().mean().item())
+    if args.dump_outputs and rank == 0:
+        # [16, 150, 1024] bf16 -> float32 (exact), 9.8 MB; the padding mask extract_finetune returns is None here
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "features.npy"), y.float().cpu().numpy())
 
     # ---- sustained leg: >= SUSTAIN_S seconds of back-to-back steps (the driver-sized region above is ~0.1 s, i.e.
     #      burst clocks); reports what the power cap does to the rate over seconds

@@ -32,6 +32,12 @@ def _grads_for(rank, params):
     return [torch.randn(p.shape, generator=g) for p in params]
 
 
+def _by_value(arrays):
+    """Workers send results as numpy arrays, which a queue pickles by value.  A CPU tensor would travel as a file
+    descriptor that the parent fetches from the worker while unpickling, and rank 0 may have exited by then."""
+    return [None if a is None else torch.from_numpy(a) for a in arrays]
+
+
 def _worker(rank, world, port, q):
     os.environ["MASTER_ADDR"] = "127.0.0.1"
     os.environ["MASTER_PORT"] = str(port)
@@ -51,9 +57,9 @@ def _worker(rank, world, port, q):
         assert red.all_reduce_grads() == 0
         assert torch.equal(params[0].grad, grads[0])     # untouched inside no_sync
     n = red.all_reduce_grads()
-    out = [None if p.grad is None else p.grad.clone() for p in params]
+    out = [None if p.grad is None else p.grad.numpy().copy() for p in params]
     if rank == 0:
-        q.put((n, out))
+        q.put((n, out))        # numpy arrays: see _by_value
     dist.barrier()
     dist.destroy_process_group()
 
@@ -66,6 +72,7 @@ def test_gradient_all_reduce_two_ranks_gloo():
     for p in procs:
         p.start()
     n, out = q.get(timeout=120)
+    out = _by_value(out)
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
@@ -104,13 +111,13 @@ def _worker_presynced(rank, world, port, q):
     # the device backward reports what it already averaged (mark_reduced): those gradients must not be reduced twice
     red.mark_reduced([params[0], params[2]])
     n1 = red.all_reduce_grads()
-    first = [p.grad.clone() for p in params]
+    first = [p.grad.numpy().copy() for p in params]
     n2 = red.all_reduce_grads()                           # the mark is per step: the next call reduces everything again
-    second = [p.grad.clone() for p in params]
+    second = [p.grad.numpy().copy() for p in params]
     # off an NCCL group (gloo here) the bucketed overlap declines and leaves the work to all_reduce_grads
     declined = red.reduce_buckets(None, None, torch.zeros(4)) is False
     if rank == 0:
-        q.put((n1, n2, first, second, declined))
+        q.put((n1, n2, first, second, declined))        # numpy arrays: see _by_value
     dist.barrier()
     dist.destroy_process_group()
 
@@ -123,6 +130,7 @@ def test_gradients_reduced_during_the_backward_are_skipped_once():
     for p in procs:
         p.start()
     n1, n2, first, second, declined = q.get(timeout=120)
+    first, second = _by_value(first), _by_value(second)
     for p in procs:
         p.join(timeout=60)
         assert p.exitcode == 0
