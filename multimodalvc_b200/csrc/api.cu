@@ -52,9 +52,6 @@ int device_sm_count() {
   if (dev != cached_dev) {
     int n = 0;
     if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) == cudaSuccess && n > 0) cached_n = n;
-    // experiment knob: persistent kernels size their grids for this many SMs (e.g. half the chip per CUDA stream)
-    const char* ev = std::getenv("AVH_SM_LIMIT");
-    if (ev != nullptr && std::atoi(ev) > 0 && std::atoi(ev) < cached_n) cached_n = std::atoi(ev);
     cached_dev = dev;
   }
   return cached_n;
@@ -151,10 +148,6 @@ struct LayerW {
   // packed for trainable handles (cfg.reserved[3] != 0), bias pointers unused
   LinearW qkvT, outT, fc1T, fc2T;
   float *ln1_g = nullptr, *ln1_b = nullptr, *ln2_g = nullptr, *ln2_b = nullptr;
-  // LayerNorm folded into the consuming GEMM (bf16 mode, pre-LN): W' = W diag(gamma), csum[n] = sum_k bf16(W'[n,k]),
-  // bias' [n] = b[n] + sum_k W[n,k] beta[k]
-  LinearW qkv_ln, fc1_ln;
-  float *qkv_csum = nullptr, *fc1_csum = nullptr;
 };
 
 // Q-Former (src/sub_model/Qformer.py) handle: BERT-style post-LN layers over the query tokens, each = self-attention,
@@ -515,26 +508,6 @@ bool pack_linear(Packer& pk, const std::string& prefix, LinearW* lw, float wscal
   return true;
 }
 
-// W [n,k], b [n] (already scaled) with the preceding LayerNorm's gamma / beta folded in (see LayerW)
-void pack_ln_folded(Packer& pk, const std::vector<float>& w, const std::vector<float>& b, int n, int k,
-                    const std::vector<float>& gamma, const std::vector<float>& beta, LinearW* lw, float** csum) {
-  std::vector<float> wf((size_t)n * k), cs(n), bf(n);
-  for (int r = 0; r < n; ++r) {
-    double c = 0.0, d = 0.0;
-    for (int j = 0; j < k; ++j) {
-      const float x = w[(size_t)r * k + j] * gamma[j];
-      wf[(size_t)r * k + j] = x;
-      c += (double)bf2f(f2bf(x));                 // the GEMM multiplies the bf16-rounded weight
-      d += (double)w[(size_t)r * k + j] * (double)beta[j];
-    }
-    cs[r] = (float)c;
-    bf[r] = (float)((double)b[r] + d);
-  }
-  lw->w = pk.pack(wf, n, k, k);
-  lw->bias = pk.upload_f(bf);
-  *csum = pk.upload_f(cs);
-}
-
 // several nn.Linear with the same input stacked along the output dim (fused q / k / v, the K / V of all layers)
 bool pack_linear_cat(Packer& pk, const std::vector<std::string>& prefixes, LinearW* lw) {
   std::vector<float> wcat, bcat;
@@ -799,20 +772,9 @@ bool pack_all(Packer& pk) {
           pk.job(pre + nm[t] + ".bias", RJ_VEC_OFF, lw.qkv.bias, D, 0, 0, (long long)t * D, t == 0 ? qscale : 1.f);
         }
       }
-      const HostTensor* g1 = pk.get(pre + "self_attn_layer_norm.weight");
-      const HostTensor* b1 = pk.get(pre + "self_attn_layer_norm.bias");
-      if (g1 && b1 && c.layer_norm_first && h->P == 1) pack_ln_folded(pk, w, b, 3 * D, D, g1->v, b1->v, &lw.qkv_ln, &lw.qkv_csum);
     } else ok = false;
     ok &= pack_linear(pk, pre + "self_attn.out_proj", &lw.out);
     ok &= pack_linear(pk, pre + "fc1", &lw.fc1);
-    {
-      const HostTensor* w1 = pk.get(pre + "fc1.weight");
-      const HostTensor* bb1 = pk.get(pre + "fc1.bias");
-      const HostTensor* g2 = pk.get(pre + "final_layer_norm.weight");
-      const HostTensor* b2 = pk.get(pre + "final_layer_norm.bias");
-      if (w1 && bb1 && g2 && b2 && c.layer_norm_first && h->P == 1)
-        pack_ln_folded(pk, w1->v, bb1->v, (int)w1->shape[0], (int)w1->shape[1], g2->v, b2->v, &lw.fc1_ln, &lw.fc1_csum);
-    }
     ok &= pack_linear(pk, pre + "fc2", &lw.fc2);
     if (c.reserved[3] != 0) {      // trainable handle: W^T operands of the dgrad GEMMs (avh_encoder_backward)
       ok &= pack_linear_T(pk, {pre + "self_attn.q_proj", pre + "self_attn.k_proj", pre + "self_attn.v_proj"},
@@ -913,20 +875,6 @@ struct Builder {
     pr.a_col_nblk = a_col_nblk;
     pr.block_n = block_n;
     pr.sk_ws = sk_ws; pr.sk_ws_bytes = sk_bytes; pr.sk_flags = sk_flags;
-    {   // tuning knob: AVH_GEMM_BN="fc1:256,qkv_proj:192" forces the tile width of a kernel class
-      static const char* ov = std::getenv("AVH_GEMM_BN");
-      if (ov != nullptr && block_n == 0) {
-        const std::string key = tag + ":";
-        const std::string all(ov);
-        size_t pos = 0;
-        while (pos < all.size()) {
-          const size_t end = all.find(',', pos) == std::string::npos ? all.size() : all.find(',', pos);
-          const std::string item = all.substr(pos, end - pos);
-          if (item.compare(0, key.size(), key) == 0) pr.block_n = std::atoi(item.c_str() + key.size());
-          pos = end + 1;
-        }
-      }
-    }
     pr.ep = ep;
     if (sizing) return true;
     GemmPlan* gp = new GemmPlan();
@@ -1032,10 +980,8 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     if (rg) CB = B;                                                  // ragged: one chunk of Nb packed frames
     const int CF = rg ? (int)N : CB * T;
     FrontendBufs fb;
-    static int stemf_env0 = -1;
-    if (stemf_env0 < 0) { const char* ev = std::getenv("AVH_STEM_FUSED"); stemf_env0 = (ev != nullptr && ev[0] == '0') ? 0 : 1; }
     const bool train = plan->train;
-    if (f32 || !stemf_env0 || train) {     // patch matrix + un-pooled stem maps: only the unfused stem needs them
+    if (f32 || train) {     // patch matrix + un-pooled stem maps: only the unfused stem needs them
       fb.im2col = b.alloc((size_t)CB * (T + 2) * 1936 * 64 * 2 * P);
       fb.stem_out = b.alloc((size_t)CB * (T + 2) * 1936 * 64 * es);      // same clip-padded row space as the patches
     }
@@ -1097,9 +1043,7 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     auto conv3x3_s1 = [&](const Act& in, const ConvUnit& cu, const Act& out, int Himg, int nimg, const float* slope1,
                           const Act* res, const float* slope2) -> bool {
       const int S = Himg + 1;
-      static int win_env = -1;
-      if (win_env < 0) { const char* ev = std::getenv("AVH_CONV_WINDOW"); win_env = (ev != nullptr && ev[0] == '0') ? 0 : 1; }
-      if (!f32 && !train && win_env && cu.cin == 64 && cu.cout == 64) {
+      if (!f32 && !train && cu.cin == 64 && cu.cout == 64) {
         // layer1: operand window resident in smem, nine taps as descriptor row offsets (conv_window.cu)
         b.tag = "conv3x3_c64";
         if (sizing) return true;
@@ -1138,9 +1082,7 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     };
 
     // bf16 mode, layers 2-4: one frame per GEMM row, dense [frames, H*H*C] maps, in-image taps only (conv_frame.cu)
-    static int frame_env = -1;
-    if (frame_env < 0) { const char* ev = std::getenv("AVH_CONV_FRAME"); frame_env = (ev != nullptr && ev[0] == '0') ? 0 : 1; }
-    const bool frame_mode = !f32 && !train && frame_env != 0;
+    const bool frame_mode = !f32 && !train;
     struct Shortcut { const void* A2 = nullptr; int Cin = 0, Sin = 0, stride = 1; const PackedW* w = nullptr;
                       const float* bias = nullptr; const float* ones = nullptr; };
     auto conv_frame = [&](const void* in, int Hin, int Sin, int Cin, const ConvUnit& cu, void* out, int Hout, int nimg,
@@ -1178,9 +1120,7 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
       const int nf = rg ? (int)N : nb * T;
       const long long f0 = rg ? 0 : (long long)b0 * T;
       // ---- stem: one fused kernel in bf16 mode (stem_fused.cu) ...
-      static int stemf_env = -1;
-      if (stemf_env < 0) { const char* ev = std::getenv("AVH_STEM_FUSED"); stemf_env = (ev != nullptr && ev[0] == '0') ? 0 : 1; }
-      if (!f32 && !train && stemf_env) {
+      if (!f32 && !train) {
         if (!sizing && b0 == 0 && stem_fused_plan(h->stem_wf.w, &plan->stemf)) return false;
         void* po = fb.pooled.data;
         b.tag = "stem_fused";
@@ -1237,19 +1177,10 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
           Act dsout;
           if (frame_mode && L > 0) {
             const int Hp = bi == 0 ? HS[L - 1] : Hn, Sp = (bi == 0 && L == 1) ? Hp + 1 : Hp, Cin = bi == 0 ? Cc / 2 : Cc;
-            static int dsf_env = -1;
-            if (dsf_env < 0) { const char* ev = std::getenv("AVH_DS_FUSED"); dsf_env = (ev != nullptr && ev[0] == '0') ? 0 : 1; }
-            const void* resp = cur.data;
-            const bool fuse_ds = bw.has_ds && dsf_env != 0;
-            if (bw.has_ds && !fuse_ds) {
-              if (!conv_frame(cur.op, Hp, Sp, Cin, bw.ds, fb.ds[L].data, Hn, nf, nullptr, nullptr, nullptr, "downsample"))
-                return false;
-              resp = fb.ds[L].data;
-            }
             if (!conv_frame(cur.op, Hp, Sp, Cin, bw.c1, mid.data, Hn, nf, bw.c1.slope, nullptr, nullptr,
                             (bi == 0 ? "conv_s2_c" : "conv3x3_c") + std::to_string(Cin)))
               return false;
-            if (fuse_ds) {
+            if (bw.has_ds) {
               // block 0 of layers 2-4: out = PReLU(BN2(conv2(mid)) + BN_ds(conv1x1_s2(x))) as ONE GEMM (the shortcut's
               // K steps read the block input x directly): no shortcut launch, no shortcut map written and re-read
               Shortcut sc;
@@ -1257,7 +1188,7 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
               if (!conv_frame(mid.data, Hn, Hn, Cc, bw.c2, out.data, Hn, nf, bw.slope2, nullptr, nullptr,
                               "conv3x3_c" + std::to_string(Cc), &sc))
                 return false;
-            } else if (!conv_frame(mid.data, Hn, Hn, Cc, bw.c2, out.data, Hn, nf, nullptr, resp, bw.slope2,
+            } else if (!conv_frame(mid.data, Hn, Hn, Cc, bw.c2, out.data, Hn, nf, nullptr, cur.data, bw.slope2,
                                    "conv3x3_c" + std::to_string(Cc)))
               return false;
             cur = out;
@@ -1486,59 +1417,25 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     if (!c.layer_norm_first) x_to_h();
   }
   const int n_layers = plan->output_layer > 0 ? std::min(plan->output_layer, c.encoder_layers) : c.encoder_layers;
-  // LayerNorm folding (gemm.h, Epilogue::ln_mode; AVH_LN_FUSED=1, off by default): bf16 mode, pre-LN layers.
-  // out_proj / fc2 write the new residual stream AND the centred bf16 operand + row partial sums; qkv / fc1 apply
-  // mean / rstd / gamma / beta in their epilogue: no LayerNorm launches inside the layer stack (48 for Large, 194 ->
-  // 147 launches per step).  Measured: results within 5e-6 of the unfused path, but 3916 vs 4127 clips/s — out_proj and
-  // fc2 are one-wave kernels whose epilogue is fully exposed, and trading the TMA reduce-add (x is never read) for a
-  // read-modify-write of x plus a second store costs +6.7 us per launch in the pipeline, more than the 3.9 us
-  // LayerNorm it removes.  AVH_LN_DBG elimination runs: ~4 us of it is the thread-per-row read of x (32 different
-  // cache lines per load instruction, even when requested a box ahead), the second store and the sums are free, the
-  // other ~2.5 us come with the smaller smem ring (4 stages) and the store-form epilogue.
-  static int lnf_env = -1;
-  if (lnf_env < 0) { const char* ev = std::getenv("AVH_LN_FUSED"); lnf_env = (ev != nullptr && ev[0] == '1') ? 1 : 0; }
-  const bool ln_fused = !f32 && !train && c.layer_norm_first && lnf_env != 0 && (D == 768 || D == 1024) && n_layers > 0 &&
-                        h->layers[0].qkv_csum != nullptr;
-  const int ln_pbn = 160;                                    // tile width of the producers (fixes the slot count)
-  const int ln_np_prod = ((D + ln_pbn - 1) / ln_pbn) * 2;
-  float* ln_mu = ln_fused ? reinterpret_cast<float*>(b.alloc((size_t)N * 4)) : nullptr;
-  float2* ln_part = ln_fused ? reinterpret_cast<float2*>(b.alloc((size_t)N * ln_np_prod * 8)) : nullptr;
-  int ln_np_cur = 1;
-  if (ln_fused) {
-    void* xc = hbuf.data;
-    b.tag = "layer_ln";
-    b.push([=](cudaStream_t s) { return launch_ln_center_stats(x, xc, ln_mu, ln_part, 1, N, D, s); });
-  }
-  auto ln_consumer = [&](Epilogue& ep, const float* csum) {
-    ep.col_scale = csum;
-    ep.ln_mode = 2; ep.ln_mu = ln_mu; ep.ln_part = ln_part; ep.ln_np = ln_np_cur; ep.ln_inv_dim = 1.0f / (float)D;
-  };
-  auto ln_producer = [&](Epilogue& ep) {
-    ep.ln_mode = 1; ep.ln_mu = ln_mu; ep.ln_part = ln_part; ep.ln_np = ln_np_prod; ep.ln_xc = hbuf.data; ep.ln_ldxc = D;
-    ln_np_cur = ln_np_prod;
-  };
-  static int att_tc_env = -1;
-  if (att_tc_env < 0) { const char* ev = std::getenv("AVH_ATT_TC"); att_tc_env = (ev != nullptr && ev[0] == '0') ? 0 : 1; }
   // measured (tools/att_bench.py, Large head count): tcgen05 11.4 vs 12.8 us at 16 x 150, 21.6 vs 29.0 at 8 x 300,
   // 31.9 vs 44.3 at 4 x 600; short clips (64 x 38 frames: 12.6 vs 9.3 us) stay on the mma.sync kernel
-  const bool att_tc = !f32 && (rg || (att_tc_env != 0 && T > 96)) && (size_t)((T + 127) / 128 * 128) * 4 <= 48 * 1024;
+  const bool att_tc = !f32 && (rg || T > 96) && (size_t)((T + 127) / 128 * 128) * 4 <= 48 * 1024;
   for (int l = 0; l < n_layers; ++l) {
     const LayerW& lw = h->layers[l];
     b.cur_layer = l;               // LayerDrop (training mode) skips every launch of a dropped layer
-    if (c.layer_norm_first && !ln_fused) ln_to_h(x, lw.ln1_g, lw.ln1_b, nullptr);
+    if (c.layer_norm_first) ln_to_h(x, lw.ln1_g, lw.ln1_b, nullptr);
     {   // fused QKV projection
       Epilogue ep = ep_base(qkv.data, 3 * D);
-      ep.col_bias = ln_fused ? lw.qkv_ln.bias : lw.qkv.bias;
-      if (ln_fused) ln_consumer(ep, lw.qkv_csum);
+      ep.col_bias = lw.qkv.bias;
       b.tag = "qkv_proj";
-      if (!b.gemm(hbuf.op, N, P * D, ln_fused ? lw.qkv_ln.w : lw.qkv.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      if (!b.gemm(hbuf.op, N, P * D, lw.qkv.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
     }
     {
       const void* q = qkv.data; void* o = ctx.data;
       b.tag = "attention";
       const double att_flops = 4.0 * (double)B * Hh * (double)T * (double)T * 64.0;   // QK^T + PV, dense (padding not excluded)
       if (att_tc) {
-        // bf16 mode: tcgen05 / TMEM kernel (attention_tc.cu); AVH_ATT_TC=0 selects the mma.sync kernel
+        // bf16 mode: tcgen05 / TMEM kernel (attention_tc.cu)
         if (!sizing && l == 0 && attention_tc_plan(q, N, B, T, D, Hh, &plan->att)) return false;
         b.push([=](cudaStream_t s) {
           return attention_tc_launch(pl->att, hm ? pl->mask_dev : nullptr, pl->ragged ? pl->rag + 16 : nullptr, o, s);
@@ -1566,13 +1463,11 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
       ep.C = c.layer_norm_first ? x : tmp; ep.ldc = D; ep.c_fp32 = 1;
       ep.col_bias = lw.out.bias; ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
       if (train) { ep.C = dtmp; ep.R = nullptr; }
-      if (ln_fused) ln_producer(ep);
       b.tag = "out_proj";
-      if (!b.gemm(ctx.op, N, P * D, lw.out.w, N, {Tap{0, 0, 0}}, D / 64, D, ep, ln_fused ? ln_pbn : 0)) return false;
+      if (!b.gemm(ctx.op, N, P * D, lw.out.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
       if (train) dropout_add(16u + 4u * (unsigned)l);
     }
-    if (c.layer_norm_first && !ln_fused) ln_to_h(x, lw.ln2_g, lw.ln2_b, nullptr);
-    else if (ln_fused) {}
+    if (c.layer_norm_first) ln_to_h(x, lw.ln2_g, lw.ln2_b, nullptr);
     else {
       float* g = lw.ln1_g; float* be = lw.ln1_b;
       b.tag = "layer_ln";
@@ -1581,10 +1476,9 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     }
     {   // fc1 + GELU (erf form, fp32: fairseq/fairseq/modules/gelu.py:95-96)
       Epilogue ep = ep_base(ffn.data, F);
-      ep.col_bias = ln_fused ? lw.fc1_ln.bias : lw.fc1.bias; ep.act = ACT_GELU;
-      if (ln_fused) ln_consumer(ep, lw.fc1_csum);
+      ep.col_bias = lw.fc1.bias; ep.act = ACT_GELU;
       b.tag = "fc1";
-      if (!b.gemm(hbuf.op, N, P * D, ln_fused ? lw.fc1_ln.w : lw.fc1.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      if (!b.gemm(hbuf.op, N, P * D, lw.fc1.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
       if (train) {      // dropout2 = activation_dropout after the GELU, wav2vec2.py:987
         void* fd = ffn.data;
         const unsigned site = 17u + 4u * (unsigned)l;
@@ -1599,11 +1493,9 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
       Epilogue ep;
       ep.C = c.layer_norm_first ? x : tmp; ep.ldc = D; ep.c_fp32 = 1;
       ep.col_bias = lw.fc2.bias; ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
-      const bool prod = ln_fused && l + 1 < n_layers;        // the last fc2 has no consumer: plain reduce-add
-      if (prod) ln_producer(ep);
       if (train) { ep.C = dtmp; ep.R = nullptr; }
       b.tag = "fc2";
-      if (!b.gemm(ffn.op, N, P * F, lw.fc2.w, N, {Tap{0, 0, 0}}, F / 64, F, ep, prod ? ln_pbn : 0)) return false;
+      if (!b.gemm(ffn.op, N, P * F, lw.fc2.w, N, {Tap{0, 0, 0}}, F / 64, F, ep)) return false;
       if (train) dropout_add(18u + 4u * (unsigned)l);
     }
     if (!c.layer_norm_first) {
@@ -1774,15 +1666,9 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
   const bool hm = plan->has_mask;
   const int tail = plan->tail;
   const bool full = tail == 2;
-  // AVH_WGRAD_SK=1: stream-K also for the ENCODER's weight-gradient GEMMs (64-256 tiles of 19 K blocks at 8 x 150 tokens).
-  // Off by default: measured slower on one box, 16.96 vs 15.96 ms per frozen-extractor step (73 launches at 24.5 us against
-  // ~13 us as whole tiles — the partial-tile round trip through the workspace costs more than the idle SMs)
-  static int wgrad_sk_env = -1;
-  if (wgrad_sk_env < 0) { const char* ev = std::getenv("AVH_WGRAD_SK"); wgrad_sk_env = (ev != nullptr && ev[0] == '1') ? 1 : 0; }
-  if (!f32 && (full || wgrad_sk_env == 1)) {
-    // stream-K workspace for the weight-gradient GEMMs (lip ResNet: a handful of output tiles, K = pixels; encoder: 64-256
-    // tiles of 19 K blocks at 8 x 150 tokens, i.e. 0.4-1.7 waves of the 148 SMs): one fp32 partial tile per SM + flags
-    // (zero from the arena's initial fill; the kernels hand the flags back as zeros)
+  if (!f32 && full) {
+    // stream-K workspace for the lip ResNet's weight-gradient GEMMs (a handful of output tiles, K = pixels): one fp32
+    // partial tile per SM + flags (zero from the arena's initial fill; the kernels hand the flags back as zeros)
     b.sk_bytes = (size_t)device_sm_count() * 128 * 256 * 4;
     b.sk_ws = reinterpret_cast<float*>(b.alloc(b.sk_bytes));
     b.sk_flags = reinterpret_cast<int*>(b.alloc(4096));
@@ -2145,10 +2031,10 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     Epilogue ep;
     ep.C = dW; ep.ldc = n_in; ep.c_fp32 = 1;
     b.tag = tag;
-    b.force_sk = (!f32 && wgrad_sk_env == 1) ? 1 : 0;      // few tiles x short K: cut the k-block space evenly over the SMs
-    const bool ok = b.gemm(tA, n_out, P * (int)Kp, xw, n_out, {Tap{0, 0, 0}}, (int)(Kp / 64), (int)Kp, ep);
-    b.force_sk = 0;
-    if (!ok) return false;
+    // whole tiles, no stream-K: measured faster for the encoder's weight gradients (64-256 tiles of 19 K blocks at
+    // 8 x 150 tokens), 15.96 vs 16.96 ms per frozen-extractor step (73 launches at ~13 us against 24.5 us with
+    // stream-K: the partial-tile round trip through the workspace costs more than the idle SMs)
+    if (!b.gemm(tA, n_out, P * (int)Kp, xw, n_out, {Tap{0, 0, 0}}, (int)(Kp / 64), (int)Kp, ep)) return false;
     if (db != nullptr) {
       b.tag = "bias_grad";
       b.push([=](cudaStream_t s) { return launch_colsum(dyv, dy_dt, n_out, N, n_out, db, 1.0f, s); });
@@ -2693,6 +2579,8 @@ bool build_qformer_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_ou
   return true;
 }
 
+constexpr int MAX_PLANS = 24;      // plans kept per handle (shape x stream); the least recently used one is evicted
+
 Plan* get_plan(avh_handle* h, int B, int T, bool has_video, bool has_audio, bool has_mask, int output_layer,
                cudaStream_t stream, long long ragged_rows = 0, bool enc_only = false, bool train = false, int qf_lk = 0,
                bool enc_train = false, int tail = 0) {
@@ -2708,9 +2596,7 @@ Plan* get_plan(avh_handle* h, int B, int T, bool has_video, bool has_audio, bool
     return it->second.get();
   }
   // bound workspace growth for ragged shape streams: evict the least recently used plan (one cudaFree, not all)
-  static int cap_env = -1;
-  if (cap_env < 0) { const char* ev = std::getenv("AVH_PLAN_CACHE"); cap_env = (ev != nullptr && std::atoi(ev) > 0) ? std::atoi(ev) : 24; }
-  while ((int)h->plans.size() >= cap_env) {
+  while ((int)h->plans.size() >= MAX_PLANS) {
     auto victim = h->plans.begin();
     for (auto jt = h->plans.begin(); jt != h->plans.end(); ++jt)
       if (jt->second->last_use < victim->second->last_use) victim = jt;

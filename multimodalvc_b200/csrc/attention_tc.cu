@@ -25,8 +25,6 @@
 #include "gemm.h"
 #include "kernels.h"
 
-#include <cstdlib>
-
 namespace avh {
 namespace {
 
@@ -47,7 +45,6 @@ struct AttnParams {
   int kv_rows;                // keys per block: round16(T) <= 160 (single block) or 128
   int stages, stage_bytes;
   int mask_floats;
-  int tiles_per_cta;          // consecutive query tiles of one (clip, head) handled by a CTA (K/V reuse, one wave)
 };
 
 __device__ __forceinline__ void tmem_st_32x16(uint32_t taddr, const uint32_t (&r)[16]) {
@@ -79,13 +76,11 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_cons
   uint64_t* full_bar = bars;                    // [MAX_STAGES]
   uint64_t* empty_bar = bars + MAX_STAGES;      // [MAX_STAGES]
   uint64_t* bar_q = bars + 2 * MAX_STAGES;      // Q tile landed (TMA -> MMA)
-  uint64_t* bar_qfree = bar_q + 1;              // last S MMA of the tile done: Q buffer reusable (MMA -> TMA)
-  uint64_t* bar_s = bar_qfree + 1;              // [2] S buffer ready (MMA -> softmax)
+  uint64_t* bar_s = bar_q + 1;                  // [2] S buffer ready (MMA -> softmax)
   uint64_t* bar_sfree = bar_s + 2;              // [2] S buffer consumed (softmax -> MMA), pass A
   uint64_t* bar_p = bar_sfree + 2;              // P written (softmax -> MMA)
   uint64_t* bar_o = bar_p + 1;                  // O complete (MMA -> epilogue)
-  uint64_t* bar_ofree = bar_o + 1;              // O read out (epilogue -> MMA)
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_ofree + 1);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bar_o + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int b = blockIdx.z, h = blockIdx.y;
@@ -94,9 +89,7 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_cons
   const int row_base = p.cu != nullptr ? __ldg(p.cu + b) : b * p.T;
   const int Tb = p.cu != nullptr ? __ldg(p.cu + b + 1) - row_base : p.T;
   const int ntiles = (Tb + QROWS - 1) / QROWS;
-  const int tile_first = blockIdx.x * p.tiles_per_cta;
-  const int tile_end = min(ntiles, tile_first + p.tiles_per_cta);
-  if (tile_first >= tile_end) return;
+  if ((int)blockIdx.x >= ntiles) return;            // clips shorter than the longest have fewer query tiles
   const int tile_rows = (Tb + ntiles - 1) / ntiles;         // balanced tiles: 150 frames -> 75 + 75
   const int kv = p.kv_rows;
   const int nkb = (Tb + kv - 1) / kv;
@@ -112,14 +105,12 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_cons
       mbar_init(&empty_bar[s], 1);
     }
     mbar_init(bar_q, 1);
-    mbar_init(bar_qfree, 1);
     for (int s = 0; s < 2; ++s) {
       mbar_init(&bar_s[s], 1);
       mbar_init(&bar_sfree[s], 4);
     }
     mbar_init(bar_p, 4);
     mbar_init(bar_o, 1);
-    mbar_init(bar_ofree, 4);
     mbar_fence_init();
   }
   if (warp == 2) tmem_alloc(tmem_slot, TMEM_COLS);
@@ -134,32 +125,28 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_cons
     const int col_q = h * HD, col_k = p.D + h * HD, col_v = 2 * p.D + h * HD;
     int stage = 0;
     uint32_t phase = 0;
-    for (int ti = tile_first, it = 0; ti < tile_end; ++ti, ++it) {
-      if (it > 0) mbar_wait(bar_qfree, (it - 1) & 1);
+    if (elect_one()) {
+      mbar_expect_tx(bar_q, Q_BYTES);
+      tma_load_2d(sQ, &tma_q, bar_q, col_q, row_base + (int)blockIdx.x * tile_rows);
+    }
+    __syncwarp();
+    const int nloads = two_pass ? 3 * nkb : 2;
+    for (int i = 0; i < nloads; ++i) {
+      // order of use: pass A K_0..K_{n-1}; pass B K_0, V_0, K_1, V_1, ...
+      int blk, col;
+      if (two_pass && i < nkb) { blk = i; col = col_k; }
+      else {
+        const int j = two_pass ? i - nkb : i;
+        blk = j >> 1;
+        col = (j & 1) ? col_v : col_k;
+      }
+      mbar_wait(&empty_bar[stage], phase ^ 1);
       if (elect_one()) {
-        mbar_expect_tx(bar_q, Q_BYTES);
-        tma_load_2d(sQ, &tma_q, bar_q, col_q, row_base + ti * tile_rows);
+        mbar_expect_tx(&full_bar[stage], (uint32_t)p.stage_bytes);
+        tma_load_2d(sKV + stage * p.stage_bytes, &tma_kv, &full_bar[stage], col, row_base + blk * kv);
       }
       __syncwarp();
-      if (!two_pass && it > 0) continue;            // single key block: K and V stay resident for every tile
-      const int nloads = two_pass ? 3 * nkb : 2;
-      for (int i = 0; i < nloads; ++i) {
-        // order of use: pass A K_0..K_{n-1}; pass B K_0, V_0, K_1, V_1, ...
-        int blk, col;
-        if (two_pass && i < nkb) { blk = i; col = col_k; }
-        else {
-          const int j = two_pass ? i - nkb : i;
-          blk = j >> 1;
-          col = (j & 1) ? col_v : col_k;
-        }
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        if (elect_one()) {
-          mbar_expect_tx(&full_bar[stage], (uint32_t)p.stage_bytes);
-          tma_load_2d(sKV + stage * p.stage_bytes, &tma_kv, &full_bar[stage], col, row_base + blk * kv);
-        }
-        __syncwarp();
-        if (++stage == p.stages) { stage = 0; phase ^= 1; }
-      }
+      if (++stage == p.stages) { stage = 0; phase ^= 1; }
     }
   } else if (warp == 1) {
     // ------------------------------------------------------------------ MMA issuer
@@ -170,74 +157,64 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_cons
     const uint64_t qdesc = umma_desc_sw128(smem_u32(sQ));
     uint32_t sfree_phase[2] = {0, 0};
     uint32_t p_phase = 0;
-    for (int ti = tile_first, it = 0; ti < tile_end; ++ti, ++it) {
-      mbar_wait(bar_q, it & 1);
-      tc_fence_after();
-      if (two_pass) {
-        // the second S buffer of pass A overlaps the O columns: the previous tile's epilogue must have read O out
-        if (it > 0) { mbar_wait(bar_ofree, (it - 1) & 1); tc_fence_after(); }
-        for (int j = 0; j < nkb; ++j) {
-          const int buf = j & 1;
-          if (j >= 2) {              // the sweep of the S that lived in this buffer two blocks ago is done
-            mbar_wait(&bar_sfree[buf], sfree_phase[buf]);
-            sfree_phase[buf] ^= 1;
-            tc_fence_after();
-          }
-          mbar_wait(&full_bar[stage], phase);
-          tc_fence_after();
-          const uint64_t kdesc = umma_desc_sw128(smem_u32(sKV + stage * p.stage_bytes));
-          if (elect_one()) {
-#pragma unroll
-            for (int k = 0; k < HD / 16; ++k)
-              umma_bf16(tmem_base + (buf ? COL_S1 : 0), qdesc + 2 * k, kdesc + 2 * k, idesc_s, k != 0);
-            umma_commit(&empty_bar[stage]);
-            umma_commit(&bar_s[buf]);
-          }
-          __syncwarp();
-          if (++stage == p.stages) { stage = 0; phase ^= 1; }
-        }
-        // pass B writes S into buffer 0 and O over buffer 1: the last sweep of either buffer must have drained
-        for (int buf = 0; buf < 2; ++buf) {
+    mbar_wait(bar_q, 0);
+    tc_fence_after();
+    if (two_pass) {
+      for (int j = 0; j < nkb; ++j) {
+        const int buf = j & 1;
+        if (j >= 2) {              // the sweep of the S that lived in this buffer two blocks ago is done
           mbar_wait(&bar_sfree[buf], sfree_phase[buf]);
           sfree_phase[buf] ^= 1;
-        }
-        tc_fence_after();
-      }
-      for (int j = 0; j < nkb; ++j) {
-        // S_j = Q K_j^T into buffer 0 (in-order execution behind PV_{j-1}, which reads P from the same columns)
-        if (two_pass || it == 0) {
-          mbar_wait(&full_bar[stage], phase);
           tc_fence_after();
         }
-        const int k_stage = two_pass ? stage : 0;
-        const uint64_t kdesc = umma_desc_sw128(smem_u32(sKV + k_stage * p.stage_bytes));
+        mbar_wait(&full_bar[stage], phase);
+        tc_fence_after();
+        const uint64_t kdesc = umma_desc_sw128(smem_u32(sKV + stage * p.stage_bytes));
         if (elect_one()) {
 #pragma unroll
-          for (int k = 0; k < HD / 16; ++k) umma_bf16(tmem_base, qdesc + 2 * k, kdesc + 2 * k, idesc_s, k != 0);
-          if (two_pass) umma_commit(&empty_bar[stage]);
-          umma_commit(&bar_s[0]);
-          if (j + 1 == nkb) umma_commit(bar_qfree);        // Q buffer free once these MMAs have run
+          for (int k = 0; k < HD / 16; ++k)
+            umma_bf16(tmem_base + (buf ? COL_S1 : 0), qdesc + 2 * k, kdesc + 2 * k, idesc_s, k != 0);
+          umma_commit(&empty_bar[stage]);
+          umma_commit(&bar_s[buf]);
         }
         __syncwarp();
-        if (two_pass || it == 0) { if (++stage == p.stages) { stage = 0; phase ^= 1; } }
-        // O += P_j V_j
-        mbar_wait(bar_p, p_phase);
-        p_phase ^= 1;
-        if (two_pass || it == 0) mbar_wait(&full_bar[stage], phase);
-        if (!two_pass && it > 0) mbar_wait(bar_ofree, (it - 1) & 1);      // previous tile's O has been read out
-        tc_fence_after();
-        const int v_stage = two_pass ? stage : 1;
-        const uint64_t vdesc = umma_desc_sw128(smem_u32(sKV + v_stage * p.stage_bytes));
-        const int ksteps = (min(kv, Tb - j * kv) + 15) >> 4;    // 16 keys per MMA; keys past the clip have P = 0
-        if (elect_one()) {
-          for (int k = 0; k < ksteps; ++k)
-            umma_bf16_ts(tmem_base + COL_O, tmem_base + 8 * k, vdesc + 128 * k, idesc_o, (j | k) != 0);
-          if (two_pass) umma_commit(&empty_bar[stage]);
-          if (j + 1 == nkb) umma_commit(bar_o);
-        }
-        __syncwarp();
-        if (two_pass || it == 0) { if (++stage == p.stages) { stage = 0; phase ^= 1; } }
+        if (++stage == p.stages) { stage = 0; phase ^= 1; }
       }
+      // pass B writes S into buffer 0 and O over buffer 1: the last sweep of either buffer must have drained
+      for (int buf = 0; buf < 2; ++buf) {
+        mbar_wait(&bar_sfree[buf], sfree_phase[buf]);
+        sfree_phase[buf] ^= 1;
+      }
+      tc_fence_after();
+    }
+    for (int j = 0; j < nkb; ++j) {
+      // S_j = Q K_j^T into buffer 0 (in-order execution behind PV_{j-1}, which reads P from the same columns)
+      mbar_wait(&full_bar[stage], phase);
+      tc_fence_after();
+      const uint64_t kdesc = umma_desc_sw128(smem_u32(sKV + stage * p.stage_bytes));
+      if (elect_one()) {
+#pragma unroll
+        for (int k = 0; k < HD / 16; ++k) umma_bf16(tmem_base, qdesc + 2 * k, kdesc + 2 * k, idesc_s, k != 0);
+        if (two_pass) umma_commit(&empty_bar[stage]);      // a single key block is loaded once: no stage is reused
+        umma_commit(&bar_s[0]);
+      }
+      __syncwarp();
+      if (++stage == p.stages) { stage = 0; phase ^= 1; }
+      // O += P_j V_j
+      mbar_wait(bar_p, p_phase);
+      p_phase ^= 1;
+      mbar_wait(&full_bar[stage], phase);
+      tc_fence_after();
+      const uint64_t vdesc = umma_desc_sw128(smem_u32(sKV + stage * p.stage_bytes));
+      const int ksteps = (min(kv, Tb - j * kv) + 15) >> 4;    // 16 keys per MMA; keys past the clip have P = 0
+      if (elect_one()) {
+        for (int k = 0; k < ksteps; ++k)
+          umma_bf16_ts(tmem_base + COL_O, tmem_base + 8 * k, vdesc + 128 * k, idesc_o, (j | k) != 0);
+        if (two_pass) umma_commit(&empty_bar[stage]);
+        if (j + 1 == nkb) umma_commit(bar_o);
+      }
+      __syncwarp();
+      if (++stage == p.stages) { stage = 0; phase ^= 1; }
     }
   } else if (warp >= 4) {
     // ------------------------------------------------------------------ softmax + epilogue: thread = query row
@@ -252,100 +229,95 @@ attention_tc_kernel(const __grid_constant__ CUtensorMap tma_q, const __grid_cons
     asm volatile("bar.sync 1, 128;" ::: "memory");
     const int nchunks = kv >> 5;                         // 32-key chunks per block (kv is a multiple of 32)
     uint32_t s_phase[2] = {0, 0};
-    for (int ti = tile_first, it = 0; ti < tile_end; ++ti, ++it) {
-      const int q0 = ti * tile_rows;
-      const int q_valid = min(tile_rows, Tb - q0);
-      const bool warp_live = quarter * 32 < q_valid;     // warps whose 32 rows are all past the tile skip the math
-      float m = -INFINITY;
-      if (two_pass) {
-        for (int j = 0; j < nkb; ++j) {
-          const int buf = j & 1;
-          mbar_wait(&bar_s[buf], s_phase[buf]);
-          s_phase[buf] ^= 1;
-          tc_fence_after();
-          if (warp_live) {
-            const int nch = (min(kv, Tb - j * kv) + 31) >> 5;
-            for (int c = 0; c < nch; ++c) {
-              uint32_t v[32];
-              tmem_ld_32x32(lane_addr + (buf ? COL_S1 : 0) + 32 * c, v);
-              tmem_ld_wait();
-              const float* mk = sMask + j * kv + 32 * c;
-#pragma unroll
-              for (int i = 0; i < 32; ++i) m = fmaxf(m, __uint_as_float(v[i]) + mk[i]);
-            }
-          }
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&bar_sfree[buf]);
-        }
-      }
-      float l = 0.f;
+    const int q0 = (int)blockIdx.x * tile_rows;
+    const int q_valid = min(tile_rows, Tb - q0);
+    const bool warp_live = quarter * 32 < q_valid;     // warps whose 32 rows are all past the tile skip the math
+    float m = -INFINITY;
+    if (two_pass) {
       for (int j = 0; j < nkb; ++j) {
-        mbar_wait(&bar_s[0], s_phase[0]);
-        s_phase[0] ^= 1;
+        const int buf = j & 1;
+        mbar_wait(&bar_s[buf], s_phase[buf]);
+        s_phase[buf] ^= 1;
         tc_fence_after();
         if (warp_live) {
-          const int nch = two_pass ? (min(kv, Tb - j * kv) + 31) >> 5 : nchunks;
-          const float* mk0 = sMask + j * kv;
-          if (!two_pass) {
-            for (int c = 0; c < nch; ++c) {
-              uint32_t v[32];
-              tmem_ld_32x32(lane_addr + 32 * c, v);
-              tmem_ld_wait();
+          const int nch = (min(kv, Tb - j * kv) + 31) >> 5;
+          for (int c = 0; c < nch; ++c) {
+            uint32_t v[32];
+            tmem_ld_32x32(lane_addr + (buf ? COL_S1 : 0) + 32 * c, v);
+            tmem_ld_wait();
+            const float* mk = sMask + j * kv + 32 * c;
 #pragma unroll
-              for (int i = 0; i < 32; ++i) m = fmaxf(m, __uint_as_float(v[i]) + mk0[32 * c + i]);
-            }
+            for (int i = 0; i < 32; ++i) m = fmaxf(m, __uint_as_float(v[i]) + mk[i]);
           }
-          const float ms = (m == -INFINITY) ? 0.f : m * LOG2E;      // fully masked row: every p = exp2(-inf) = 0
+        }
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&bar_sfree[buf]);
+      }
+    }
+    float l = 0.f;
+    for (int j = 0; j < nkb; ++j) {
+      mbar_wait(&bar_s[0], s_phase[0]);
+      s_phase[0] ^= 1;
+      tc_fence_after();
+      if (warp_live) {
+        const int nch = two_pass ? (min(kv, Tb - j * kv) + 31) >> 5 : nchunks;
+        const float* mk0 = sMask + j * kv;
+        if (!two_pass) {
           for (int c = 0; c < nch; ++c) {
             uint32_t v[32];
             tmem_ld_32x32(lane_addr + 32 * c, v);
             tmem_ld_wait();
-            uint32_t pk[16];
-            const float* mk = mk0 + 32 * c;
 #pragma unroll
-            for (int i = 0; i < 16; ++i) {
-              const float p0 = ex2(fmaf(__uint_as_float(v[2 * i]) + mk[2 * i], LOG2E, -ms));
-              const float p1 = ex2(fmaf(__uint_as_float(v[2 * i + 1]) + mk[2 * i + 1], LOG2E, -ms));
-              l += p0 + p1;
-              pk[i] = pack_bf16(p0, p1);
-            }
-            tmem_st_32x16(lane_addr + 16 * c, pk);      // P chunk c over S columns already consumed
+            for (int i = 0; i < 32; ++i) m = fmaxf(m, __uint_as_float(v[i]) + mk0[32 * c + i]);
           }
-          tmem_st_wait();
         }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(bar_p);
-      }
-      // ---- epilogue: O / l -> bf16 -> global (128 B per row)
-      mbar_wait(bar_o, it & 1);
-      tc_fence_after();
-      uint32_t o0[32], o1[32];
-      if (warp_live) {
-        tmem_ld_32x32(lane_addr + COL_O, o0);
-        tmem_ld_32x32(lane_addr + COL_O + 32, o1);
-        tmem_ld_wait();
+        const float ms = (m == -INFINITY) ? 0.f : m * LOG2E;      // fully masked row: every p = exp2(-inf) = 0
+        for (int c = 0; c < nch; ++c) {
+          uint32_t v[32];
+          tmem_ld_32x32(lane_addr + 32 * c, v);
+          tmem_ld_wait();
+          uint32_t pk[16];
+          const float* mk = mk0 + 32 * c;
+#pragma unroll
+          for (int i = 0; i < 16; ++i) {
+            const float p0 = ex2(fmaf(__uint_as_float(v[2 * i]) + mk[2 * i], LOG2E, -ms));
+            const float p1 = ex2(fmaf(__uint_as_float(v[2 * i + 1]) + mk[2 * i + 1], LOG2E, -ms));
+            l += p0 + p1;
+            pk[i] = pack_bf16(p0, p1);
+          }
+          tmem_st_32x16(lane_addr + 16 * c, pk);      // P chunk c over S columns already consumed
+        }
+        tmem_st_wait();
       }
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(bar_ofree);            // the next tile may overwrite O
-      if (warp_live && row < q_valid) {
-        const float inv = l > 0.f ? 1.f / l : 0.f;
-        uint4* dst = reinterpret_cast<uint4*>(p.out + (long long)(row_base + q0 + row) * p.D + h * HD);
+      if (lane == 0) mbar_arrive(bar_p);
+    }
+    // ---- epilogue: O / l -> bf16 -> global (128 B per row)
+    mbar_wait(bar_o, 0);
+    tc_fence_after();
+    uint32_t o0[32], o1[32];
+    if (warp_live) {
+      tmem_ld_32x32(lane_addr + COL_O, o0);
+      tmem_ld_32x32(lane_addr + COL_O + 32, o1);
+      tmem_ld_wait();
+    }
+    if (warp_live && row < q_valid) {
+      const float inv = l > 0.f ? 1.f / l : 0.f;
+      uint4* dst = reinterpret_cast<uint4*>(p.out + (long long)(row_base + q0 + row) * p.D + h * HD);
 #pragma unroll
-        for (int i = 0; i < 4; ++i)
-          dst[i] = make_uint4(pack_bf16(__uint_as_float(o0[8 * i]) * inv, __uint_as_float(o0[8 * i + 1]) * inv),
-                              pack_bf16(__uint_as_float(o0[8 * i + 2]) * inv, __uint_as_float(o0[8 * i + 3]) * inv),
-                              pack_bf16(__uint_as_float(o0[8 * i + 4]) * inv, __uint_as_float(o0[8 * i + 5]) * inv),
-                              pack_bf16(__uint_as_float(o0[8 * i + 6]) * inv, __uint_as_float(o0[8 * i + 7]) * inv));
+      for (int i = 0; i < 4; ++i)
+        dst[i] = make_uint4(pack_bf16(__uint_as_float(o0[8 * i]) * inv, __uint_as_float(o0[8 * i + 1]) * inv),
+                            pack_bf16(__uint_as_float(o0[8 * i + 2]) * inv, __uint_as_float(o0[8 * i + 3]) * inv),
+                            pack_bf16(__uint_as_float(o0[8 * i + 4]) * inv, __uint_as_float(o0[8 * i + 5]) * inv),
+                            pack_bf16(__uint_as_float(o0[8 * i + 6]) * inv, __uint_as_float(o0[8 * i + 7]) * inv));
 #pragma unroll
-        for (int i = 0; i < 4; ++i)
-          dst[4 + i] = make_uint4(pack_bf16(__uint_as_float(o1[8 * i]) * inv, __uint_as_float(o1[8 * i + 1]) * inv),
-                                  pack_bf16(__uint_as_float(o1[8 * i + 2]) * inv, __uint_as_float(o1[8 * i + 3]) * inv),
-                                  pack_bf16(__uint_as_float(o1[8 * i + 4]) * inv, __uint_as_float(o1[8 * i + 5]) * inv),
-                                  pack_bf16(__uint_as_float(o1[8 * i + 6]) * inv, __uint_as_float(o1[8 * i + 7]) * inv));
-      }
+      for (int i = 0; i < 4; ++i)
+        dst[4 + i] = make_uint4(pack_bf16(__uint_as_float(o1[8 * i]) * inv, __uint_as_float(o1[8 * i + 1]) * inv),
+                                pack_bf16(__uint_as_float(o1[8 * i + 2]) * inv, __uint_as_float(o1[8 * i + 3]) * inv),
+                                pack_bf16(__uint_as_float(o1[8 * i + 4]) * inv, __uint_as_float(o1[8 * i + 5]) * inv),
+                                pack_bf16(__uint_as_float(o1[8 * i + 6]) * inv, __uint_as_float(o1[8 * i + 7]) * inv));
     }
   }
   tc_fence_before();
@@ -366,7 +338,7 @@ int attention_tc_plan(const void* qkv, long long rows, int B, int T, int D, int 
   plan->stage_bytes = plan->kv_rows * HD * 2;
   const int nkb = (T + plan->kv_rows - 1) / plan->kv_rows;
   plan->mask_floats = nkb * plan->kv_rows;
-  plan->smem = 1024 + Q_BYTES + (size_t)plan->stages * plan->stage_bytes + (size_t)plan->mask_floats * 4 + 256;      // 17 mbarriers + TMEM slot
+  plan->smem = 1024 + Q_BYTES + (size_t)plan->stages * plan->stage_bytes + (size_t)plan->mask_floats * 4 + 256;      // 15 mbarriers + TMEM slot
   AVH_CHECK(plan->smem <= 113 * 1024, "clip too long for the attention kernel's key-mask buffer");
   if (encode_2d(&plan->tma_q, qkv, rows, 3 * D, 3ll * D, QROWS)) return 1;
   if (encode_2d(&plan->tma_kv, qkv, rows, 3 * D, 3ll * D, plan->kv_rows)) return 1;
@@ -383,15 +355,11 @@ int attention_tc_launch(const AttnTcPlan& plan, const unsigned char* kpm, const 
   p.stages = plan.stages; p.stage_bytes = plan.stage_bytes;
   p.mask_floats = plan.mask_floats;
   if (ensure_dyn_smem(reinterpret_cast<const void*>(attention_tc_kernel), 113 * 1024)) return 1;
-  // One query tile per CTA.  (Several consecutive tiles of a head per CTA — K/V loaded once, 256 CTAs = one wave at
-  // T = 150 — was measured: 11.4 vs 11.7 us at 16 x 150 and 38 vs 32 us at 4 x 600; the tiles of a CTA run back to
-  // back, so the softmax of one cannot overlap the MMAs of the next.  The kernel keeps the loop; AVH_ATT_TPC sets it.)
+  // One query tile per CTA.  Several consecutive tiles of a head per CTA (K/V loaded once, 256 CTAs = one wave at
+  // T = 150) measured slower or no better: 11.4 vs 11.7 us at 16 x 150 and 38 vs 32 us at 4 x 600; the tiles of a CTA
+  // run back to back, so the softmax of one cannot overlap the MMAs of the next.
   const int ntiles = (plan.T + QROWS - 1) / QROWS;
-  static int tpc_env = -1;
-  if (tpc_env < 0) { const char* ev = std::getenv("AVH_ATT_TPC"); tpc_env = ev != nullptr ? std::atoi(ev) : 1; }
-  const int tpc = tpc_env >= 1 && tpc_env <= ntiles ? tpc_env : 1;
-  p.tiles_per_cta = tpc;
-  dim3 grid((ntiles + tpc - 1) / tpc, plan.H, plan.B);
+  dim3 grid(ntiles, plan.H, plan.B);
   AVH_CUDA_OK(launch_pdl(attention_tc_kernel, grid, dim3(256), plan.smem, stream, plan.tma_q, plan.tma_kv, p));
   AVH_CUDA_OK(cudaGetLastError());
   count_launch(1);

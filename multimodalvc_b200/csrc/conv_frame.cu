@@ -405,12 +405,10 @@ int conv_frame_plan(const ConvFrameProblem& pr, ConvFramePlan* plan) {
   const int pad = pr.ks == 3 ? 1 : 0;
   int bn = pr.block_n, occ = pr.occ;
   if (bn == 0) bn = pr.Cout >= 256 ? 256 : pr.Cout;
-  // CTA pairs (cta_group::2) for the 256-wide tiles of layers 3-4; AVH_FRAME_PAIR=1 selects single-CTA tiles everywhere,
-  // =2 pairs wherever the tile allows.  Measured per step (2400 frames): 256-channel 3x3 convs 0.204 vs 0.232 ms,
-  // 512-channel 0.175 vs 0.179, but the 128-channel layer (BN 128) 0.300 vs 0.284 ms against two single CTAs per SM.
-  static int pair_env = -1;
-  if (pair_env < 0) { const char* ev = std::getenv("AVH_FRAME_PAIR"); pair_env = ev != nullptr ? std::atoi(ev) : 0; }
-  int pair = pr.pair != 0 ? pr.pair : (pair_env == 1 ? 1 : (pair_env == 2 ? 2 : (bn == 256 ? 2 : 1)));
+  // CTA pairs (cta_group::2) for the 256-wide tiles of layers 3-4, single CTAs elsewhere.  Measured per step (2400
+  // frames), pairs against single CTAs: 256-channel 3x3 convs 0.204 vs 0.232 ms, 512-channel 0.175 vs 0.179, but the
+  // 128-channel layer (BN 128) 0.300 vs 0.284 ms against two single CTAs per SM.
+  int pair = pr.pair != 0 ? pr.pair : (bn == 256 ? 2 : 1);
   if (device_sm_count() < 2 || bn % 128 != 0) pair = 1;        // each CTA of a pair stages bn / 2 weight rows (64-row boxes)
   if (pair == 2) occ = 1;
   if (occ == 0) occ = bn <= 128 ? 2 : 1;

@@ -57,15 +57,11 @@ __device__ __forceinline__ void wait_dbg(uint64_t* bar, uint32_t parity, unsigne
   acc += clock64() - c0;
 }
 
-// PAIR = 2: a cluster of two CTAs on the SMs of one TPC runs ONE tcgen05.mma.cta_group::2 of 256 rows per tap and
-// K step — each CTA stages the window of its own 128-row tile and holds HALF of every weight tap (32 of the 64 output
-// channels).  A 128 x 64 x 16 MMA needs 32 clk of tensor pipe but ~53 clk of its issuing thread, so the single-CTA
-// form looked issue-bound (36 MMAs = 1900 clk per tile).  Measured: bit-identical results, 0.487 vs 0.468 ms per step.
 // The stall counters (AVH_WIN_DBG=1) show the producer waiting for free stages 78 % of the time and the MMA warp busy
-// 93 %: ~64 clk per 128 x 64 x 16 MMA in either form, i.e. the tensor core is fed at half rate — an SS-form MMA with
-// N = 64 re-reads its 4 KB A slice from shared memory for only 64 output columns (the same bound the first fused stem
-// hit).  PAIR = 1 stays the default (AVH_WINDOW_PAIR=2 selects this form).
-template <bool RES, int PAIR>
+// 93 %: ~64 clk per 128 x 64 x 16 MMA, i.e. the tensor core is fed at half rate — an SS-form MMA with N = 64 re-reads
+// its 4 KB A slice from shared memory for only 64 output columns (the same bound the first fused stem hit).  Running
+// each tap as one 256-row MMA of a CTA pair does not lift that bound (DESIGN.md, tried and rejected).
+template <bool RES>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 conv_window_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                    const __grid_constant__ CUtensorMap tma_c, const WinParams p) {
@@ -73,7 +69,7 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_const
   const uint32_t raw = smem_u32(smem_raw);
   uint8_t* smem = smem_raw + (((raw + 1023u) & ~1023u) - raw);
   uint8_t* smem_b = smem;
-  uint8_t* smem_a = smem + B_BYTES / PAIR;
+  uint8_t* smem_a = smem + B_BYTES;
   uint8_t* epi_stage = smem_a + p.stages * p.win_bytes;
   float* colvec = reinterpret_cast<float*>(epi_stage + EPI_BYTES);     // scale | bias | slope1 | slope2, 64 each
   uint64_t* b_full = reinterpret_cast<uint64_t*>(colvec + 4 * CH);
@@ -85,11 +81,7 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_const
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const int cta_rank = PAIR == 2 ? (int)cluster_ctarank() : 0;
-  const bool leader = cta_rank == 0;
-  const int unit = blockIdx.x / PAIR, num_units = gridDim.x / PAIR;
-  const int num_work = (p.num_tiles + PAIR - 1) / PAIR;          // tiles (PAIR 1) or tile pairs
-  constexpr int B_TAP = B_TAP_BYTES / PAIR;                        // bytes of one tap held by this CTA
+  const int unit = blockIdx.x, num_units = gridDim.x;      // persistent CTAs: tiles unit, unit + num_units, ...
   pdl_launch_dependents();
   const long long k_start = clock64();
   long long st0 = 0, st1 = 0;
@@ -107,14 +99,11 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_const
     }
     for (int s = 0; s < 2; ++s) {
       mbar_init(&tmem_full[s], 1);
-      mbar_init(&tmem_empty[s], 4 * PAIR);
+      mbar_init(&tmem_empty[s], 4);
     }
     mbar_fence_init();
   }
-  if (warp == 2) {
-    if (PAIR == 2) tmem_alloc_pair(tmem_slot, 128);
-    else tmem_alloc(tmem_slot, 128);
-  }
+  if (warp == 2) tmem_alloc(tmem_slot, 128);
   if (threadIdx.x < CH) {           // launch-constant per-channel vectors
     const int c = threadIdx.x;
     colvec[c] = __ldg(p.scale + c);
@@ -123,80 +112,64 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_const
     colvec[3 * CH + c] = p.slope2 != nullptr ? __ldg(p.slope2 + c) : 1.f;
   }
   tc_fence_before();
-  if (PAIR == 2) cluster_sync_all();
-  else __syncthreads();
+  __syncthreads();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   if (warp == 0) {                  // the resident weights are launch constants: request them before the wait
     if (elect_one()) {
-      if (leader) mbar_expect_tx(b_full, B_BYTES);                 // both halves report to the leader's barrier
-      for (int t = 0; t < 9; ++t) {
-        if (PAIR == 2) tma_load_2d_pair(smem_b + t * B_TAP, &tma_b, b_full, t * CH, cta_rank * (CH / 2));
-        else tma_load_2d(smem_b + t * B_TAP, &tma_b, b_full, t * CH, 0);
-      }
+      mbar_expect_tx(b_full, B_BYTES);
+      for (int t = 0; t < 9; ++t) tma_load_2d(smem_b + t * B_TAP_BYTES, &tma_b, b_full, t * CH, 0);
     }
     __syncwarp();
   }
   pdl_wait();                       // from here on: activations of the previous kernel
 
   if (warp == 0) {
-    // ------------------------------------------------------------------ TMA producer (both CTAs)
+    // ------------------------------------------------------------------ TMA producer
     int stage = 0;
     uint32_t phase = 0;
-    for (int w = unit; w < num_work; w += num_units) {
-      const int tile = w * PAIR + cta_rank;       // a tile past the end loads zeros (TMA out-of-bounds fill)
+    for (int tile = unit; tile < p.num_tiles; tile += num_units) {
       wait_dbg(&a_empty[stage], phase ^ 1, p.dbg, st0);
       if (elect_one()) {
-        if (leader) mbar_expect_tx(&a_full[stage], (uint32_t)PAIR * (uint32_t)p.win_rows * 128u);
-        if (PAIR == 2) tma_load_2d_pair(smem_a + stage * p.win_bytes, &tma_a, &a_full[stage], 0, tile * BM - p.S - 1);
-        else tma_load_2d(smem_a + stage * p.win_bytes, &tma_a, &a_full[stage], 0, tile * BM - p.S - 1);
+        mbar_expect_tx(&a_full[stage], (uint32_t)p.win_rows * 128u);
+        tma_load_2d(smem_a + stage * p.win_bytes, &tma_a, &a_full[stage], 0, tile * BM - p.S - 1);
       }
       __syncwarp();
       if (++stage == p.stages) { stage = 0; phase ^= 1; }
     }
     if (p.dbg != nullptr && lane == 0) p.dbg[blockIdx.x * 8 + 1] = st0;
   } else if (warp == 1) {
-    // ------------------------------------------------------------------ MMA issuer (leader CTA only)
-    if (leader) {
-      constexpr uint32_t idesc = umma_idesc_bf16(BM * PAIR, CH);
-      mbar_wait(b_full, 0);
-      int stage = 0;
-      uint32_t phase = 0;
-      int it = 0;
-      for (int w = unit; w < num_work; w += num_units, ++it) {
-        const int acc = it & 1;
-        const uint32_t acc_phase = (it >> 1) & 1;
-        wait_dbg(&tmem_empty[acc], acc_phase ^ 1, p.dbg, st0);
-        wait_dbg(&a_full[stage], phase, p.dbg, st1);
-        tc_fence_after();
-        const uint32_t tmem_d = tmem_base + acc * CH;
-        const uint32_t a_base = smem_u32(smem_a + stage * p.win_bytes);
-        const uint32_t b_base = smem_u32(smem_b);
-        if (elect_one()) {
+    // ------------------------------------------------------------------ MMA issuer
+    constexpr uint32_t idesc = umma_idesc_bf16(BM, CH);
+    mbar_wait(b_full, 0);
+    int stage = 0;
+    uint32_t phase = 0;
+    int it = 0;
+    for (int tile = unit; tile < p.num_tiles; tile += num_units, ++it) {
+      const int acc = it & 1;
+      const uint32_t acc_phase = (it >> 1) & 1;
+      wait_dbg(&tmem_empty[acc], acc_phase ^ 1, p.dbg, st0);
+      wait_dbg(&a_full[stage], phase, p.dbg, st1);
+      tc_fence_after();
+      const uint32_t tmem_d = tmem_base + acc * CH;
+      const uint32_t a_base = smem_u32(smem_a + stage * p.win_bytes);
+      const uint32_t b_base = smem_u32(smem_b);
+      if (elect_one()) {
 #pragma unroll
-          for (int t = 0; t < 9; ++t) {
-            // tap (kh, kw): rows of the window starting at kh*S + kw
-            const uint64_t adesc = umma_desc_sw128(a_base + (uint32_t)((t / 3) * p.S + (t % 3)) * 128u);
-            const uint64_t bdesc = umma_desc_sw128(b_base + t * B_TAP);
+        for (int t = 0; t < 9; ++t) {
+          // tap (kh, kw): rows of the window starting at kh*S + kw
+          const uint64_t adesc = umma_desc_sw128(a_base + (uint32_t)((t / 3) * p.S + (t % 3)) * 128u);
+          const uint64_t bdesc = umma_desc_sw128(b_base + t * B_TAP_BYTES);
 #pragma unroll
-            for (int k = 0; k < CH / 16; ++k) {
-              if (PAIR == 2) umma_bf16_pair(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (t | k) != 0);
-              else umma_bf16(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (t | k) != 0);
-            }
-          }
-          if (PAIR == 2) {
-            umma_commit_pair(&a_empty[stage]);      // windows of BOTH CTAs reusable once these MMAs have read them
-            umma_commit_pair(&tmem_full[acc]);
-          } else {
-            umma_commit(&a_empty[stage]);
-            umma_commit(&tmem_full[acc]);
-          }
+          for (int k = 0; k < CH / 16; ++k) umma_bf16(tmem_d, adesc + 2 * k, bdesc + 2 * k, idesc, (t | k) != 0);
         }
-        __syncwarp();
-        if (++stage == p.stages) { stage = 0; phase ^= 1; }
+        umma_commit(&a_empty[stage]);
+        umma_commit(&tmem_full[acc]);
       }
-      if (p.dbg != nullptr && lane == 0) { p.dbg[blockIdx.x * 8 + 2] = st0; p.dbg[blockIdx.x * 8 + 3] = st1; p.dbg[blockIdx.x * 8 + 6] = it; }
+      __syncwarp();
+      if (++stage == p.stages) { stage = 0; phase ^= 1; }
     }
+    if (p.dbg != nullptr && lane == 0) { p.dbg[blockIdx.x * 8 + 2] = st0; p.dbg[blockIdx.x * 8 + 3] = st1; p.dbg[blockIdx.x * 8 + 6] = it; }
   } else if (warp >= 4) {
     // ------------------------------------------------------------------ epilogue: thread = row
     // two warp sets alternate tiles (set e owns accumulator stage e), so each set has two tile times for its epilogue
@@ -205,9 +178,8 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_const
     uint8_t* stg = epi_stage + (warp - 4) * 4096;
     const int S = p.S, H = p.S - 1;
     int it = 0;
-    for (int w = unit; w < num_work; w += num_units, ++it) {
+    for (int tile = unit; tile < p.num_tiles; tile += num_units, ++it) {
       if ((it & 1) != eset) continue;
-      const int tile = w * PAIR + cta_rank;
       const int acc = it & 1;
       const uint32_t acc_phase = (it >> 1) & 1;
       const int row0 = tile * BM + q * 32;
@@ -234,10 +206,7 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_const
         if (sub == 1) {
           tc_fence_before();
           __syncwarp();
-          if (lane == 0) {
-            if (PAIR == 2) mbar_arrive_leader(&tmem_empty[acc]);
-            else mbar_arrive(&tmem_empty[acc]);
-          }
+          if (lane == 0) mbar_arrive(&tmem_empty[acc]);
         }
         float v[32];
 #pragma unroll
@@ -299,13 +268,9 @@ conv_window_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_const
   }
 
   tc_fence_before();
-  if (PAIR == 2) cluster_sync_all();
-  else __syncthreads();
+  __syncthreads();
   tc_fence_after();
-  if (warp == 2) {
-    if (PAIR == 2) tmem_dealloc_pair(tmem_base, 128);
-    else tmem_dealloc(tmem_base, 128);
-  }
+  if (warp == 2) tmem_dealloc(tmem_base, 128);
   if (p.dbg != nullptr && threadIdx.x == 0) p.dbg[blockIdx.x * 8] = clock64() - k_start;
 }
 
@@ -319,23 +284,18 @@ int conv_window_plan(const ConvWinProblem& pr, ConvWinPlan* plan) {
   plan->win_rows = BM + 2 * (pr.S + 1);
   AVH_CHECK(plan->win_rows <= 256, "window exceeds the TMA box limit");
   const int win_bytes = ((plan->win_rows * 128 + 1023) / 1024) * 1024;
-  static int pair_env = -1;
-  if (pair_env < 0) { const char* ev = std::getenv("AVH_WINDOW_PAIR"); pair_env = (ev != nullptr && ev[0] == '2') ? 2 : 1; }
-  const int sms0 = device_sm_count();
-  plan->pair = (pair_env == 2 && sms0 >= 2) ? 2 : 1;
-  const int fixed = 1024 + B_BYTES / plan->pair + EPI_BYTES + 4 * CH * 4 + (1 + 2 * MAX_STAGES + 4) * 8 + 16;
+  const int fixed = 1024 + B_BYTES + EPI_BYTES + 4 * CH * 4 + (1 + 2 * MAX_STAGES + 4) * 8 + 16;
   int stages = (SMEM_LIMIT - fixed) / win_bytes;
   if (stages > MAX_STAGES) stages = MAX_STAGES;
   AVH_CHECK(stages >= 2, "window too large for shared memory");
   plan->stages = stages;
   plan->smem = (size_t)fixed + (size_t)stages * win_bytes;
   if (encode_2d(&plan->tma_a, pr.A, pr.rows, CH, CH, plan->win_rows)) return 1;
-  if (encode_2d(&plan->tma_b, pr.B, CH, 9 * CH, 9 * CH, CH / plan->pair)) return 1;
+  if (encode_2d(&plan->tma_b, pr.B, CH, 9 * CH, 9 * CH, CH)) return 1;
   if (encode_c(&plan->tma_c, pr.C, pr.rows, CH, CH, 0)) return 1;
   const long long tiles = (pr.rows + BM - 1) / BM;
-  const long long work = (tiles + plan->pair - 1) / plan->pair;
-  const long long units = sms0 / plan->pair;
-  plan->grid = (int)(work < units ? work : units) * plan->pair;
+  const long long sms = device_sm_count();
+  plan->grid = (int)(tiles < sms ? tiles : sms);
   return 0;
 }
 
@@ -354,8 +314,7 @@ int conv_window_launch(const ConvWinPlan& plan, cudaStream_t stream) {
   p.slope2 = pr.slope2;
   p.R = reinterpret_cast<const __nv_bfloat16*>(pr.R);
   typedef void (*WinFn)(CUtensorMap, CUtensorMap, CUtensorMap, WinParams);
-  WinFn fn = plan.pair == 2 ? (pr.R != nullptr ? conv_window_kernel<true, 2> : conv_window_kernel<false, 2>)
-                            : (pr.R != nullptr ? conv_window_kernel<true, 1> : conv_window_kernel<false, 1>);
+  WinFn fn = pr.R != nullptr ? conv_window_kernel<true> : conv_window_kernel<false>;
   if (ensure_dyn_smem(reinterpret_cast<const void*>(fn), SMEM_LIMIT)) return 1;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)plan.grid);
@@ -364,7 +323,7 @@ int conv_window_launch(const ConvWinPlan& plan, cudaStream_t stream) {
   cfg.stream = stream;
   cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = (unsigned)plan.pair;
+  attr[0].val.clusterDim.x = 1;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;

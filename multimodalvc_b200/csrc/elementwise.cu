@@ -329,39 +329,6 @@ __global__ void avgpool_kernel(const void* __restrict__ in, void* __restrict__ o
   store_lp(out, dt, i, s / (float)(H * W));
 }
 
-// Entry point of the LayerNorm-folded encoder (gemm.h, Epilogue::ln_mode): for every fp32 row x of width VEC*128
-// writes the centred bf16 operand xc = bf16(x - mean), mu[row] = mean, and the partial-sum slots the consuming GEMM
-// reads: slot 0 = (0, sum (x - mean)^2), slots 1..np-1 = 0.
-template <int VEC>
-__global__ void ln_center_stats_kernel(const float* __restrict__ in, __nv_bfloat16* __restrict__ xc, float* __restrict__ mu,
-                                       float2* __restrict__ part, int np, long long rows) {
-  pdl_launch_dependents();
-  pdl_wait();
-  constexpr int C = VEC * 128;
-  const long long row = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (row >= rows) return;
-  const int lane = threadIdx.x & 31;
-  const float4* x = reinterpret_cast<const float4*>(in + row * C);
-  float4 v[VEC];
-  float s = 0.f;
-#pragma unroll
-  for (int i = 0; i < VEC; ++i) {
-    v[i] = x[lane + 32 * i];
-    s += (v[i].x + v[i].y) + (v[i].z + v[i].w);
-  }
-  const float mean = warp_sum(s) * (1.f / C);
-  float q = 0.f;
-#pragma unroll
-  for (int i = 0; i < VEC; ++i) {
-    v[i].x -= mean; v[i].y -= mean; v[i].z -= mean; v[i].w -= mean;
-    q += (v[i].x * v[i].x + v[i].y * v[i].y) + (v[i].z * v[i].z + v[i].w * v[i].w);
-    reinterpret_cast<uint2*>(xc + row * C)[lane + 32 * i] = make_uint2(pack_bf16(v[i].x, v[i].y), pack_bf16(v[i].z, v[i].w));
-  }
-  q = warp_sum(q);
-  if (lane == 0) mu[row] = mean;
-  for (int i = lane; i < np; i += 32) part[row * np + i] = make_float2(0.f, i == 0 ? q : 0.f);
-}
-
 // Video pre-processing of the dataset's eval transform (avhubert/hubert_dataset.py:222-226,298-302;
 // avhubert/utils.py:56-95): uint8 gray frames [n, src_h, src_w] -> x/255 -> centre crop -> (x - mean)/std.  The
 // reference does this in float64 numpy and casts to float32 (hubert_dataset.py:432): the 256 possible results are
@@ -634,23 +601,6 @@ int launch_layernorm(const void* in, int in_dt, long long ld_in, const float* ga
     AVH_CUDA_OK(launch_pdl(layernorm_kernel, dim3(grid), dim3(wpb * 32), 0, stream, in, in_dt, ld_in, gamma, beta, eps,
                            out_f32, out_lp, lp_dt, row_zero, rows, C));
 #undef AVH_LN_VEC
-  AVH_CUDA_OK(cudaGetLastError());
-  count_launch(1);
-  return 0;
-}
-
-int launch_ln_center_stats(const float* in, void* xc, float* mu, void* part, int np, long long rows, int C,
-                           cudaStream_t stream) {
-  if (rows <= 0) return 0;
-  AVH_CHECK(C == 768 || C == 1024, "LayerNorm folding supports D = 768 / 1024");
-  const int wpb = 4;
-  const int grid = blocks_for(rows, wpb);
-  if (C == 1024)
-    AVH_CUDA_OK(launch_pdl(ln_center_stats_kernel<8>, dim3(grid), dim3(wpb * 32), 0, stream, in,
-                           reinterpret_cast<__nv_bfloat16*>(xc), mu, reinterpret_cast<float2*>(part), np, rows));
-  else
-    AVH_CUDA_OK(launch_pdl(ln_center_stats_kernel<6>, dim3(grid), dim3(wpb * 32), 0, stream, in,
-                           reinterpret_cast<__nv_bfloat16*>(xc), mu, reinterpret_cast<float2*>(part), np, rows));
   AVH_CUDA_OK(cudaGetLastError());
   count_launch(1);
   return 0;

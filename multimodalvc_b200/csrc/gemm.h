@@ -35,21 +35,6 @@ struct Epilogue {
   long long O0 = 0, O1 = 0, O2 = 0;
   int invalid_zero = 0;                 // invalid rows: 1 -> store zeros, 0 -> skip
   const int* row_map = nullptr;         // device [M]: tile row -> output row, -1 = skip (overrides map_mode; ragged pos-conv)
-  // ---- LayerNorm of the residual stream folded into the GEMMs around it (bf16 mode, pre-LN layers) ----
-  // ln_mode 1, PRODUCER (x = x + A B^T + bias, fp32): also writes xc = bf16(x - mu[row]) (the next GEMM's operand,
-  //   centred on the row mean of the PREVIOUS x) and, per row and per (N tile, epilogue warp set), the partial sums
-  //   (sum, sum of squares) of (x - mu[row]) over the columns it owns: ln_part[row * ln_np + n_tile * 2 + set].
-  // ln_mode 2, CONSUMER (weights pre-multiplied by gamma): out = act(r * (acc - delta * col_scale) + col_bias) with
-  //   delta = mean(x) - mu[row] and r = rsqrt(var(x) + eps) from the ln_np partials (summed in a fixed order);
-  //   col_scale[n] = sum_k W'[n,k], col_bias[n] = b[n] + sum_k W[n,k] beta[k].  The n-tile-0 CTA updates
-  //   mu[row] += delta.  LN(x) W^T = r ((x - mu) gamma) W^T + beta W^T, exactly.
-  int ln_mode = 0;
-  float* ln_mu = nullptr;               // [rows]
-  float2* ln_part = nullptr;            // [rows, ln_np]
-  int ln_np = 0;
-  void* ln_xc = nullptr;                // producer: bf16 [rows, N], row stride ln_ldxc
-  long long ln_ldxc = 0;
-  float ln_inv_dim = 0.f, ln_eps = 1e-5f;
 };
 
 // One K-block (64 bf16 along K) of the contraction: A box at (col, m0 + row_off), B box at (col, n0 + row_off).
@@ -86,7 +71,7 @@ struct GemmProblem {
 };
 
 struct GemmPlan {
-  CUtensorMap tma_a, tma_b, tma_c, tma_c2;      // tma_c2: bf16 centred copy of an ln_mode-1 producer (32-column boxes)
+  CUtensorMap tma_a, tma_b, tma_c;
   int c_mode = 0;
   int sk = 0;                     // stream-K partition in use
   GemmProblem prob;
@@ -117,7 +102,6 @@ struct ConvWinPlan {
   CUtensorMap tma_a, tma_b, tma_c;
   ConvWinProblem prob;
   int grid = 0, stages = 0, win_rows = 0;
-  int pair = 1;                   // 1 = single CTAs (default); 2 = CTA pairs (tcgen05 cta_group::2, AVH_WINDOW_PAIR=2)
   size_t smem = 0;
 };
 int conv_window_plan(const ConvWinProblem& prob, ConvWinPlan* plan);

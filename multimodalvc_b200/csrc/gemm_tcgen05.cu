@@ -81,8 +81,6 @@ struct KernelParams {
   int sk;
   float* sk_ws;                 // [units][PAIR * 128][block_n] fp32
   int* sk_flags;                // [units], zero between launches
-  int lnf_dbg;                  // debug (AVH_LN_DBG bits, timing experiments only — results become wrong): 1 skip the
-                                // centred bf16 store, 2 skip the statistics, 4 skip the residual loads
   Epilogue ep;
 };
 
@@ -143,14 +141,12 @@ struct SegIter {
 
 // ACT (ACT_*), RES (residual add), S2 (second PReLU), SCALE (per-column scale) and OUTF32 (fp32 output and
 // residual, else bf16) are compile-time when >= 0 and read from the Epilogue struct when -1.
-// LNF: LayerNorm folding (Epilogue::ln_mode): 0 none, 1 producer (centred bf16 copy + row partial sums), 2 consumer.
 // SK: stream-K code compiled in (only the instantiations the planner picks for a stream-K launch carry it: with the
 // code in every kernel the epilogue spilled registers and the encoder GEMMs ran ~9 % slower — tools/ab_bench.sh).
-template <int PAIR, int OCC, int ACT, int RES, int S2, int SCALE, int OUTF32, int LNF = 0, int SK = 0>
+template <int PAIR, int OCC, int ACT, int RES, int S2, int SCALE, int OUTF32, int SK = 0>
 __global__ void __launch_bounds__(Occ<OCC>::NUM_THREADS, OCC)
 gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
-            const __grid_constant__ CUtensorMap tma_c, const __grid_constant__ CUtensorMap tma_c2,
-            const KernelParams p) {
+            const __grid_constant__ CUtensorMap tma_c, const KernelParams p) {
   constexpr int EPI_WARPS = Occ<OCC>::EPI_WARPS;
   constexpr int NUM_THREADS = Occ<OCC>::NUM_THREADS;
   constexpr int TMEM_COLS = Occ<OCC>::TMEM_COLS;
@@ -166,8 +162,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
   uint8_t* smem_a = smem;
   uint8_t* smem_b = smem + STAGES * A_STAGE_BYTES;
   uint8_t* epi_stage = smem_b + STAGES * b_stage_bytes;
-  uint8_t* epi_stage2 = epi_stage + EPI_STAGE_BYTES;                  // LNF 1: 2 KB per epilogue warp (bf16 32 x 32 box)
-  float* colvec = reinterpret_cast<float*>(epi_stage2 + (LNF == 1 ? EPI_WARPS * 2048 : 0));
+  float* colvec = reinterpret_cast<float*>(epi_stage + EPI_STAGE_BYTES);
   int4* ktab = reinterpret_cast<int4*>(reinterpret_cast<uint8_t*>(colvec) + COLVEC_BYTES);
   uint64_t* full_bar = reinterpret_cast<uint64_t*>(reinterpret_cast<uint8_t*>(ktab) + p.ktab_bytes);
   uint64_t* empty_bar = full_bar + MAX_STAGES;
@@ -418,27 +413,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
         store = mr >= 0;
       }
       if (store && ep.row_zero != nullptr && ep.row_zero[orow]) zero = true;
-      // LayerNorm folding: per-row quantities of this thread's row
-      float ln_a = 1.f, ln_b = 0.f;          // consumer: r, -delta;  producer: ln_b = mu[row]
-      float ln_s1 = 0.f, ln_s2 = 0.f;        // producer: partial sums of this warp's columns
-      if (LNF == 2) {
-        float s1 = 0.f, s2 = 0.f;
-        if (store) {
-          const float2* pp = ep.ln_part + orow * ep.ln_np;
-          for (int i = 0; i < ep.ln_np; ++i) {
-            const float2 q2 = __ldg(pp + i);
-            s1 += q2.x;
-            s2 += q2.y;
-          }
-        }
-        const float delta = s1 * ep.ln_inv_dim;
-        const float var = fmaxf(s2 * ep.ln_inv_dim - delta * delta, 0.f);
-        ln_a = rsqrtf(var + ep.ln_eps);
-        ln_b = -delta;
-        if (store && n_blk == 0 && half == 0) ep.ln_mu[orow] += delta;      // mean of x for the next producer
-      } else if (LNF == 1) {
-        ln_b = store ? __ldg(ep.ln_mu + orow) : 0.f;
-      }
       // per-column epilogue vectors of this tile -> smem while the main loop runs: every CTA reads the same few
       // cache lines at the same moment; from global inside the box loop that costs ~1 us of L2 queueing per box
       float* cv = colvec + acc * 1024;
@@ -452,17 +426,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
       }
       asm volatile("bar.sync 1, %0;" ::"n"(32 * EPI_WARPS) : "memory");
 
-      // LNF 1: the residual (x) of this warp's first 32-column box is requested while the main loop still runs, and
-      // inside the box loop the next box's residual is requested before the current one is consumed
-      uint4 rpre[8];
-      if (LNF == 1) {
-        const int pc0 = n_blk * BN + half * 32;
-        if (store && !zero && half * 32 < BN && pc0 < p.N && !(p.lnf_dbg & 4)) {
-          const uint4* rp = reinterpret_cast<const uint4*>(reinterpret_cast<const float*>(ep.R) + orow * ep.ldr + pc0);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) rpre[j] = __ldg(rp + j);
-        }
-      }
       mbar_wait(&tmem_full[acc], acc_phase);
       tc_fence_after();
       if (warp == 4 && lane == 0) {
@@ -482,7 +445,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
         for (int bx = half; bx < nboxes; bx += HSTRIDE) {
           const int cbase = bx * box_cols;                 // column offset inside the tile
           uint32_t packed[32];
-          uint32_t cpk[16];                                // LNF 1: centred bf16 pairs of this 32-column box
 #pragma unroll
           for (int sub = 0; sub < 2; ++sub) {
             if (sub == 1 && out_f32) break;
@@ -493,16 +455,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
             // residual row segment (32 columns) straight from global while the TMEM load is in flight
             uint4 rres[8];
             if (has_res && live && col0 < p.N) {
-              if (LNF == 1) {
-#pragma unroll
-                for (int j = 0; j < 8; ++j) rres[j] = rpre[j];
-                const int nc0 = col0 + HSTRIDE * 32;            // this warp's next box
-                if (c0 + HSTRIDE * 32 < BN && nc0 < p.N && !(p.lnf_dbg & 4)) {
-                  const uint4* rp = reinterpret_cast<const uint4*>(reinterpret_cast<const float*>(ep.R) + orow * ep.ldr + nc0);
-#pragma unroll
-                  for (int j = 0; j < 8; ++j) rpre[j] = __ldg(rp + j);
-                }
-              } else if (out_f32) {
+              if (out_f32) {
                 const uint4* rp = reinterpret_cast<const uint4*>(reinterpret_cast<const float*>(ep.R) + orow * ep.ldr + col0);
 #pragma unroll
                 for (int j = 0; j < 8; ++j) rres[j] = __ldg(rp + j);
@@ -545,14 +498,7 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
 #pragma unroll
               for (int j = 0; j < 8; ++j) {
                 const float4 bi = *reinterpret_cast<const float4*>(cv + c0 + 4 * j);
-                if (LNF == 2) {
-                  // r * (acc - delta * c_n) + d_n
-                  const float4 sc = *reinterpret_cast<const float4*>(cv + 256 + c0 + 4 * j);
-                  v[4 * j] = fmaf(ln_a, fmaf(ln_b, sc.x, v[4 * j]), bi.x);
-                  v[4 * j + 1] = fmaf(ln_a, fmaf(ln_b, sc.y, v[4 * j + 1]), bi.y);
-                  v[4 * j + 2] = fmaf(ln_a, fmaf(ln_b, sc.z, v[4 * j + 2]), bi.z);
-                  v[4 * j + 3] = fmaf(ln_a, fmaf(ln_b, sc.w, v[4 * j + 3]), bi.w);
-                } else if (has_scale) {
+                if (has_scale) {
                   const float4 sc = *reinterpret_cast<const float4*>(cv + 256 + c0 + 4 * j);
                   v[4 * j] = fmaf(v[4 * j], sc.x, bi.x); v[4 * j + 1] = fmaf(v[4 * j + 1], sc.y, bi.y);
                   v[4 * j + 2] = fmaf(v[4 * j + 2], sc.z, bi.z); v[4 * j + 3] = fmaf(v[4 * j + 3], sc.w, bi.w);
@@ -608,22 +554,6 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
 #pragma unroll
               for (int j = 0; j < 32; ++j) v[j] = 0.f;
             }
-            if (LNF == 1) {
-              // centred bf16 copy of the new residual-stream values + this warp's share of the row sums
-              if (col0 < p.N && live && !(p.lnf_dbg & 2)) {
-                float d1 = 0.f, d2 = 0.f;
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                  const float d = v[j] - ln_b;
-                  d1 += d;
-                  d2 = fmaf(d, d, d2);
-                }
-                ln_s1 += d1;
-                ln_s2 += d2;
-              }
-#pragma unroll
-              for (int j = 0; j < 16; ++j) cpk[j] = pack_bf16(v[2 * j] - ln_b, v[2 * j + 1] - ln_b);
-            }
             if (out_f32) {
 #pragma unroll
               for (int j = 0; j < 32; ++j) packed[j] = __float_as_uint(v[j]);
@@ -649,26 +579,16 @@ gemm_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ C
           for (int j = 0; j < 8; ++j)
             *reinterpret_cast<uint4*>(sbox + lane * 128 + ((j ^ (lane & 7)) << 4)) =
                 make_uint4(packed[4 * j], packed[4 * j + 1], packed[4 * j + 2], packed[4 * j + 3]);
-          if (LNF == 1) {
-            uint8_t* stg2 = epi_stage2 + (warp - 4) * 2048;      // row-major 32 x 32 bf16 box (64-byte rows)
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-              *reinterpret_cast<uint4*>(stg2 + lane * 64 + ((j ^ ((lane >> 1) & 3)) << 4)) =
-                  make_uint4(cpk[4 * j], cpk[4 * j + 1], cpk[4 * j + 2], cpk[4 * j + 3]);
-          }
           fence_proxy_async_smem();
           __syncwarp();
           if (lane == 0) {
             if (row0 < p.M) {
               if (p.c_mode == 2) tma_reduce_add_2d(&tma_c, sbox, n_blk * BN + cbase, row0);
               else tma_store_2d(&tma_c, sbox, n_blk * BN + cbase, row0);
-              if (LNF == 1 && n_blk * BN + cbase < p.N && !(p.lnf_dbg & 1)) tma_store_2d(&tma_c2, epi_stage2 + (warp - 4) * 2048, n_blk * BN + cbase, row0);
             }
             tma_commit_group();       // one group per box, stored or not: "all but the newest group" = the box before
           }
         }
-        if (LNF == 1 && store)
-          ep.ln_part[orow * ep.ln_np + n_blk * HSTRIDE + half] = make_float2(ln_s1, ln_s2);
         if (half >= nboxes) {
           tc_fence_before();
           __syncwarp();
@@ -834,23 +754,6 @@ int encode_c(CUtensorMap* map, const void* base, long long rows, int cols, long 
   return 0;
 }
 
-// bf16 output map with 32-column boxes (64-byte rows, 64B swizzle) x 32 rows: the centred copy an ln_mode-1 GEMM
-// writes next to its fp32 output (whose boxes are 32 columns wide too)
-int encode_c_bf16_32(CUtensorMap* map, const void* base, long long rows, int cols, long long ld) {
-  EncodeTiledFn fn = get_encode_fn();
-  AVH_CHECK(fn != nullptr, "cuTensorMapEncodeTiled entry point not available");
-  AVH_CHECK((reinterpret_cast<uintptr_t>(base) & 15) == 0 && (ld * 2) % 16 == 0, "TMA store alignment");
-  cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)ld * 2};
-  cuuint32_t box[2] = {32u, 32u};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  AVH_CHECK(r == CUDA_SUCCESS, "cuTensorMapEncodeTiled (C2) failed (code " + std::to_string((int)r) + ")");
-  return 0;
-}
-
 // 2-D bf16 row-major tensor [rows, cols] (row stride ld elements), box = 64 cols x box_rows, 128B swizzle.
 int encode_2d(CUtensorMap* map, const void* base, long long rows, int cols, long long ld, int box_rows) {
   EncodeTiledFn fn = get_encode_fn();
@@ -892,19 +795,6 @@ double model_cycles(long long M, int N, int num_kb, int bn, int pair, int occ, i
   const long long nt = (N + bn - 1) / bn;
   const long long units = (long long)sms * occ / pair;
   const long long tiles = mt * nt;
-  static int model_env = -1;
-  if (model_env < 0) { const char* ev = std::getenv("AVH_GEMM_MODEL"); model_env = ev ? std::atoi(ev) : 0; }
-  if (model_env == 1 && !sk) {
-    // round-1 model (whole-step A/B, tools/ab_bench.sh): ~80 B/clk operand stream, no fill / tail asymmetry
-    const long long rounds = (tiles + units - 1) / units;
-    double kb1 = 415.0;
-    if (2.0 * bn > kb1) kb1 = 2.0 * bn;
-    const double pipe1 = occ * 4.0 * (bn / 2.0);
-    const double l2 = occ * (double)(A_STAGE_BYTES + (bn / pair) * BK * 2) / 80.0;
-    if (pipe1 > kb1) kb1 = pipe1;
-    if (l2 > kb1) kb1 = l2;
-    return rounds * (num_kb * kb1 + 400.0) + 8.0 * bn + 2500.0;
-  }
   double kblock = 415.0;
   if (2.0 * bn > kblock) kblock = 2.0 * bn;
   const double ingress = occ * (double)(A_STAGE_BYTES + (bn / pair) * BK * 2) / 66.0;
@@ -943,19 +833,7 @@ int gemm_plan(const GemmProblem& pr, GemmPlan* plan) {
   if (sms < 2) pair = 1;
   int bn = pr.block_n;
   int occ = pr.occ;
-  static int occ_env = -1;
-  if (occ_env < 0) { const char* ev = std::getenv("AVH_GEMM_OCC"); occ_env = ev ? std::atoi(ev) : 0; }
-  if (occ == 0) occ = occ_env;
   if (pair == 2) occ = 1;
-  if (pr.ep.ln_mode != 0) {
-    AVH_CHECK(pair == 1, "LayerNorm folding needs single-CTA tiles");
-    AVH_CHECK(pr.ep.ln_mu != nullptr && pr.ep.ln_part != nullptr && pr.ep.ln_np >= 1, "LayerNorm folding buffers missing");
-    AVH_CHECK(pr.ep.ln_mode != 1 || (pr.ep.c_fp32 && pr.ep.R == pr.ep.C && pr.ep.ln_xc != nullptr && pr.ep.act == ACT_NONE),
-              "ln producer must be an in-place fp32 residual GEMM");
-    AVH_CHECK(pr.ep.ln_mode != 2 || (!pr.ep.c_fp32 && pr.ep.col_scale != nullptr && pr.ep.R == nullptr),
-              "ln consumer must be a bf16-output GEMM with the column sums in col_scale");
-    occ = 1;
-  }
   // Stream-K is OFF unless AVH_GEMM_SK=1 (forced where applicable) or AVH_GEMM_SK=2 (cost model decides).  Measured at
   // M = 2400 (profiles/r2_gemm_streamk.txt): correct and bit-reproducible, but slower than whole tiles in rounds — qkv
   // 22.6 vs 18.1 us, fc1 22.0 vs 20.6, fc2 24.8 vs 23.0 (BN 160) — although it removes the idle part of the last round:
@@ -964,10 +842,10 @@ int gemm_plan(const GemmProblem& pr, GemmPlan* plan) {
   static int sk_env = -2;
   if (sk_env == -2) { const char* ev = std::getenv("AVH_GEMM_SK"); sk_env = ev ? std::atoi(ev) : 0; }
   if (sk_env == 2) sk_env = -1;      // -1 = model decides
-  // stream-K needs the TMA epilogue (tile rows = output rows), no LayerNorm folding and a workspace
+  // stream-K needs the TMA epilogue (tile rows = output rows) and a workspace
   const Epilogue& e0 = pr.ep;
   const bool sk_possible = pr.sk_ws != nullptr && pr.sk_flags != nullptr && pr.streamk >= 0 && (sk_env != 0 || pr.streamk == 1) &&
-                           e0.ln_mode == 0 && e0.row_map == nullptr && e0.map_mode != MAP_2LEVEL && e0.row_zero == nullptr &&
+                           e0.row_map == nullptr && e0.map_mode != MAP_2LEVEL && e0.row_zero == nullptr &&
                            (e0.R == nullptr || (e0.R == e0.C && e0.slope2 == nullptr && e0.c_fp32));
   int sk = 0;
   {
@@ -1027,11 +905,6 @@ int gemm_plan(const GemmProblem& pr, GemmPlan* plan) {
         mode = (e.ldr == e.ldc && e.c_fp32 && e.slope2 == nullptr && e.row_zero == nullptr) ? 2 : 0;
       }
     }
-    if (e.ln_mode == 1) mode = 1;          // residual read per thread, fp32 + centred bf16 boxes stored by TMA
-    static int force = -1;
-    if (force < 0) { const char* ev = std::getenv("AVH_GEMM_CMODE"); force = ev ? std::atoi(ev) : 9; }
-    if (force == 0 && e.ln_mode == 0) mode = 0;
-    AVH_CHECK(e.ln_mode == 0 || mode == 1, "LayerNorm folding needs the TMA-store epilogue");
     if (mode == 0) plan->sk = 0;
     plan->c_mode = mode;
     if (mode != 0) {
@@ -1039,8 +912,6 @@ int gemm_plan(const GemmProblem& pr, GemmPlan* plan) {
     } else {
       plan->tma_c = plan->tma_a;
     }
-    plan->tma_c2 = plan->tma_a;
-    if (e.ln_mode == 1 && encode_c_bf16_32(&plan->tma_c2, e.ln_xc, pr.M, pr.N, e.ln_ldxc)) return 1;
   }
   const long long mt = (pr.M + (long long)BM * pair - 1) / ((long long)BM * pair);
   const long long nt = (pr.N + bn - 1) / bn;
@@ -1050,8 +921,7 @@ int gemm_plan(const GemmProblem& pr, GemmPlan* plan) {
   const int stage_bytes = A_STAGE_BYTES + (bn / pair) * BK * 2;
   const int ktab_bytes = pr.ktable != nullptr ? ((pr.num_kb * 16 + 1023) / 1024) * 1024 : 0;
   const int smem_limit = occ == 2 ? Occ<2>::SMEM_LIMIT : Occ<1>::SMEM_LIMIT;
-  const int epi_bytes = (occ == 2 ? Occ<2>::EPI_STAGE_BYTES : Occ<1>::EPI_STAGE_BYTES) +
-                        (pr.ep.ln_mode == 1 ? Occ<1>::EPI_WARPS * 2048 : 0);
+  const int epi_bytes = occ == 2 ? Occ<2>::EPI_STAGE_BYTES : Occ<1>::EPI_STAGE_BYTES;
   int stages = (smem_limit - 1024 - epi_bytes - COLVEC_BYTES - ktab_bytes - BAR_BYTES) / stage_bytes;
   if (stages > MAX_STAGES) stages = MAX_STAGES;
   AVH_CHECK(stages >= 2, "tile too large for shared memory");
@@ -1082,9 +952,6 @@ int gemm_launch(const GemmPlan& plan, cudaStream_t stream) {
   kp.sk_flags = pr.sk_flags;
 
   kp.trace = g_trace;
-  static int lnf_dbg_env = -1;
-  if (lnf_dbg_env < 0) { const char* ev = std::getenv("AVH_LN_DBG"); lnf_dbg_env = ev ? std::atoi(ev) : 0; }
-  kp.lnf_dbg = lnf_dbg_env;
   kp.ep = pr.ep;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)plan.grid);
@@ -1103,17 +970,14 @@ int gemm_launch(const GemmPlan& plan, cudaStream_t stream) {
   cfg.numAttrs = pdl_enabled() ? 2 : 1;
   const Epilogue& e = pr.ep;
   const int act = e.act, res = e.R != nullptr, s2 = e.slope2 != nullptr, scl = e.col_scale != nullptr, f32 = e.c_fp32;
-  typedef void (*KernelFn)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, KernelParams);
+  typedef void (*KernelFn)(CUtensorMap, CUtensorMap, CUtensorMap, KernelParams);
   KernelFn fn = nullptr;
-  if (e.ln_mode == 1) fn = gemm_kernel<1, 1, ACT_NONE, 1, 0, 0, 1, 1>;                   // out_proj / fc2 producing xc + sums
-  else if (e.ln_mode == 2 && act == ACT_GELU) fn = gemm_kernel<1, 1, ACT_GELU, 0, 0, 1, 0, 2>;   // fc1 on LayerNorm'd rows
-  else if (e.ln_mode == 2) fn = gemm_kernel<1, 1, ACT_NONE, 0, 0, 1, 0, 2>;                      // qkv on LayerNorm'd rows
   if (plan.sk != 0) {      // stream-K launches (AVH_GEMM_SK): single CTA per SM or CTA pairs, the three encoder epilogues
-    if (pair == 2) fn = gemm_kernel<2, 1, -1, -1, -1, -1, -1, 0, 1>;
-    else if (act == ACT_NONE && !res && !s2 && !scl && !f32) fn = gemm_kernel<1, 1, ACT_NONE, 0, 0, 0, 0, 0, 1>;
-    else if (act == ACT_GELU && !res && !s2 && !scl && !f32) fn = gemm_kernel<1, 1, ACT_GELU, 0, 0, 0, 0, 0, 1>;
-    else if (act == ACT_NONE && res && !s2 && !scl && f32) fn = gemm_kernel<1, 1, ACT_NONE, 1, 0, 0, 1, 0, 1>;
-    else fn = gemm_kernel<1, 1, -1, -1, -1, -1, -1, 0, 1>;
+    if (pair == 2) fn = gemm_kernel<2, 1, -1, -1, -1, -1, -1, 1>;
+    else if (act == ACT_NONE && !res && !s2 && !scl && !f32) fn = gemm_kernel<1, 1, ACT_NONE, 0, 0, 0, 0, 1>;
+    else if (act == ACT_GELU && !res && !s2 && !scl && !f32) fn = gemm_kernel<1, 1, ACT_GELU, 0, 0, 0, 0, 1>;
+    else if (act == ACT_NONE && res && !s2 && !scl && f32) fn = gemm_kernel<1, 1, ACT_NONE, 1, 0, 0, 1, 1>;
+    else fn = gemm_kernel<1, 1, -1, -1, -1, -1, -1, 1>;
   }
 #define AVH_SPEC(O, A, R, S, C, F)                                                                     \
   if (fn == nullptr && pair == 1 && occ == O && act == A && res == R && s2 == S && scl == C && f32 == F) \
@@ -1145,7 +1009,7 @@ int gemm_launch(const GemmPlan& plan, cudaStream_t stream) {
     else fn = gemm_kernel<1, 1, -1, -1, -1, -1, -1>;
   }
   if (ensure_dyn_smem(reinterpret_cast<const void*>(fn), occ == 2 ? Occ<2>::SMEM_LIMIT : Occ<1>::SMEM_LIMIT)) return 1;
-  AVH_CUDA_OK(cudaLaunchKernelEx(&cfg, fn, plan.tma_a, plan.tma_b, plan.tma_c, plan.tma_c2, kp));
+  AVH_CUDA_OK(cudaLaunchKernelEx(&cfg, fn, plan.tma_a, plan.tma_b, plan.tma_c, kp));
   count_launch(1);
   return 0;
 }

@@ -67,8 +67,6 @@ int launch_im2col_s2(const void* in, void* out, int n, int H, int W, int C, cuda
 // flagged in frame_zero ([n], may be null: the key-padding mask) are written as 0.0, as the collater's zero padding is
 int launch_video_preprocess(const unsigned char* frames, long long n_frames, int src_h, int src_w, int crop, double mean,
                             double stdv, void* out, int out_dt, const unsigned char* frame_zero, cudaStream_t stream);
-int launch_ln_center_stats(const float* in, void* xc, float* mu, void* part, int np, long long rows, int C,
-                           cudaStream_t stream);
 int launch_avgpool(const void* in, void* out, int n, int H, int W, int C, int pitch, int fp32, cudaStream_t stream);
 
 // ---- training-mode forward (train_ops.cu): BatchNorm with batch statistics, Philox dropout
