@@ -179,32 +179,49 @@ struct CallArgs {          // per-call pointers the steps read through the plan
   int pitch = 0;             // ragged plans: time pitch of the caller's padded tensors (baked into captured launches)
   void* grads_out = nullptr; // training backward: the caller's gradient buffer, filled bucket by bucket (never captured)
   int grads_dt = 0;
-  // graph-cache key: the INPUT pointers (the output is written by the last step, which stays outside the graph)
-  bool operator<(const CallArgs& o) const {
-    return std::tie(video, video_dt, audio, audio_dt, as[0], as[1], as[2], mask, pitch, xin, xin_dt) <
-           std::tie(o.video, o.video_dt, o.audio, o.audio_dt, o.as[0], o.as[1], o.as[2], o.mask, o.pitch, o.xin, o.xin_dt);
+};
+
+enum class PlanKind {
+  Forward,        // avh_forward: AVHubertModel.extract_finetune
+  // avh_forward_ragged: packed ragged batches.  Every buffer holds Nb = round_up(sum of clip lengths, 128) token /
+  // frame rows with the clips back to back; T is then the longest clip the plan serves (attention tiling).  The
+  // per-call geometry lives in a small device descriptor `rag` (int32): [0] stem work items, [1] rows in use,
+  // [16..16+B] first row of every clip (cu), then the stem's (clip, band, t0, t1) item list.
+  Ragged,
+  EncoderOnly,    // avh_encoder_forward: TransformerEncoder on caller-provided features [B,T,D]
+  // avh_forward_train: BatchNorm batch statistics through the generic convolution path, Philox dropout at the
+  // reference's dropout sites, LayerDrop by skipping a layer's launches; never graph-captured
+  TrainForward,
+  // training plans (forward with saved activations + backward, avh_encoder_backward): steps [0, fwd_steps) are the
+  // forward, the rest the backward; gradients accumulate in a plan-owned fp32 buffer
+  EncoderTrain,   // TransformerEncoder on caller-provided features
+  TailTrain,      // trainable tail of AV-HuBERT (fusion LayerNorm + post_extract_proj + encoder) on caller-provided fused features
+  FullTrain,      // the whole model (lip ResNet + projections computed in the plan, feature_grad_mult > 0)
+  QFormer,        // avh_qformer_forward: T = query rows per clip, Lk = AV feature rows per clip
+};
+
+// One plan (= workspace + launch list) per key: shape, inputs present, kind AND CUDA stream.  Forwards enqueued on
+// different streams never share scratch memory, so a caller can keep several batches in flight on one device.
+struct PlanKey {
+  PlanKind kind = PlanKind::Forward;
+  int B = 0, T = 0;
+  bool has_video = false, has_audio = false, has_mask = false;
+  int output_layer = 0;
+  long long ragged_rows = 0;      // Ragged: Nb
+  int Lk = 0;                     // QFormer
+  cudaStream_t stream = nullptr;
+  bool training() const { return kind == PlanKind::EncoderTrain || kind == PlanKind::TailTrain || kind == PlanKind::FullTrain; }
+  bool operator<(const PlanKey& o) const {
+    return std::tie(kind, B, T, has_video, has_audio, has_mask, output_layer, ragged_rows, Lk, stream) <
+           std::tie(o.kind, o.B, o.T, o.has_video, o.has_audio, o.has_mask, o.output_layer, o.ragged_rows, o.Lk, o.stream);
   }
 };
 
 struct Plan {
-  int B = 0, T = 0, output_layer = 0;
-  bool has_video = false, has_audio = false, has_mask = false;
-  // packed ragged batches (avh_forward_ragged): every buffer holds Nb = round_up(sum of clip lengths, 128) token /
-  // frame rows with the clips back to back; T is then the longest clip the plan serves (attention tiling).  The
-  // per-call geometry lives in a small device descriptor `rag` (int32): [0] stem work items, [1] rows in use,
-  // [16..16+B] first row of every clip (cu), then the stem's (clip, band, t0, t1) item list.
-  // training-mode forward (avh_forward_train): BatchNorm batch statistics through the generic convolution path,
-  // Philox dropout at the reference's dropout sites, LayerDrop by skipping a layer's launches; never graph-captured
-  bool train = false;
-  float p_in = 0.f, p_enc = 0.f, p_act = 0.f, bn_momentum = 0.1f;     // set per call
+  PlanKey key;
+  float p_in = 0.f, p_enc = 0.f, p_act = 0.f, bn_momentum = 0.1f;     // training-mode forward: set per call
   unsigned long long seed = 0;
   std::vector<unsigned char> layer_skip;
-  bool enc_only = false;           // avh_encoder_forward: TransformerEncoder on caller-provided features [B,T,D]
-  // encoder training plans (avh_encoder_train_forward / avh_encoder_backward): steps [0, fwd_steps) are the forward
-  // with saved activations, the rest the backward; gradients accumulate in a plan-owned fp32 buffer
-  bool enc_train = false;
-  int tail = 0;                    // 1: trainable tail of AV-HuBERT (fusion LayerNorm + post_extract_proj + encoder) on caller-provided
-                                   // fused features; 2: the whole model (lip ResNet + projections computed in the plan, feature_grad_mult > 0)
   size_t fwd_steps = 0;
   float* grads = nullptr;
   long long grad_floats = 0;
@@ -212,11 +229,8 @@ struct Plan {
   float* dy_in = nullptr;          // gradient w.r.t. the output, staged fp32 [B*T, D]
   float fgm = 1.f;                 // mode 2: feature_grad_mult (GradMultiply on the extractor outputs), set per call
   bool fwd_done = false;
-  int Lk = 0;                      // Q-Former plans: T = query rows per clip, Lk = AV feature rows per clip
   unsigned char* qmask_dev = nullptr;    // Q-Former plans: [B*T] 1 = padded query, [B*Lk] 1 = padded AV frame
   unsigned char* kmask_dev = nullptr;
-  bool ragged = false;
-  long long Nb = 0;
   int* rag = nullptr;
   int rag_ints = 0, rag_items_off = 0, rag_max_items = 0;
   static constexpr int RAG_SLOTS = 4;
@@ -255,7 +269,6 @@ struct Plan {
   unsigned char* mask_dev = nullptr;   // staged copy of the caller's padding mask [B*T]
   int direct_runs = 0;              // un-captured forwards so far (the first one also configures the kernels)
   long long last_use = 0;           // LRU clock value of the most recent forward through this plan
-  cudaStream_t stream = nullptr;
   void drop_graphs() {
     for (auto& sg : segments)
       if (sg.exec) cudaGraphExecDestroy(sg.exec);
@@ -326,7 +339,7 @@ struct avh_handle {
   std::vector<QfLayerW> qf_layers;
   LinearW qf_ckv;                  // cross-attention key / value projections of ALL layers: [L * 2D, encoder_width]
   float *qf_emb_g = nullptr, *qf_emb_b = nullptr, *qf_tokens = nullptr;
-  std::map<std::string, std::unique_ptr<Plan>> plans;
+  std::map<PlanKey, std::unique_ptr<Plan>> plans;
   long long plan_clock = 0;
   bool profiling = false;
   std::vector<cudaEvent_t> prof_events;      // 2 per step of the last profiled forward
@@ -813,6 +826,22 @@ struct Tap {
   int a_row_off, a_col, b_col;
 };
 
+// GEMM epilogue writing [M, N] rows of stride ldc (fp32 or bf16); the other fields are filled per call site
+Epilogue epilogue(void* C, long long ldc, bool c_fp32) {
+  Epilogue ep;
+  ep.C = C; ep.ldc = ldc; ep.c_fp32 = c_fp32 ? 1 : 0;
+  return ep;
+}
+
+// activation tensor: `data` holds the values ([rows, C], bf16 in bf16 mode / fp32 in fp32 mode); `op` is the
+// GEMM-operand form (bf16 [rows, P*C]); identical to data in bf16 mode.
+struct Act {
+  void* data = nullptr;
+  void* op = nullptr;
+  long long rows = 0;
+  int C = 0;
+};
+
 struct Builder {
   avh_handle* h;
   Plan* plan;
@@ -820,11 +849,20 @@ struct Builder {
   Sizer sizer;
   int P;
   bool f32;      // fp32-faithful mode
+  size_t es;     // bytes per activation value
+  int act_dt;    // dtype of activation values
   bool linear_k = false;         // next gemm(): plain K loop without a step table (bf16 mode, single zero tap)
   int force_sk = 0;              // next gemm(): GemmProblem::streamk
   float* sk_ws = nullptr;        // stream-K workspace of the plan's GEMMs (launches of a plan are serialised on its stream)
   size_t sk_bytes = 0;
   int* sk_flags = nullptr;
+  int cur_layer = -1;           // encoder layer of the steps pushed next (LayerDrop skips a dropped layer's steps)
+
+  Builder(avh_handle* h_, Plan* plan_, bool sizing_)
+      : h(h_), plan(plan_), sizing(sizing_), P(h_->P), f32(h_->cfg.compute_mode == AVH_COMPUTE_FP32) {
+    es = f32 ? 4 : 2;
+    act_dt = f32 ? DT_F32 : DT_BF16;
+  }
 
   void* alloc(size_t bytes) {
     if (sizing) {
@@ -833,11 +871,52 @@ struct Builder {
     }
     return plan->arena.take(bytes);
   }
-  std::string tag = "misc";     // name given to the steps pushed next
-  int cur_layer = -1;           // encoder layer of the steps pushed next
-  bool cur_direct = false;      // the steps pushed next touch caller pointers (kept out of the CUDA graphs)
-  void push(std::function<int(cudaStream_t)> f, double flops = 0.0) {
-    if (!sizing) plan->steps.push_back(Step{std::move(f), tag, flops, cur_layer, cur_direct});
+  float* f32buf(long long n) { return reinterpret_cast<float*>(alloc((size_t)n * 4)); }
+  Act act(long long rows, int C) {
+    Act a;
+    a.rows = rows; a.C = C;
+    a.data = alloc((size_t)rows * C * es);
+    a.op = f32 ? alloc((size_t)rows * C * 2 * P) : a.data;
+    return a;
+  }
+  // plan-owned copy of a [rows] byte mask (padding masks are staged into it before the launch list runs)
+  unsigned char* mask_buf(long long rows) { return reinterpret_cast<unsigned char*>(alloc((size_t)rows + 16)); }
+  // stream-K workspace: one fp32 partial tile (128 x 256) per SM + flags (zero from the arena's initial fill; the
+  // kernels hand the flags back as zeros)
+  void stream_k_workspace() {
+    sk_bytes = (size_t)device_sm_count() * 128 * 256 * 4;
+    sk_ws = f32buf((long long)sk_bytes / 4);
+    sk_flags = reinterpret_cast<int*>(alloc(4096));
+  }
+  void stage(const char* name, const void* p, int dt, long long n) {
+    if (!sizing) plan->stages[name] = {p, {dt, n}};
+  }
+
+  // `direct`: the step reads or writes caller pointers, so it is launched outside the CUDA graphs
+  void push(const std::string& tag, std::function<int(cudaStream_t)> f, double flops = 0.0, bool direct = false) {
+    if (!sizing) plan->steps.push_back(Step{std::move(f), tag, flops, cur_layer, direct});
+  }
+  void push_direct(const std::string& tag, std::function<int(cudaStream_t)> f, double flops = 0.0) {
+    push(tag, std::move(f), flops, true);
+  }
+  // fp32 [rows, C] (row stride ld) -> GEMM-operand form (bf16 [rows, P*C])
+  void split(const float* src, int ld, void* dst, long long rows, int C) {
+    const int planes = P;
+    push("split", [=](cudaStream_t s) { return launch_split_rows(src, ld, dst, planes, rows, C, 0, 0, s); });
+  }
+  // fp32 mode: refresh the split bf16 operand planes of an activation (bf16 mode: op is data)
+  void sync_op(const Act& a) {
+    if (f32) split(reinterpret_cast<const float*>(a.data), a.C, a.op, a.rows, a.C);
+  }
+  // LayerNorm over the rows of src ([dst.rows, dst.C] of dtype src_dt) into an activation and its operand form
+  void layernorm(const std::string& tag, const void* src, int src_dt, const float* g, const float* be, float eps,
+                 const Act& dst) {
+    float* of = f32 ? reinterpret_cast<float*>(dst.data) : nullptr;
+    void* ol = f32 ? nullptr : dst.data;
+    const long long rows = dst.rows;
+    const int C = dst.C;
+    push(tag, [=](cudaStream_t s) { return launch_layernorm(src, src_dt, C, g, be, eps, of, ol, DT_BF16, nullptr, rows, C, s); });
+    sync_op(dst);
   }
 
   // K-step table for one GEMM: every tap x every 64-wide K chunk (x 3 split-precision products in fp32 mode)
@@ -858,9 +937,9 @@ struct Builder {
   }
 
   // enqueue one GEMM; returns false on planning failure
-  bool gemm(const void* A, long long a_rows, int a_cols, const PackedW& W, long long M, const std::vector<Tap>& taps,
-            int chunks, int a_plane_stride, Epilogue ep, int block_n = 0, const int* a_col_nblk = nullptr,
-            long long lda = 0) {
+  bool gemm(const std::string& tag, const void* A, long long a_rows, int a_cols, const PackedW& W, long long M,
+            const std::vector<Tap>& taps, int chunks, int a_plane_stride, const Epilogue& ep, int block_n = 0,
+            const int* a_col_nblk = nullptr, long long lda = 0) {
     GemmProblem pr;
     pr.A = A; pr.a_rows = a_rows; pr.a_cols = a_cols; pr.lda = lda > 0 ? lda : a_cols;
     pr.B = W.w; pr.b_rows = W.n; pr.b_cols = P * W.kpad; pr.ldb = (long long)P * W.kpad;
@@ -880,25 +959,13 @@ struct Builder {
     GemmPlan* gp = new GemmPlan();
     plan->gemms.push_back(gp);
     if (gemm_plan(pr, gp)) return false;
-    const bool wants_mask = ep.row_zero != nullptr;     // sentinel: bind the caller's mask at launch
-    Plan* pl = plan;
-    plan->steps.push_back(Step{[gp, pl, wants_mask](cudaStream_t s) {
-      if (wants_mask) gp->prob.ep.row_zero = pl->mask_dev;
-      return gemm_launch(*gp, s);
-    }, tag, 2.0 * (double)M * (double)W.n * 64.0 * (double)pr.num_kb, cur_layer});
+    push(tag, [gp](cudaStream_t s) { return gemm_launch(*gp, s); }, 2.0 * (double)M * (double)W.n * 64.0 * (double)pr.num_kb);
     return true;
   }
-};
-
-const unsigned char* const MASK_SENTINEL = reinterpret_cast<const unsigned char*>(0x1);
-
-// activation tensor: `data` holds the values ([rows, C], bf16 in bf16 mode / fp32 in fp32 mode); `op` is the
-// GEMM-operand form (bf16 [rows, P*C]); identical to data in bf16 mode.
-struct Act {
-  void* data = nullptr;
-  void* op = nullptr;
-  long long rows = 0;
-  int C = 0;
+  // dense single-tap GEMM: A [rows, P*K] (operand form) x W^T
+  bool linear(const std::string& tag, const void* A, long long rows, int K, const PackedW& W, const Epilogue& ep) {
+    return gemm(tag, A, rows, P * K, W, rows, {Tap{0, 0, 0}}, K / 64, K, ep);
+  }
 };
 
 struct FrontendBufs {
@@ -911,56 +978,30 @@ struct FrontendBufs {
 };
 
 bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
-  Builder b;
-  b.h = h; b.plan = plan; b.sizing = sizing; b.P = h->P; b.f32 = (h->cfg.compute_mode == AVH_COMPUTE_FP32);
+  Builder b(h, plan, sizing);
   const avh_config& c = h->cfg;
+  const PlanKey& key = plan->key;
   const int P = b.P;
   const bool f32 = b.f32;
-  const int B = plan->B, T = plan->T, D = c.encoder_embed_dim, F = c.encoder_ffn_embed_dim;
+  const int B = key.B, T = key.T, D = c.encoder_embed_dim, F = c.encoder_ffn_embed_dim;
   const int Hh = c.encoder_attention_heads;
-  const bool rg = plan->ragged;
-  const long long N = rg ? plan->Nb : (long long)B * T;
+  const bool rg = key.kind == PlanKind::Ragged;
+  const bool enc_only = key.kind == PlanKind::EncoderOnly;
+  const bool train = key.kind == PlanKind::TrainForward;
+  const bool hm = key.has_mask;
+  const long long N = rg ? key.ragged_rows : (long long)B * T;
   const int E = c.modality_fuse == AVH_FUSE_CONCAT ? 2 * D : D;
-  const size_t es = f32 ? 4 : 2;            // bytes per activation value
-  const int act_dt = f32 ? DT_F32 : DT_BF16;
+  const size_t es = b.es;
+  const int act_dt = b.act_dt;
   Plan* pl = plan;
 
-  auto new_act = [&](long long rows, int C) {
-    Act a;
-    a.rows = rows; a.C = C;
-    a.data = b.alloc((size_t)rows * C * es);
-    a.op = f32 ? b.alloc((size_t)rows * C * 2 * P) : a.data;
-    return a;
-  };
-  // fp32 mode: refresh the split bf16 operand planes of an activation
-  auto sync_op = [&](const Act& a) {
-    if (!f32) return;
-    const float* src = reinterpret_cast<const float*>(a.data);
-    void* dst = a.op;
-    const long long rows = a.rows;
-    const int C = a.C, planes = P;
-    const std::string keep = b.tag;
-    b.tag = "split";
-    b.push([=](cudaStream_t s) { return launch_split_rows(src, C, dst, planes, rows, C, 0, 0, s); });
-    b.tag = keep;
-  };
-  auto ep_base = [&](void* Cptr, long long ldc) {
-    Epilogue ep;
-    ep.C = Cptr; ep.ldc = ldc; ep.c_fp32 = f32 ? 1 : 0;
-    return ep;
-  };
-
-  // stream-K workspace: one fp32 partial tile (128 x 256) per SM + flags (zero from the arena's initial fill; the
-  // kernels hand the flags back as zeros)
-  b.sk_bytes = (size_t)device_sm_count() * 128 * 256 * 4;
-  b.sk_ws = reinterpret_cast<float*>(b.alloc(b.sk_bytes));
-  b.sk_flags = reinterpret_cast<int*>(b.alloc(4096));
+  b.stream_k_workspace();
   {
-    unsigned char* md = reinterpret_cast<unsigned char*>(b.alloc((size_t)B * T + 16));
+    unsigned char* md = b.mask_buf((long long)B * T);
     if (!sizing) plan->mask_dev = md;
   }
   // fused token features [N, E]: audio arm in columns [0,D), video arm in [D,2D) (concat) or summed (add)
-  Act fused = new_act(N, E);
+  Act fused = b.act(N, E);
   if (rg) {
     plan->rag_items_off = 16 + ((B + 1 + 3) / 4) * 4;
     plan->rag_max_items = 11 * (int)(N / 2 + B);
@@ -972,7 +1013,7 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
   const int a_off = 0;
 
   // ========================================================================== lip frontend
-  if (plan->has_video) {
+  if (key.has_video) {
     // chunks of whole clips (the stem's temporal taps are row shifts inside a clip-padded layout)
     const int target = c.frontend_chunk_frames > 0 ? c.frontend_chunk_frames : 2400;
     int CB = std::max(1, target / T);
@@ -980,23 +1021,22 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     if (rg) CB = B;                                                  // ragged: one chunk of Nb packed frames
     const int CF = rg ? (int)N : CB * T;
     FrontendBufs fb;
-    const bool train = plan->train;
     if (f32 || train) {     // patch matrix + un-pooled stem maps: only the unfused stem needs them
       fb.im2col = b.alloc((size_t)CB * (T + 2) * 1936 * 64 * 2 * P);
       fb.stem_out = b.alloc((size_t)CB * (T + 2) * 1936 * 64 * es);      // same clip-padded row space as the patches
     }
     static const int HS[4] = {22, 11, 6, 3};
-    fb.pooled = new_act((long long)CF * 23 * 23, 64);
+    fb.pooled = b.act((long long)CF * 23 * 23, 64);
     for (int L = 0; L < 4; ++L) {
       const int S = HS[L] + 1, Cc = 64 << L;
-      for (int i = 0; i < 4; ++i) fb.a[L][i] = new_act((long long)CF * S * S, Cc);
+      for (int i = 0; i < 4; ++i) fb.a[L][i] = b.act((long long)CF * S * S, Cc);
       if (L > 0) {
-        fb.ds[L] = new_act((long long)CF * S * S, Cc);
+        fb.ds[L] = b.act((long long)CF * S * S, Cc);
         fb.col[L] = b.alloc((size_t)CF * HS[L] * HS[L] * 9 * (Cc / 2) * P * 2);
       }
     }
-    Act pooled_feat = new_act(N, 512);     // avgpool output = ResEncoder output [B*T, 512]
-    if (!sizing) plan->stages["resnet"] = {pooled_feat.data, {act_dt, N * 512}};
+    Act pooled_feat = b.act(N, 512);     // avgpool output = ResEncoder output [B*T, 512]
+    b.stage("resnet", pooled_feat.data, act_dt, N * 512);
 
     // ---- training mode: BatchNorm with batch statistics.  The convolution writes its raw output into a scratch map of
     // the output's own layout, bn_stats / bn_finalize produce scale + bias (and update the running statistics),
@@ -1007,8 +1047,8 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     if (train) {
       bn_raw = b.alloc((size_t)CB * (T + 2) * 1936 * 64 * es);          // the stem's map is the largest
       bn_sums = reinterpret_cast<double*>(b.alloc((size_t)BN_SLOTS * 2 * 512 * sizeof(double)));
-      bn_scale = reinterpret_cast<float*>(b.alloc(512 * 4));
-      bn_bias = reinterpret_cast<float*>(b.alloc(512 * 4));
+      bn_scale = b.f32buf(512);
+      bn_bias = b.f32buf(512);
     }
     // launch(ep) enqueues the convolution with epilogue `ep`; in training mode it is called with a raw epilogue
     auto conv_bn = [&](Epilogue ep, const ConvUnit& cu, long long out_rows, double count, long long period, long long valid,
@@ -1026,16 +1066,15 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
       const float* s2 = ep.slope2;
       const float *gm = cu.gamma, *bt = cu.beta;
       float *rm = cu.rmean, *rv = cu.rvar;
-      const std::string keep = b.tag;
-      b.tag = "bn_train";
-      b.push([=](cudaStream_t s) { return launch_bn_stats(bn_raw, act_dt, out_rows, Cc, period, valid, S, Himg, bn_sums, s); });
-      b.push([=](cudaStream_t s) {
+      b.push("bn_train", [=](cudaStream_t s) {
+        return launch_bn_stats(bn_raw, act_dt, out_rows, Cc, period, valid, S, Himg, bn_sums, s);
+      });
+      b.push("bn_train", [=](cudaStream_t s) {
         return launch_bn_finalize(bn_sums, count, gm, bt, 1e-5f, pl->bn_momentum, rm, rv, bn_scale, bn_bias, Cc, s);
       });
-      b.push([=](cudaStream_t s) {
+      b.push("bn_train", [=](cudaStream_t s) {
         return launch_bn_apply(bn_raw, outp, act_dt, out_rows, Cc, bn_scale, bn_bias, s1, res, s2, S, Himg, s);
       });
-      b.tag = keep;
       return true;
     };
 
@@ -1045,7 +1084,6 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
       const int S = Himg + 1;
       if (!f32 && !train && cu.cin == 64 && cu.cout == 64) {
         // layer1: operand window resident in smem, nine taps as descriptor row offsets (conv_window.cu)
-        b.tag = "conv3x3_c64";
         if (sizing) return true;
         ConvWinProblem wp;
         wp.A = in.op; wp.B = cu.w.w; wp.rows = (long long)nimg * S * S; wp.S = S;
@@ -1054,15 +1092,14 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
         ConvWinPlan* cp = new ConvWinPlan();
         plan->convwins.push_back(cp);
         if (conv_window_plan(wp, cp)) return false;
-        const double fl = 2.0 * (double)wp.rows * 64.0 * 576.0;
-        plan->steps.push_back(Step{[cp](cudaStream_t s) { return conv_window_launch(*cp, s); }, b.tag, fl});
+        b.push("conv3x3_c64", [cp](cudaStream_t s) { return conv_window_launch(*cp, s); }, 2.0 * (double)wp.rows * 64.0 * 576.0);
         return true;
       }
       std::vector<Tap> taps;
       for (int kh = 0; kh < 3; ++kh)
         for (int kw = 0; kw < 3; ++kw)
           taps.push_back(Tap{(kh - 1) * S + (kw - 1), 0, (kh * 3 + kw) * cu.cin});
-      Epilogue ep = ep_base(out.data, cu.cout);
+      Epilogue ep = epilogue(out.data, cu.cout, f32);
       ep.col_scale = cu.scale; ep.col_bias = cu.bias;
       if (slope1) { ep.act = ACT_PRELU; ep.slope1 = slope1; }
       if (res) { ep.R = res->data; ep.ldr = cu.cout; ep.r_fp32 = f32 ? 1 : 0; }
@@ -1070,14 +1107,14 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
       ep.map_mode = MAP_2LEVEL; ep.S2 = S * S; ep.S1 = S; ep.H = Himg; ep.W = Himg;
       ep.O2 = S * S; ep.O1 = S; ep.O0 = 0; ep.invalid_zero = 1;
       const long long rows = (long long)nimg * S * S;
-      b.tag = "conv3x3_c" + std::to_string(cu.cin);
+      const std::string tag = "conv3x3_c" + std::to_string(cu.cin);
       const void* a_op = in.op;
       const int a_cols = P * cu.cin, chunks = cu.cin / 64, aps = cu.cin;
       if (!conv_bn(ep, cu, rows, (double)nimg * Himg * Himg, 0, 0, S, Himg, [&](const Epilogue& e) {
-            return b.gemm(a_op, rows, a_cols, cu.w, rows, taps, chunks, aps, e);
+            return b.gemm(tag, a_op, rows, a_cols, cu.w, rows, taps, chunks, aps, e);
           }))
         return false;
-      sync_op(out);
+      b.sync_op(out);
       return true;
     };
 
@@ -1097,7 +1134,6 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
         fp.B = sc->w->w; fp.scale = sc->ones; fp.bias = sc->bias;
         fp.A2 = sc->A2; fp.ds_Cin = sc->Cin; fp.ds_Sin = sc->Sin; fp.ds_Pin = sc->Sin * sc->Sin; fp.ds_stride = sc->stride;
       }
-      b.tag = tg;
       void* table = b.alloc(conv_frame_table_bytes(fp));
       if (sizing) return true;
       ConvFramePlan* cp = new ConvFramePlan();
@@ -1111,7 +1147,7 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
         }
       const double fl = 2.0 * (double)nimg * taps * taps * (double)Cin * (double)cu.cout +
                         (sc != nullptr ? 2.0 * (double)nimg * Hout * Hout * (double)sc->Cin * (double)cu.cout : 0.0);
-      plan->steps.push_back(Step{[cp](cudaStream_t s) { return conv_frame_launch(*cp, s); }, b.tag, fl});
+      b.push(tg, [cp](cudaStream_t s) { return conv_frame_launch(*cp, s); }, fl);
       return true;
     };
 
@@ -1123,47 +1159,41 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
       if (!f32 && !train) {
         if (!sizing && b0 == 0 && stem_fused_plan(h->stem_wf.w, &plan->stemf)) return false;
         void* po = fb.pooled.data;
-        b.tag = "stem_fused";
         const double fl = 2.0 * (double)nf * 1936.0 * 64.0 * 245.0;
-        if (!sizing && rg)
-          plan->steps.push_back(Step{[=](cudaStream_t s) {
+        if (rg)
+          b.push_direct("stem_fused", [=](cudaStream_t s) {
             return stem_fused_launch_ragged(pl->stemf, pl->args.video, pl->args.video_dt, pl->args.pitch,
                                             reinterpret_cast<const int4*>(pl->rag + pl->rag_items_off), pl->rag, pl->rag + 16,
                                             h->stem.scale, h->stem.bias, h->stem.slope, po, s);
-          }, b.tag, fl, -1, true});
-        else if (!sizing)
-          plan->steps.push_back(Step{[=](cudaStream_t s) {
+          }, fl);
+        else
+          b.push_direct("stem_fused", [=](cudaStream_t s) {
             return stem_fused_launch(pl->stemf, pl->args.video, pl->args.video_dt, T, b0, nb, h->stem.scale, h->stem.bias,
                                      h->stem.slope, po, s);
-          }, b.tag, fl, -1, true});
+          }, fl);
       } else
       // ---- ... else (kh,kw) patches -> GEMM over 5 temporal row-shift taps (+BN+PReLU) -> maxpool
       {
         void* col = fb.im2col;
         const int planes = P;
-        b.tag = "stem_patches";
-        b.cur_direct = true;
-        b.push([=](cudaStream_t s) {
+        b.push_direct("stem_patches", [=](cudaStream_t s) {
           return launch_stem_patches(pl->args.video, pl->args.video_dt, T, b0, nb, col, planes, s);
         });
-        b.cur_direct = false;
-        Epilogue ep = ep_base(fb.stem_out, 64);
+        Epilogue ep = epilogue(fb.stem_out, 64, f32);
         ep.col_scale = h->stem.scale; ep.col_bias = h->stem.bias; ep.act = ACT_PRELU; ep.slope1 = h->stem.slope;
         const long long rows = (long long)nb * (T + 2) * 1936;       // tile rows include the gap frames
         // rows map 1:1 (TMA-store epilogue); rows of the gap frames hold don't-care values nobody reads
         std::vector<Tap> taps;
         for (int dt = 0; dt < 5; ++dt) taps.push_back(Tap{(dt - 2) * 1936, 0, dt * 64});
-        b.tag = "stem_gemm";
         // batch statistics over the frames of the chunk (gap frames of the clip-padded row space excluded)
         if (!conv_bn(ep, h->stem, rows, (double)nf * 1936.0, (long long)(T + 2) * 1936, (long long)T * 1936, 0, 0,
-                     [&](const Epilogue& e) { return b.gemm(fb.im2col, rows, P * 64, h->stem.w, rows, taps, 1, 64, e); }))
+                     [&](const Epilogue& e) { return b.gemm("stem_gemm", fb.im2col, rows, P * 64, h->stem.w, rows, taps, 1, 64, e); }))
           return false;
         void* so = fb.stem_out;
         void* po = fb.pooled.data;
-        b.tag = "maxpool";
-        b.push([=](cudaStream_t s) { return launch_maxpool_stem(so, po, nf, T, f32 ? 1 : 0, s); });
+        b.push("maxpool", [=](cudaStream_t s) { return launch_maxpool_stem(so, po, nf, T, f32 ? 1 : 0, s); });
         Act pv = fb.pooled; pv.rows = (long long)nf * 529;
-        sync_op(pv);
+        b.sync_op(pv);
       }
       // ---- trunk
       Act cur = fb.pooled;
@@ -1200,31 +1230,29 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
             void* col = fb.col[L];
             const void* src = cur.op;
             const int CinP = Cin * P;
-            b.tag = "im2col_s2";
-            b.push([=](cudaStream_t s) { return launch_im2col_s2(src, col, nf, Hp, Hp, CinP, s); });
+            b.push("im2col_s2", [=](cudaStream_t s) { return launch_im2col_s2(src, col, nf, Hp, Hp, CinP, s); });
             const long long rows = (long long)nf * Hn * Hn;
             std::vector<Tap> taps;
             for (int t = 0; t < 9; ++t) taps.push_back(Tap{0, t * CinP, t * Cin});
-            Epilogue ep = ep_base(mid.data, Cc);
+            Epilogue ep = epilogue(mid.data, Cc, f32);
             ep.col_scale = bw.c1.scale; ep.col_bias = bw.c1.bias; ep.act = ACT_PRELU; ep.slope1 = bw.c1.slope;
             ep.map_mode = MAP_2LEVEL; ep.S2 = Hn * Hn; ep.S1 = Hn; ep.H = Hn; ep.W = Hn;
             ep.O2 = S * S; ep.O1 = S; ep.O0 = 0;
-            b.tag = "conv_s2_c" + std::to_string(Cin);
+            const std::string tag = "conv_s2_c" + std::to_string(Cin);
             const long long out_rows = (long long)nf * S * S;
             if (!conv_bn(ep, bw.c1, out_rows, (double)nf * Hn * Hn, 0, 0, S, Hn, [&](const Epilogue& e) {
-                  return b.gemm(col, rows, 9 * CinP, bw.c1.w, rows, taps, Cin / 64, Cin, e);
+                  return b.gemm(tag, col, rows, 9 * CinP, bw.c1.w, rows, taps, Cin / 64, Cin, e);
                 }))
               return false;
-            sync_op(mid);
+            b.sync_op(mid);
             dsout = fb.ds[L];
             dsout.rows = mid.rows;
-            Epilogue epd = ep_base(dsout.data, Cc);
+            Epilogue epd = epilogue(dsout.data, Cc, f32);
             epd.col_scale = bw.ds.scale; epd.col_bias = bw.ds.bias;
             epd.map_mode = MAP_2LEVEL; epd.S2 = Hn * Hn; epd.S1 = Hn; epd.H = Hn; epd.W = Hn;
             epd.O2 = S * S; epd.O1 = S; epd.O0 = 0;
-            b.tag = "downsample";
             if (!conv_bn(epd, bw.ds, out_rows, (double)nf * Hn * Hn, 0, 0, S, Hn, [&](const Epilogue& e) {
-                  return b.gemm(col, rows, 9 * CinP, bw.ds.w, rows, {Tap{0, 4 * CinP, 0}}, Cin / 64, Cin, e);
+                  return b.gemm("downsample", col, rows, 9 * CinP, bw.ds.w, rows, {Tap{0, 4 * CinP, 0}}, Cin / 64, Cin, e);
                 }))
               return false;
             res = &dsout;
@@ -1239,107 +1267,80 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
       {
         const void* src = cur.data;
         char* dst = reinterpret_cast<char*>(pooled_feat.data) + (size_t)f0 * 512 * es;
-        b.tag = "avgpool";
         const int pitch = frame_mode ? 3 : 4;
-        b.push([=](cudaStream_t s) { return launch_avgpool(src, dst, nf, 3, 3, 512, pitch, f32 ? 1 : 0, s); });
+        b.push("avgpool", [=](cudaStream_t s) { return launch_avgpool(src, dst, nf, 3, 3, 512, pitch, f32 ? 1 : 0, s); });
       }
     }
-    sync_op(pooled_feat);
+    b.sync_op(pooled_feat);
     // ---- SubModel.proj (hubert.py:321,327): Linear 512 -> D into the video columns of the fused buffer
-    {
-      Epilogue ep = ep_base(reinterpret_cast<char*>(fused.data) + (size_t)v_off * es, E);
-      ep.col_bias = h->proj_v.bias;
-      b.tag = "proj_video";
-      if (!b.gemm(pooled_feat.op, N, P * 512, h->proj_v.w, N, {Tap{0, 0, 0}}, 512 / 64, 512, ep)) return false;
-    }
+    Epilogue ep = epilogue(reinterpret_cast<char*>(fused.data) + (size_t)v_off * es, E, f32);
+    ep.col_bias = h->proj_v.bias;
+    if (!b.linear("proj_video", pooled_feat.op, N, 512, h->proj_v.w, ep)) return false;
   }
   // ========================================================================== audio arm
-  if (plan->has_audio) {
+  if (key.has_audio) {
     const int Fa = c.audio_feat_dim, Fp = round_up(Fa, 64);
-    Act arows = new_act(N, Fp);       // zero-initialised; only the first Fa columns are ever written
-    {
-      void* dst = arows.data;
-      b.tag = "audio_rows";
-      b.cur_direct = true;
-      if (rg)
-        b.push([=](cudaStream_t s) {
-          return launch_bct_to_rows_ragged(pl->args.audio, pl->args.audio_dt, pl->args.as[0], pl->args.as[1], pl->args.as[2],
-                                           B, Fa, pl->rag + 16, dst, act_dt, Fp, N, s);
-        });
-      else
-        b.push([=](cudaStream_t s) {
-          return launch_bct_to_rows(pl->args.audio, pl->args.audio_dt, pl->args.as[0], pl->args.as[1], pl->args.as[2],
-                                    B, Fa, T, dst, act_dt, Fp, s);
-        });
-      b.cur_direct = false;
-      sync_op(arows);
-    }
-    Epilogue ep = ep_base(reinterpret_cast<char*>(fused.data) + (size_t)a_off * es, E);
+    Act arows = b.act(N, Fp);       // zero-initialised; only the first Fa columns are ever written
+    void* dst = arows.data;
+    if (rg)
+      b.push_direct("audio_rows", [=](cudaStream_t s) {
+        return launch_bct_to_rows_ragged(pl->args.audio, pl->args.audio_dt, pl->args.as[0], pl->args.as[1], pl->args.as[2],
+                                         B, Fa, pl->rag + 16, dst, act_dt, Fp, N, s);
+      });
+    else
+      b.push_direct("audio_rows", [=](cudaStream_t s) {
+        return launch_bct_to_rows(pl->args.audio, pl->args.audio_dt, pl->args.as[0], pl->args.as[1], pl->args.as[2],
+                                  B, Fa, T, dst, act_dt, Fp, s);
+      });
+    b.sync_op(arows);
+    Epilogue ep = epilogue(reinterpret_cast<char*>(fused.data) + (size_t)a_off * es, E, f32);
     ep.col_bias = h->proj_a.bias;
-    if (c.modality_fuse == AVH_FUSE_ADD && plan->has_video) {     // features_audio + features_video
+    if (c.modality_fuse == AVH_FUSE_ADD && key.has_video) {     // features_audio + features_video
       ep.R = ep.C; ep.ldr = E; ep.r_fp32 = f32 ? 1 : 0;
     }
-    b.tag = "proj_audio";
-    if (!b.gemm(arows.op, N, P * Fp, h->proj_a.w, N, {Tap{0, 0, 0}}, Fp / 64, Fp, ep)) return false;
+    if (!b.linear("proj_audio", arows.op, N, Fp, h->proj_a.w, ep)) return false;
   }
   // a missing modality contributes zeros [B,D,T] (hubert.py:703-708): with concat its columns stay at the
   // arena's zero fill (nothing ever writes them for this plan); with add there is nothing to add.
 
   // ========================================================================== fusion LN + post_extract_proj
-  float* x = reinterpret_cast<float*>(b.alloc((size_t)N * D * 4));      // residual stream, fp32
-  if (plan->enc_only) {
+  float* x = b.f32buf(N * D);      // residual stream, fp32
+  if (enc_only) {
     // TransformerEncoder.forward on the caller's features: x = features with padded frames zeroed (wav2vec2.py:869-870)
-    const bool hm0 = plan->has_mask;
-    b.tag = "load_features";
-    b.cur_direct = true;
-    b.push([=](cudaStream_t s) {
-      return launch_load_rows(pl->args.xin, pl->args.xin_dt, x, hm0 ? pl->mask_dev : nullptr, N, D, s);
+    b.push_direct("load_features", [=](cudaStream_t s) {
+      return launch_load_rows(pl->args.xin, pl->args.xin_dt, x, hm ? pl->mask_dev : nullptr, N, D, s);
     });
-    b.cur_direct = false;
-  }
-  Act lnE = plan->enc_only ? Act() : new_act(N, E);
-  if (!plan->enc_only) {
-    const void* src = fused.data;
-    if (!sizing) plan->stages["fused"] = {fused.data, {act_dt, N * E}};     // pre-LayerNorm features (features_pen)
-    float* of = f32 ? reinterpret_cast<float*>(lnE.data) : nullptr;
-    void* ol = f32 ? nullptr : lnE.data;
-    float* g = h->fuse_ln_g; float* be = h->fuse_ln_b;
-    b.tag = "fuse_ln";
+  } else {
+    b.stage("fused", fused.data, act_dt, N * E);     // pre-LayerNorm features (features_pen)
+    Act lnE = b.act(N, E);
     if (h->has_post_proj) {
-      b.push([=](cudaStream_t s) {
-        return launch_layernorm(src, act_dt, E, g, be, 1e-5f, of, ol, DT_BF16, nullptr, N, E, s);
-      });
-      sync_op(lnE);
-      if (!sizing) plan->stages["fused_ln"] = {lnE.data, {act_dt, N * E}};
-      Epilogue ep;
-      ep.C = x; ep.ldc = D; ep.c_fp32 = 1;
+      b.layernorm("fuse_ln", fused.data, act_dt, h->fuse_ln_g, h->fuse_ln_b, 1e-5f, lnE);
+      b.stage("fused_ln", lnE.data, act_dt, N * E);
+      Epilogue ep = epilogue(x, D, true);
       ep.col_bias = h->post_proj.bias;
-      if (plan->has_mask) ep.row_zero = MASK_SENTINEL;      // index_put(x, padding_mask, 0), wav2vec2.py:869-870
-      b.tag = "post_extract_proj";
-      if (!b.gemm(lnE.op, N, P * E, h->post_proj.w, N, {Tap{0, 0, 0}}, E / 64, E, ep)) return false;
+      ep.row_zero = hm ? plan->mask_dev : nullptr;      // index_put(x, padding_mask, 0), wav2vec2.py:869-870
+      if (!b.linear("post_extract_proj", lnE.op, N, E, h->post_proj.w, ep)) return false;
     } else {
       // no post_extract_proj (embed == D): the LN output is the encoder input; zero padded rows here
-      const bool hm = plan->has_mask;
-      b.push([=](cudaStream_t s) {
+      const void* src = fused.data;
+      float* g = h->fuse_ln_g; float* be = h->fuse_ln_b;
+      b.push("fuse_ln", [=](cudaStream_t s) {
         return launch_layernorm(src, act_dt, E, g, be, 1e-5f, x, nullptr, DT_BF16, hm ? pl->mask_dev : nullptr, N, E, s);
       });
-      if (!sizing) plan->stages["fused_ln"] = {x, {DT_F32, N * E}};
+      b.stage("fused_ln", x, DT_F32, N * E);
     }
   }
-  const bool train = plan->train;
   if (train) {      // features = self.dropout_input(features), hubert.py:729
-    b.tag = "dropout";
-    b.push([=](cudaStream_t s) {
+    b.push("dropout", [=](cudaStream_t s) {
       return pl->p_in > 0.f ? launch_dropout(x, DT_F32, nullptr, N * D, pl->p_in, pl->seed, 1u, s) : 0;
     });
   }
   if (c.capture_stages) {      // x is overwritten in place by the encoder: keep a copy for stage-level tests
-    b.tag = "stage_copy";
-    float* enc_in_copy = reinterpret_cast<float*>(b.alloc((size_t)N * D * 4));
-    b.push([=](cudaStream_t s) {
+    float* enc_in_copy = b.f32buf(N * D);
+    b.push("stage_copy", [=](cudaStream_t s) {
       return cudaMemcpyAsync(enc_in_copy, x, (size_t)N * D * 4, cudaMemcpyDeviceToDevice, s) == cudaSuccess ? 0 : 1;
     });
-    if (!sizing) plan->stages["enc_in"] = {enc_in_copy, {DT_F32, N * D}};
+    b.stage("enc_in", enc_in_copy, DT_F32, N * D);
   }
 
   // ========================================================================== positional conv + GELU + residual
@@ -1348,197 +1349,151 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     const long long pad_rows = rg ? N + (long long)G * B : (long long)B * Tp;
     void* xpad = b.alloc((size_t)pad_rows * P * D * 2);      // bf16 [B*(T+64), P*D], gap rows stay zero
     const int planes = P;
-    b.tag = "pos_pad";
     int* row_map = nullptr;
     if (rg) {
       // packed clips: clip b at padded rows [cu[b] + 64 b, +T_b); the kernel also zeroes the gap rows (they move from
       // call to call) and writes the padded-row -> packed-row map the convolution's epilogue stores through
       row_map = reinterpret_cast<int*>(b.alloc((size_t)pad_rows * 4));
       if (!sizing) plan->pos_row_map = row_map;
-      b.push([=](cudaStream_t s) { return launch_pos_pad_ragged(x, D, xpad, row_map, pl->rag + 16, B, D, G, pad_rows, s); });
+      b.push("pos_pad", [=](cudaStream_t s) { return launch_pos_pad_ragged(x, D, xpad, row_map, pl->rag + 16, B, D, G, pad_rows, s); });
     } else
-    b.push([=](cudaStream_t s) { return launch_split_rows(x, D, xpad, planes, N, D, T, Tp, s); });
-    b.tag = "pos_conv";
+    b.push("pos_pad", [=](cudaStream_t s) { return launch_split_rows(x, D, xpad, planes, N, D, T, Tp, s); });
     const int KT = c.conv_pos, win = h->pos_window;
     std::vector<Tap> taps;
     for (int k = 0; k < KT; ++k) taps.push_back(Tap{k - KT / 2, 0, k * win});
-    Epilogue ep;
-    ep.C = x; ep.ldc = D; ep.c_fp32 = 1;
+    Epilogue ep = epilogue(x, D, true);
     ep.col_bias = h->pos_bias; ep.act = ACT_GELU;
     ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
     if (rg) ep.row_map = row_map;
     else { ep.map_mode = MAP_2LEVEL; ep.S2 = Tp; ep.S1 = Tp; ep.H = 1; ep.W = T; ep.O2 = T; ep.O1 = 0; ep.O0 = 0; }
-    if (!b.gemm(xpad, pad_rows, P * D, h->pos_w, pad_rows, taps, win / 64, D, ep, 64, h->pos_acol))
+    if (!b.gemm("pos_conv", xpad, pad_rows, P * D, h->pos_w, pad_rows, taps, win / 64, D, ep, 64, h->pos_acol))
       return false;
   }
 
   // ========================================================================== transformer layers
-  float* dtmp = train ? reinterpret_cast<float*>(b.alloc((size_t)N * D * 4)) : nullptr;     // block output before dropout + add
-  Act hbuf = new_act(N, D);          // LayerNorm output / post-LN operand copy of x
-  Act qkv = new_act(N, 3 * D);
-  Act ctx = new_act(N, D);
-  Act ffn = new_act(N, F);
-  float* tmp = c.layer_norm_first ? nullptr : reinterpret_cast<float*>(b.alloc((size_t)N * D * 4));
-  const bool hm = plan->has_mask;
+  float* dtmp = train ? b.f32buf(N * D) : nullptr;     // block output before dropout + add
+  Act hbuf = b.act(N, D);          // LayerNorm output / post-LN operand copy of x
+  Act qkv = b.act(N, 3 * D);
+  Act ctx = b.act(N, D);
+  Act ffn = b.act(N, F);
+  float* tmp = c.layer_norm_first ? nullptr : b.f32buf(N * D);
 
-  auto ln_to_h = [&](const float* src, const float* g, const float* be, float* also_f32) {
-    // LN(src) -> hbuf (operand form) and optionally an fp32 copy (post-LN: the new residual stream)
-    float* of = f32 ? reinterpret_cast<float*>(hbuf.data) : also_f32;
-    void* ol = f32 ? nullptr : hbuf.data;
-    b.tag = "layer_ln";
-    b.push([=](cudaStream_t s) { return launch_layernorm(src, DT_F32, D, g, be, 1e-5f, of, ol, DT_BF16, nullptr, N, D, s); });
-    if (f32 && also_f32 != nullptr) {
-      float* hd = reinterpret_cast<float*>(hbuf.data);
-      b.push([=](cudaStream_t s) {
-        return cudaMemcpyAsync(also_f32, hd, (size_t)N * D * 4, cudaMemcpyDeviceToDevice, s) == cudaSuccess ? 0 : 1;
-      });
-    }
-    sync_op(hbuf);
+  // post-LN: x = LayerNorm(src) in place of the residual stream (src = x or tmp)
+  auto post_ln = [&](const float* src, const float* g, const float* be) {
+    b.push("layer_ln", [=](cudaStream_t s) { return launch_layernorm(src, DT_F32, D, g, be, 1e-5f, x, nullptr, DT_BF16, nullptr, N, D, s); });
   };
-  auto x_to_h = [&]() {   // operand copy of the residual stream (post-LN blocks read x itself)
-    void* dst = hbuf.op;
-    const int planes = P;
-    b.tag = "split";
-    b.push([=](cudaStream_t s) { return launch_split_rows(x, D, dst, planes, N, D, 0, 0, s); });
-  };
-
   if (!c.layer_norm_first) {
     // encoder-level LayerNorm right after the positional conv (wav2vec2.py:876-877)
-    float* g = h->enc_ln_g; float* be = h->enc_ln_b;
-    b.tag = "layer_ln";
-    b.push([=](cudaStream_t s) { return launch_layernorm(x, DT_F32, D, g, be, 1e-5f, x, nullptr, DT_BF16, nullptr, N, D, s); });
-    if (!train) x_to_h();
+    post_ln(x, h->enc_ln_g, h->enc_ln_b);
+    if (!train) b.split(x, D, hbuf.op, N, D);      // operand copy of the residual stream (post-LN blocks read x itself)
   }
   if (train) {      // x = F.dropout(x, p=self.dropout, training=self.training), wav2vec2.py:879
-    b.tag = "dropout";
-    b.push([=](cudaStream_t s) {
+    b.push("dropout", [=](cudaStream_t s) {
       return pl->p_enc > 0.f ? launch_dropout(x, DT_F32, nullptr, N * D, pl->p_enc, pl->seed, 2u, s) : 0;
     });
-    if (!c.layer_norm_first) x_to_h();
+    if (!c.layer_norm_first) b.split(x, D, hbuf.op, N, D);
   }
-  const int n_layers = plan->output_layer > 0 ? std::min(plan->output_layer, c.encoder_layers) : c.encoder_layers;
+  const int n_layers = key.output_layer > 0 ? std::min(key.output_layer, c.encoder_layers) : c.encoder_layers;
   // measured (tools/att_bench.py, Large head count): tcgen05 11.4 vs 12.8 us at 16 x 150, 21.6 vs 29.0 at 8 x 300,
   // 31.9 vs 44.3 at 4 x 600; short clips (64 x 38 frames: 12.6 vs 9.3 us) stay on the mma.sync kernel
   const bool att_tc = !f32 && (rg || T > 96) && (size_t)((T + 127) / 128 * 128) * 4 <= 48 * 1024;
   for (int l = 0; l < n_layers; ++l) {
     const LayerW& lw = h->layers[l];
     b.cur_layer = l;               // LayerDrop (training mode) skips every launch of a dropped layer
-    if (c.layer_norm_first) ln_to_h(x, lw.ln1_g, lw.ln1_b, nullptr);
+    if (c.layer_norm_first) b.layernorm("layer_ln", x, DT_F32, lw.ln1_g, lw.ln1_b, 1e-5f, hbuf);
     {   // fused QKV projection
-      Epilogue ep = ep_base(qkv.data, 3 * D);
+      Epilogue ep = epilogue(qkv.data, 3 * D, f32);
       ep.col_bias = lw.qkv.bias;
-      b.tag = "qkv_proj";
-      if (!b.gemm(hbuf.op, N, P * D, lw.qkv.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      if (!b.linear("qkv_proj", hbuf.op, N, D, lw.qkv.w, ep)) return false;
     }
     {
       const void* q = qkv.data; void* o = ctx.data;
-      b.tag = "attention";
       const double att_flops = 4.0 * (double)B * Hh * (double)T * (double)T * 64.0;   // QK^T + PV, dense (padding not excluded)
       if (att_tc) {
         // bf16 mode: tcgen05 / TMEM kernel (attention_tc.cu)
         if (!sizing && l == 0 && attention_tc_plan(q, N, B, T, D, Hh, &plan->att)) return false;
-        b.push([=](cudaStream_t s) {
-          return attention_tc_launch(pl->att, hm ? pl->mask_dev : nullptr, pl->ragged ? pl->rag + 16 : nullptr, o, s);
+        b.push("attention", [=](cudaStream_t s) {
+          return attention_tc_launch(pl->att, hm ? pl->mask_dev : nullptr, rg ? pl->rag + 16 : nullptr, o, s);
         }, att_flops);
       } else {
-        b.push([=](cudaStream_t s) {
+        b.push("attention", [=](cudaStream_t s) {
           return launch_attention(q, hm ? pl->mask_dev : nullptr, o, B, T, D, Hh, f32 ? 1 : 0, s);
         }, att_flops);
       }
-      sync_op(ctx);
+      b.sync_op(ctx);
     }
     // training mode: block output -> dtmp, then target (+)= dropout(dtmp) (dropout1 / dropout3, wav2vec2.py:980,990);
     // with p = 0 this is the eval arithmetic (fp32 block output added to the fp32 residual stream)
     auto dropout_add = [&](unsigned site) {
       float* target = c.layer_norm_first ? x : tmp;
-      b.tag = "dropout";
       if (!c.layer_norm_first)
-        b.push([=](cudaStream_t s) {
+        b.push("dropout", [=](cudaStream_t s) {
           return cudaMemcpyAsync(tmp, x, (size_t)N * D * 4, cudaMemcpyDeviceToDevice, s) == cudaSuccess ? 0 : 1;
         });
-      b.push([=](cudaStream_t s) { return launch_dropout(target, DT_F32, dtmp, N * D, pl->p_enc, pl->seed, site, s); });
+      b.push("dropout", [=](cudaStream_t s) { return launch_dropout(target, DT_F32, dtmp, N * D, pl->p_enc, pl->seed, site, s); });
     };
     {   // out_proj + residual
-      Epilogue ep;
-      ep.C = c.layer_norm_first ? x : tmp; ep.ldc = D; ep.c_fp32 = 1;
+      Epilogue ep = epilogue(c.layer_norm_first ? x : tmp, D, true);
       ep.col_bias = lw.out.bias; ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
       if (train) { ep.C = dtmp; ep.R = nullptr; }
-      b.tag = "out_proj";
-      if (!b.gemm(ctx.op, N, P * D, lw.out.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      if (!b.linear("out_proj", ctx.op, N, D, lw.out.w, ep)) return false;
       if (train) dropout_add(16u + 4u * (unsigned)l);
     }
-    if (c.layer_norm_first) ln_to_h(x, lw.ln2_g, lw.ln2_b, nullptr);
+    if (c.layer_norm_first) b.layernorm("layer_ln", x, DT_F32, lw.ln2_g, lw.ln2_b, 1e-5f, hbuf);
     else {
-      float* g = lw.ln1_g; float* be = lw.ln1_b;
-      b.tag = "layer_ln";
-      b.push([=](cudaStream_t s) { return launch_layernorm(tmp, DT_F32, D, g, be, 1e-5f, x, nullptr, DT_BF16, nullptr, N, D, s); });
-      x_to_h();
+      post_ln(tmp, lw.ln1_g, lw.ln1_b);
+      b.split(x, D, hbuf.op, N, D);
     }
     {   // fc1 + GELU (erf form, fp32: fairseq/fairseq/modules/gelu.py:95-96)
-      Epilogue ep = ep_base(ffn.data, F);
+      Epilogue ep = epilogue(ffn.data, F, f32);
       ep.col_bias = lw.fc1.bias; ep.act = ACT_GELU;
-      b.tag = "fc1";
-      if (!b.gemm(hbuf.op, N, P * D, lw.fc1.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      if (!b.linear("fc1", hbuf.op, N, D, lw.fc1.w, ep)) return false;
       if (train) {      // dropout2 = activation_dropout after the GELU, wav2vec2.py:987
         void* fd = ffn.data;
         const unsigned site = 17u + 4u * (unsigned)l;
-        b.tag = "dropout";
-        b.push([=](cudaStream_t s) {
+        b.push("dropout", [=](cudaStream_t s) {
           return pl->p_act > 0.f ? launch_dropout(fd, act_dt, nullptr, N * F, pl->p_act, pl->seed, site, s) : 0;
         });
       }
-      sync_op(ffn);
+      b.sync_op(ffn);
     }
     {   // fc2 + residual
-      Epilogue ep;
-      ep.C = c.layer_norm_first ? x : tmp; ep.ldc = D; ep.c_fp32 = 1;
+      Epilogue ep = epilogue(c.layer_norm_first ? x : tmp, D, true);
       ep.col_bias = lw.fc2.bias; ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
       if (train) { ep.C = dtmp; ep.R = nullptr; }
-      b.tag = "fc2";
-      if (!b.gemm(ffn.op, N, P * F, lw.fc2.w, N, {Tap{0, 0, 0}}, F / 64, F, ep)) return false;
+      if (!b.linear("fc2", ffn.op, N, F, lw.fc2.w, ep)) return false;
       if (train) dropout_add(18u + 4u * (unsigned)l);
     }
     if (!c.layer_norm_first) {
-      float* g = lw.ln2_g; float* be = lw.ln2_b;
-      b.tag = "layer_ln";
-      b.push([=](cudaStream_t s) { return launch_layernorm(tmp, DT_F32, D, g, be, 1e-5f, x, nullptr, DT_BF16, nullptr, N, D, s); });
-      if (l + 1 < n_layers) x_to_h();
+      post_ln(tmp, lw.ln2_g, lw.ln2_b);
+      if (l + 1 < n_layers) b.split(x, D, hbuf.op, N, D);
     }
   }
   b.cur_layer = -1;
   // ========================================================================== output
-  b.tag = "final_ln";
+  const bool final_ln = c.layer_norm_first && key.output_layer == 0;
+  float* g = h->enc_ln_g; float* be = h->enc_ln_b;
   if (rg) {
     // packed rows -> the caller's [B, pitch_T, D] tensor, zeros at the pad positions
     float* y = x;
-    if (c.layer_norm_first && plan->output_layer == 0) {
-      y = reinterpret_cast<float*>(b.alloc((size_t)N * D * 4));
-      float* g = h->enc_ln_g; float* be = h->enc_ln_b;
-      b.push([=](cudaStream_t s) { return launch_layernorm(x, DT_F32, D, g, be, 1e-5f, y, nullptr, DT_BF16, nullptr, N, D, s); });
+    if (final_ln) {
+      y = b.f32buf(N * D);
+      b.push("final_ln", [=](cudaStream_t s) { return launch_layernorm(x, DT_F32, D, g, be, 1e-5f, y, nullptr, DT_BF16, nullptr, N, D, s); });
     }
-    b.tag = "unpack";
-    b.cur_direct = true;
-    b.push([=](cudaStream_t s) {
+    b.push_direct("unpack", [=](cudaStream_t s) {
       return launch_unpack_rows(y, pl->rag + 16, pl->args.out, pl->args.out_dt, B, pl->args.pitch, D, s);
     });
-  } else
-  if (c.layer_norm_first && plan->output_layer == 0) {
-    b.cur_direct = true;
-    float* g = h->enc_ln_g; float* be = h->enc_ln_b;
-    b.push([=](cudaStream_t s) {
+  } else if (final_ln) {
+    b.push_direct("final_ln", [=](cudaStream_t s) {
       return launch_layernorm(x, DT_F32, D, g, be, 1e-5f, nullptr, pl->args.out, pl->args.out_dt, nullptr, N, D, s);
     });
   } else {
-    b.cur_direct = true;
-    b.push([=](cudaStream_t s) { return launch_convert(x, DT_F32, pl->args.out, pl->args.out_dt, N * D, s); });
+    b.push_direct("final_ln", [=](cudaStream_t s) { return launch_convert(x, DT_F32, pl->args.out, pl->args.out_dt, N * D, s); });
   }
-  b.cur_direct = false;
   if (bytes_out) *bytes_out = b.sizer.used;
   return true;
 }
 
-// One plan (= workspace + launch list) per shape AND per CUDA stream: forwards enqueued on different streams
-// never share scratch memory, so a caller can keep several batches in flight on one device.
 // ============================================================================ encoder training plan
 // TransformerEncoder forward with saved activations + its backward (pre-LN layers; dropout / LayerDrop 0 as BASELINE
 // config 5 states).  Forward: x0 = index_put(features, mask, 0); c = pos_conv(x0) + b; x1 = x0 + GELU(c); per layer
@@ -1567,8 +1522,8 @@ long long enc_grad_floats(const avh_config& c, int tail = 0, bool has_video = tr
 // dw[o, i, k] = sum_{b,t} dc[b,t,o] x0[b, t + k - KT/2, g(o) cg + i].  Per group one GEMM over K = the zero-gapped token
 // axis: A = rows [g cg, +cg) of dc^T, B = the (tap, input channel) rows of the group — shifted copies of x0^T — so that
 // N = KT cg; output [cg, KT cg] = dw of the group as (o, tap, in).  Then dg, dv of w = g v / ||v||.
-bool posconv_wgrad(Builder& b, avh_handle* h, Plan* plan, const float* dc, const float* x0, long long N, int B, int T,
-                   float* g_wg, float* g_wv) {
+bool posconv_wgrad(Builder& b, avh_handle* h, const float* dc, const float* x0, long long N, int B, int T, float* g_wg,
+                   float* g_wv) {
   const avh_config& c = h->cfg;
   const int D = c.encoder_embed_dim, KT = c.conv_pos, G = c.conv_pos_groups, cg = D / G, P = b.P;
   const int Tp = T + 64;
@@ -1576,27 +1531,21 @@ bool posconv_wgrad(Builder& b, avh_handle* h, Plan* plan, const float* dc, const
   void* dcT = b.alloc((size_t)D * P * kp * 2);
   void* x0T = b.alloc((size_t)D * P * kp * 2);
   void* XS = b.alloc((size_t)KT * cg * P * kp * 2);
-  float* dw = reinterpret_cast<float*>(b.alloc((size_t)D * KT * cg * 4));
-  float* norms = reinterpret_cast<float*>(b.alloc((size_t)KT * 4));
+  float* dw = b.f32buf((long long)D * KT * cg);
+  float* norms = b.f32buf(KT);
   const int planes = P;
-  b.tag = "transpose";
-  b.push([=](cudaStream_t s) { return launch_transpose_split(dc, DT_F32, D, N, D, dcT, planes, kp, 1.0f, s, T, Tp); });
-  b.push([=](cudaStream_t s) { return launch_transpose_split(x0, DT_F32, D, N, D, x0T, planes, kp, 1.0f, s, T, Tp); });
+  b.push("transpose", [=](cudaStream_t s) { return launch_transpose_split(dc, DT_F32, D, N, D, dcT, planes, kp, 1.0f, s, T, Tp); });
+  b.push("transpose", [=](cudaStream_t s) { return launch_transpose_split(x0, DT_F32, D, N, D, x0T, planes, kp, 1.0f, s, T, Tp); });
   for (int g = 0; g < G; ++g) {
-    b.tag = "pos_conv_shift";
-    b.push([=](cudaStream_t s) { return launch_posconv_shift(x0T, XS, g, cg, KT, planes, kp, s); });
+    b.push("pos_conv_shift", [=](cudaStream_t s) { return launch_posconv_shift(x0T, XS, g, cg, KT, planes, kp, s); });
     PackedW xw;
     xw.w = reinterpret_cast<bf16*>(XS); xw.n = KT * cg; xw.k = (int)kp; xw.kpad = (int)kp;
-    Epilogue ep;
-    ep.C = dw + (size_t)g * cg * KT * cg; ep.ldc = (long long)KT * cg; ep.c_fp32 = 1;
+    const Epilogue ep = epilogue(dw + (size_t)g * cg * KT * cg, (long long)KT * cg, true);
     const char* a = reinterpret_cast<const char*>(dcT) + (size_t)g * cg * P * kp * 2;
-    b.tag = "pos_conv_wgrad";
-    if (!b.gemm(a, cg, P * (int)kp, xw, cg, {Tap{0, 0, 0}}, (int)(kp / 64), (int)kp, ep)) return false;
+    if (!b.linear("pos_conv_wgrad", a, cg, (int)kp, xw, ep)) return false;
   }
   const float* v = h->pos_v_raw; const float* gg = h->pos_g_raw;
-  b.tag = "weight_norm_bwd";
-  b.push([=](cudaStream_t s) { return launch_posconv_weightnorm_bwd(dw, v, gg, D, cg, KT, g_wg, g_wv, norms, s); });
-  (void)plan;
+  b.push("weight_norm_bwd", [=](cudaStream_t s) { return launch_posconv_weightnorm_bwd(dw, v, gg, D, cg, KT, g_wg, g_wv, norms, s); });
   return true;
 }
 
@@ -1626,58 +1575,33 @@ long long frontend_grad_floats(const avh_config& c, bool has_video, bool has_aud
 }
 
 bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
-  Builder b;
-  b.h = h; b.plan = plan; b.sizing = sizing; b.P = h->P; b.f32 = (h->cfg.compute_mode == AVH_COMPUTE_FP32);
+  Builder b(h, plan, sizing);
   const avh_config& c = h->cfg;
+  const PlanKey& key = plan->key;
   const int P = b.P;
   const bool f32 = b.f32;
-  const int B = plan->B, T = plan->T, D = c.encoder_embed_dim, F = c.encoder_ffn_embed_dim, Hh = c.encoder_attention_heads;
+  const int B = key.B, T = key.T, D = c.encoder_embed_dim, F = c.encoder_ffn_embed_dim, Hh = c.encoder_attention_heads;
   const int L = c.encoder_layers;
   const long long N = (long long)B * T;
   const long long Kp = (N + 63) / 64 * 64;                  // token count padded to whole K blocks (wgrad GEMMs)
-  const size_t es = f32 ? 4 : 2;
-  const int act_dt = f32 ? DT_F32 : DT_BF16;
+  const size_t es = b.es;
+  const int act_dt = b.act_dt;
   Plan* pl = plan;
   if (!c.layer_norm_first) { set_last_error("the encoder backward is built for pre-LN layers (layer_norm_first)"); return false; }
-  auto new_act = [&](long long rows, int C) {
-    Act a;
-    a.rows = rows; a.C = C;
-    a.data = b.alloc((size_t)rows * C * es);
-    a.op = f32 ? b.alloc((size_t)rows * C * 2 * P) : a.data;
-    return a;
-  };
-  auto sync_op = [&](const Act& a) {
-    if (!f32) return;
-    const float* src = reinterpret_cast<const float*>(a.data);
-    void* dst = a.op;
-    const long long rows = a.rows;
-    const int C = a.C, planes = P;
-    const std::string keep = b.tag;
-    b.tag = "split";
-    b.push([=](cudaStream_t s) { return launch_split_rows(src, C, dst, planes, rows, C, 0, 0, s); });
-    b.tag = keep;
-  };
-  auto f32buf = [&](long long n) { return reinterpret_cast<float*>(b.alloc((size_t)n * 4)); };
-  b.sk_bytes = 0; b.sk_ws = nullptr; b.sk_flags = nullptr;
   {
-    unsigned char* md = reinterpret_cast<unsigned char*>(b.alloc((size_t)N + 16));
+    unsigned char* md = b.mask_buf(N);
     if (!sizing) plan->mask_dev = md;
   }
-  const bool hm = plan->has_mask;
-  const int tail = plan->tail;
+  const bool hm = key.has_mask;
+  const int tail = key.kind == PlanKind::FullTrain ? 2 : (key.kind == PlanKind::TailTrain ? 1 : 0);
   const bool full = tail == 2;
-  if (!f32 && full) {
-    // stream-K workspace for the lip ResNet's weight-gradient GEMMs (a handful of output tiles, K = pixels): one fp32
-    // partial tile per SM + flags (zero from the arena's initial fill; the kernels hand the flags back as zeros)
-    b.sk_bytes = (size_t)device_sm_count() * 128 * 256 * 4;
-    b.sk_ws = reinterpret_cast<float*>(b.alloc(b.sk_bytes));
-    b.sk_flags = reinterpret_cast<int*>(b.alloc(4096));
-  }
+  // stream-K workspace for the lip ResNet's weight-gradient GEMMs (a handful of output tiles, K = pixels)
+  if (!f32 && full) b.stream_k_workspace();
   const int E = c.modality_fuse == AVH_FUSE_CONCAT ? 2 * D : D;
-  const long long GF = enc_grad_floats(c, tail, plan->has_video, plan->has_audio);
-  float* grads = f32buf(GF);
-  float* dy = f32buf(N * D);
-  float* dxo = f32buf(N * D);
+  const long long GF = enc_grad_floats(c, tail, key.has_video, key.has_audio);
+  float* grads = b.f32buf(GF);
+  float* dy = b.f32buf(N * D);
+  float* dxo = b.f32buf(N * D);
   if (!sizing) { plan->grads = grads; plan->grad_floats = GF; plan->dy_in = dy; plan->dx_out = dxo; }
   // gradient bucket [begin, end) of the flat buffer is final here: a direct (never captured) step hands it to the caller —
   // converted into the caller's buffer when avh_encoder_backward_buckets runs the plan — and records the bucket's event,
@@ -1691,10 +1615,7 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       plan->buckets.push_back(gb);
       k = (int)plan->buckets.size() - 1;
     }
-    const std::string keep = b.tag;
-    b.tag = "grad_bucket";
-    b.cur_direct = true;
-    b.push([=](cudaStream_t s) {
+    b.push_direct("grad_bucket", [=](cudaStream_t s) {
       const CallArgs& a = pl->args;
       if (a.grads_out == nullptr) return 0;
       const Plan::GradBucket& gb = pl->buckets[k];
@@ -1704,22 +1625,20 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
         return 1;
       return cudaEventRecord(gb.ev, s) == cudaSuccess ? 0 : 1;
     });
-    b.cur_direct = false;
-    b.tag = keep;
   };
 
   // ---------------------------------------------------------------- saved activations
-  float* x0 = f32buf(N * D);
-  float* cpre = f32buf(N * D);                               // positional conv output before the GELU
+  float* x0 = b.f32buf(N * D);
+  float* cpre = b.f32buf(N * D);                               // positional conv output before the GELU
   std::vector<float*> xin(L + 1), xmid(L);
   std::vector<Act> h1(L), qkv(L), ctx(L), h2(L), u(L), g(L);
   std::vector<float*> lse(L);
-  for (int l = 0; l <= L; ++l) xin[l] = f32buf(N * D);
+  for (int l = 0; l <= L; ++l) xin[l] = b.f32buf(N * D);
   for (int l = 0; l < L; ++l) {
-    xmid[l] = f32buf(N * D);
-    h1[l] = new_act(N, D); qkv[l] = new_act(N, 3 * D); ctx[l] = new_act(N, D); h2[l] = new_act(N, D);
-    u[l] = new_act(N, F); g[l] = new_act(N, F);
-    lse[l] = f32buf((long long)B * Hh * T);
+    xmid[l] = b.f32buf(N * D);
+    h1[l] = b.act(N, D); qkv[l] = b.act(N, 3 * D); ctx[l] = b.act(N, D); h2[l] = b.act(N, D);
+    u[l] = b.act(N, F); g[l] = b.act(N, F);
+    lse[l] = b.f32buf((long long)B * Hh * T);
   }
 
   // ================================================================ forward
@@ -1743,13 +1662,12 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
   float *bn_scale = nullptr, *bn_bias = nullptr;
   const int v_off = c.modality_fuse == AVH_FUSE_CONCAT ? D : 0;
   const int Fa = c.audio_feat_dim, Fp = round_up(Fa > 0 ? Fa : 64, 64);
-  static const int HSd[5] = {22, 22, 11, 6, 3};
   if (full) {
-    fused = f32buf(N * E);
-    fln = new_act(N, E);
+    fused = b.f32buf(N * E);
+    fln = b.act(N, E);
     bn_sums = reinterpret_cast<double*>(b.alloc((size_t)BN_SLOTS * 3 * 512 * sizeof(double)));
-    bn_scale = f32buf(512); bn_bias = f32buf(512);
-    if (plan->has_video) {
+    bn_scale = b.f32buf(512); bn_bias = b.f32buf(512);
+    if (key.has_video) {
       colbuf = b.alloc((size_t)nfr * 484 * 576 * P * 2);
       stemcol = b.alloc((size_t)nfr * 1936 * 320 * P * 2);      // stem patches: kept for the weight gradient
       if (!f32) pool_arg = reinterpret_cast<unsigned char*>(b.alloc((size_t)nfr * 484 * 64));
@@ -1760,58 +1678,49 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
         const void* resp = res ? res->data : nullptr;
         const float *gm = cu->gamma, *bt = cu->beta;
         float *rm = cu->rmean, *rv = cu->rvar;
-        float* st = f32buf(2 * Cc);
+        float* st = b.f32buf(2 * Cc);
         cs.stat = st; cs.out = out; cs.slope = slope1 ? slope1 : slope2;
         if (res) cs.res = *res;
-        b.tag = "bn_train";
-        b.push([=](cudaStream_t s) { return launch_bn_stats(rawp, act_dt, rows, Cc, 0, 0, 0, 0, bn_sums, s); });
-        b.push([=](cudaStream_t s) {
+        b.push("bn_train", [=](cudaStream_t s) { return launch_bn_stats(rawp, act_dt, rows, Cc, 0, 0, 0, 0, bn_sums, s); });
+        b.push("bn_train", [=](cudaStream_t s) {
           return launch_bn_finalize(bn_sums, (double)rows, gm, bt, 1e-5f, pl->bn_momentum, rm, rv, bn_scale, bn_bias, Cc, s);
         });
-        b.push([=](cudaStream_t s) { return launch_bn_stat_from_affine(bn_scale, bn_bias, gm, bt, Cc, st, s); });
-        b.push([=](cudaStream_t s) {
+        b.push("bn_train", [=](cudaStream_t s) { return launch_bn_stat_from_affine(bn_scale, bn_bias, gm, bt, Cc, st, s); });
+        b.push("bn_train", [=](cudaStream_t s) {
           return launch_bn_apply(rawp, outp, act_dt, rows, Cc, bn_scale, bn_bias, slope1, resp, slope2, 0, 0, s);
         });
-        sync_op(out);
+        b.sync_op(out);
       };
       auto conv_fwd = [&](const ConvUnit& cu, const Act& in, int H, int pad, ConvSave* cs) -> bool {
         const int Ho = (H + 2 * pad - cu.ks) / cu.stride + 1;
         const int K = cu.ks * cu.ks * cu.cin;
         const long long rows = nfr * Ho * Ho;
         cs->cu = &cu; cs->in = in; cs->H = H; cs->Ho = Ho; cs->pad = pad;
-        cs->raw = new_act(rows, cu.cout);
+        cs->raw = b.act(rows, cu.cout);
         const void* xin = in.data;
         const int planes = P, ks = cu.ks, st = cu.stride, cin = cu.cin;
-        b.tag = "im2col";
-        b.push([=](cudaStream_t s) { return launch_im2col2d(xin, act_dt, nfr, H, cin, ks, st, pad, Ho, colbuf, planes, s); });
-        Epilogue ep;
-        ep.C = cs->raw.data; ep.ldc = cu.cout; ep.c_fp32 = f32 ? 1 : 0;
-        b.tag = "conv_gemm";
-        return b.gemm(colbuf, rows, P * K, cu.w, rows, {Tap{0, 0, 0}}, K / 64, K, ep);
+        b.push("im2col", [=](cudaStream_t s) { return launch_im2col2d(xin, act_dt, nfr, H, cin, ks, st, pad, Ho, colbuf, planes, s); });
+        return b.linear("conv_gemm", colbuf, rows, K, cu.w, epilogue(cs->raw.data, cu.cout, f32));
       };
       // stem: Conv3d as patches [frames * 1936, 5 * 64] x the packed stem weights
       {
         ConvSave cs;
         cs.cu = &h->stem; cs.H = 88; cs.Ho = 44;
         const long long rows = nfr * 1936;
-        cs.raw = new_act(rows, 64);
+        cs.raw = b.act(rows, 64);
         const int planes = P;
-        b.tag = "stem_patches";
-        b.cur_direct = true;
-        b.push([=](cudaStream_t s) { return launch_im2col_stem(pl->args.video, pl->args.video_dt, B, T, stemcol, planes, s); });
-        b.cur_direct = false;
-        Epilogue ep;
-        ep.C = cs.raw.data; ep.ldc = 64; ep.c_fp32 = f32 ? 1 : 0;
-        b.tag = "stem_gemm";
-        if (!b.gemm(stemcol, rows, P * 320, h->stem_wf, rows, {Tap{0, 0, 0}}, 5, 320, ep)) return false;      // K = dt*64 + kh*8 + kw
-        act0 = new_act(rows, 64);
+        b.push_direct("stem_patches", [=](cudaStream_t s) {
+          return launch_im2col_stem(pl->args.video, pl->args.video_dt, B, T, stemcol, planes, s);
+        });
+        // K = dt*64 + kh*8 + kw
+        if (!b.linear("stem_gemm", stemcol, rows, 320, h->stem_wf, epilogue(cs.raw.data, 64, f32))) return false;
+        act0 = b.act(rows, 64);
         bn_fwd(cs, rows, h->stem.slope, nullptr, nullptr, act0);
         convs.push_back(cs);
-        p0 = new_act(nfr * 484, 64);
+        p0 = b.act(nfr * 484, 64);
         const void* a0 = act0.data; void* pp = p0.data;
-        b.tag = "maxpool";
-        b.push([=](cudaStream_t s) { return launch_maxpool_dense(a0, pp, act_dt, nfr, 44, 64, 22, s, pool_arg); });
-        sync_op(p0);
+        b.push("maxpool", [=](cudaStream_t s) { return launch_maxpool_dense(a0, pp, act_dt, nfr, 44, 64, 22, s, pool_arg); });
+        b.sync_op(p0);
       }
       Act cur = p0;
       int H = 22;
@@ -1822,90 +1731,75 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
           if (!conv_fwd(bw.c1, cur, H, 1, &c1)) return false;
           const int Ho = c1.Ho, Cc = bw.c1.cout;
           const long long rows = nfr * Ho * Ho;
-          Act a1 = new_act(rows, Cc);
+          Act a1 = b.act(rows, Cc);
           bn_fwd(c1, rows, bw.c1.slope, nullptr, nullptr, a1);
           convs.push_back(c1);
           Act resid = cur;
           if (bw.has_ds) {
             if (!conv_fwd(bw.ds, cur, H, 0, &cd)) return false;
-            Act dso = new_act(rows, Cc);
+            Act dso = b.act(rows, Cc);
             bn_fwd(cd, rows, nullptr, nullptr, nullptr, dso);
             convs.push_back(cd);
             resid = dso;
           }
           if (!conv_fwd(bw.c2, a1, Ho, 1, &c2)) return false;
-          Act outb = new_act(rows, Cc);
+          Act outb = b.act(rows, Cc);
           bn_fwd(c2, rows, nullptr, &resid, bw.slope2, outb);
           convs.push_back(c2);
           cur = outb;
           H = Ho;
-          (void)HSd;
         }
-      feat = new_act(N, 512);
-      if (!sizing) plan->stages["resnet"] = {feat.data, {act_dt, N * 512}};
+      feat = b.act(N, 512);
+      b.stage("resnet", feat.data, act_dt, N * 512);
       {
         const void* src = cur.data; void* dst = feat.data;
-        b.tag = "avgpool";
-        b.push([=](cudaStream_t s) { return launch_avgpool_dense(src, dst, act_dt, nfr, 9, 512, s); });
-        sync_op(feat);
+        b.push("avgpool", [=](cudaStream_t s) { return launch_avgpool_dense(src, dst, act_dt, nfr, 9, 512, s); });
+        b.sync_op(feat);
       }
-      Epilogue ep;
-      ep.C = fused + v_off; ep.ldc = E; ep.c_fp32 = 1; ep.col_bias = h->proj_v.bias;
-      b.tag = "proj_video";
-      if (!b.gemm(feat.op, N, P * 512, h->proj_v.w, N, {Tap{0, 0, 0}}, 512 / 64, 512, ep)) return false;
+      Epilogue ep = epilogue(fused + v_off, E, true);
+      ep.col_bias = h->proj_v.bias;
+      if (!b.linear("proj_video", feat.op, N, 512, h->proj_v.w, ep)) return false;
     }
-    if (plan->has_audio) {
-      arows = new_act(N, Fp);
+    if (key.has_audio) {
+      arows = b.act(N, Fp);
       void* dst = arows.data;
-      b.tag = "audio_rows";
-      b.cur_direct = true;
-      b.push([=](cudaStream_t s) {
+      b.push_direct("audio_rows", [=](cudaStream_t s) {
         return launch_bct_to_rows(pl->args.audio, pl->args.audio_dt, pl->args.as[0], pl->args.as[1], pl->args.as[2], B, Fa, T, dst,
                                   act_dt, Fp, s);
       });
-      b.cur_direct = false;
-      sync_op(arows);
-      Epilogue ep;
-      ep.C = fused; ep.ldc = E; ep.c_fp32 = 1; ep.col_bias = h->proj_a.bias;
-      if (c.modality_fuse == AVH_FUSE_ADD && plan->has_video) { ep.R = ep.C; ep.ldr = E; ep.r_fp32 = 1; }
-      b.tag = "proj_audio";
-      if (!b.gemm(arows.op, N, P * Fp, h->proj_a.w, N, {Tap{0, 0, 0}}, Fp / 64, Fp, ep)) return false;
+      b.sync_op(arows);
+      Epilogue ep = epilogue(fused, E, true);
+      ep.col_bias = h->proj_a.bias;
+      if (c.modality_fuse == AVH_FUSE_ADD && key.has_video) { ep.R = ep.C; ep.ldr = E; ep.r_fp32 = 1; }
+      if (!b.linear("proj_audio", arows.op, N, Fp, h->proj_a.w, ep)) return false;
     }
   }
   if (tail) {
     // AVHubertModel.extract_finetune after the feature extractors: features = layer_norm(fused);
     // features = post_extract_proj(features) (concat fusion); index_put(padded frames, 0)   (hubert.py:719-727, wav2vec2.py:869)
     if (!full) {
-      fused = f32buf(N * E);
-      fln = new_act(N, E);
-      b.tag = "load_features";
-      b.cur_direct = true;
-      b.push([=](cudaStream_t s) { return launch_load_rows(pl->args.xin, pl->args.xin_dt, fused, nullptr, N, E, s); });
-      b.cur_direct = false;
+      fused = b.f32buf(N * E);
+      fln = b.act(N, E);
+      b.push_direct("load_features", [=](cudaStream_t s) {
+        return launch_load_rows(pl->args.xin, pl->args.xin_dt, fused, nullptr, N, E, s);
+      });
     }
-    float* of = f32 ? reinterpret_cast<float*>(fln.data) : nullptr;
-    void* ol = f32 ? nullptr : fln.data;
-    float* gm = h->fuse_ln_g; float* be = h->fuse_ln_b;
-    b.tag = "fuse_ln";
     if (h->has_post_proj) {
-      b.push([=](cudaStream_t s) { return launch_layernorm(fused, DT_F32, E, gm, be, 1e-5f, of, ol, DT_BF16, nullptr, N, E, s); });
-      sync_op(fln);
-      Epilogue ep;
-      ep.C = x0; ep.ldc = D; ep.c_fp32 = 1;
+      b.layernorm("fuse_ln", fused, DT_F32, h->fuse_ln_g, h->fuse_ln_b, 1e-5f, fln);
+      Epilogue ep = epilogue(x0, D, true);
       ep.col_bias = h->post_proj.bias;
-      if (hm) ep.row_zero = MASK_SENTINEL;
-      b.tag = "post_extract_proj";
-      if (!b.gemm(fln.op, N, P * E, h->post_proj.w, N, {Tap{0, 0, 0}}, E / 64, E, ep)) return false;
+      ep.row_zero = hm ? plan->mask_dev : nullptr;
+      if (!b.linear("post_extract_proj", fln.op, N, E, h->post_proj.w, ep)) return false;
     } else {
-      b.push([=](cudaStream_t s) {
+      float* gm = h->fuse_ln_g; float* be = h->fuse_ln_b;
+      b.push("fuse_ln", [=](cudaStream_t s) {
         return launch_layernorm(fused, DT_F32, E, gm, be, 1e-5f, x0, nullptr, DT_BF16, hm ? pl->mask_dev : nullptr, N, E, s);
       });
     }
   } else {
-    b.tag = "load_features";
-    b.cur_direct = true;
-    b.push([=](cudaStream_t s) { return launch_load_rows(pl->args.xin, pl->args.xin_dt, x0, hm ? pl->mask_dev : nullptr, N, D, s); });
-    b.cur_direct = false;
+    b.push_direct("load_features", [=](cudaStream_t s) {
+      return launch_load_rows(pl->args.xin, pl->args.xin_dt, x0, hm ? pl->mask_dev : nullptr, N, D, s);
+    });
   }
   const int G = 64, Tp = T + G;
   const long long pad_rows = (long long)B * Tp;
@@ -1913,146 +1807,106 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
   void* xpad = b.alloc((size_t)pad_rows * P * D * 2);         // zero-gapped operand layout of the positional conv
   {
     const int planes = P;
-    b.tag = "pos_pad";
-    b.push([=](cudaStream_t s) { return launch_split_rows(x0, D, xpad, planes, N, D, T, Tp, s); });
+    b.push("pos_pad", [=](cudaStream_t s) { return launch_split_rows(x0, D, xpad, planes, N, D, T, Tp, s); });
     std::vector<Tap> taps;
     for (int k = 0; k < KT; ++k) taps.push_back(Tap{k - KT / 2, 0, k * win});
-    Epilogue ep;
-    ep.C = cpre; ep.ldc = D; ep.c_fp32 = 1;
+    Epilogue ep = epilogue(cpre, D, true);
     ep.col_bias = h->pos_bias;
     ep.map_mode = MAP_2LEVEL; ep.S2 = Tp; ep.S1 = Tp; ep.H = 1; ep.W = T; ep.O2 = T; ep.O1 = 0; ep.O0 = 0;
-    b.tag = "pos_conv";
-    if (!b.gemm(xpad, pad_rows, P * D, h->pos_w, pad_rows, taps, win / 64, D, ep, 64, h->pos_acol)) return false;
+    if (!b.gemm("pos_conv", xpad, pad_rows, P * D, h->pos_w, pad_rows, taps, win / 64, D, ep, 64, h->pos_acol)) return false;
     float* x1 = xin[0];
-    b.tag = "gelu";
-    b.push([=](cudaStream_t s) { return launch_gelu_fwd(cpre, DT_F32, x0, x1, DT_F32, N * D, s); });
+    b.push("gelu", [=](cudaStream_t s) { return launch_gelu_fwd(cpre, DT_F32, x0, x1, DT_F32, N * D, s); });
   }
-  auto ln_fwd = [&](const float* src, const float* gm, const float* be, const Act& dst) {
-    float* of = f32 ? reinterpret_cast<float*>(dst.data) : nullptr;
-    void* ol = f32 ? nullptr : dst.data;
-    b.tag = "layer_ln";
-    b.push([=](cudaStream_t s) { return launch_layernorm(src, DT_F32, D, gm, be, 1e-5f, of, ol, DT_BF16, nullptr, N, D, s); });
-    sync_op(dst);
-  };
   for (int l = 0; l < L; ++l) {
     const LayerW& lw = h->layers[l];
     b.cur_layer = l;
     float* x = xin[l];
-    ln_fwd(x, lw.ln1_g, lw.ln1_b, h1[l]);
+    b.layernorm("layer_ln", x, DT_F32, lw.ln1_g, lw.ln1_b, 1e-5f, h1[l]);
     {
-      Epilogue ep;
-      ep.C = qkv[l].data; ep.ldc = 3 * D; ep.c_fp32 = f32 ? 1 : 0; ep.col_bias = lw.qkv.bias;
-      b.tag = "qkv_proj";
-      if (!b.gemm(h1[l].op, N, P * D, lw.qkv.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      Epilogue ep = epilogue(qkv[l].data, 3 * D, f32);
+      ep.col_bias = lw.qkv.bias;
+      if (!b.linear("qkv_proj", h1[l].op, N, D, lw.qkv.w, ep)) return false;
       const char* q = reinterpret_cast<const char*>(qkv[l].data);
       void* o = ctx[l].data;
       float* ls = lse[l];
-      b.tag = "attention";
-      b.push([=](cudaStream_t s) {
+      b.push("attention", [=](cudaStream_t s) {
         if (!f32)      // bf16 mode: the mma.sync forward kernel, also writing the log-sum-exp of every query row
           return launch_attention(q, hm ? pl->mask_dev : nullptr, o, B, T, D, Hh, 0, s, ls);
         return launch_attention_x(q, 3 * D, q + (size_t)D * es, 3 * D, q + (size_t)2 * D * es, 3 * D, act_dt,
                                   hm ? pl->mask_dev : nullptr, o, D, act_dt, B, Hh, T, T, 1.0f, s, ls);
       });
-      sync_op(ctx[l]);
+      b.sync_op(ctx[l]);
     }
     {
-      Epilogue ep;
-      ep.C = xmid[l]; ep.ldc = D; ep.c_fp32 = 1; ep.col_bias = lw.out.bias; ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
-      b.tag = "out_proj";
-      if (!b.gemm(ctx[l].op, N, P * D, lw.out.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      Epilogue ep = epilogue(xmid[l], D, true);
+      ep.col_bias = lw.out.bias; ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
+      if (!b.linear("out_proj", ctx[l].op, N, D, lw.out.w, ep)) return false;
     }
-    ln_fwd(xmid[l], lw.ln2_g, lw.ln2_b, h2[l]);
+    b.layernorm("layer_ln", xmid[l], DT_F32, lw.ln2_g, lw.ln2_b, 1e-5f, h2[l]);
     {
-      Epilogue ep;
-      ep.C = u[l].data; ep.ldc = F; ep.c_fp32 = f32 ? 1 : 0; ep.col_bias = lw.fc1.bias;
-      b.tag = "fc1";
-      if (!b.gemm(h2[l].op, N, P * D, lw.fc1.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      Epilogue ep = epilogue(u[l].data, F, f32);
+      ep.col_bias = lw.fc1.bias;
+      if (!b.linear("fc1", h2[l].op, N, D, lw.fc1.w, ep)) return false;
       const void* uu = u[l].data; void* gg = g[l].data;
-      b.tag = "gelu";
-      b.push([=](cudaStream_t s) { return launch_gelu_fwd(uu, act_dt, nullptr, gg, act_dt, N * F, s); });
-      sync_op(g[l]);
+      b.push("gelu", [=](cudaStream_t s) { return launch_gelu_fwd(uu, act_dt, nullptr, gg, act_dt, N * F, s); });
+      b.sync_op(g[l]);
     }
     {
-      Epilogue ep;
-      ep.C = xin[l + 1]; ep.ldc = D; ep.c_fp32 = 1; ep.col_bias = lw.fc2.bias; ep.R = xmid[l]; ep.ldr = D; ep.r_fp32 = 1;
-      b.tag = "fc2";
-      if (!b.gemm(g[l].op, N, P * F, lw.fc2.w, N, {Tap{0, 0, 0}}, F / 64, F, ep)) return false;
+      Epilogue ep = epilogue(xin[l + 1], D, true);
+      ep.col_bias = lw.fc2.bias; ep.R = xmid[l]; ep.ldr = D; ep.r_fp32 = 1;
+      if (!b.linear("fc2", g[l].op, N, F, lw.fc2.w, ep)) return false;
     }
   }
   b.cur_layer = -1;
   {
     float* xl = xin[L];
     float* gm = h->enc_ln_g; float* be = h->enc_ln_b;
-    b.tag = "final_ln";
-    b.cur_direct = true;
-    b.push([=](cudaStream_t s) {
+    b.push_direct("final_ln", [=](cudaStream_t s) {
       return launch_layernorm(xl, DT_F32, D, gm, be, 1e-5f, nullptr, pl->args.out, pl->args.out_dt, nullptr, N, D, s);
     });
-    b.cur_direct = false;
   }
   if (!sizing) plan->fwd_steps = plan->steps.size();
 
   // ================================================================ backward
   float2* stats = reinterpret_cast<float2*>(b.alloc((size_t)N * 8));
-  float* Dbuf = f32buf((long long)B * Hh * T);
-  float* dx = f32buf(N * D);             // gradient of the residual stream (ping)
-  float* dxm = f32buf(N * D);            // ... at the middle of a layer (pong)
-  float* dh = f32buf(N * D);             // gradient of a LayerNorm output
-  Act dxa = new_act(N, D);               // operand form of dx / dxm
-  Act dga = new_act(N, F);               // dL/dg
-  Act dua = new_act(N, F);               // dL/du
-  Act dctx = new_act(N, D);
-  Act dqkv = new_act(N, 3 * D);
+  float* Dbuf = b.f32buf((long long)B * Hh * T);
+  float* dx = b.f32buf(N * D);             // gradient of the residual stream (ping)
+  float* dxm = b.f32buf(N * D);            // ... at the middle of a layer (pong)
+  float* dh = b.f32buf(N * D);             // gradient of a LayerNorm output
+  Act dxa = b.act(N, D);                   // operand form of dx / dxm
+  Act dga = b.act(N, F);                   // dL/dg
+  Act dua = b.act(N, F);                   // dL/du
+  Act dctx = b.act(N, D);
+  Act dqkv = b.act(N, 3 * D);
   void* tA = b.alloc((size_t)std::max(3 * D, F) * P * Kp * 2);      // transposed dY operand
   void* tB = b.alloc((size_t)std::max(std::max(D, F), E) * P * Kp * 2);      // transposed X operand
-  // fp32 [N, C] -> operand form (bf16 or split planes)
-  auto to_op = [&](const float* src, const Act& dst, int C) {
-    void* d = dst.op;
-    const int planes = P;
-    b.tag = "split";
-    b.push([=](cudaStream_t s) { return launch_split_rows(src, C, d, planes, N, C, 0, 0, s); });
-  };
   // dX [N, n_in] = dY [N, n_out] W: A = dY operand, B = W^T (packed [n_in, n_out])
   auto dgrad = [&](const void* dy_op, int n_out, const LinearW& wT, void* out, bool out_f32, const char* tag) {
-    Epilogue ep;
-    ep.C = out; ep.ldc = wT.w.n; ep.c_fp32 = out_f32 ? 1 : 0;
-    b.tag = tag;
-    return b.gemm(dy_op, N, P * n_out, wT.w, N, {Tap{0, 0, 0}}, wT.w.kpad / 64, n_out, ep);
+    return b.linear(tag, dy_op, N, n_out, wT.w, epilogue(out, wT.w.n, out_f32));
   };
   // dW [n_out, n_in] = dY^T X (+ bias gradient = column sums of dY)
   auto wgrad = [&](const void* dyv, int dy_dt, int n_out, const void* xv, int x_dt, int n_in, float* dW, float* db, const char* tag) {
     const int planes = P;
-    b.tag = "transpose";
-    b.push([=](cudaStream_t s) { return launch_transpose_split(dyv, dy_dt, n_out, N, n_out, tA, planes, Kp, 1.0f, s); });
-    b.push([=](cudaStream_t s) { return launch_transpose_split(xv, x_dt, n_in, N, n_in, tB, planes, Kp, 1.0f, s); });
+    b.push("transpose", [=](cudaStream_t s) { return launch_transpose_split(dyv, dy_dt, n_out, N, n_out, tA, planes, Kp, 1.0f, s); });
+    b.push("transpose", [=](cudaStream_t s) { return launch_transpose_split(xv, x_dt, n_in, N, n_in, tB, planes, Kp, 1.0f, s); });
     PackedW xw;
     xw.w = reinterpret_cast<bf16*>(tB); xw.n = n_in; xw.k = (int)Kp; xw.kpad = (int)Kp;
-    Epilogue ep;
-    ep.C = dW; ep.ldc = n_in; ep.c_fp32 = 1;
-    b.tag = tag;
     // whole tiles, no stream-K: measured faster for the encoder's weight gradients (64-256 tiles of 19 K blocks at
     // 8 x 150 tokens), 15.96 vs 16.96 ms per frozen-extractor step (73 launches at ~13 us against 24.5 us with
     // stream-K: the partial-tile round trip through the workspace costs more than the idle SMs)
-    if (!b.gemm(tA, n_out, P * (int)Kp, xw, n_out, {Tap{0, 0, 0}}, (int)(Kp / 64), (int)Kp, ep)) return false;
-    if (db != nullptr) {
-      b.tag = "bias_grad";
-      b.push([=](cudaStream_t s) { return launch_colsum(dyv, dy_dt, n_out, N, n_out, db, 1.0f, s); });
-    }
+    if (!b.linear(tag, tA, n_out, (int)Kp, xw, epilogue(dW, n_in, true))) return false;
+    if (db != nullptr)
+      b.push("bias_grad", [=](cudaStream_t s) { return launch_colsum(dyv, dy_dt, n_out, N, n_out, db, 1.0f, s); });
     return true;
   };
   const float qscale = 1.0f / std::sqrt(64.0f);
   const long long LG = enc_layer_grad_floats(D, F);
-  b.tag = "load_grad";
-  b.cur_direct = true;
   // (the caller's dL/dy is staged into `dy` by avh_encoder_backward before the steps run)
-  b.cur_direct = false;
   {   // final LayerNorm
     float* gfin = grads + (long long)L * LG;
     float* xl = xin[L];
     float* gm = h->enc_ln_g;
-    b.tag = "ln_bwd";
-    b.push([=](cudaStream_t s) { return launch_ln_bwd(xl, gm, dy, nullptr, dx, stats, gfin, gfin + D, N, D, 1e-5f, s); });
+    b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(xl, gm, dy, nullptr, dx, stats, gfin, gfin + D, N, D, 1e-5f, s); });
   }
   for (int l = L - 1; l >= 0; --l) {
     const LayerW& lw = h->layers[l];
@@ -2070,53 +1924,48 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     float* g_ln2 = g_fc2_b + D;
     // ---- fc2: x' = xm + g W2^T + b2
     if (!wgrad(dx, DT_F32, D, g[l].data, act_dt, F, g_fc2_w, g_fc2_b, "fc2_wgrad")) return false;
-    to_op(dx, dxa, D);
+    b.split(dx, D, dxa.op, N, D);
     if (!dgrad(dxa.op, D, lw.fc2T, dga.data, f32, "fc2_dgrad")) return false;
     {
       const void* uu = u[l].data; const void* dgv = dga.data; void* duv = dua.data;
-      b.tag = "gelu_bwd";
-      b.push([=](cudaStream_t s) { return launch_gelu_bwd(uu, act_dt, dgv, act_dt, duv, act_dt, N * F, s); });
-      sync_op(dua);
+      b.push("gelu_bwd", [=](cudaStream_t s) { return launch_gelu_bwd(uu, act_dt, dgv, act_dt, duv, act_dt, N * F, s); });
+      b.sync_op(dua);
     }
     // ---- fc1: u = h2 W1^T + b1
     if (!wgrad(dua.data, act_dt, F, h2[l].data, act_dt, D, g_fc1_w, g_fc1_b, "fc1_wgrad")) return false;
     if (!dgrad(dua.op, F, lw.fc1T, dh, true, "fc1_dgrad")) return false;
     {   // LN2: dxm = dx + dLN(dh; xm)
       float* xm = xmid[l]; float* gm = lw.ln2_g;
-      b.tag = "ln_bwd";
-      b.push([=](cudaStream_t s) { return launch_ln_bwd(xm, gm, dh, dx, dxm, stats, g_ln2, g_ln2 + D, N, D, 1e-5f, s); });
+      b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(xm, gm, dh, dx, dxm, stats, g_ln2, g_ln2 + D, N, D, 1e-5f, s); });
     }
     // ---- out_proj: xm = x + ctx Wo^T + bo
     if (!wgrad(dxm, DT_F32, D, ctx[l].data, act_dt, D, g_out_w, g_out_b, "out_wgrad")) return false;
-    to_op(dxm, dxa, D);
+    b.split(dxm, D, dxa.op, N, D);
     if (!dgrad(dxa.op, D, lw.outT, dctx.data, f32, "out_dgrad")) return false;
     {   // attention
       const char* q = reinterpret_cast<const char*>(qkv[l].data);
       char* dq = reinterpret_cast<char*>(dqkv.data);
       const void* dO = dctx.data; const void* O = ctx[l].data;
       float* ls = lse[l];
-      b.tag = "attention_bwd";
-      b.push([=](cudaStream_t s) {
+      b.push("attention_bwd", [=](cudaStream_t s) {
         if (!f32)      // bf16 mode: tensor-core backward (attention.cu); fp32 mode: the fp32 CUDA-core kernels
           return launch_attention_bwd_tc(q, dO, O, ls, hm ? pl->mask_dev : nullptr, dq, Dbuf, B, T, D, Hh, s);
         return launch_attention_bwd(q, 3 * D, q + (size_t)D * es, 3 * D, q + (size_t)2 * D * es, 3 * D, act_dt, dO, O, D, act_dt, ls,
                                     hm ? pl->mask_dev : nullptr, dq, dq + (size_t)D * es, dq + (size_t)2 * D * es, 3 * D, act_dt,
                                     Dbuf, B, Hh, T, s);
       });
-      sync_op(dqkv);
+      b.sync_op(dqkv);
     }
     // ---- qkv: [q', k, v] = h1 Wqkv'^T + b' with q' = s q (the scaling is folded into Wq', bq')
     if (!wgrad(dqkv.data, act_dt, 3 * D, h1[l].data, act_dt, D, g_qkv_w, g_qkv_b, "qkv_wgrad")) return false;
-    b.tag = "scale";
-    b.push([=](cudaStream_t s) {     // d/dWq = s d/dWq', d/dbq = s d/dbq'
+    b.push("scale", [=](cudaStream_t s) {     // d/dWq = s d/dWq', d/dbq = s d/dbq'
       if (launch_scale(g_qkv_w, (long long)D * D, qscale, s)) return 1;
       return launch_scale(g_qkv_b, D, qscale, s);
     });
     if (!dgrad(dqkv.op, 3 * D, lw.qkvT, dh, true, "qkv_dgrad")) return false;
     {   // LN1: dx = dxm + dLN(dh; x)
       float* xl = xin[l]; float* gm = lw.ln1_g;
-      b.tag = "ln_bwd";
-      b.push([=](cudaStream_t s) { return launch_ln_bwd(xl, gm, dh, dxm, dx, stats, g_ln1, g_ln1 + D, N, D, 1e-5f, s); });
+      b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(xl, gm, dh, dxm, dx, stats, g_ln1, g_ln1 + D, N, D, 1e-5f, s); });
     }
     if (l % 4 == 0) {      // layers l .. l+3 are final: one gradient bucket (Large: 4 x 12.6 M floats)
       b.cur_layer = -1;
@@ -2128,27 +1977,22 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
   {
     float* gpos = grads + (long long)L * LG + 2ll * D;       // bias [D], weight_g [KT], weight_v [D, D/G, KT]
     float* dc = dh;                                          // dL/dc = dx * GELU'(c)
-    b.tag = "gelu_bwd";
-    b.push([=](cudaStream_t s) { return launch_gelu_bwd(cpre, DT_F32, dx, DT_F32, dc, DT_F32, N * D, s); });
-    b.tag = "bias_grad";
-    b.push([=](cudaStream_t s) { return launch_colsum(dc, DT_F32, D, N, D, gpos, 1.0f, s); });
+    b.push("gelu_bwd", [=](cudaStream_t s) { return launch_gelu_bwd(cpre, DT_F32, dx, DT_F32, dc, DT_F32, N * D, s); });
+    b.push("bias_grad", [=](cudaStream_t s) { return launch_colsum(dc, DT_F32, D, N, D, gpos, 1.0f, s); });
     // dgrad: dx0[t, i] = dx[t, i] + sum_k sum_o dc[t + 64 - k, o] w[o, i, k]: the same shifted-row GEMM over the
     // zero-gapped layout with the taps mirrored and the weights transposed inside every group (pos_wT)
     void* dcpad = b.alloc((size_t)pad_rows * P * D * 2);     // zero-gapped operand layout of dL/dc (gap rows stay zero)
     const int planes = P;
-    b.tag = "pos_pad";
-    b.push([=](cudaStream_t s) { return launch_split_rows(dc, D, dcpad, planes, N, D, T, Tp, s); });
+    b.push("pos_pad", [=](cudaStream_t s) { return launch_split_rows(dc, D, dcpad, planes, N, D, T, Tp, s); });
     std::vector<Tap> taps;
     for (int k = 0; k < KT; ++k) taps.push_back(Tap{KT / 2 - k, 0, k * win});
-    Epilogue ep;
-    ep.C = dxo; ep.ldc = D; ep.c_fp32 = 1;
+    Epilogue ep = epilogue(dxo, D, true);
     ep.R = dx; ep.ldr = D; ep.r_fp32 = 1;
-    if (hm) ep.row_zero = MASK_SENTINEL;                     // x0 = index_put(features, mask, 0): no gradient into pad rows
+    ep.row_zero = hm ? plan->mask_dev : nullptr;             // x0 = index_put(features, mask, 0): no gradient into pad rows
     ep.map_mode = MAP_2LEVEL; ep.S2 = Tp; ep.S1 = Tp; ep.H = 1; ep.W = T; ep.O2 = T; ep.O1 = 0; ep.O0 = 0;
-    b.tag = "pos_conv_dgrad";
-    if (!b.gemm(dcpad, pad_rows, P * D, h->pos_wT, pad_rows, taps, win / 64, D, ep, 64, h->pos_acol)) return false;
+    if (!b.gemm("pos_conv_dgrad", dcpad, pad_rows, P * D, h->pos_wT, pad_rows, taps, win / 64, D, ep, 64, h->pos_acol)) return false;
     // weight gradients of the grouped convolution + weight-norm backward
-    if (!posconv_wgrad(b, h, plan, dc, x0, N, B, T, gpos + D, gpos + D + KT)) return false;
+    if (!posconv_wgrad(b, h, dc, x0, N, B, T, gpos + D, gpos + D + KT)) return false;
     if (tail) {
       // dxo = dL/dx0 (rows of padded frames already zero).  post_extract_proj: x0 = fln Wp^T + bp; then the fusion LayerNorm
       // (its input comes from the frozen extractors: only dgamma / dbeta are needed)
@@ -2159,31 +2003,27 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
         float* g_pw = gt; float* g_pb = gt + (long long)D * E;
         g_ln = g_pb + D;
         if (!wgrad(dxo, DT_F32, D, fln.data, act_dt, E, g_pw, g_pb, "post_proj_wgrad")) return false;
-        to_op(dxo, dxa, D);
-        dfl = f32buf(N * E);
+        b.split(dxo, D, dxa.op, N, D);
+        dfl = b.f32buf(N * E);
         if (!dgrad(dxa.op, D, h->post_projT, dfl, true, "post_proj_dgrad")) return false;
       } else {
         dfl = dxo;
       }
-      float* dfused = f32buf(N * E);       // dL/d(fused): used by mode 2, a by-product otherwise
+      float* dfused = b.f32buf(N * E);       // dL/d(fused): used by mode 2, a by-product otherwise
       float* gm = h->fuse_ln_g;
-      b.tag = "ln_bwd";
-      b.push([=](cudaStream_t s) { return launch_ln_bwd(fused, gm, dfl, nullptr, dfused, stats, g_ln, g_ln + E, N, E, 1e-5f, s); });
+      b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(fused, gm, dfl, nullptr, dfused, stats, g_ln, g_ln + E, N, E, 1e-5f, s); });
       // final LayerNorm, positional conv, post_extract_proj, fusion LayerNorm: one bucket; the feature extractors' another
       grad_mark((long long)L * LG, full ? (g_ln + 2ll * E) - grads : GF);
       if (full) {
         // ============================================================ backward of the feature extractors (mode 2)
         float* gf = g_ln + 2ll * E;                         // frontend gradients follow layer_norm.{weight,bias}
-        b.tag = "scale";
-        b.push([=](cudaStream_t s) {                        // GradMultiply on the extractor outputs (grad_multiply.py:105-114)
+        b.push("scale", [=](cudaStream_t s) {               // GradMultiply on the extractor outputs (grad_multiply.py:105-114)
           return pl->fgm != 1.f ? launch_scale(dfused, N * E, pl->fgm, s) : 0;
         });
         // generic dW [n_out, n_in] (+)= dY^T X over `rows` rows; X either a plain matrix (x_op = false) or an operand-form
         // matrix [rows, P * n_in] (planes side by side); K = rows is cut into segments the GEMM's K-step table holds
-        long long max_rows = N;
         long long max_a = (long long)D * ((N + 63) / 64 * 64), max_b = (long long)std::max(Fp, 512) * ((N + 63) / 64 * 64);
-        if (plan->has_video) {
-          max_rows = nfr * 1936;
+        if (key.has_video) {
           max_a = std::max(max_a, 64ll * ((nfr * 1936 + 63) / 64 * 64));
           max_b = std::max(max_b, 320ll * ((nfr * 1936 + 63) / 64 * 64));
           int cin = 64, Hh2 = 22;
@@ -2204,39 +2044,40 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
                               int n_in, long long rows, float* dW, float* db, const char* tag, int dy_dt = DT_F32) -> bool {
           const long long kp = (rows + 63) / 64 * 64;
           const int planes = P;
-          b.tag = "transpose";
           if (!f32 && n_out % 8 == 0 && ld_dy % 8 == 0) {
-            b.push([=](cudaStream_t s) { return launch_transposeT(dyv, dy_dt, ld_dy, rows, n_out, ftA, kp, kp, s); });
+            b.push("transpose", [=](cudaStream_t s) { return launch_transposeT(dyv, dy_dt, ld_dy, rows, n_out, ftA, kp, kp, s); });
           } else {
-            b.push([=](cudaStream_t s) { return launch_transpose_split(dyv, dy_dt, ld_dy, rows, n_out, ftA, planes, kp, 1.0f, s); });
+            b.push("transpose", [=](cudaStream_t s) {
+              return launch_transpose_split(dyv, dy_dt, ld_dy, rows, n_out, ftA, planes, kp, 1.0f, s);
+            });
           }
           if (x_mode == 1) {
             for (int pp = 0; pp < P; ++pp) {
               const __nv_bfloat16* src = reinterpret_cast<const __nv_bfloat16*>(xv) + (long long)pp * n_in;
               __nv_bfloat16* dst = reinterpret_cast<__nv_bfloat16*>(ftB) + (long long)pp * kp;
               if (!f32 && n_in % 8 == 0 && ld_x % 8 == 0)
-                b.push([=](cudaStream_t s) { return launch_transposeT(src, DT_BF16, ld_x, rows, n_in, dst, kp, kp, s); });
+                b.push("transpose", [=](cudaStream_t s) { return launch_transposeT(src, DT_BF16, ld_x, rows, n_in, dst, kp, kp, s); });
               else
-                b.push([=](cudaStream_t s) {
+                b.push("transpose", [=](cudaStream_t s) {
                   return launch_transpose_split(src, DT_BF16, ld_x, rows, n_in, dst, 1, kp, 1.0f, s, 0, 0, (long long)planes * kp);
                 });
             }
           } else if (x_mode == 0) {
             if (!f32 && x_dt == DT_BF16 && n_in % 8 == 0 && ld_x % 8 == 0)
-              b.push([=](cudaStream_t s) { return launch_transposeT(xv, DT_BF16, ld_x, rows, n_in, ftB, kp, kp, s); });
+              b.push("transpose", [=](cudaStream_t s) { return launch_transposeT(xv, DT_BF16, ld_x, rows, n_in, ftB, kp, kp, s); });
             else
-              b.push([=](cudaStream_t s) { return launch_transpose_split(xv, x_dt, ld_x, rows, n_in, ftB, planes, kp, 1.0f, s); });
+              b.push("transpose", [=](cudaStream_t s) {
+                return launch_transpose_split(xv, x_dt, ld_x, rows, n_in, ftB, planes, kp, 1.0f, s);
+              });
           }
           if (!f32) {
             // bf16 mode: ONE launch over the whole K extent (no step table), stream-K over the SMs: the output is a handful
             // of tiles (dW of a 64-channel conv: 1 x 5) while K is the pixel count (580 800 in layer1 at 8 x 150 frames)
             PackedW xw;
             xw.w = reinterpret_cast<bf16*>(ftB); xw.n = n_in; xw.k = (int)kp; xw.kpad = (int)kp;
-            Epilogue ep;
-            ep.C = dW; ep.ldc = n_in; ep.c_fp32 = 1;
-            b.tag = tag;
             b.linear_k = true; b.force_sk = 1;
-            const bool ok = b.gemm(ftA, n_out, (int)kp, xw, n_out, {Tap{0, 0, 0}}, (int)(kp / 64), (int)kp, ep, 0, nullptr, kp);
+            const bool ok = b.gemm(tag, ftA, n_out, (int)kp, xw, n_out, {Tap{0, 0, 0}}, (int)(kp / 64), (int)kp,
+                                   epilogue(dW, n_in, true), 0, nullptr, kp);
             b.linear_k = false; b.force_sk = 0;
             if (!ok) return false;
           } else {
@@ -2245,39 +2086,29 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
               const long long kl = std::min(seg, kp - k0);
               PackedW xw;
               xw.w = reinterpret_cast<bf16*>(ftB) + k0; xw.n = n_in; xw.k = (int)kp; xw.kpad = (int)kp;
-              Epilogue ep;
-              ep.C = dW; ep.ldc = n_in; ep.c_fp32 = 1;
+              Epilogue ep = epilogue(dW, n_in, true);
               if (k0 > 0) { ep.R = dW; ep.ldr = n_in; ep.r_fp32 = 1; }
-              b.tag = tag;
               const char* a = reinterpret_cast<const char*>(ftA) + (size_t)k0 * 2;
-              if (!b.gemm(a, n_out, (int)(P * kp - k0), xw, n_out, {Tap{0, 0, 0}}, (int)(kl / 64), (int)kp, ep, 0, nullptr, P * kp))
+              if (!b.gemm(tag, a, n_out, (int)(P * kp - k0), xw, n_out, {Tap{0, 0, 0}}, (int)(kl / 64), (int)kp, ep, 0, nullptr, P * kp))
                 return false;
             }
           }
-          if (db != nullptr) {
-            b.tag = "bias_grad";
-            b.push([=](cudaStream_t s) { return launch_colsum(dyv, dy_dt, ld_dy, rows, n_out, db, 1.0f, s); });
-          }
+          if (db != nullptr)
+            b.push("bias_grad", [=](cudaStream_t s) { return launch_colsum(dyv, dy_dt, ld_dy, rows, n_out, db, 1.0f, s); });
           return true;
         };
-        if (plan->has_audio) {
+        if (key.has_audio) {
           float* g_w = gf; float* g_b = g_w + (long long)D * Fp;
           gf = g_b + D;
           if (!wgrad_rows(dfused, E, D, arows.data, act_dt, Fp, 0, Fp, N, g_w, g_b, "proj_audio_wgrad")) return false;
         }
-        if (plan->has_video) {
+        if (key.has_video) {
           float* g_w = gf; float* g_b = g_w + (long long)D * 512;
           gf = g_b + D;
           if (!wgrad_rows(dfused + v_off, E, D, feat.data, act_dt, 512, 0, 512, N, g_w, g_b, "proj_video_wgrad")) return false;
           // d(feat) = d(fused_video) Wv
-          {
-            void* d = dxa.op;
-            const float* src = dfused + v_off;
-            const int planes = P;
-            b.tag = "split";
-            b.push([=](cudaStream_t s) { return launch_split_rows(src, E, d, planes, N, D, 0, 0, s); });
-          }
-          float* dfeat = f32buf(N * 512);
+          b.split(dfused + v_off, E, dxa.op, N, D);
+          float* dfeat = b.f32buf(N * 512);
           if (!dgrad(dxa.op, D, h->proj_vT, dfeat, true, "proj_video_dgrad")) return false;
           // gradient slots of the ResNet, in forward (state-dict) order
           float* g_stem_w = gf; float* g_stem_bn = g_stem_w + 64 * 320; float* g_stem_slope = g_stem_bn + 128;
@@ -2302,7 +2133,7 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
               }
             }
           }
-          float* tot = f32buf(3 * 512);
+          float* tot = b.f32buf(3 * 512);
           size_t dcol_elems = 0, dop_elems = 0;
           for (const ConvSave& cs : convs) {
             if (cs.cu == &h->stem) continue;
@@ -2310,19 +2141,18 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
             dcol_elems = std::max(dcol_elems, (size_t)rows * cs.cu->ks * cs.cu->ks * cs.cu->cin);
             dop_elems = std::max(dop_elems, (size_t)rows * cs.cu->cout);
           }
-          float* dcol = f32buf((long long)dcol_elems);
+          float* dcol = b.f32buf((long long)dcol_elems);
           void* dop = b.alloc(dop_elems * P * 2);
           // BatchNorm (+ residual) (+ PReLU) backward of one saved conv: dz -> d_raw (returned), d_res, parameter gradients
           const int graw_dt = f32 ? DT_F32 : DT_BF16;     // bf16 mode: d(raw conv output) is only ever a GEMM operand
           auto bn_bwd = [&](const ConvSave& cs, const float* dz, float* d_res, int res_acc, float* g_bn, float* g_slope) {
             const long long rows = nfr * cs.Ho * cs.Ho;
             const int Cc = cs.cu->cout;
-            float* d_raw = f32buf(f32 ? rows * Cc : (rows * Cc + 1) / 2);
+            float* d_raw = b.f32buf(f32 ? rows * Cc : (rows * Cc + 1) / 2);
             const void* rawp = cs.raw.data;
             const void* resp = cs.res.data;
             const float* st = cs.stat; const float* gm = cs.cu->gamma; const float* bt = cs.cu->beta; const float* sl = cs.slope;
-            b.tag = "bn_bwd";
-            b.push([=](cudaStream_t s) {
+            b.push("bn_bwd", [=](cudaStream_t s) {
               return launch_bn_act_bwd(rawp, act_dt, resp, dz, st, gm, bt, sl, rows, Cc, bn_sums, tot, d_raw, d_res, res_acc,
                                        g_bn, g_bn + Cc, g_slope, s, graw_dt);
             });
@@ -2336,38 +2166,31 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
             const long long rows = nfr * cs.Ho * cs.Ho;
             const void* xin = cs.in.data;
             const int planes = P, ks = cu.ks, st = cu.stride, cin = cu.cin, H = cs.H, Ho = cs.Ho, pad = cs.pad;
-            b.tag = "im2col";
             if (!f32) {
               // bf16 mode: the patches are written transposed straight from the map (no patch matrix, no transpose pass)
               const long long kp = (rows + 63) / 64 * 64;
-              b.push([=](cudaStream_t s) { return launch_im2colT(xin, nfr, H, cin, ks, st, pad, Ho, ftB, kp, s); });
+              b.push("im2col", [=](cudaStream_t s) { return launch_im2colT(xin, nfr, H, cin, ks, st, pad, Ho, ftB, kp, s); });
               if (!wgrad_rows(d_raw, Cc, Cc, nullptr, DT_BF16, 0, 2, K, rows, dW, nullptr, "conv_wgrad", graw_dt)) return false;
             } else {
-              b.push([=](cudaStream_t s) { return launch_im2col2d(xin, act_dt, nfr, H, cin, ks, st, pad, Ho, colbuf, planes, s); });
+              b.push("im2col", [=](cudaStream_t s) {
+                return launch_im2col2d(xin, act_dt, nfr, H, cin, ks, st, pad, Ho, colbuf, planes, s);
+              });
               if (!wgrad_rows(d_raw, Cc, Cc, colbuf, DT_BF16, (long long)P * K, 1, K, rows, dW, nullptr, "conv_wgrad")) return false;
             }
             if (dx == nullptr) return true;
             const void* dopv = dop;
-            if (f32) {
-              b.tag = "split";
-              b.push([=](cudaStream_t s) { return launch_split_rows(d_raw, Cc, dop, planes, rows, Cc, 0, 0, s); });
-            } else {
-              dopv = d_raw;                                          // already the bf16 operand
-            }
-            Epilogue ep;
-            ep.C = dcol; ep.ldc = K; ep.c_fp32 = f32 ? 1 : 0;        // bf16 mode: patch gradients in bf16 (half the traffic)
-            b.tag = "conv_dgrad";
-            if (!b.gemm(dopv, rows, P * Cc, cu.wT, rows, {Tap{0, 0, 0}}, cu.wT.kpad / 64, Cc, ep)) return false;
-            b.tag = "col2im";
-            b.push([=](cudaStream_t s) { return launch_col2im2d(dcol, act_dt, nfr, H, cin, ks, st, pad, Ho, dx, dx_acc, s); });
+            if (f32) b.split(d_raw, Cc, dop, rows, Cc);
+            else dopv = d_raw;                                     // already the bf16 operand
+            // bf16 mode: patch gradients in bf16 (half the traffic)
+            if (!b.linear("conv_dgrad", dopv, rows, Cc, cu.wT, epilogue(dcol, K, f32))) return false;
+            b.push("col2im", [=](cudaStream_t s) { return launch_col2im2d(dcol, act_dt, nfr, H, cin, ks, st, pad, Ho, dx, dx_acc, s); });
             return true;
           };
           // avgpool
-          float* dcur = f32buf(nfr * 9 * 512);
-          b.tag = "avgpool_bwd";
+          float* dcur = b.f32buf(nfr * 9 * 512);
           {
             float* dc4 = dcur;
-            b.push([=](cudaStream_t s) { return launch_avgpool_bwd(dfeat, dc4, nfr, 9, 512, s); });
+            b.push("avgpool_bwd", [=](cudaStream_t s) { return launch_avgpool_bwd(dfeat, dc4, nfr, 9, 512, s); });
           }
           // blocks in reverse; convs = [stem, (c1, [ds], c2) x 8]
           int ci = (int)convs.size() - 1;
@@ -2381,15 +2204,15 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
               ci -= bw.has_ds ? 3 : 2;
               const long long rows_out = nfr * c2.Ho * c2.Ho;
               const long long rows_in = nfr * c1.H * c1.H;
-              float* d_res = f32buf(rows_out * c2.cu->cout);
+              float* d_res = b.f32buf(rows_out * c2.cu->cout);
               float* d_raw2 = bn_bwd(c2, dcur, d_res, 0, g.bn2, g.s2);
-              float* d_a1 = f32buf(rows_out * c2.cu->cin);
+              float* d_a1 = b.f32buf(rows_out * c2.cu->cin);
               if (!conv_bwd(c2, d_raw2, g.c2w, d_a1, 0)) return false;
               float* d_raw1 = bn_bwd(c1, d_a1, nullptr, 0, g.bn1, g.s1);
-              float* d_in = f32buf(rows_in * c1.cu->cin);
-              if (!sizing && L == 3 && bi == 1) {      // gradient maps of the last block, for the kink-attribution test
-                plan->stages["grad_layer4_1_conv2_in"] = {d_a1, {DT_F32, rows_out * 512}};
-                plan->stages["grad_layer4_1_conv1_out"] = {d_raw1, {DT_F32, rows_out * 512}};
+              float* d_in = b.f32buf(rows_in * c1.cu->cin);
+              if (L == 3 && bi == 1) {      // gradient maps of the last block, for the kink-attribution test
+                b.stage("grad_layer4_1_conv2_in", d_a1, DT_F32, rows_out * 512);
+                b.stage("grad_layer4_1_conv1_out", d_raw1, DT_F32, rows_out * 512);
               }
               if (!conv_bwd(c1, d_raw1, g.c1w, d_in, 0)) return false;
               if (cd != nullptr) {
@@ -2397,19 +2220,17 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
                 if (!conv_bwd(*cd, d_rawd, g.dsw, d_in, 1)) return false;
               } else {
                 const long long n_el = rows_in * c1.cu->cin;
-                b.tag = "add";
-                b.push([=](cudaStream_t s) { return launch_add_f32(d_in, d_res, n_el, s); });
+                b.push("add", [=](cudaStream_t s) { return launch_add_f32(d_in, d_res, n_el, s); });
               }
               dcur = d_in;
             }
           // max-pool, stem BatchNorm + PReLU, stem weights
           {
             const ConvSave& cs = convs[0];
-            float* d_act0 = f32buf(nfr * 1936 * 64);
+            float* d_act0 = b.f32buf(nfr * 1936 * 64);
             const void* a0 = act0.data;
             float* dp0 = dcur;
-            b.tag = "maxpool_bwd";
-            b.push([=](cudaStream_t s) { return launch_maxpool_bwd(a0, act_dt, dp0, d_act0, nfr, 44, 64, 22, s, pool_arg); });
+            b.push("maxpool_bwd", [=](cudaStream_t s) { return launch_maxpool_bwd(a0, act_dt, dp0, d_act0, nfr, 44, 64, 22, s, pool_arg); });
             float* d_raw0 = bn_bwd(cs, d_act0, nullptr, 0, g_stem_bn, g_stem_slope);
             if (!wgrad_rows(d_raw0, 64, 64, stemcol, DT_BF16, (long long)P * 320, 1, 320, nfr * 1936, g_stem_w, nullptr, "stem_wgrad",
                             graw_dt))
@@ -2433,163 +2254,113 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
 // Every Linear is a tcgen05 GEMM (the K / V projections of the AV features for ALL layers are one GEMM: they are
 // ~80 % of the block's FLOPs); attention is launch_attention_x (qformer.cu).
 bool build_qformer_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
-  Builder b;
-  b.h = h; b.plan = plan; b.sizing = sizing; b.P = h->P; b.f32 = (h->cfg.compute_mode == AVH_COMPUTE_FP32);
+  Builder b(h, plan, sizing);
   const avh_config& c = h->cfg;
-  const int P = b.P;
+  const PlanKey& key = plan->key;
   const bool f32 = b.f32;
-  const int B = plan->B, T = plan->T, Lk = plan->Lk, D = c.encoder_embed_dim, F = c.encoder_ffn_embed_dim;
+  const int B = key.B, T = key.T, Lk = key.Lk, D = c.encoder_embed_dim, F = c.encoder_ffn_embed_dim;
   const int Hh = c.encoder_attention_heads, Ew = c.reserved[1], L = c.encoder_layers;
   const long long N = (long long)B * T, NK = (long long)B * Lk;
-  const size_t es = f32 ? 4 : 2;
-  const int act_dt = f32 ? DT_F32 : DT_BF16;
+  const size_t es = b.es;
+  const int act_dt = b.act_dt;
   const float eps = 1e-12f;                                   // BertConfig.layer_norm_eps
   Plan* pl = plan;
-  auto new_act = [&](long long rows, int C) {
-    Act a;
-    a.rows = rows; a.C = C;
-    a.data = b.alloc((size_t)rows * C * es);
-    a.op = f32 ? b.alloc((size_t)rows * C * 2 * P) : a.data;
-    return a;
-  };
-  auto sync_op = [&](const Act& a) {
-    if (!f32) return;
-    const float* src = reinterpret_cast<const float*>(a.data);
-    void* dst = a.op;
-    const long long rows = a.rows;
-    const int C = a.C, planes = P;
-    const std::string keep = b.tag;
-    b.tag = "split";
-    b.push([=](cudaStream_t s) { return launch_split_rows(src, C, dst, planes, rows, C, 0, 0, s); });
-    b.tag = keep;
-  };
-  b.sk_bytes = 0; b.sk_ws = nullptr; b.sk_flags = nullptr;
-  unsigned char* qm = reinterpret_cast<unsigned char*>(b.alloc((size_t)N + 16));
-  unsigned char* km = reinterpret_cast<unsigned char*>(b.alloc((size_t)NK + 16));
+  unsigned char* qm = b.mask_buf(N);
+  unsigned char* km = b.mask_buf(NK);
   if (!sizing) { plan->qmask_dev = qm; plan->kmask_dev = km; }
-  float* x = reinterpret_cast<float*>(b.alloc((size_t)N * D * 4));       // hidden states (fp32)
-  float* tmp = reinterpret_cast<float*>(b.alloc((size_t)N * D * 4));     // dense(...) + residual, before the LayerNorm
-  float* emb = reinterpret_cast<float*>(b.alloc((size_t)T * D * 4));     // LayerNorm(query_tokens[:T])
-  Act hbuf = new_act(N, D), qkv = new_act(N, 3 * D), cq = new_act(N, D), ctx = new_act(N, D), ffn = new_act(N, F);
-  Act enc = new_act(NK, Ew), ckv = new_act(NK, 2 * D * L);
-  const bool hm = plan->has_mask;
+  float* x = b.f32buf(N * D);       // hidden states (fp32)
+  float* tmp = b.f32buf(N * D);     // dense(...) + residual, before the LayerNorm
+  float* emb = b.f32buf((long long)T * D);     // LayerNorm(query_tokens[:T])
+  Act hbuf = b.act(N, D), qkv = b.act(N, 3 * D), cq = b.act(N, D), ctx = b.act(N, D), ffn = b.act(N, F);
+  Act enc = b.act(NK, Ew), ckv = b.act(NK, 2 * D * L);
+  const bool hm = key.has_mask;
 
   // ---- AV features -> operand form (the only step that reads a caller pointer besides the output store)
-  b.tag = "load_features";
-  b.cur_direct = true;
   {
     void* dst = enc.data;
-    b.push([=](cudaStream_t s) { return launch_convert(pl->args.xin, pl->args.xin_dt, dst, act_dt, NK * Ew, s); });
+    b.push_direct("load_features", [=](cudaStream_t s) { return launch_convert(pl->args.xin, pl->args.xin_dt, dst, act_dt, NK * Ew, s); });
   }
-  b.cur_direct = false;
-  sync_op(enc);
+  b.sync_op(enc);
   // ---- embeddings: LayerNorm(query_embeds) (no position embeddings on the query-only path, Qformer.py:98-110)
   {
     const float* qt = h->qf_tokens; const float* g = h->qf_emb_g; const float* be = h->qf_emb_b;
-    b.tag = "layer_ln";
-    b.push([=](cudaStream_t s) { return launch_layernorm(qt, DT_F32, D, g, be, eps, emb, nullptr, DT_BF16, nullptr, T, D, s); });
-    b.push([=](cudaStream_t s) { return launch_rows_broadcast(emb, x, (long long)T * D, B, s); });
+    b.push("layer_ln", [=](cudaStream_t s) { return launch_layernorm(qt, DT_F32, D, g, be, eps, emb, nullptr, DT_BF16, nullptr, T, D, s); });
+    b.push("layer_ln", [=](cudaStream_t s) { return launch_rows_broadcast(emb, x, (long long)T * D, B, s); });
   }
-  auto x_to_h = [&]() {
-    void* dst = hbuf.op;
-    const int planes = P;
-    b.tag = "split";
-    b.push([=](cudaStream_t s) { return launch_split_rows(x, D, dst, planes, N, D, 0, 0, s); });
-  };
-  auto post_ln = [&](const float* g, const float* be) {      // x = LayerNorm(tmp), then its operand copy
-    b.tag = "layer_ln";
-    b.push([=](cudaStream_t s) { return launch_layernorm(tmp, DT_F32, D, g, be, eps, x, nullptr, DT_BF16, nullptr, N, D, s); });
+  // x = LayerNorm(tmp), then (unless it is the output) its operand copy
+  auto post_ln = [&](const float* g, const float* be, bool to_op) {
+    b.push("layer_ln", [=](cudaStream_t s) { return launch_layernorm(tmp, DT_F32, D, g, be, eps, x, nullptr, DT_BF16, nullptr, N, D, s); });
+    if (to_op) b.split(x, D, hbuf.op, N, D);
   };
   auto dense_res = [&](const Act& a, int K, const LinearW& w, const char* tag) {      // tmp = a W^T + b + x
-    Epilogue ep;
-    ep.C = tmp; ep.ldc = D; ep.c_fp32 = 1;
+    Epilogue ep = epilogue(tmp, D, true);
     ep.col_bias = w.bias; ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
-    b.tag = tag;
-    return b.gemm(a.op, N, P * K, w.w, N, {Tap{0, 0, 0}}, K / 64, K, ep);
+    return b.linear(tag, a.op, N, K, w.w, ep);
   };
-  x_to_h();
+  b.split(x, D, hbuf.op, N, D);
   // ---- K / V of the AV features for every layer's cross-attention
   {
-    Epilogue ep;
-    ep.C = ckv.data; ep.ldc = 2 * D * L; ep.c_fp32 = f32 ? 1 : 0;
+    Epilogue ep = epilogue(ckv.data, 2 * D * L, f32);
     ep.col_bias = h->qf_ckv.bias;
-    b.tag = "cross_kv_proj";
-    if (!b.gemm(enc.op, NK, P * Ew, h->qf_ckv.w, NK, {Tap{0, 0, 0}}, Ew / 64, Ew, ep)) return false;
+    if (!b.linear("cross_kv_proj", enc.op, NK, Ew, h->qf_ckv.w, ep)) return false;
   }
   const float scale = 0.125f;                                 // 1 / sqrt(attention_head_size = 64), Qformer.py:246
   for (int l = 0; l < L; ++l) {
     const QfLayerW& lw = h->qf_layers[l];
     b.cur_layer = l;
     {   // self-attention over the queries
-      Epilogue ep;
-      ep.C = qkv.data; ep.ldc = 3 * D; ep.c_fp32 = f32 ? 1 : 0;
+      Epilogue ep = epilogue(qkv.data, 3 * D, f32);
       ep.col_bias = lw.sqkv.bias;
-      b.tag = "qkv_proj";
-      if (!b.gemm(hbuf.op, N, P * D, lw.sqkv.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      if (!b.linear("qkv_proj", hbuf.op, N, D, lw.sqkv.w, ep)) return false;
       const char* q = reinterpret_cast<const char*>(qkv.data);
       void* o = ctx.data;
-      b.tag = "attention";
-      b.push([=](cudaStream_t s) {
+      b.push("attention", [=](cudaStream_t s) {
         return launch_attention_x(q, 3 * D, q + (size_t)D * es, 3 * D, q + (size_t)2 * D * es, 3 * D, act_dt, pl->qmask_dev, o, D,
                                   act_dt, B, Hh, T, T, scale, s);
       }, 4.0 * (double)B * Hh * (double)T * (double)T * 64.0);
-      sync_op(ctx);
+      b.sync_op(ctx);
       if (!dense_res(ctx, D, lw.sout, "out_proj")) return false;
-      post_ln(lw.ln1_g, lw.ln1_b);
-      x_to_h();
+      post_ln(lw.ln1_g, lw.ln1_b, true);
     }
     {   // cross-attention to the AV features
-      Epilogue ep;
-      ep.C = cq.data; ep.ldc = D; ep.c_fp32 = f32 ? 1 : 0;
+      Epilogue ep = epilogue(cq.data, D, f32);
       ep.col_bias = lw.cq.bias;
-      b.tag = "cross_q_proj";
-      if (!b.gemm(hbuf.op, N, P * D, lw.cq.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
+      if (!b.linear("cross_q_proj", hbuf.op, N, D, lw.cq.w, ep)) return false;
       const void* q = cq.data;
       const char* kvp = reinterpret_cast<const char*>(ckv.data) + (size_t)l * 2 * D * es;
       const long long ldkv = 2ll * D * L;
       void* o = ctx.data;
-      b.tag = "cross_attention";
-      b.push([=](cudaStream_t s) {
+      b.push("cross_attention", [=](cudaStream_t s) {
         return launch_attention_x(q, D, kvp, ldkv, kvp + (size_t)D * es, ldkv, act_dt, hm ? pl->kmask_dev : nullptr, o, D, act_dt,
                                   B, Hh, T, Lk, scale, s);
       }, 4.0 * (double)B * Hh * (double)T * (double)Lk * 64.0);
-      sync_op(ctx);
+      b.sync_op(ctx);
       if (!dense_res(ctx, D, lw.cout, "cross_out_proj")) return false;
-      post_ln(lw.ln2_g, lw.ln2_b);
-      x_to_h();
+      post_ln(lw.ln2_g, lw.ln2_b, true);
     }
     {   // feed-forward of the query branch (intermediate_query / output_query, Qformer.py:482-485), erf GELU
-      Epilogue ep;
-      ep.C = ffn.data; ep.ldc = F; ep.c_fp32 = f32 ? 1 : 0;
+      Epilogue ep = epilogue(ffn.data, F, f32);
       ep.col_bias = lw.fc1.bias; ep.act = ACT_GELU;
-      b.tag = "fc1";
-      if (!b.gemm(hbuf.op, N, P * D, lw.fc1.w, N, {Tap{0, 0, 0}}, D / 64, D, ep)) return false;
-      sync_op(ffn);
+      if (!b.linear("fc1", hbuf.op, N, D, lw.fc1.w, ep)) return false;
+      b.sync_op(ffn);
       if (!dense_res(ffn, F, lw.fc2, "fc2")) return false;
-      post_ln(lw.ln3_g, lw.ln3_b);
-      if (l + 1 < L) x_to_h();
+      post_ln(lw.ln3_g, lw.ln3_b, l + 1 < L);
     }
   }
   b.cur_layer = -1;
-  b.tag = "output";
-  b.cur_direct = true;
-  b.push([=](cudaStream_t s) { return launch_convert(x, DT_F32, pl->args.out, pl->args.out_dt, N * D, s); });
-  b.cur_direct = false;
+  b.push_direct("output", [=](cudaStream_t s) { return launch_convert(x, DT_F32, pl->args.out, pl->args.out_dt, N * D, s); });
   if (bytes_out) *bytes_out = b.sizer.used;
   return true;
 }
 
 constexpr int MAX_PLANS = 24;      // plans kept per handle (shape x stream); the least recently used one is evicted
 
-Plan* get_plan(avh_handle* h, int B, int T, bool has_video, bool has_audio, bool has_mask, int output_layer,
-               cudaStream_t stream, long long ragged_rows = 0, bool enc_only = false, bool train = false, int qf_lk = 0,
-               bool enc_train = false, int tail = 0) {
-  const std::string key = (ragged_rows > 0 ? "r" + std::to_string(ragged_rows) + ":" : std::string()) + (enc_only ? "e:" : "") +
-                          (train ? "t:" : "") + (qf_lk > 0 ? "q" + std::to_string(qf_lk) + ":" : std::string()) +
-                          (enc_train ? (tail == 2 ? "gf:" : (tail ? "gt:" : "g:")) : "") +
-                          std::to_string(B) + "x" + std::to_string(T) + (has_video ? "v" : "-") +
-                          (has_audio ? "a" : "-") + (has_mask ? "m" : "-") + std::to_string(output_layer) + "@" +
-                          std::to_string(reinterpret_cast<uintptr_t>(stream));
+void forget_plan(avh_handle* h, const Plan* p) {
+  if (h->last_plan == p) h->last_plan = nullptr;
+  if (h->prof_plan == p) h->prof_plan = nullptr;
+}
+
+Plan* get_plan(avh_handle* h, const PlanKey& key) {
   auto it = h->plans.find(key);
   if (it != h->plans.end()) {
     it->second->last_use = ++h->plan_clock;
@@ -2600,44 +2371,43 @@ Plan* get_plan(avh_handle* h, int B, int T, bool has_video, bool has_audio, bool
     auto victim = h->plans.begin();
     for (auto jt = h->plans.begin(); jt != h->plans.end(); ++jt)
       if (jt->second->last_use < victim->second->last_use) victim = jt;
-    if (h->last_plan == victim->second.get()) h->last_plan = nullptr;
-    if (h->prof_plan == victim->second.get()) h->prof_plan = nullptr;
+    forget_plan(h, victim->second.get());
     h->plans.erase(victim);
   }
-  if (enc_train) {
+  if (key.training()) {
     // training plans keep every activation of the step (GBs for Large): at most two of them live per handle
     for (;;) {
       int n_train = 0;
       auto victim = h->plans.end();
       for (auto jt = h->plans.begin(); jt != h->plans.end(); ++jt)
-        if (jt->second->enc_train) {
+        if (jt->first.training()) {
           ++n_train;
           if (victim == h->plans.end() || jt->second->last_use < victim->second->last_use) victim = jt;
         }
       if (n_train < 2) break;
-      if (h->last_plan == victim->second.get()) h->last_plan = nullptr;
-      if (h->prof_plan == victim->second.get()) h->prof_plan = nullptr;
+      forget_plan(h, victim->second.get());
       h->plans.erase(victim);
     }
   }
   std::unique_ptr<Plan> p(new Plan());
   p->last_use = ++h->plan_clock;
-  p->stream = stream;
-  p->B = B; p->T = T; p->has_video = has_video; p->has_audio = has_audio; p->has_mask = has_mask;
-  p->output_layer = output_layer;
-  p->ragged = ragged_rows > 0;
-  p->Nb = ragged_rows;
-  p->enc_only = enc_only;
-  p->train = train;
-  p->Lk = qf_lk;
-  p->enc_train = enc_train;
-  p->tail = tail;
+  p->key = key;
+  bool (*build)(avh_handle*, Plan*, bool, size_t*) = nullptr;
+  switch (key.kind) {
+    case PlanKind::Forward:
+    case PlanKind::Ragged:
+    case PlanKind::EncoderOnly:
+    case PlanKind::TrainForward: build = build_plan; break;
+    case PlanKind::EncoderTrain:
+    case PlanKind::TailTrain:
+    case PlanKind::FullTrain: build = build_encoder_train_plan; break;
+    case PlanKind::QFormer: build = build_qformer_plan; break;
+  }
   size_t bytes = 0;
-  auto build = qf_lk > 0 ? build_qformer_plan : (enc_train ? build_encoder_train_plan : build_plan);
   if (!build(h, p.get(), true, &bytes)) return nullptr;
   if (p->arena.init(bytes + (1 << 20))) return nullptr;
   if (!build(h, p.get(), false, nullptr)) return nullptr;
-  if (p->ragged) {
+  if (key.kind == PlanKind::Ragged) {
     for (int i = 0; i < Plan::RAG_SLOTS; ++i) {
       if (cudaMallocHost(reinterpret_cast<void**>(&p->rag_host[i]), (size_t)p->rag_ints * 4) != cudaSuccess ||
           cudaEventCreateWithFlags(&p->rag_done[i], cudaEventDisableTiming) != cudaSuccess) {
@@ -2850,20 +2620,28 @@ static int replay_range(avh::Plan* p, size_t begin, size_t end, cudaStream_t s) 
   return 0;
 }
 
-static int run_plan(avh_handle* h, avh::Plan* p, cudaStream_t s) {
+// Steps [begin, end) of a plan: a whole forward, or the forward or backward half of a training plan.  The first run of
+// a plan launches its steps directly (it also configures the kernels); the second captures every maximal run of
+// plan-internal steps into a CUDA graph, later runs replay them (in a training plan the direct final-LayerNorm store
+// separates the forward from the backward, so no graph straddles the two ranges).  Training-mode forwards (LayerDrop,
+// per-call dropout) and profiled forwards always launch directly.
+static int run_steps(avh_handle* h, avh::Plan* p, size_t begin, size_t end, cudaStream_t s) {
   read_graphs_env();
+  const avh::PlanKey& key = p->key;
+  const bool train_fwd = key.kind == avh::PlanKind::TrainForward;
+  const bool profiled = h->profiling && !key.training();     // avh_profile_json covers the forward plans
   // the caller's padding mask -> plan-owned copy (every later read is pointer-independent)
-  if (p->has_mask && p->args.mask != nullptr)
-    AVH_CUDA_OK(cudaMemcpyAsync(p->mask_dev, p->args.mask, (size_t)p->B * p->T, cudaMemcpyDeviceToDevice, s));
+  if (begin == 0 && p->args.mask != nullptr)
+    AVH_CUDA_OK(cudaMemcpyAsync(p->mask_dev, p->args.mask, (size_t)key.B * key.T, cudaMemcpyDeviceToDevice, s));
   // a caller that is itself capturing this stream (e.g. torch.cuda.graph) gets plain launches recorded into ITS graph
   cudaStreamCaptureStatus cap_status = cudaStreamCaptureStatusNone;
   if (s != nullptr && s != cudaStreamLegacy && s != cudaStreamPerThread) cudaStreamIsCapturing(s, &cap_status);
-  const bool graphs_ok = graphs_env == 1 && !h->profiling && !p->train && s != nullptr && s != cudaStreamLegacy &&
+  const bool graphs_ok = graphs_env == 1 && !profiled && !train_fwd && s != nullptr && s != cudaStreamLegacy &&
                          s != cudaStreamPerThread && cap_status == cudaStreamCaptureStatusNone;
-  if (graphs_ok && !p->segments_ready && p->direct_runs >= 1) capture_segments(p, s);      // second forward of this plan
-  if (graphs_ok && graphs_env == 1 && p->segments_ready) return replay_range(p, 0, p->steps.size(), s);
-  ++p->direct_runs;
-  if (h->profiling) {
+  if (graphs_ok && begin == 0 && !p->segments_ready && p->direct_runs >= 1) capture_segments(p, s);
+  if (graphs_ok && graphs_env == 1 && p->segments_ready) return replay_range(p, begin, end, s);
+  if (begin == 0) ++p->direct_runs;
+  if (profiled) {
     while (h->prof_events.size() < 2 * p->steps.size()) {
       cudaEvent_t e;
       AVH_CUDA_OK(cudaEventCreate(&e));
@@ -2871,16 +2649,15 @@ static int run_plan(avh_handle* h, avh::Plan* p, cudaStream_t s) {
     }
     h->prof_plan = p;
   }
-  size_t i = 0;
-  for (auto& st : p->steps) {
-    if (h->profiling) cudaEventRecord(h->prof_events[2 * i], s);
-    const bool dropped = p->train && st.layer >= 0 && st.layer < (int)p->layer_skip.size() && p->layer_skip[st.layer] != 0;
+  for (size_t i = begin; i < end; ++i) {
+    const avh::Step& st = p->steps[i];
+    if (profiled) cudaEventRecord(h->prof_events[2 * i], s);
+    const bool dropped = train_fwd && st.layer >= 0 && st.layer < (int)p->layer_skip.size() && p->layer_skip[st.layer] != 0;
     if (!dropped && st.run(s)) {
       if (avh::g_err.empty()) avh::set_last_error("kernel launch failed");
       return 1;
     }
-    if (h->profiling) cudaEventRecord(h->prof_events[2 * i + 1], s);
-    ++i;
+    if (profiled) cudaEventRecord(h->prof_events[2 * i + 1], s);
   }
   return 0;
 }
@@ -2896,9 +2673,8 @@ int avh_release_stream(avh_handle* h, void* stream) {
   AVH_CUDA_OK(cudaSetDevice(h->device));
   AVH_CUDA_OK(cudaStreamSynchronize(reinterpret_cast<cudaStream_t>(stream)));
   for (auto it = h->plans.begin(); it != h->plans.end();) {
-    if (it->second->stream == reinterpret_cast<cudaStream_t>(stream)) {
-      if (h->last_plan == it->second.get()) h->last_plan = nullptr;
-      if (h->prof_plan == it->second.get()) h->prof_plan = nullptr;
+    if (it->first.stream == reinterpret_cast<cudaStream_t>(stream)) {
+      avh::forget_plan(h, it->second.get());
       it = h->plans.erase(it);
     } else ++it;
   }
@@ -2939,8 +2715,13 @@ int avh_forward(avh_handle* h, const void* video, int video_dtype, const void* a
     video_dtype = pdt;
   }
   AVH_CHECK(video == nullptr || video_dtype == AVH_F32 || video_dtype == AVH_F16 || video_dtype == AVH_BF16, "bad video dtype");
-  avh::Plan* p = avh::get_plan(h, B, T, video != nullptr, audio != nullptr, padding_mask != nullptr, output_layer,
-                               reinterpret_cast<cudaStream_t>(stream));
+  avh::PlanKey key;
+  key.kind = avh::PlanKind::Forward;
+  key.B = B; key.T = T;
+  key.has_video = video != nullptr; key.has_audio = audio != nullptr; key.has_mask = padding_mask != nullptr;
+  key.output_layer = output_layer;
+  key.stream = reinterpret_cast<cudaStream_t>(stream);
+  avh::Plan* p = avh::get_plan(h, key);
   if (p == nullptr) return 1;
   h->last_plan = p;
   p->args.video = video; p->args.video_dt = video_dtype;
@@ -2948,7 +2729,7 @@ int avh_forward(avh_handle* h, const void* video, int video_dtype, const void* a
   if (audio) for (int i = 0; i < 3; ++i) p->args.as[i] = audio_strides[i];
   p->args.mask = padding_mask;
   p->args.out = out; p->args.out_dt = out_dtype;
-  return run_plan(h, p, reinterpret_cast<cudaStream_t>(stream));
+  return run_steps(h, p, 0, p->steps.size(), reinterpret_cast<cudaStream_t>(stream));
 }
 
 int avh_forward_train(avh_handle* h, const void* video, int video_dtype, const void* audio, int audio_dtype,
@@ -2970,8 +2751,13 @@ int avh_forward_train(avh_handle* h, const void* video, int video_dtype, const v
   AVH_CHECK(ta->bn_momentum > 0.f && ta->bn_momentum <= 1.f, "bad BatchNorm momentum");
   AVH_CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  avh::Plan* p = avh::get_plan(h, B, T, video != nullptr, audio != nullptr, padding_mask != nullptr, output_layer, s, 0,
-                               false, true);
+  avh::PlanKey key;
+  key.kind = avh::PlanKind::TrainForward;
+  key.B = B; key.T = T;
+  key.has_video = video != nullptr; key.has_audio = audio != nullptr; key.has_mask = padding_mask != nullptr;
+  key.output_layer = output_layer;
+  key.stream = s;
+  avh::Plan* p = avh::get_plan(h, key);
   if (p == nullptr) return 1;
   h->last_plan = p;
   p->args = avh::CallArgs();
@@ -2986,7 +2772,7 @@ int avh_forward_train(avh_handle* h, const void* video, int video_dtype, const v
   p->layer_skip.assign(h->cfg.encoder_layers, 0);
   if (ta->layer_skip != nullptr)
     for (int l = 0; l < h->cfg.encoder_layers; ++l) p->layer_skip[l] = ta->layer_skip[l];
-  return run_plan(h, p, s);
+  return run_steps(h, p, 0, p->steps.size(), s);
 }
 
 int avh_interp_linear(const void* x, int dtype, int B, int T, int C, const int32_t* len_in, const int32_t* len_out,
@@ -3085,34 +2871,20 @@ int avh_encoder_forward(avh_handle* h, const void* x, int x_dtype, const uint8_t
   AVH_CHECK(output_layer >= 0 && output_layer <= h->cfg.encoder_layers, "output_layer out of range");
   AVH_CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  avh::Plan* p = avh::get_plan(h, B, T, false, false, padding_mask != nullptr, output_layer, s, 0, true);
+  avh::PlanKey key;
+  key.kind = avh::PlanKind::EncoderOnly;
+  key.B = B; key.T = T;
+  key.has_mask = padding_mask != nullptr;
+  key.output_layer = output_layer;
+  key.stream = s;
+  avh::Plan* p = avh::get_plan(h, key);
   if (p == nullptr) return 1;
   h->last_plan = p;
   p->args = avh::CallArgs();
   p->args.xin = x; p->args.xin_dt = x_dtype;
   p->args.mask = padding_mask;
   p->args.out = out; p->args.out_dt = out_dtype;
-  return run_plan(h, p, s);
-}
-
-static int run_steps(avh_handle* h, avh::Plan* p, size_t begin, size_t end, cudaStream_t s) {
-  (void)h;
-  read_graphs_env();
-  cudaStreamCaptureStatus cap_status = cudaStreamCaptureStatusNone;
-  if (s != nullptr && s != cudaStreamLegacy && s != cudaStreamPerThread) cudaStreamIsCapturing(s, &cap_status);
-  const bool graphs_ok = graphs_env == 1 && s != nullptr && s != cudaStreamLegacy && s != cudaStreamPerThread &&
-                         cap_status == cudaStreamCaptureStatusNone;
-  // training plans: the first step of a shape runs directly (it also configures the kernels), the second captures the
-  // forward and the backward launch lists (the direct final-LayerNorm store separates them), later ones replay
-  if (graphs_ok && begin == 0 && !p->segments_ready && p->direct_runs >= 1) capture_segments(p, s);
-  if (graphs_ok && graphs_env == 1 && p->segments_ready) return replay_range(p, begin, end, s);
-  if (begin == 0) ++p->direct_runs;
-  for (size_t i = begin; i < end; ++i)
-    if (p->steps[i].run(s)) {
-      if (avh::g_err.empty()) avh::set_last_error("kernel launch failed");
-      return 1;
-    }
-  return 0;
+  return run_steps(h, p, 0, p->steps.size(), s);
 }
 
 int avh_encoder_grad_count(avh_handle* h, int64_t* n_floats) {
@@ -3165,8 +2937,12 @@ int avh_full_train_forward(avh_handle* h, const void* video, int video_dtype, co
   AVH_CHECK(B >= 1 && T >= 1 && (long long)B * T < (1ll << 20), "bad batch");
   AVH_CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  avh::Plan* p = avh::get_plan(h, B, T, video != nullptr, audio != nullptr, padding_mask != nullptr, 0, s, 0, false, false, 0,
-                               true, 2);
+  avh::PlanKey key;
+  key.kind = avh::PlanKind::FullTrain;
+  key.B = B; key.T = T;
+  key.has_video = video != nullptr; key.has_audio = audio != nullptr; key.has_mask = padding_mask != nullptr;
+  key.stream = s;
+  avh::Plan* p = avh::get_plan(h, key);
   if (p == nullptr) return 1;
   h->last_plan = p;
   p->args = avh::CallArgs();
@@ -3177,8 +2953,6 @@ int avh_full_train_forward(avh_handle* h, const void* video, int video_dtype, co
   p->args.out = out; p->args.out_dt = out_dtype;
   p->bn_momentum = bn_momentum;
   p->fgm = feature_grad_mult;
-  if (padding_mask != nullptr)
-    AVH_CUDA_OK(cudaMemcpyAsync(p->mask_dev, padding_mask, (size_t)B * T, cudaMemcpyDeviceToDevice, s));
   p->fwd_done = false;
   if (run_steps(h, p, 0, p->fwd_steps, s)) return 1;
   p->fwd_done = true;
@@ -3196,67 +2970,62 @@ static int encoder_train_forward(avh_handle* h, const void* x, int x_dtype, cons
   AVH_CHECK(B >= 1 && T >= 1 && (long long)B * T < (1ll << 24), "bad batch");
   AVH_CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  avh::Plan* p = avh::get_plan(h, B, T, false, false, padding_mask != nullptr, 0, s, 0, true, false, 0, true, tail);
+  avh::PlanKey key;
+  key.kind = tail ? avh::PlanKind::TailTrain : avh::PlanKind::EncoderTrain;
+  key.B = B; key.T = T;
+  key.has_mask = padding_mask != nullptr;
+  key.stream = s;
+  avh::Plan* p = avh::get_plan(h, key);
   if (p == nullptr) return 1;
   h->last_plan = p;
   p->args = avh::CallArgs();
   p->args.xin = x; p->args.xin_dt = x_dtype;
   p->args.mask = padding_mask;
   p->args.out = out; p->args.out_dt = out_dtype;
-  if (padding_mask != nullptr)
-    AVH_CUDA_OK(cudaMemcpyAsync(p->mask_dev, padding_mask, (size_t)B * T, cudaMemcpyDeviceToDevice, s));
   p->fwd_done = false;
   if (run_steps(h, p, 0, p->fwd_steps, s)) return 1;
   p->fwd_done = true;
   return 0;
 }
 
-int avh_encoder_backward(avh_handle* h, const void* dout, int dout_dtype, void* dx, int dx_dtype, float* grads,
-                         int64_t grads_capacity, void* stream) {
+// The backward half of the last training plan.  `buckets`: the gradient buckets are converted into the caller's `grads`
+// (of dtype grads_dtype) as the backward completes them; otherwise the whole fp32 buffer is copied at the end, if asked.
+static int encoder_backward(avh_handle* h, const void* dout, int dout_dtype, void* dx, int dx_dtype, void* grads, int grads_dtype,
+                            int64_t grads_capacity, bool buckets, void* stream) {
   AVH_CHECK(h != nullptr, "null handle");
-  AVH_CHECK(dout != nullptr, "null argument");
+  AVH_CHECK(dout != nullptr && (grads != nullptr || !buckets), "null argument");
+  AVH_CHECK(!buckets || grads_dtype == AVH_F32 || grads_dtype == AVH_BF16 || grads_dtype == AVH_F16, "bad gradient dtype");
   avh::Plan* p = h->last_plan;
-  AVH_CHECK(p != nullptr && p->enc_train && p->fwd_done, "avh_encoder_backward follows avh_encoder_train_forward on the same handle");
+  AVH_CHECK(p != nullptr && p->key.training() && p->fwd_done, "the backward follows a training forward on the same handle");
   AVH_CHECK(grads == nullptr || grads_capacity >= p->grad_floats, "gradient buffer too small (avh_encoder_grad_count)");
   AVH_CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  AVH_CHECK(s == p->stream, "backward must run on the stream of its forward");
-  const long long N = (long long)p->B * p->T;
+  AVH_CHECK(s == p->key.stream, "backward must run on the stream of its forward");
+  const long long N = (long long)p->key.B * p->key.T;
   const int D = h->cfg.encoder_embed_dim;
   // dL/dy -> fp32.  Rows of padded frames are taken as given, as autograd does: the dense forward computed those rows
   // (their queries attend to the valid keys), so a loss that reads them sends gradient through them too
   if (avh::launch_load_rows(dout, dout_dtype, p->dy_in, nullptr, N, D, s)) return 1;
-  p->args.grads_out = nullptr;
-  if (run_steps(h, p, p->fwd_steps, p->steps.size(), s)) return 1;
-  if (dx != nullptr && avh::launch_convert(p->dx_out, avh::DT_F32, dx, dx_dtype, N * D, s)) return 1;
-  if (grads != nullptr)
-    AVH_CUDA_OK(cudaMemcpyAsync(grads, p->grads, (size_t)p->grad_floats * 4, cudaMemcpyDeviceToDevice, s));
-  p->fwd_done = false;
-  return 0;
-}
-
-int avh_encoder_backward_buckets(avh_handle* h, const void* dout, int dout_dtype, void* dx, int dx_dtype, void* grads,
-                                 int grads_dtype, int64_t grads_capacity, void* stream) {
-  AVH_CHECK(h != nullptr, "null handle");
-  AVH_CHECK(dout != nullptr && grads != nullptr, "null argument");
-  AVH_CHECK(grads_dtype == AVH_F32 || grads_dtype == AVH_BF16 || grads_dtype == AVH_F16, "bad gradient dtype");
-  avh::Plan* p = h->last_plan;
-  AVH_CHECK(p != nullptr && p->enc_train && p->fwd_done, "avh_encoder_backward_buckets follows a training forward on the same handle");
-  AVH_CHECK(grads_capacity >= p->grad_floats, "gradient buffer too small (avh_encoder_grad_count)");
-  AVH_CUDA_OK(cudaSetDevice(h->device));
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  AVH_CHECK(s == p->stream, "backward must run on the stream of its forward");
-  const long long N = (long long)p->B * p->T;
-  const int D = h->cfg.encoder_embed_dim;
-  if (avh::launch_load_rows(dout, dout_dtype, p->dy_in, nullptr, N, D, s)) return 1;
-  p->args.grads_out = grads;
+  p->args.grads_out = buckets ? grads : nullptr;
   p->args.grads_dt = grads_dtype;
   const int rc = run_steps(h, p, p->fwd_steps, p->steps.size(), s);
   p->args.grads_out = nullptr;
   if (rc) return 1;
   if (dx != nullptr && avh::launch_convert(p->dx_out, avh::DT_F32, dx, dx_dtype, N * D, s)) return 1;
+  if (!buckets && grads != nullptr)
+    AVH_CUDA_OK(cudaMemcpyAsync(grads, p->grads, (size_t)p->grad_floats * 4, cudaMemcpyDeviceToDevice, s));
   p->fwd_done = false;
   return 0;
+}
+
+int avh_encoder_backward(avh_handle* h, const void* dout, int dout_dtype, void* dx, int dx_dtype, float* grads,
+                         int64_t grads_capacity, void* stream) {
+  return encoder_backward(h, dout, dout_dtype, dx, dx_dtype, grads, AVH_F32, grads_capacity, false, stream);
+}
+
+int avh_encoder_backward_buckets(avh_handle* h, const void* dout, int dout_dtype, void* dx, int dx_dtype, void* grads,
+                                 int grads_dtype, int64_t grads_capacity, void* stream) {
+  return encoder_backward(h, dout, dout_dtype, dx, dx_dtype, grads, grads_dtype, grads_capacity, true, stream);
 }
 
 int avh_refresh_weights_device(avh_handle* h, const char* const* names, const void* const* ptrs, const int32_t* dtypes,
@@ -3364,7 +3133,7 @@ int avh_refresh_weights_device(avh_handle* h, const char* const* names, const vo
 int avh_grad_bucket_count(avh_handle* h, int32_t* count) {
   AVH_CHECK(h != nullptr && count != nullptr, "null argument");
   avh::Plan* p = h->last_plan;
-  AVH_CHECK(p != nullptr && p->enc_train, "no training plan on this handle yet (run a training forward first)");
+  AVH_CHECK(p != nullptr && p->key.training(), "no training plan on this handle yet (run a training forward first)");
   *count = (int32_t)p->buckets.size();
   return 0;
 }
@@ -3372,7 +3141,7 @@ int avh_grad_bucket_count(avh_handle* h, int32_t* count) {
 int avh_grad_bucket_range(avh_handle* h, int k, int64_t* begin, int64_t* end) {
   AVH_CHECK(h != nullptr && begin != nullptr && end != nullptr, "null argument");
   avh::Plan* p = h->last_plan;
-  AVH_CHECK(p != nullptr && p->enc_train && k >= 0 && k < (int)p->buckets.size(), "bucket index out of range");
+  AVH_CHECK(p != nullptr && p->key.training() && k >= 0 && k < (int)p->buckets.size(), "bucket index out of range");
   *begin = p->buckets[k].begin;
   *end = p->buckets[k].end;
   return 0;
@@ -3381,7 +3150,7 @@ int avh_grad_bucket_range(avh_handle* h, int k, int64_t* begin, int64_t* end) {
 int avh_grad_bucket_wait(avh_handle* h, int k, void* stream) {
   AVH_CHECK(h != nullptr, "null handle");
   avh::Plan* p = h->last_plan;
-  AVH_CHECK(p != nullptr && p->enc_train && k >= 0 && k < (int)p->buckets.size(), "bucket index out of range");
+  AVH_CHECK(p != nullptr && p->key.training() && k >= 0 && k < (int)p->buckets.size(), "bucket index out of range");
   AVH_CUDA_OK(cudaSetDevice(h->device));
   AVH_CUDA_OK(cudaStreamWaitEvent(reinterpret_cast<cudaStream_t>(stream), p->buckets[k].ev, 0));
   return 0;
@@ -3398,7 +3167,12 @@ int avh_qformer_forward(avh_handle* h, const void* enc, int enc_dtype, const uin
   AVH_CHECK(Lq <= h->cfg.reserved[2], "more queries than query_tokens holds");
   AVH_CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-  avh::Plan* p = avh::get_plan(h, B, Lq, false, false, enc_padding != nullptr, 0, s, 0, false, false, Lk);
+  avh::PlanKey key;
+  key.kind = avh::PlanKind::QFormer;
+  key.B = B; key.T = Lq; key.Lk = Lk;
+  key.has_mask = enc_padding != nullptr;
+  key.stream = s;
+  avh::Plan* p = avh::get_plan(h, key);
   if (p == nullptr) return 1;
   h->last_plan = p;
   // query attention mask (src/model.py:588-590): row i of clip b is a key for the queries iff i < len_queries[b]
@@ -3414,11 +3188,7 @@ int avh_qformer_forward(avh_handle* h, const void* enc, int enc_dtype, const uin
   p->args = avh::CallArgs();
   p->args.xin = enc; p->args.xin_dt = enc_dtype;
   p->args.out = out; p->args.out_dt = out_dtype;
-  const bool keep = p->has_mask;
-  p->has_mask = false;                 // run_plan's generic [B,T] mask staging does not apply (masks staged above)
-  const int rc = run_plan(h, p, s);
-  p->has_mask = keep;
-  return rc;
+  return run_steps(h, p, 0, p->steps.size(), s);
 }
 
 int avh_forward_ragged(avh_handle* h, const void* video, int video_dtype, const void* audio, int audio_dtype,
@@ -3456,7 +3226,14 @@ int avh_forward_ragged(avh_handle* h, const void* video, int video_dtype, const 
   // one plan per (clips, 128-row bucket of the packed rows, attention tiling class of the longest clip)
   const long long Nb = (N + 127) / 128 * 128;
   const int Tcap = tmax <= 160 ? 160 : (tmax + 127) / 128 * 128;
-  avh::Plan* p = avh::get_plan(h, B, Tcap, video != nullptr, audio != nullptr, false, output_layer, s, Nb);
+  avh::PlanKey key;
+  key.kind = avh::PlanKind::Ragged;
+  key.B = B; key.T = Tcap;
+  key.has_video = video != nullptr; key.has_audio = audio != nullptr;
+  key.output_layer = output_layer;
+  key.ragged_rows = Nb;
+  key.stream = s;
+  avh::Plan* p = avh::get_plan(h, key);
   if (p == nullptr) return 1;
   h->last_plan = p;
   // per-call geometry -> pinned mirror -> device descriptor (ordered on the stream before the launches that read it)
@@ -3484,7 +3261,7 @@ int avh_forward_ragged(avh_handle* h, const void* video, int video_dtype, const 
   p->args.mask = nullptr;
   p->args.out = out; p->args.out_dt = out_dtype;
   p->args.pitch = T;
-  return run_plan(h, p, s);
+  return run_steps(h, p, 0, p->steps.size(), s);
 }
 
 int avh_set_video_preprocess(avh_handle* h, int src_h, int src_w, double mean, double stdv) {

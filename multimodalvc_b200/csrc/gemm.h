@@ -171,7 +171,6 @@ constexpr int GEMM_MAX_KSTEPS = 768;
 
 int gemm_plan(const GemmProblem& prob, GemmPlan* plan);       // builds tensor maps; 0 on success
 int gemm_launch(const GemmPlan& plan, cudaStream_t stream);  // enqueue; 0 on success
-int gemm_pick_block_n(long long M, int N);
-void gemm_set_trace(unsigned long long* dev_buf);             // debug: per-CTA globaltimer stamps [grid][16]                    // tile heuristic
+void gemm_set_trace(unsigned long long* dev_buf);             // debug: per-CTA globaltimer stamps [grid][16]
 
 }  // namespace avh

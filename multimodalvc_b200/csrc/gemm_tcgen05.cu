@@ -817,8 +817,6 @@ double model_cycles(long long M, int N, int num_kb, int bn, int pair, int occ, i
 
 void gemm_set_trace(unsigned long long* dev_buf) { g_trace = dev_buf; }
 
-int gemm_pick_block_n(long long M, int N) { return 0; (void)M; (void)N; }      // 0 = let gemm_plan choose
-
 int gemm_plan(const GemmProblem& pr, GemmPlan* plan) {
   AVH_CHECK(pr.N % 32 == 0, "N must be a multiple of 32");
   AVH_CHECK(pr.num_kb >= 1, "num_kb must be >= 1");

@@ -632,24 +632,29 @@ class AVHubertModel(nn.Module):
             raise NotImplementedError("the training step takes normalised float video")
         params, spec = self.full_parameters(video is not None, audio is not None)
         y = _FullTrainFn.apply(self, video, audio, pm_u8, float(c.feature_grad_mult), spec, *params)
-        if video is not None:          # running statistics of the training-mode BatchNorms back into the module's buffers
-            with torch.no_grad():
-                lib = _lib.load()
-                n = ctypes.c_int64()
-                _lib.check(lib.avh_bn_stats_count(handle, ctypes.byref(n)))
-                flat = torch.empty(n.value, device=dev, dtype=torch.float32)
-                with torch.cuda.device(dev):
-                    stream = torch.cuda.current_stream(dev).cuda_stream
-                    _lib.check(lib.avh_read_bn_stats(handle, ctypes.c_void_p(flat.data_ptr()), n.value, ctypes.c_void_p(stream)))
-                off = 0
-                for bn in self._bn_modules():
-                    C = bn.num_features
-                    bn.running_mean.copy_(flat[off:off + C])
-                    bn.running_var.copy_(flat[off + C:off + 2 * C])
-                    bn.num_batches_tracked += 1
-                    off += 2 * C
-                self._eval_stale = True
+        if video is not None:
+            self._read_back_bn_stats(handle, dev)
         return y, pm
+
+    @torch.no_grad()
+    def _read_back_bn_stats(self, handle, dev):
+        """Running statistics of the training-mode BatchNorms, updated on the device by the last forward, back into the
+        module's buffers (the next eval forward folds them again)."""
+        lib = _lib.load()
+        n = ctypes.c_int64()
+        _lib.check(lib.avh_bn_stats_count(handle, ctypes.byref(n)))
+        flat = torch.empty(n.value, device=dev, dtype=torch.float32)
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _lib.check(lib.avh_read_bn_stats(handle, ctypes.c_void_p(flat.data_ptr()), n.value, ctypes.c_void_p(stream)))
+        off = 0
+        for bn in self._bn_modules():
+            C = bn.num_features
+            bn.running_mean.copy_(flat[off:off + C])
+            bn.running_var.copy_(flat[off + C:off + 2 * C])
+            bn.num_batches_tracked += 1
+            off += 2 * C
+        self._eval_stale = True
 
     def _extract_finetune_trainable(self, source, padding_mask, mask, output_layer):
         """Fine-tuning step with frozen feature extractors (feature_grad_mult <= 0: the reference runs them under
@@ -725,19 +730,8 @@ class AVHubertModel(nn.Module):
                     _DTYPES[src_audio.dtype] if src_audio is not None else 0, strides,
                     ctypes.c_void_p(pm_u8.data_ptr()) if pm_u8 is not None else None,
                     B, T, ol, ctypes.byref(ta), ctypes.c_void_p(out.data_ptr()), _DTYPES[out_dtype], ctypes.c_void_p(stream)))
-                if src_video is not None:
-                    n = ctypes.c_int64()
-                    _lib.check(lib.avh_bn_stats_count(handle, ctypes.byref(n)))
-                    flat = torch.empty(n.value, device=dev, dtype=torch.float32)
-                    _lib.check(lib.avh_read_bn_stats(handle, ctypes.c_void_p(flat.data_ptr()), n.value, ctypes.c_void_p(stream)))
-                    off = 0
-                    for bn in self._bn_modules():
-                        C = bn.num_features
-                        bn.running_mean.copy_(flat[off:off + C])
-                        bn.running_var.copy_(flat[off + C:off + 2 * C])
-                        bn.num_batches_tracked += 1
-                        off += 2 * C
-                    self._eval_stale = True
+            if src_video is not None:
+                self._read_back_bn_stats(handle, dev)
             return out, padding_mask
         if self.cfg.ragged not in ("dense", "packed"):
             raise ValueError(f"cfg.ragged must be 'dense' or 'packed', got {self.cfg.ragged}")
