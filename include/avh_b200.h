@@ -176,10 +176,11 @@ AVH_API int avh_read_bn_stats(avh_handle* h, float* dst, int64_t capacity, void*
 AVH_API int avh_encoder_forward(avh_handle* h, const void* x, int x_dtype, const uint8_t* padding_mask, int B, int T,
                                 int output_layer, void* out, int out_dtype, void* stream);
 
-/* Training step of the TransformerEncoder (SURVEY 8(a) row A18, encoder part of BASELINE config 5; dropout and LayerDrop 0
- * as that config states; pre-LN layers): forward with saved activations, then the backward of exactly that graph —
- * wav2vec2.py:859-902 (positional conv + GELU + residual, index_put on padded frames), :974-992 (pre-LN layer),
- * multihead_attention.py:170-192, the final LayerNorm (:862-863) — what torch.autograd computes for the reference module.
+/* Training step of the TransformerEncoder (SURVEY 8(a) row A18, encoder part of BASELINE config 5; pre-LN layers): forward
+ * with saved activations, then the backward of exactly that graph — wav2vec2.py:859-902 (positional conv + GELU +
+ * residual, index_put on padded frames), :974-992 (pre-LN layer), multihead_attention.py:170-192, the final LayerNorm
+ * (:862-863) — what torch.autograd computes for the reference module.  Dropout and LayerDrop as avh_set_train_args
+ * leaves them for the call (none without it).
  * Handle: any handle with encoder weights created with avh_config.reserved[3] = 1 (packs W^T for the dX = dY W GEMMs).
  * avh_encoder_train_forward: as avh_encoder_forward (all layers + final LayerNorm); avh_encoder_backward: dout [B,T,D] =
  * dL/d(out) (every row counts, padded frames too, as under autograd), dx [B,T,D] = dL/d(x) (may be NULL), grads = fp32 [avh_encoder_grad_count]
@@ -215,6 +216,18 @@ AVH_API int avh_refresh_weights_device(avh_handle* h, const char* const* names, 
 AVH_API int avh_grad_bucket_range(avh_handle* h, int k, int64_t* begin, int64_t* end);       /* [begin, end) elements */
 AVH_API int avh_grad_bucket_wait(avh_handle* h, int k, void* stream);
 
+/* Regularisation of the NEXT avh_encoder_train_forward / avh_tail_train_forward / avh_full_train_forward on the handle,
+ * which consumes it (without this call a training step has no dropout and drops no layer).  Same masks and sites as
+ * avh_forward_train: dropout_input on the post_extract_proj output (tail and full steps only; ignored by the bare
+ * encoder), dropout after the positional conv block and on the attention / FFN block outputs, activation_dropout after
+ * the FFN GELU — element i of a site's [B*T, C] tensor keeps lane i % 4 of Philox4x32-10(seed, i / 4, site), exactly as
+ * avh_dropout.  layer_skip (HOST [encoder_layers], or NULL = no LayerDrop) holds the LayerDrop coins: a dropped layer is
+ * the identity, dx passes through it, and its 16 gradient tensors are zero in the flat buffer.  The backward
+ * (avh_encoder_backward*) uses the seed and coins of its forward and regenerates the masks.  Probabilities select the
+ * launch plan (and so its CUDA graphs), the seed and coins do not: a step replays its graphs for any seed and any set of
+ * dropped layers.  attention_dropout must be 0; bn_momentum is not read (avh_full_train_forward takes its own). */
+AVH_API int avh_set_train_args(avh_handle* h, const avh_train_args* args);
+
 /* The trainable tail of AVHubertModel.extract_finetune when the feature extractors are frozen (feature_grad_mult <= 0: the
  * reference runs them under no_grad, avhubert/hubert.py:538-547): fused [B,T,E] = the concatenated / summed extractor
  * outputs BEFORE the fusion LayerNorm (avh_read_stage "fused"), then layer_norm -> post_extract_proj -> index_put ->
@@ -223,9 +236,10 @@ AVH_API int avh_grad_bucket_wait(avh_handle* h, int k, void* stream);
  * gradient at the ENCODER input (post_extract_proj output).  AV-HuBERT handle created with reserved[3] = 1. */
 AVH_API int avh_tail_grad_count(avh_handle* h, int64_t* n_floats);
 AVH_API int avh_tail_train_forward(avh_handle* h, const void* fused, int dtype, const uint8_t* padding_mask, int B, int T,
-                                   void* out, int out_dtype, void* stream);
+                                   void* out, int out_dtype, void* stream);      /* regularisation: avh_set_train_args */
 
-/* The whole fine-tuning step (feature_grad_mult > 0, BASELINE config 5 as stated): lip ResNet (training-mode BatchNorm:
+/* The whole fine-tuning step (feature_grad_mult > 0, BASELINE config 5; dropout / LayerDrop: avh_set_train_args): lip
+ * ResNet (training-mode BatchNorm:
  * batch statistics, running statistics updated with bn_momentum — read them back with avh_read_bn_stats), modality
  * projections, fusion, encoder, with saved activations; avh_encoder_backward then also returns, after the tail's
  * gradients, those of the feature extractors (scaled by feature_grad_mult as fairseq's GradMultiply does,

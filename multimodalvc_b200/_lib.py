@@ -24,6 +24,7 @@ EXPORTS = [
     "avh_encoder_backward_buckets", "avh_grad_bucket_count", "avh_grad_bucket_range", "avh_grad_bucket_wait",
     "avh_refresh_weights_device",
     "avh_tail_grad_count", "avh_tail_train_forward", "avh_full_grad_count", "avh_full_train_forward",
+    "avh_set_train_args",
 ]
 
 
@@ -84,6 +85,7 @@ def load():
                                        i32, vp]
     lib.avh_forward_train.argtypes = [vp, vp, i32, vp, i32, ctypes.POINTER(i64), vp, i32, i32, i32, ctypes.POINTER(AvhTrainArgs),
                                       vp, i32, vp]
+    lib.avh_set_train_args.argtypes = [vp, ctypes.POINTER(AvhTrainArgs)]
     lib.avh_interp_linear.argtypes = [vp, i32, i32, i32, i32, vp, vp, i32, vp, vp, vp]
     lib.avh_encoder_grad_count.argtypes = [vp, ctypes.POINTER(i64)]
     lib.avh_tail_grad_count.argtypes = [vp, ctypes.POINTER(i64)]

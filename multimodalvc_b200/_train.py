@@ -5,11 +5,50 @@ soon as the library has recorded the bucket's event, so that the collective over
 (fairseq legacy_distributed_data_parallel.py:76-165 does the reduction after the backward; same result)."""
 import ctypes
 
+import numpy as np
 import torch
 
 from . import _lib
 
 _DTYPES = {torch.float32: _lib.AVH_F32, torch.float16: _lib.AVH_F16, torch.bfloat16: _lib.AVH_BF16}
+PARAMS_PER_LAYER = 16      # gradient tensors of one encoder layer, first in every training step's parameter list
+
+
+class StepRegularization:
+    """Dropout and LayerDrop of one training step (avh_set_train_args).  The LayerDrop coins are drawn here, one
+    np.random.random() per layer in layer order, as the reference draws them (wav2vec2.py:886-888) whatever the
+    probability; the dropout seed comes from torch's CPU generator, and only when some dropout probability is non-zero."""
+
+    def __init__(self, n_layers, dropout_input=0.0, dropout=0.0, activation_dropout=0.0, attention_dropout=0.0,
+                 layerdrop=0.0):
+        if float(attention_dropout or 0.0) != 0.0:
+            raise NotImplementedError("attention_dropout > 0 in training mode is not implemented (0.0 in every "
+                                      "shipped fine-tune config, avhubert/conf/finetune/*.yaml)")
+        self.p = (float(dropout_input or 0.0), float(dropout or 0.0), float(activation_dropout or 0.0))
+        self.layerdrop = float(layerdrop or 0.0)
+        self.skip = [0 if np.random.random() > self.layerdrop else 1 for _ in range(n_layers)]
+        if self.layerdrop <= 0.0:
+            self.skip = [0] * n_layers
+        self.seed = int(torch.randint(0, 2 ** 62, (1,)).item()) if any(p > 0.0 for p in self.p) else 0
+
+    def set_on(self, handle):
+        """Leaves the regularisation for the next training forward on `handle`."""
+        skip = (ctypes.c_uint8 * len(self.skip))(*self.skip) if self.layerdrop > 0.0 else None
+        ta = _lib.AvhTrainArgs(dropout_input=self.p[0], dropout=self.p[1], activation_dropout=self.p[2], attention_dropout=0.0,
+                               bn_momentum=0.1, seed=self.seed,
+                               layer_skip=ctypes.cast(skip, ctypes.c_void_p) if skip is not None else None)
+        _lib.check(_lib.load().avh_set_train_args(handle, ctypes.byref(ta)))
+
+    def layer_grads(self, grads, reduced):
+        """autograd's view of a dropped layer: its parameters took no part in the step, so their gradients are None —
+        unless the all-reducer has reduced the bucket, whose values (the other ranks' gradients) they then get."""
+        if reduced:
+            return grads
+        grads = list(grads)
+        for l, dropped in enumerate(self.skip):
+            if dropped:
+                grads[l * PARAMS_PER_LAYER:(l + 1) * PARAMS_PER_LAYER] = [None] * PARAMS_PER_LAYER
+        return grads
 
 
 def backward_flat(handle, dout, dx, n_floats, dtypes, fwd_stream, owner):

@@ -15,7 +15,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "_build")
 LIB = os.path.join(HERE, "libavh_b200.so")
-SOURCES = ["api.cu", "gemm_tcgen05.cu", "conv_window.cu", "conv_frame.cu", "stem_fused.cu", "attention.cu", "attention_tc.cu", "elementwise.cu", "train_ops.cu", "pretrain_ops.cu", "qformer.cu", "backward_ops.cu", "frontend_train.cu", "refresh.cu", "fbank.cu"]
+SOURCES = ["api.cu", "gemm_tcgen05.cu", "conv_window.cu", "conv_frame.cu", "stem_fused.cu", "attention.cu", "attention_tc.cu", "elementwise.cu", "train_ops.cu", "train_dropout.cu", "pretrain_ops.cu", "qformer.cu", "backward_ops.cu", "frontend_train.cu", "refresh.cu", "fbank.cu"]
 NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr",
               "-I", os.path.join(ROOT, "include"), "-I", CSRC]

@@ -163,6 +163,7 @@ struct Step {
   double flops = 0;       // executed tensor-core FLOPs (GEMM steps)
   int layer = -1;         // encoder layer the step belongs to (LayerDrop skips it in training mode), -1 = none
   bool direct = false;    // reads or writes a CALLER pointer (video, audio, features, output): never part of a CUDA graph
+  bool on_drop = false;   // runs only when its layer is dropped (the identity that stands in for the layer)
 };
 
 struct CallArgs {          // per-call pointers the steps read through the plan
@@ -210,10 +211,17 @@ struct PlanKey {
   long long ragged_rows = 0;      // Ragged: Nb
   int Lk = 0;                     // QFormer
   cudaStream_t stream = nullptr;
+  // training plans (avh_set_train_args): dropout_input (tail modes), dropout, activation_dropout, and whether the
+  // caller draws LayerDrop coins; all 0 / false: the launch list of a step without regularisation
+  float p_in = 0.f, p_enc = 0.f, p_act = 0.f;
+  bool layerdrop = false;
   bool training() const { return kind == PlanKind::EncoderTrain || kind == PlanKind::TailTrain || kind == PlanKind::FullTrain; }
+  bool dropout() const { return p_in > 0.f || p_enc > 0.f || p_act > 0.f; }
   bool operator<(const PlanKey& o) const {
-    return std::tie(kind, B, T, has_video, has_audio, has_mask, output_layer, ragged_rows, Lk, stream) <
-           std::tie(o.kind, o.B, o.T, o.has_video, o.has_audio, o.has_mask, o.output_layer, o.ragged_rows, o.Lk, o.stream);
+    return std::tie(kind, B, T, has_video, has_audio, has_mask, output_layer, ragged_rows, Lk, stream, p_in, p_enc, p_act,
+                    layerdrop) <
+           std::tie(o.kind, o.B, o.T, o.has_video, o.has_audio, o.has_mask, o.output_layer, o.ragged_rows, o.Lk, o.stream, o.p_in,
+                    o.p_enc, o.p_act, o.layerdrop);
   }
 };
 
@@ -241,6 +249,12 @@ struct Plan {
   struct GradBucket { long long begin, end; cudaEvent_t ev; };
   std::vector<GradBucket> buckets;
   int rag_next = 0;
+  // training plans with dropout: the seed of the current step in a device word the kernels read (captured graphs
+  // replay for any seed), written from pinned mirrors used round robin like rag_host
+  unsigned long long* seed_dev = nullptr;
+  unsigned long long* seed_host[RAG_SLOTS] = {nullptr, nullptr, nullptr, nullptr};
+  cudaEvent_t seed_done[RAG_SLOTS] = {nullptr, nullptr, nullptr, nullptr};
+  int seed_next = 0;
   int* pos_row_map = nullptr;
 
   Arena arena;
@@ -283,6 +297,8 @@ struct Plan {
     for (int i = 0; i < RAG_SLOTS; ++i) {
       if (rag_host[i]) cudaFreeHost(rag_host[i]);
       if (rag_done[i]) cudaEventDestroy(rag_done[i]);
+      if (seed_host[i]) cudaFreeHost(seed_host[i]);
+      if (seed_done[i]) cudaEventDestroy(seed_done[i]);
     }
     for (GradBucket& gb : buckets)
       if (gb.ev) cudaEventDestroy(gb.ev);
@@ -354,6 +370,13 @@ struct avh_handle {
   // raw-video geometry and normalisation for video_dtype == AVH_U8 (avh_set_video_preprocess)
   int vp_src_h = 88, vp_src_w = 88;
   double vp_mean = 0.421, vp_std = 0.165;
+  // avh_set_train_args: regularisation of the next training step on this handle, consumed by it
+  struct NextTrain {
+    float p_in = 0.f, p_enc = 0.f, p_act = 0.f;
+    unsigned long long seed = 0;
+    std::vector<unsigned char> skip;      // LayerDrop coins (1 = dropped); empty = LayerDrop off
+  };
+  NextTrain next_train;
 };
 
 namespace avh {
@@ -898,6 +921,11 @@ struct Builder {
   }
   void push_direct(const std::string& tag, std::function<int(cudaStream_t)> f, double flops = 0.0) {
     push(tag, std::move(f), flops, true);
+  }
+  // a step of layer cur_layer that runs only when LayerDrop drops that layer (launched directly, between the graphs
+  // of the layers around it)
+  void push_on_drop(const std::string& tag, std::function<int(cudaStream_t)> f) {
+    if (!sizing) plan->steps.push_back(Step{std::move(f), tag, 0.0, cur_layer, true, true});
   }
   // fp32 [rows, C] (row stride ld) -> GEMM-operand form (bf16 [rows, P*C])
   void split(const float* src, int ld, void* dst, long long rows, int C) {
@@ -1495,12 +1523,16 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
 }
 
 // ============================================================================ encoder training plan
-// TransformerEncoder forward with saved activations + its backward (pre-LN layers; dropout / LayerDrop 0 as BASELINE
-// config 5 states).  Forward: x0 = index_put(features, mask, 0); c = pos_conv(x0) + b; x1 = x0 + GELU(c); per layer
-// h1 = LN1(x); qkv = h1 Wqkv^T + b; ctx = Attn(qkv) (+ log-sum-exp per row); xm = x + ctx Wo^T + bo; h2 = LN2(xm);
-// u = h2 W1^T + b1; g = GELU(u); x' = xm + g W2^T + b2; y = LN(x_L).  Backward: the chain rule of exactly that graph
-// — every contraction on the tcgen05 GEMM (dX = dY W with W^T packed at finalisation; dW = dY^T X with both operands
-// transposed by transpose_split, K = tokens), the rest in backward_ops.cu.
+// TransformerEncoder forward with saved activations + its backward (pre-LN layers).  Forward: x0 = index_put(features,
+// mask, 0); c = pos_conv(x0) + b; x1 = m2 (x0 + GELU(c)); per layer h1 = LN1(x); qkv = h1 Wqkv^T + b; ctx = Attn(qkv)
+// (+ log-sum-exp per row); xm = x + m(16+4l) (ctx Wo^T + bo); h2 = LN2(xm); u = h2 W1^T + b1; g = m(17+4l) GELU(u);
+// x' = xm + m(18+4l) (g W2^T + b2); y = LN(x_L).  Tail modes: x0 = m1 post_extract_proj(LN(fused)) before the zeroing.
+// m_site = the dropout mask of that site (philox.cuh, p = key.p_in for site 1, p_act for 17+4l, p_enc otherwise; a
+// site with p = 0 is no mask and no launch).  A layer dropped by LayerDrop is the identity: its steps are skipped, an
+// on-drop step copies x into x' and zeroes the layer's gradients.  Backward: the chain rule of exactly that graph —
+// every contraction on the tcgen05 GEMM (dX = dY W with W^T packed at finalisation; dW = dY^T X with both operands
+// transposed by transpose_split, K = tokens), the rest in backward_ops.cu / train_dropout.cu, every mask regenerated
+// from (seed, site, element).
 // Gradient layout (fp32, `grad_floats` values), in this order — the Python mirror walks the same list:
 //   per layer l: [q,k,v]_proj.weight (3 x [D,D], contiguous), [q,k,v]_proj.bias (3 x [D]), out_proj.weight [D,D],
 //   out_proj.bias [D], self_attn_layer_norm.{weight,bias}, fc1.weight [F,D], fc1.bias [F], fc2.weight [D,F], fc2.bias [D],
@@ -1595,6 +1627,11 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
   const bool hm = key.has_mask;
   const int tail = key.kind == PlanKind::FullTrain ? 2 : (key.kind == PlanKind::TailTrain ? 1 : 0);
   const bool full = tail == 2;
+  const float p_in = key.p_in, p_enc = key.p_enc, p_act = key.p_act;
+  const bool ldrop = key.layerdrop;
+  unsigned long long* seed = key.dropout() ? reinterpret_cast<unsigned long long*>(b.alloc(16)) : nullptr;
+  if (!sizing) plan->seed_dev = seed;
+  float* dtmp = p_enc > 0.f ? b.f32buf(N * D) : nullptr;     // block output before dropout + residual; backward: m * dx
   // stream-K workspace for the lip ResNet's weight-gradient GEMMs (a handful of output tiles, K = pixels)
   if (!f32 && full) b.stream_k_workspace();
   const int E = c.modality_fuse == AVH_FUSE_CONCAT ? 2 * D : D;
@@ -1796,6 +1833,8 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
         return launch_layernorm(fused, DT_F32, E, gm, be, 1e-5f, x0, nullptr, DT_BF16, hm ? pl->mask_dev : nullptr, N, E, s);
       });
     }
+    if (p_in > 0.f)      // features = self.dropout_input(features), hubert.py:729
+      b.push("dropout", [=](cudaStream_t s) { return launch_dropout_residual(nullptr, x0, x0, N * D, p_in, seed, 1u, s); });
   } else {
     b.push_direct("load_features", [=](cudaStream_t s) {
       return launch_load_rows(pl->args.xin, pl->args.xin_dt, x0, hm ? pl->mask_dev : nullptr, N, D, s);
@@ -1815,12 +1854,26 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     ep.map_mode = MAP_2LEVEL; ep.S2 = Tp; ep.S1 = Tp; ep.H = 1; ep.W = T; ep.O2 = T; ep.O1 = 0; ep.O0 = 0;
     if (!b.gemm("pos_conv", xpad, pad_rows, P * D, h->pos_w, pad_rows, taps, win / 64, D, ep, 64, h->pos_acol)) return false;
     float* x1 = xin[0];
-    b.push("gelu", [=](cudaStream_t s) { return launch_gelu_fwd(cpre, DT_F32, x0, x1, DT_F32, N * D, s); });
+    if (p_enc > 0.f)     // x = F.dropout(x + GELU(conv(x))), wav2vec2.py:879
+      b.push("gelu", [=](cudaStream_t s) { return launch_masked_gelu(cpre, DT_F32, x0, x1, DT_F32, N * D, p_enc, seed, 2u, s); });
+    else
+      b.push("gelu", [=](cudaStream_t s) { return launch_gelu_fwd(cpre, DT_F32, x0, x1, DT_F32, N * D, s); });
   }
   for (int l = 0; l < L; ++l) {
     const LayerW& lw = h->layers[l];
     b.cur_layer = l;
     float* x = xin[l];
+    if (ldrop) {
+      float* xn = xin[l + 1];
+      b.push_on_drop("layerdrop", [=](cudaStream_t s) {
+        return cudaMemcpyAsync(xn, x, (size_t)N * D * 4, cudaMemcpyDeviceToDevice, s) == cudaSuccess ? 0 : 1;
+      });
+    }
+    const unsigned site = 16u + 4u * (unsigned)l;
+    // block output + bias into dtmp, then target = res + m * dtmp (dropout1 / dropout3, wav2vec2.py:980,990)
+    auto block_dropout = [&](const float* res, float* target, unsigned st) {
+      b.push("dropout", [=](cudaStream_t s) { return launch_dropout_residual(res, dtmp, target, N * D, p_enc, seed, st, s); });
+    };
     b.layernorm("layer_ln", x, DT_F32, lw.ln1_g, lw.ln1_b, 1e-5f, h1[l]);
     {
       Epilogue ep = epilogue(qkv[l].data, 3 * D, f32);
@@ -1837,7 +1890,12 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       });
       b.sync_op(ctx[l]);
     }
-    {
+    if (p_enc > 0.f) {
+      Epilogue ep = epilogue(dtmp, D, true);
+      ep.col_bias = lw.out.bias;
+      if (!b.linear("out_proj", ctx[l].op, N, D, lw.out.w, ep)) return false;
+      block_dropout(x, xmid[l], site);
+    } else {
       Epilogue ep = epilogue(xmid[l], D, true);
       ep.col_bias = lw.out.bias; ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
       if (!b.linear("out_proj", ctx[l].op, N, D, lw.out.w, ep)) return false;
@@ -1848,10 +1906,20 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       ep.col_bias = lw.fc1.bias;
       if (!b.linear("fc1", h2[l].op, N, D, lw.fc1.w, ep)) return false;
       const void* uu = u[l].data; void* gg = g[l].data;
-      b.push("gelu", [=](cudaStream_t s) { return launch_gelu_fwd(uu, act_dt, nullptr, gg, act_dt, N * F, s); });
+      if (p_act > 0.f)   // dropout2 = activation_dropout after the GELU, wav2vec2.py:987
+        b.push("gelu", [=](cudaStream_t s) {
+          return launch_masked_gelu(uu, act_dt, nullptr, gg, act_dt, N * F, p_act, seed, site + 1u, s);
+        });
+      else
+        b.push("gelu", [=](cudaStream_t s) { return launch_gelu_fwd(uu, act_dt, nullptr, gg, act_dt, N * F, s); });
       b.sync_op(g[l]);
     }
-    {
+    if (p_enc > 0.f) {
+      Epilogue ep = epilogue(dtmp, D, true);
+      ep.col_bias = lw.fc2.bias;
+      if (!b.linear("fc2", g[l].op, N, F, lw.fc2.w, ep)) return false;
+      block_dropout(xmid[l], xin[l + 1], site + 2u);
+    } else {
       Epilogue ep = epilogue(xin[l + 1], D, true);
       ep.col_bias = lw.fc2.bias; ep.R = xmid[l]; ep.ldr = D; ep.r_fp32 = 1;
       if (!b.linear("fc2", g[l].op, N, F, lw.fc2.w, ep)) return false;
@@ -1922,13 +1990,39 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     float* g_fc2_w = g_fc1_b + F;                // [D, F]
     float* g_fc2_b = g_fc2_w + (long long)D * F;
     float* g_ln2 = g_fc2_b + D;
-    // ---- fc2: x' = xm + g W2^T + b2
-    if (!wgrad(dx, DT_F32, D, g[l].data, act_dt, F, g_fc2_w, g_fc2_b, "fc2_wgrad")) return false;
-    b.split(dx, D, dxa.op, N, D);
+    const unsigned site = 16u + 4u * (unsigned)l;
+    if (ldrop)      // a dropped layer passes dx through unchanged; its parameters get zero gradients
+      b.push_on_drop("layerdrop", [=](cudaStream_t s) {
+        return cudaMemsetAsync(gl, 0, (size_t)LG * 4, s) == cudaSuccess ? 0 : 1;
+      });
+    // gradient of a block output behind a dropout: dtmp = m * dy and its operand form, or (p = 0) dy and its split
+    auto block_grad = [&](float* dyv, unsigned st) -> float* {
+      if (p_enc <= 0.f) {
+        b.split(dyv, D, dxa.op, N, D);
+        return dyv;
+      }
+      void* op = dxa.op;
+      const int planes = P;
+      b.push("dropout_bwd", [=](cudaStream_t s) { return launch_dropout_grad(dyv, dtmp, op, planes, N, D, p_enc, seed, st, s); });
+      return dtmp;
+    };
+    // ---- fc2: x' = xm + m (g W2^T + b2)
+    if (p_enc > 0.f) {
+      float* d3 = block_grad(dx, site + 2u);
+      if (!wgrad(d3, DT_F32, D, g[l].data, act_dt, F, g_fc2_w, g_fc2_b, "fc2_wgrad")) return false;
+    } else {
+      if (!wgrad(dx, DT_F32, D, g[l].data, act_dt, F, g_fc2_w, g_fc2_b, "fc2_wgrad")) return false;
+      block_grad(dx, site + 2u);
+    }
     if (!dgrad(dxa.op, D, lw.fc2T, dga.data, f32, "fc2_dgrad")) return false;
     {
       const void* uu = u[l].data; const void* dgv = dga.data; void* duv = dua.data;
-      b.push("gelu_bwd", [=](cudaStream_t s) { return launch_gelu_bwd(uu, act_dt, dgv, act_dt, duv, act_dt, N * F, s); });
+      if (p_act > 0.f)
+        b.push("gelu_bwd", [=](cudaStream_t s) {
+          return launch_masked_gelu_bwd(uu, act_dt, dgv, act_dt, duv, act_dt, N * F, p_act, seed, site + 1u, s);
+        });
+      else
+        b.push("gelu_bwd", [=](cudaStream_t s) { return launch_gelu_bwd(uu, act_dt, dgv, act_dt, duv, act_dt, N * F, s); });
       b.sync_op(dua);
     }
     // ---- fc1: u = h2 W1^T + b1
@@ -1938,9 +2032,14 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       float* xm = xmid[l]; float* gm = lw.ln2_g;
       b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(xm, gm, dh, dx, dxm, stats, g_ln2, g_ln2 + D, N, D, 1e-5f, s); });
     }
-    // ---- out_proj: xm = x + ctx Wo^T + bo
-    if (!wgrad(dxm, DT_F32, D, ctx[l].data, act_dt, D, g_out_w, g_out_b, "out_wgrad")) return false;
-    b.split(dxm, D, dxa.op, N, D);
+    // ---- out_proj: xm = x + m (ctx Wo^T + bo)
+    if (p_enc > 0.f) {
+      float* d1 = block_grad(dxm, site);
+      if (!wgrad(d1, DT_F32, D, ctx[l].data, act_dt, D, g_out_w, g_out_b, "out_wgrad")) return false;
+    } else {
+      if (!wgrad(dxm, DT_F32, D, ctx[l].data, act_dt, D, g_out_w, g_out_b, "out_wgrad")) return false;
+      block_grad(dxm, site);
+    }
     if (!dgrad(dxa.op, D, lw.outT, dctx.data, f32, "out_dgrad")) return false;
     {   // attention
       const char* q = reinterpret_cast<const char*>(qkv[l].data);
@@ -1973,9 +2072,11 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     }
   }
   b.cur_layer = -1;
-  // ---- positional conv block: x1 = x0 + GELU(c), c = conv(x0) + bias  (pos-conv weight gradients: see posconv_bwd)
+  // ---- positional conv block: x1 = m2 (x0 + GELU(c)), c = conv(x0) + bias  (pos-conv weight gradients: see posconv_bwd)
   {
     float* gpos = grads + (long long)L * LG + 2ll * D;       // bias [D], weight_g [KT], weight_v [D, D/G, KT]
+    if (p_enc > 0.f)     // dx = m2 dL/dx1 in place: the gradient of both the residual and the GELU input
+      b.push("dropout_bwd", [=](cudaStream_t s) { return launch_dropout_grad(dx, dx, nullptr, 1, N, D, p_enc, seed, 2u, s); });
     float* dc = dh;                                          // dL/dc = dx * GELU'(c)
     b.push("gelu_bwd", [=](cudaStream_t s) { return launch_gelu_bwd(cpre, DT_F32, dx, DT_F32, dc, DT_F32, N * D, s); });
     b.push("bias_grad", [=](cudaStream_t s) { return launch_colsum(dc, DT_F32, D, N, D, gpos, 1.0f, s); });
@@ -1994,16 +2095,22 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     // weight gradients of the grouped convolution + weight-norm backward
     if (!posconv_wgrad(b, h, dc, x0, N, B, T, gpos + D, gpos + D + KT)) return false;
     if (tail) {
-      // dxo = dL/dx0 (rows of padded frames already zero).  post_extract_proj: x0 = fln Wp^T + bp; then the fusion LayerNorm
-      // (its input comes from the frozen extractors: only dgamma / dbeta are needed)
+      // dxo = dL/dx0 (rows of padded frames already zero).  post_extract_proj: x0 = m1 (fln Wp^T + bp); then the fusion
+      // LayerNorm (its input comes from the frozen extractors: only dgamma / dbeta are needed)
       float* gt = gpos + D + KT + (long long)D * (D / c.conv_pos_groups) * KT;
       float* dfl = nullptr;
       float* g_ln = gt;
-      if (h->has_post_proj) {
+      const bool pp = h->has_post_proj;
+      if (p_in > 0.f) {  // dxo = m1 dxo in place (+ the operand form post_extract_proj's dgrad reads)
+        void* op = pp ? dxa.op : nullptr;
+        const int planes = P;
+        b.push("dropout_bwd", [=](cudaStream_t s) { return launch_dropout_grad(dxo, dxo, op, planes, N, D, p_in, seed, 1u, s); });
+      }
+      if (pp) {
         float* g_pw = gt; float* g_pb = gt + (long long)D * E;
         g_ln = g_pb + D;
         if (!wgrad(dxo, DT_F32, D, fln.data, act_dt, E, g_pw, g_pb, "post_proj_wgrad")) return false;
-        b.split(dxo, D, dxa.op, N, D);
+        if (p_in <= 0.f) b.split(dxo, D, dxa.op, N, D);
         dfl = b.f32buf(N * E);
         if (!dgrad(dxa.op, D, h->post_projT, dfl, true, "post_proj_dgrad")) return false;
       } else {
@@ -2416,6 +2523,15 @@ Plan* get_plan(avh_handle* h, const PlanKey& key) {
       }
     }
   }
+  if (p->seed_dev != nullptr) {
+    for (int i = 0; i < Plan::RAG_SLOTS; ++i) {
+      if (cudaMallocHost(reinterpret_cast<void**>(&p->seed_host[i]), sizeof(unsigned long long)) != cudaSuccess ||
+          cudaEventCreateWithFlags(&p->seed_done[i], cudaEventDisableTiming) != cudaSuccess) {
+        set_last_error("pinned seed allocation failed");
+        return nullptr;
+      }
+    }
+  }
   Plan* raw = p.get();
   h->plans[key] = std::move(p);
   return raw;
@@ -2563,14 +2679,23 @@ static void read_graphs_env() {
   graphs_env = ((ev != nullptr && ev[0] == '0') || dbg != nullptr || dbg2 != nullptr) ? 0 : 1;
 }
 
-// capture every maximal run of plan-internal steps (they only enqueue kernels / async copies) into its own graph
+// LayerDrop: a step of a dropped layer is skipped and an on-drop step of a kept one; steps outside the layers always run
+// (plans without LayerDrop have an empty layer_skip)
+static bool step_runs(const avh::Plan* p, const avh::Step& st) {
+  const bool dropped = st.layer >= 0 && st.layer < (int)p->layer_skip.size() && p->layer_skip[st.layer] != 0;
+  return dropped == st.on_drop;
+}
+
+// capture every maximal run of plan-internal steps (they only enqueue kernels / async copies) into its own graph; in a
+// plan with LayerDrop a run also ends where the layer changes, so that a dropped layer's graphs are skipped whole
 static bool capture_segments(avh::Plan* p, cudaStream_t s) {
   bool ok = true;
   size_t i = 0;
+  const bool by_layer = p->key.layerdrop;
   while (ok && i < p->steps.size()) {
     if (p->steps[i].direct) { ++i; continue; }
     size_t j = i;
-    while (j < p->steps.size() && !p->steps[j].direct) ++j;
+    while (j < p->steps.size() && !p->steps[j].direct && (!by_layer || p->steps[j].layer == p->steps[i].layer)) ++j;
     const long long before = avh::g_launches.load();
     cudaGraph_t graph = nullptr;
     ok = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
@@ -2604,13 +2729,15 @@ static int replay_range(avh::Plan* p, size_t begin, size_t end, cudaStream_t s) 
   while (sg < p->segments.size() && p->segments[sg].begin < begin) ++sg;
   while (i < end) {
     if (sg < p->segments.size() && p->segments[sg].begin == i && p->segments[sg].end <= end) {
-      AVH_CUDA_OK(cudaGraphLaunch(p->segments[sg].exec, s));
-      avh::count_launch(p->segments[sg].kernels);
-      avh::g_graph_launches.fetch_add(1, std::memory_order_relaxed);
+      if (step_runs(p, p->steps[i])) {      // a segment holds the steps of one layer when LayerDrop is possible
+        AVH_CUDA_OK(cudaGraphLaunch(p->segments[sg].exec, s));
+        avh::count_launch(p->segments[sg].kernels);
+        avh::g_graph_launches.fetch_add(1, std::memory_order_relaxed);
+      }
       i = p->segments[sg].end;
       ++sg;
     } else {
-      if (p->steps[i].run(s)) {
+      if (step_runs(p, p->steps[i]) && p->steps[i].run(s)) {
         if (avh::g_err.empty()) avh::set_last_error("kernel launch failed");
         return 1;
       }
@@ -2623,8 +2750,9 @@ static int replay_range(avh::Plan* p, size_t begin, size_t end, cudaStream_t s) 
 // Steps [begin, end) of a plan: a whole forward, or the forward or backward half of a training plan.  The first run of
 // a plan launches its steps directly (it also configures the kernels); the second captures every maximal run of
 // plan-internal steps into a CUDA graph, later runs replay them (in a training plan the direct final-LayerNorm store
-// separates the forward from the backward, so no graph straddles the two ranges).  Training-mode forwards (LayerDrop,
-// per-call dropout) and profiled forwards always launch directly.
+// separates the forward from the backward, so no graph straddles the two ranges).  The no-grad training-mode forward
+// (its dropout seed is a launch argument) and profiled forwards always launch directly.  LayerDrop (step_runs) holds for
+// every plan that has coins: direct runs and replays skip a dropped layer's steps alike.
 static int run_steps(avh_handle* h, avh::Plan* p, size_t begin, size_t end, cudaStream_t s) {
   read_graphs_env();
   const avh::PlanKey& key = p->key;
@@ -2652,8 +2780,7 @@ static int run_steps(avh_handle* h, avh::Plan* p, size_t begin, size_t end, cuda
   for (size_t i = begin; i < end; ++i) {
     const avh::Step& st = p->steps[i];
     if (profiled) cudaEventRecord(h->prof_events[2 * i], s);
-    const bool dropped = train_fwd && st.layer >= 0 && st.layer < (int)p->layer_skip.size() && p->layer_skip[st.layer] != 0;
-    if (!dropped && st.run(s)) {
+    if (step_runs(p, st) && st.run(s)) {
       if (avh::g_err.empty()) avh::set_last_error("kernel launch failed");
       return 1;
     }
@@ -2897,6 +3024,49 @@ int avh_encoder_grad_count(avh_handle* h, int64_t* n_floats) {
 static int encoder_train_forward(avh_handle* h, const void* x, int x_dtype, const uint8_t* padding_mask, int B, int T, void* out,
                                  int out_dtype, void* stream, bool tail);
 
+int avh_set_train_args(avh_handle* h, const avh_train_args* ta) {
+  AVH_CHECK(h != nullptr && ta != nullptr, "null argument");
+  AVH_CHECK(ta->attention_dropout == 0.f, "attention_dropout > 0 is not implemented (0.0 in every shipped fine-tune config)");
+  for (float pr : {ta->dropout_input, ta->dropout, ta->activation_dropout})
+    AVH_CHECK(pr >= 0.f && pr < 1.f, "dropout probabilities must be in [0, 1)");
+  avh_handle::NextTrain nt;
+  nt.p_in = ta->dropout_input; nt.p_enc = ta->dropout; nt.p_act = ta->activation_dropout;
+  nt.seed = ta->seed;
+  if (ta->layer_skip != nullptr) nt.skip.assign(ta->layer_skip, ta->layer_skip + h->cfg.encoder_layers);
+  h->next_train = std::move(nt);
+  return 0;
+}
+
+// The plan of a training step with the regularisation avh_set_train_args left for it (consumed here; none: a plain
+// step): probabilities and "LayerDrop possible" select the plan, the seed goes to its device word and the coins to its
+// layer_skip, which the backward of this step reads too.  site1: the plan has dropout_input (tail modes).
+static avh::Plan* training_plan(avh_handle* h, avh::PlanKey key, bool site1, cudaStream_t s) {
+  avh_handle::NextTrain nt = std::move(h->next_train);
+  h->next_train = avh_handle::NextTrain();
+  key.p_in = site1 ? nt.p_in : 0.f;
+  key.p_enc = nt.p_enc;
+  key.p_act = nt.p_act;
+  key.layerdrop = !nt.skip.empty();
+  avh::Plan* p = avh::get_plan(h, key);
+  if (p == nullptr) return nullptr;
+  p->layer_skip = std::move(nt.skip);
+  if (p->seed_dev != nullptr) {
+    const int slot = p->seed_next;
+    p->seed_next = (slot + 1) % avh::Plan::RAG_SLOTS;
+    cudaError_t e = cudaEventSynchronize(p->seed_done[slot]);      // the copy that last read this mirror has run
+    if (e == cudaSuccess) {
+      *p->seed_host[slot] = nt.seed;
+      e = cudaMemcpyAsync(p->seed_dev, p->seed_host[slot], sizeof(unsigned long long), cudaMemcpyHostToDevice, s);
+    }
+    if (e == cudaSuccess) e = cudaEventRecord(p->seed_done[slot], s);
+    if (e != cudaSuccess) {
+      avh::set_last_error(std::string("dropout seed upload failed: ") + cudaGetErrorString(e));
+      return nullptr;
+    }
+  }
+  return p;
+}
+
 int avh_tail_grad_count(avh_handle* h, int64_t* n_floats) {
   AVH_CHECK(h != nullptr && n_floats != nullptr, "null argument");
   AVH_CHECK(h->cfg.reserved[0] == 0, "the trainable tail belongs to an AV-HuBERT handle");
@@ -2942,7 +3112,7 @@ int avh_full_train_forward(avh_handle* h, const void* video, int video_dtype, co
   key.B = B; key.T = T;
   key.has_video = video != nullptr; key.has_audio = audio != nullptr; key.has_mask = padding_mask != nullptr;
   key.stream = s;
-  avh::Plan* p = avh::get_plan(h, key);
+  avh::Plan* p = training_plan(h, key, true, s);
   if (p == nullptr) return 1;
   h->last_plan = p;
   p->args = avh::CallArgs();
@@ -2975,7 +3145,7 @@ static int encoder_train_forward(avh_handle* h, const void* x, int x_dtype, cons
   key.B = B; key.T = T;
   key.has_mask = padding_mask != nullptr;
   key.stream = s;
-  avh::Plan* p = avh::get_plan(h, key);
+  avh::Plan* p = training_plan(h, key, tail, s);
   if (p == nullptr) return 1;
   h->last_plan = p;
   p->args = avh::CallArgs();

@@ -80,6 +80,20 @@ int launch_bn_apply(const void* raw, void* out, int dt, long long rows, int C, c
 // x = dropout(x) in place (any dtype), or x += dropout(add) (fp32); mask = Philox4x32-10(seed, site, element)
 int launch_dropout(void* x, int dt, const float* add, long long n, float p, unsigned long long seed, unsigned int site,
                    cudaStream_t stream);
+// ---- dropout of the training step (train_dropout.cu): the same masks, the seed read from DEVICE memory (`seed`),
+// 0 < p < 1, n and C multiples of 4; dtypes fp32 / bf16
+// out = m * ((res ? res : 0) + gelu(u))
+int launch_masked_gelu(const void* u, int u_dt, const float* res, void* out, int out_dt, long long n, float p,
+                       const unsigned long long* seed, unsigned int site, cudaStream_t stream);
+// y = (r ? r : 0) + m * a (fp32; y may alias a)
+int launch_dropout_residual(const float* r, const float* a, float* y, long long n, float p, const unsigned long long* seed,
+                            unsigned int site, cudaStream_t stream);
+// du = m * dg * gelu'(u)
+int launch_masked_gelu_bwd(const void* u, int u_dt, const void* dg, int dg_dt, void* du, int du_dt, long long n, float p,
+                           const unsigned long long* seed, unsigned int site, cudaStream_t stream);
+// out = m * dx over [rows, C] fp32 (out may alias dx); op != null: also its GEMM operand form (bf16 [rows, planes * C])
+int launch_dropout_grad(const float* dx, float* out, void* op, int planes, long long rows, int C, float p,
+                        const unsigned long long* seed, unsigned int site, cudaStream_t stream);
 
 // ---- pretraining-mode extras (pretrain_ops.cu): span-mask substitution, masked-prediction logits, features_pen
 // out unit u ([units, U] contiguous) = in unit code[u] (>= 0) | own (-1) | zeros (-2) | emb (-3); chan_zero [units / T, U]

@@ -14,6 +14,7 @@
 // LayerDrop (wav2vec2.py:887-888) is a host coin: the plan skips the layer's launches.
 #include "common.cuh"
 #include "kernels.h"
+#include "philox.cuh"
 
 #include <cuda_fp16.h>
 
@@ -196,23 +197,6 @@ bn_apply_kernel(const void* __restrict__ raw, void* __restrict__ out, int dt, lo
     for (int k = 0; k < 8; ++k) st_any(out, dt, i0 + k, v[k]);
   }
 }
-
-// ---- Philox4x32-10 (Salmon et al.): counter = (element block, site), key = seed
-__device__ __forceinline__ uint4 philox4x32(unsigned long long seed, unsigned long long ctr_lo, unsigned int site) {
-  unsigned int k0 = (unsigned int)seed, k1 = (unsigned int)(seed >> 32);
-  unsigned int c0 = (unsigned int)ctr_lo, c1 = (unsigned int)(ctr_lo >> 32), c2 = site, c3 = 0x5eedu;
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const unsigned int hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
-    const unsigned int hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
-    const unsigned int n0 = hi1 ^ c1 ^ k0, n1 = lo1, n2 = hi0 ^ c3 ^ k1, n3 = lo0;
-    c0 = n0; c1 = n1; c2 = n2; c3 = n3;
-    k0 += 0x9E3779B9u;
-    k1 += 0xBB67AE85u;
-  }
-  return make_uint4(c0, c1, c2, c3);
-}
-__device__ __forceinline__ float u01(unsigned int x) { return (float)(x >> 8) * (1.0f / 16777216.0f); }
 
 // x = dropout(x) in place, or x += dropout(t) when `add` is given (dropout1 / dropout3 before the residual add)
 __global__ void dropout_kernel(void* __restrict__ x, int dt, const float* __restrict__ add, long long n, float p,

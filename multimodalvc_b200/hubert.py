@@ -19,7 +19,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib, masking
-from ._train import backward_flat, refresh_weights_device
+from ._train import StepRegularization, backward_flat, refresh_weights_device
 
 _DTYPES = {torch.float32: _lib.AVH_F32, torch.float16: _lib.AVH_F16, torch.bfloat16: _lib.AVH_BF16}
 _U8 = _lib.AVH_U8        # raw uint8 video frames (normalised + centre-cropped on the device)
@@ -195,7 +195,7 @@ class _TailTrainFn(torch.autograd.Function):
     backward; the parameters are arguments only so that autograd routes their gradients."""
 
     @staticmethod
-    def forward(ctx, model, fused, pm_u8, *params):
+    def forward(ctx, model, reg, fused, pm_u8, *params):
         handle = model._ensure_handle()
         dev = fused.device
         B, T, _ = fused.shape
@@ -206,11 +206,12 @@ class _TailTrainFn(torch.autograd.Function):
         fused = fused.contiguous()
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
+            reg.set_on(handle)
             _lib.check(_lib.load().avh_tail_train_forward(
                 handle, ctypes.c_void_p(fused.data_ptr()), _DTYPES[fused.dtype],
                 ctypes.c_void_p(pm_u8.data_ptr()) if pm_u8 is not None else None, B, T,
                 ctypes.c_void_p(out.data_ptr()), _DTYPES[out_dtype], ctypes.c_void_p(stream)))
-        ctx.handle, ctx.stream, ctx.model, ctx.params = handle, stream, model, params
+        ctx.handle, ctx.stream, ctx.model, ctx.params, ctx.reg = handle, stream, model, params, reg
         ctx.shapes = [tuple(p.shape) for p in params]
         ctx.dtypes = [p.dtype for p in params]
         return out
@@ -235,7 +236,7 @@ class _TailTrainFn(torch.autograd.Function):
         assert off == n.value
         if flat.reduced:
             ctx.model._grad_sync.mark_reduced(ctx.params)
-        return (None, None, None, *grads)
+        return (None, None, None, None, *ctx.reg.layer_grads(grads, flat.reduced))
 
 
 class _FullTrainFn(torch.autograd.Function):
@@ -244,7 +245,7 @@ class _FullTrainFn(torch.autograd.Function):
     gradient buffer maps onto the parameters that follow."""
 
     @staticmethod
-    def forward(ctx, model, video, audio, pm_u8, fgm, spec, *params):
+    def forward(ctx, model, reg, video, audio, pm_u8, fgm, spec, *params):
         handle = model._ensure_handle()
         ref = video if video is not None else audio
         dev = ref.device
@@ -257,12 +258,13 @@ class _FullTrainFn(torch.autograd.Function):
         vp = ctypes.c_void_p
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
+            reg.set_on(handle)
             _lib.check(_lib.load().avh_full_train_forward(
                 handle, vp(video.data_ptr()) if video is not None else None, _DTYPES[video.dtype] if video is not None else 0,
                 vp(audio.data_ptr()) if audio is not None else None, _DTYPES[audio.dtype] if audio is not None else 0, strides,
                 vp(pm_u8.data_ptr()) if pm_u8 is not None else None, B, T, float(fgm), 0.1, vp(out.data_ptr()),
                 _DTYPES[out_dtype], vp(stream)))
-        ctx.handle, ctx.stream, ctx.spec = handle, stream, spec
+        ctx.handle, ctx.stream, ctx.spec, ctx.reg = handle, stream, spec, reg
         ctx.model, ctx.params = model, params
         ctx.flags = (int(video is not None), int(audio is not None))
         ctx.keep = (video, audio)                      # the backward re-reads the frames (stem patches are recomputed)
@@ -289,7 +291,7 @@ class _FullTrainFn(torch.autograd.Function):
         assert off == n.value, (off, n.value)
         if flat.reduced:
             ctx.model._grad_sync.mark_reduced(ctx.params)
-        return (None, None, None, None, None, None, *grads)
+        return (None, None, None, None, None, None, None, *ctx.reg.layer_grads(grads, flat.reduced))
 
 
 class AVHubertModel(nn.Module):
@@ -484,12 +486,18 @@ class AVHubertModel(nn.Module):
                     out.append(blk.downsample[1])
         return out
 
-    def _train_args(self, output_layer):
+    def _train_args(self, output_layer, regularise=True):
         """Per-call arguments of the training-mode forward: dropout probabilities of the config, a seed from torch's
         CPU generator, and the LayerDrop coins — drawn with np.random.random() in layer order up to the exit layer,
-        exactly as the reference does (wav2vec2.py:886-888), so the same numpy seed drops the same layers."""
+        exactly as the reference does (wav2vec2.py:886-888), so the same numpy seed drops the same layers.
+        regularise=False: no dropout, no layer dropped, nothing drawn (a pass that only reads an early stage)."""
         import numpy as np
         c = self.cfg
+        if not regularise:
+            skip_arr = (ctypes.c_uint8 * c.encoder_layers)()
+            ta = _lib.AvhTrainArgs(dropout_input=0.0, dropout=0.0, activation_dropout=0.0, attention_dropout=0.0,
+                                   bn_momentum=0.1, seed=0, layer_skip=ctypes.cast(skip_arr, ctypes.c_void_p))
+            return ta, skip_arr, [0] * c.encoder_layers
         if c.attention_dropout > 0:
             raise NotImplementedError("attention_dropout > 0 in training mode is not implemented (0.0 in every "
                                       "shipped fine-tune config, avhubert/conf/finetune/*.yaml)")
@@ -614,6 +622,12 @@ class AVHubertModel(nn.Module):
                     cin = C
         return params, spec
 
+    def _step_regularization(self):
+        c = self.cfg
+        return StepRegularization(c.encoder_layers, dropout_input=c.dropout_input, dropout=c.dropout,
+                                  activation_dropout=c.activation_dropout, attention_dropout=c.attention_dropout,
+                                  layerdrop=c.encoder_layerdrop)
+
     def _extract_finetune_full(self, source, padding_mask, mask):
         """The whole model differentiable (feature_grad_mult > 0, hubert.py:538-547 with GradMultiply): SURVEY row A18 /
         BASELINE config 5 as stated."""
@@ -631,7 +645,9 @@ class AVHubertModel(nn.Module):
         if video is not None and video_dt == _U8:
             raise NotImplementedError("the training step takes normalised float video")
         params, spec = self.full_parameters(video is not None, audio is not None)
-        y = _FullTrainFn.apply(self, video, audio, pm_u8, float(c.feature_grad_mult), spec, *params)
+        reg = self._step_regularization()
+        y = _FullTrainFn.apply(self, reg, video, audio, pm_u8, float(c.feature_grad_mult), spec, *params)
+        self._last_train_args = (reg.seed, list(reg.skip))      # what the step used: tests rebuild its masks from it
         if video is not None:
             self._read_back_bn_stats(handle, dev)
         return y, pm
@@ -665,20 +681,24 @@ class AVHubertModel(nn.Module):
             raise NotImplementedError("the training step runs the whole encoder (output_layer=None)")
         if not c.layer_norm_first:
             raise NotImplementedError("the device backward is built for pre-LN layers (layer_norm_first=True)")
-        for name in ("dropout_input", "dropout", "activation_dropout", "attention_dropout", "encoder_layerdrop"):
-            if float(getattr(c, name)) != 0.0:
-                raise NotImplementedError(f"{name} must be 0 for the device training step (BASELINE config 5)")
+        if c.attention_dropout > 0:
+            raise NotImplementedError("attention_dropout > 0 in training mode is not implemented (0.0 in every "
+                                      "shipped fine-tune config, avhubert/conf/finetune/*.yaml)")
         if c.feature_grad_mult > 0:
             return self._extract_finetune_full(source, padding_mask, mask)
         self._sync_trained_weights()                             # an optimizer step changed the weights: refresh
         with torch.no_grad():
-            y1, pm = self._extract_finetune_nograd(source, padding_mask, mask=mask, output_layer=1)
+            # only the "fused" stage is read: no regularisation and no draws, so the step draws its coins once
+            y1, pm = self._extract_finetune_nograd(source, padding_mask, mask=mask, output_layer=1, _regularise=False)
             B, T, _ = y1.shape
             fused = self.read_stage("fused", B * T * self.embed).view(B, T, self.embed)
         self._param_versions = [p._version for p in self.parameters()]
         dev = fused.device
         pm_u8 = pm.to(device=dev, dtype=torch.bool).contiguous().view(torch.uint8) if pm is not None else None
-        return _TailTrainFn.apply(self, fused, pm_u8, *self.tail_parameters()), pm
+        reg = self._step_regularization()
+        y = _TailTrainFn.apply(self, reg, fused, pm_u8, *self.tail_parameters())
+        self._last_train_args = (reg.seed, list(reg.skip))      # what the step used: tests rebuild its masks from it
+        return y, pm
 
     def extract_finetune(self, source, padding_mask=None, mask=False, ret_conv=False, output_layer=None, lengths=None):
         """avhubert/hubert.py:694-745 (see _extract_finetune_nograd).  In .train() with gradients enabled and
@@ -690,7 +710,8 @@ class AVHubertModel(nn.Module):
                                              lengths=lengths)
 
     @torch.no_grad()
-    def _extract_finetune_nograd(self, source, padding_mask=None, mask=False, ret_conv=False, output_layer=None, lengths=None):
+    def _extract_finetune_nograd(self, source, padding_mask=None, mask=False, ret_conv=False, output_layer=None, lengths=None,
+                                 _regularise=True):
         """avhubert/hubert.py:694-745.  source = {'audio': [B,F,T] | None, 'video': [B,1,T,88,88] | None};
         padding_mask bool [B,T] (True = padded).  Returns (x [B,T,D], padding_mask).  With cfg.ragged == "packed" (bf16
         mode) ragged batches run packed; `lengths` (valid frames per clip) may be given to skip reading the mask back."""
@@ -719,7 +740,7 @@ class AVHubertModel(nn.Module):
             # frozen-encoder-in-train-mode forward (src/model.py:96-100,280): batch-statistics BatchNorm, dropout, LayerDrop
             if video_dt == _U8:
                 raise NotImplementedError("the training-mode forward takes normalised float video")
-            ta, skip_arr, _ = self._train_args(output_layer)
+            ta, skip_arr, _ = self._train_args(output_layer, regularise=_regularise)
             lib = _lib.load()
             with torch.cuda.device(dev):
                 stream = torch.cuda.current_stream(dev).cuda_stream

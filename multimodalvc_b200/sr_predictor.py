@@ -11,8 +11,9 @@
 Inference by default (eval mode: LayerDrop and dropout are identity, as in the reference's ``self.training`` gates).
 ``TransformerEncoder(args, trainable=True)`` also differentiates: in ``.train()`` with gradients enabled ``forward`` is a
 ``torch.autograd.Function`` whose backward is the library's (``avh_encoder_train_forward`` / ``avh_encoder_backward``:
-SURVEY row A18, encoder part of BASELINE config 5 — dropout / LayerDrop must be 0, pre-LN layers), so ``loss.backward()``
-fills ``.grad`` of the input and of every encoder parameter.  No CPU path.
+SURVEY row A18, encoder part of BASELINE config 5; pre-LN layers; ``dropout``, ``activation_dropout`` and
+``encoder_layerdrop`` of the args as the reference applies them, ``attention_dropout`` must be 0), so ``loss.backward()``
+fills ``.grad`` of the input and of every encoder parameter (None for the layers LayerDrop dropped).  No CPU path.
 """
 import ctypes
 from types import SimpleNamespace
@@ -21,7 +22,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from ._train import backward_flat, refresh_weights_device
+from ._train import StepRegularization, backward_flat, refresh_weights_device
 from .hubert import _DTYPES, _EncoderParams
 from .hubert_asr import _project
 
@@ -31,7 +32,7 @@ class _EncoderTrainFn(torch.autograd.Function):
     The parameters are passed only so that autograd routes their gradients; the arithmetic uses the packed copies."""
 
     @staticmethod
-    def forward(ctx, enc, x, pm_u8, *params):
+    def forward(ctx, enc, reg, x, pm_u8, *params):
         handle = enc._ensure_handle()
         dev = x.device
         B, T, D = x.shape
@@ -39,11 +40,12 @@ class _EncoderTrainFn(torch.autograd.Function):
         out = torch.empty(B, T, D, device=dev, dtype=out_dtype)
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
+            reg.set_on(handle)
             _lib.check(_lib.load().avh_encoder_train_forward(
                 handle, ctypes.c_void_p(x.data_ptr()), _DTYPES[x.dtype],
                 ctypes.c_void_p(pm_u8.data_ptr()) if pm_u8 is not None else None, B, T,
                 ctypes.c_void_p(out.data_ptr()), _DTYPES[out_dtype], ctypes.c_void_p(stream)))
-        ctx.enc, ctx.handle, ctx.x_dtype, ctx.stream = enc, handle, x.dtype, stream
+        ctx.enc, ctx.reg, ctx.handle, ctx.x_dtype, ctx.stream = enc, reg, handle, x.dtype, stream
         ctx.shapes = [tuple(p.shape) for p in params]
         ctx.dtypes = [p.dtype for p in params]
         ctx.params = params
@@ -71,7 +73,7 @@ class _EncoderTrainFn(torch.autograd.Function):
         assert off == n.value
         if flat.reduced:
             enc._grad_sync.mark_reduced(ctx.params)
-        return (None, dx, None, *grads)
+        return (None, None, dx, None, *ctx.reg.layer_grads(grads, flat.reduced))
 
 
 class TransformerEncoder(nn.Module):
@@ -176,10 +178,6 @@ class TransformerEncoder(nn.Module):
             raise NotImplementedError("the training-mode forward runs the whole stack (layer=None)")
         if not self.layer_norm_first:
             raise NotImplementedError("the device backward is built for pre-LN layers (layer_norm_first=True)")
-        for name in ("dropout", "attention_dropout", "activation_dropout", "encoder_layerdrop"):
-            if float(getattr(a, name, 0.0) or 0.0) != 0.0:
-                raise NotImplementedError(f"{name} must be 0 for the device training step (BASELINE config 5 sets "
-                                          "dropout / layerdrop 0)")
         dev = self.layer_norm.weight.device
         if x.device != dev or x.dim() != 3 or x.size(2) != self.embedding_dim:
             raise ValueError(f"x must be [B,T,{self.embedding_dim}] on {dev}, got {tuple(x.shape)} on {x.device}")
@@ -200,9 +198,15 @@ class TransformerEncoder(nn.Module):
                 self._eval_stale = True
             else:
                 self._dirty = True
+        reg = StepRegularization(a.encoder_layers, dropout=getattr(a, "dropout", 0.0),
+                                 activation_dropout=getattr(a, "activation_dropout", 0.0),
+                                 attention_dropout=getattr(a, "attention_dropout", 0.0),
+                                 layerdrop=getattr(a, "encoder_layerdrop", 0.0))
         self._ensure_handle()
         self._versions = [p._version for p in self.parameters()]
-        return _EncoderTrainFn.apply(self, x, pm, *self.grad_parameters()), []
+        y = _EncoderTrainFn.apply(self, reg, x, pm, *self.grad_parameters())
+        self._last_train_args = (reg.seed, list(reg.skip))      # what the step used: tests rebuild its masks from it
+        return y, []
 
     def forward(self, x, padding_mask=None, layer=None):
         """wav2vec2.py:859-902: returns (x [B,T,D], layer_results) — layer_results is empty (nobody on this path reads
