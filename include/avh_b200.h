@@ -176,14 +176,15 @@ AVH_API int avh_read_bn_stats(avh_handle* h, float* dst, int64_t capacity, void*
 AVH_API int avh_encoder_forward(avh_handle* h, const void* x, int x_dtype, const uint8_t* padding_mask, int B, int T,
                                 int output_layer, void* out, int out_dtype, void* stream);
 
-/* Training step of the TransformerEncoder (SURVEY 8(a) row A18, encoder part of BASELINE config 5; pre-LN layers): forward
- * with saved activations, then the backward of exactly that graph — wav2vec2.py:859-902 (positional conv + GELU +
- * residual, index_put on padded frames), :974-992 (pre-LN layer), multihead_attention.py:170-192, the final LayerNorm
- * (:862-863) — what torch.autograd computes for the reference module.  Dropout and LayerDrop as avh_set_train_args
+/* Training step of the TransformerEncoder (SURVEY 8(a) row A18, encoder part of BASELINE config 5; pre-LN or post-LN
+ * layers as layer_norm_first says): forward with saved activations, then the backward of exactly that graph —
+ * wav2vec2.py:859-902 (positional conv + GELU + residual, index_put on padded frames), :974-992 (pre-LN layer) or
+ * :993-1012 (post-LN layer), multihead_attention.py:170-192, the final LayerNorm (:862-863, pre-LN) or the LayerNorm after
+ * the positional conv (:876-877, post-LN) — what torch.autograd computes for the reference module.  Dropout and LayerDrop as avh_set_train_args
  * leaves them for the call (none without it).
  * Handle: any handle with encoder weights created with avh_config.reserved[3] = 1 (packs W^T for the dX = dY W GEMMs).
- * avh_encoder_train_forward: as avh_encoder_forward (all layers + final LayerNorm); avh_encoder_backward: dout [B,T,D] =
- * dL/d(out) (every row counts, padded frames too, as under autograd), dx [B,T,D] = dL/d(x) (may be NULL), grads = fp32 [avh_encoder_grad_count]
+ * avh_encoder_train_forward: as avh_encoder_forward (all layers, + final LayerNorm when pre-LN); avh_encoder_backward:
+ * dout [B,T,D] = dL/d(out) (every row counts, padded frames too, as under autograd), dx [B,T,D] = dL/d(x) (may be NULL), grads = fp32 [avh_encoder_grad_count]
  * (may be NULL) in this order: per layer {q,k,v}_proj.weight, {q,k,v}_proj.bias, out_proj.weight, out_proj.bias,
  * self_attn_layer_norm.{weight,bias}, fc1.weight, fc1.bias, fc2.weight, fc2.bias, final_layer_norm.{weight,bias}; then
  * encoder.layer_norm.{weight,bias}; then pos_conv.0.{bias, weight_g, weight_v}.  Same stream as the forward. */

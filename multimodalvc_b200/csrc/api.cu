@@ -1523,10 +1523,16 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
 }
 
 // ============================================================================ encoder training plan
-// TransformerEncoder forward with saved activations + its backward (pre-LN layers).  Forward: x0 = index_put(features,
-// mask, 0); c = pos_conv(x0) + b; x1 = m2 (x0 + GELU(c)); per layer h1 = LN1(x); qkv = h1 Wqkv^T + b; ctx = Attn(qkv)
-// (+ log-sum-exp per row); xm = x + m(16+4l) (ctx Wo^T + bo); h2 = LN2(xm); u = h2 W1^T + b1; g = m(17+4l) GELU(u);
-// x' = xm + m(18+4l) (g W2^T + b2); y = LN(x_L).  Tail modes: x0 = m1 post_extract_proj(LN(fused)) before the zeroing.
+// TransformerEncoder forward with saved activations + its backward, pre-LN or post-LN layers.  Pre-LN forward:
+// x0 = index_put(features, mask, 0); c = pos_conv(x0) + b; x1 = m2 (x0 + GELU(c)); per layer h1 = LN1(x);
+// qkv = h1 Wqkv^T + b; ctx = Attn(qkv) (+ log-sum-exp per row); xm = x + m(16+4l) (ctx Wo^T + bo); h2 = LN2(xm);
+// u = h2 W1^T + b1; g = m(17+4l) GELU(u); x' = xm + m(18+4l) (g W2^T + b2); y = LN(x_L).
+// Post-LN forward (wav2vec2.py:872-879, 993-1012): s = x0 + GELU(c); x1 = m2 LN(s); per layer qkv = x Wqkv^T + b (h1 = x);
+// r1 = x + m(16+4l) (ctx Wo^T + bo); y1 = LN1(r1) (h2 = y1); r2 = y1 + m(18+4l) (g W2^T + b2); x' = LN2(r2); y = x_L
+// (no final LayerNorm; encoder.layer_norm is the one after the positional conv and keeps its gradient slot).  Its
+// backward: dr2 = LN2^T(dx; r2), dr1 = LN1^T(dr2 + dL/dy1; r1), dx = dr1 + dL/dx through qkv, ds = LN^T(m2 dx1; s), each
+// LayerNorm backward also writing the masked gradient of the block that feeds it (launch_ln_post_bwd).
+// Tail modes: x0 = m1 post_extract_proj(LN(fused)) before the zeroing.
 // m_site = the dropout mask of that site (philox.cuh, p = key.p_in for site 1, p_act for 17+4l, p_enc otherwise; a
 // site with p = 0 is no mask and no launch).  A layer dropped by LayerDrop is the identity: its steps are skipped, an
 // on-drop step copies x into x' and zeroes the layer's gradients.  Backward: the chain rule of exactly that graph —
@@ -1619,7 +1625,7 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
   const size_t es = b.es;
   const int act_dt = b.act_dt;
   Plan* pl = plan;
-  if (!c.layer_norm_first) { set_last_error("the encoder backward is built for pre-LN layers (layer_norm_first)"); return false; }
+  const bool post = !c.layer_norm_first;
   {
     unsigned char* md = b.mask_buf(N);
     if (!sizing) plan->mask_dev = md;
@@ -1671,9 +1677,27 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
   std::vector<Act> h1(L), qkv(L), ctx(L), h2(L), u(L), g(L);
   std::vector<float*> lse(L);
   for (int l = 0; l <= L; ++l) xin[l] = b.f32buf(N * D);
+  // post-LN: h1 = x_l itself, h2 = y1 = LN1(r1) (both also the residual stream, fp32); r2 = y1 + block before LN2;
+  // spre = x0 + GELU(c) before the encoder LayerNorm
+  std::vector<float*> y1(post ? L : 0), r2(post ? L : 0);
+  float* spre = post ? b.f32buf(N * D) : nullptr;
+  // fp32 residual-stream tensor as a GEMM input: fp32 mode reads the tensor itself, bf16 mode a bf16 copy
+  auto stream_act = [&](float* v) {
+    Act a;
+    a.rows = N; a.C = D;
+    a.data = f32 ? v : b.alloc((size_t)N * D * 2);
+    a.op = f32 ? b.alloc((size_t)N * D * 2 * P) : a.data;
+    return a;
+  };
   for (int l = 0; l < L; ++l) {
     xmid[l] = b.f32buf(N * D);
-    h1[l] = b.act(N, D); qkv[l] = b.act(N, 3 * D); ctx[l] = b.act(N, D); h2[l] = b.act(N, D);
+    if (post) {
+      y1[l] = b.f32buf(N * D); r2[l] = b.f32buf(N * D);
+      h1[l] = stream_act(xin[l]); h2[l] = stream_act(y1[l]);
+      qkv[l] = b.act(N, 3 * D); ctx[l] = b.act(N, D);
+    } else {
+      h1[l] = b.act(N, D); qkv[l] = b.act(N, 3 * D); ctx[l] = b.act(N, D); h2[l] = b.act(N, D);
+    }
     u[l] = b.act(N, F); g[l] = b.act(N, F);
     lse[l] = b.f32buf((long long)B * Hh * T);
   }
@@ -1854,7 +1878,15 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     ep.map_mode = MAP_2LEVEL; ep.S2 = Tp; ep.S1 = Tp; ep.H = 1; ep.W = T; ep.O2 = T; ep.O1 = 0; ep.O0 = 0;
     if (!b.gemm("pos_conv", xpad, pad_rows, P * D, h->pos_w, pad_rows, taps, win / 64, D, ep, 64, h->pos_acol)) return false;
     float* x1 = xin[0];
-    if (p_enc > 0.f)     // x = F.dropout(x + GELU(conv(x))), wav2vec2.py:879
+    if (post) {          // x = F.dropout(LN(x + GELU(conv(x)))), wav2vec2.py:872-879
+      float* gm = h->enc_ln_g; float* be = h->enc_ln_b;
+      b.push("gelu", [=](cudaStream_t s) { return launch_gelu_fwd(cpre, DT_F32, x0, spre, DT_F32, N * D, s); });
+      b.push("layer_ln", [=](cudaStream_t s) {
+        return launch_layernorm(spre, DT_F32, D, gm, be, 1e-5f, x1, nullptr, DT_BF16, nullptr, N, D, s);
+      });
+      if (p_enc > 0.f)
+        b.push("dropout", [=](cudaStream_t s) { return launch_dropout_residual(nullptr, x1, x1, N * D, p_enc, seed, 2u, s); });
+    } else if (p_enc > 0.f)     // x = F.dropout(x + GELU(conv(x))), wav2vec2.py:879
       b.push("gelu", [=](cudaStream_t s) { return launch_masked_gelu(cpre, DT_F32, x0, x1, DT_F32, N * D, p_enc, seed, 2u, s); });
     else
       b.push("gelu", [=](cudaStream_t s) { return launch_gelu_fwd(cpre, DT_F32, x0, x1, DT_F32, N * D, s); });
@@ -1874,7 +1906,10 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     auto block_dropout = [&](const float* res, float* target, unsigned st) {
       b.push("dropout", [=](cudaStream_t s) { return launch_dropout_residual(res, dtmp, target, N * D, p_enc, seed, st, s); });
     };
-    b.layernorm("layer_ln", x, DT_F32, lw.ln1_g, lw.ln1_b, 1e-5f, h1[l]);
+    // post-LN: the qkv GEMM reads x_l itself; its operand form is made here, in layer l's own steps, so that a
+    // dropped layer's on-drop copy is all LayerDrop needs
+    if (post) b.split(x, D, h1[l].op, N, D);
+    else b.layernorm("layer_ln", x, DT_F32, lw.ln1_g, lw.ln1_b, 1e-5f, h1[l]);
     {
       Epilogue ep = epilogue(qkv[l].data, 3 * D, f32);
       ep.col_bias = lw.qkv.bias;
@@ -1900,7 +1935,17 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       ep.col_bias = lw.out.bias; ep.R = x; ep.ldr = D; ep.r_fp32 = 1;
       if (!b.linear("out_proj", ctx[l].op, N, D, lw.out.w, ep)) return false;
     }
-    b.layernorm("layer_ln", xmid[l], DT_F32, lw.ln2_g, lw.ln2_b, 1e-5f, h2[l]);
+    if (post) {          // y1 = self_attn_layer_norm(r1): fp32 residual stream of the FFN block + the fc1 operand
+      const float* r1 = xmid[l]; float* yv = y1[l];
+      void* yl = f32 ? nullptr : h2[l].data;
+      const float* gm = lw.ln1_g; const float* be = lw.ln1_b;
+      b.push("layer_ln", [=](cudaStream_t s) {
+        return launch_layernorm(r1, DT_F32, D, gm, be, 1e-5f, yv, yl, DT_BF16, nullptr, N, D, s);
+      });
+      b.sync_op(h2[l]);
+    } else {
+      b.layernorm("layer_ln", xmid[l], DT_F32, lw.ln2_g, lw.ln2_b, 1e-5f, h2[l]);
+    }
     {
       Epilogue ep = epilogue(u[l].data, F, f32);
       ep.col_bias = lw.fc1.bias;
@@ -1914,31 +1959,43 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
         b.push("gelu", [=](cudaStream_t s) { return launch_gelu_fwd(uu, act_dt, nullptr, gg, act_dt, N * F, s); });
       b.sync_op(g[l]);
     }
+    float* res2 = post ? y1[l] : xmid[l];          // FFN block: residual input, sum (post-LN: r2, before LN2)
+    float* out2 = post ? r2[l] : xin[l + 1];
     if (p_enc > 0.f) {
       Epilogue ep = epilogue(dtmp, D, true);
       ep.col_bias = lw.fc2.bias;
       if (!b.linear("fc2", g[l].op, N, F, lw.fc2.w, ep)) return false;
-      block_dropout(xmid[l], xin[l + 1], site + 2u);
+      block_dropout(res2, out2, site + 2u);
     } else {
-      Epilogue ep = epilogue(xin[l + 1], D, true);
-      ep.col_bias = lw.fc2.bias; ep.R = xmid[l]; ep.ldr = D; ep.r_fp32 = 1;
+      Epilogue ep = epilogue(out2, D, true);
+      ep.col_bias = lw.fc2.bias; ep.R = res2; ep.ldr = D; ep.r_fp32 = 1;
       if (!b.linear("fc2", g[l].op, N, F, lw.fc2.w, ep)) return false;
+    }
+    if (post) {          // x_{l+1} = final_layer_norm(r2)
+      float* xn = xin[l + 1];
+      const float* gm = lw.ln2_g; const float* be = lw.ln2_b;
+      b.push("layer_ln", [=](cudaStream_t s) {
+        return launch_layernorm(out2, DT_F32, D, gm, be, 1e-5f, xn, nullptr, DT_BF16, nullptr, N, D, s);
+      });
     }
   }
   b.cur_layer = -1;
   {
     float* xl = xin[L];
     float* gm = h->enc_ln_g; float* be = h->enc_ln_b;
-    b.push_direct("final_ln", [=](cudaStream_t s) {
-      return launch_layernorm(xl, DT_F32, D, gm, be, 1e-5f, nullptr, pl->args.out, pl->args.out_dt, nullptr, N, D, s);
-    });
+    if (post)            // no final LayerNorm after post-LN layers (wav2vec2.py:862-863)
+      b.push_direct("output", [=](cudaStream_t s) { return launch_convert(xl, DT_F32, pl->args.out, pl->args.out_dt, N * D, s); });
+    else
+      b.push_direct("final_ln", [=](cudaStream_t s) {
+        return launch_layernorm(xl, DT_F32, D, gm, be, 1e-5f, nullptr, pl->args.out, pl->args.out_dt, nullptr, N, D, s);
+      });
   }
   if (!sizing) plan->fwd_steps = plan->steps.size();
 
   // ================================================================ backward
   float2* stats = reinterpret_cast<float2*>(b.alloc((size_t)N * 8));
   float* Dbuf = b.f32buf((long long)B * Hh * T);
-  float* dx = b.f32buf(N * D);             // gradient of the residual stream (ping)
+  float* dx = post ? dy : b.f32buf(N * D);  // gradient of the residual stream (ping; post-LN: starts as dL/dy itself)
   float* dxm = b.f32buf(N * D);            // ... at the middle of a layer (pong)
   float* dh = b.f32buf(N * D);             // gradient of a LayerNorm output
   Act dxa = b.act(N, D);                   // operand form of dx / dxm
@@ -1970,7 +2027,7 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
   const float qscale = 1.0f / std::sqrt(64.0f);
   const long long LG = enc_layer_grad_floats(D, F);
   // (the caller's dL/dy is staged into `dy` by avh_encoder_backward before the steps run)
-  {   // final LayerNorm
+  if (!post) {   // final LayerNorm
     float* gfin = grads + (long long)L * LG;
     float* xl = xin[L];
     float* gm = h->enc_ln_g;
@@ -2006,8 +2063,23 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       b.push("dropout_bwd", [=](cudaStream_t s) { return launch_dropout_grad(dyv, dtmp, op, planes, N, D, p_enc, seed, st, s); });
       return dtmp;
     };
-    // ---- fc2: x' = xm + m (g W2^T + b2)
-    if (p_enc > 0.f) {
+    // post-LN: gradient of a LayerNorm input r = res + m * block from its output's gradients (dya + dyb), written to
+    // dr, with m * dr into dtmp (p > 0) and its operand form; returns what the block's weight gradient reads
+    auto post_ln_grad = [&](const float* r, const float* gm, const float* dya, const float* dyb, float* dr, float* g_ln,
+                            unsigned st) -> float* {
+      float* mo = p_enc > 0.f ? dtmp : nullptr;
+      void* op = dxa.op;
+      const int planes = P;
+      b.push("ln_bwd", [=](cudaStream_t s) {
+        return launch_ln_post_bwd(r, gm, dya, dyb, dr, mo, op, planes, stats, g_ln, g_ln + D, N, D, 1e-5f, p_enc, seed, st, s);
+      });
+      return mo ? mo : dr;
+    };
+    // ---- fc2: x' = xm + m (g W2^T + b2)   (post-LN: r2 = y1 + m (g W2^T + b2), x' = LN2(r2); dr2 -> dxm)
+    if (post) {
+      float* d3 = post_ln_grad(r2[l], lw.ln2_g, dx, nullptr, dxm, g_ln2, site + 2u);
+      if (!wgrad(d3, DT_F32, D, g[l].data, act_dt, F, g_fc2_w, g_fc2_b, "fc2_wgrad")) return false;
+    } else if (p_enc > 0.f) {
       float* d3 = block_grad(dx, site + 2u);
       if (!wgrad(d3, DT_F32, D, g[l].data, act_dt, F, g_fc2_w, g_fc2_b, "fc2_wgrad")) return false;
     } else {
@@ -2028,17 +2100,22 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     // ---- fc1: u = h2 W1^T + b1
     if (!wgrad(dua.data, act_dt, F, h2[l].data, act_dt, D, g_fc1_w, g_fc1_b, "fc1_wgrad")) return false;
     if (!dgrad(dua.op, F, lw.fc1T, dh, true, "fc1_dgrad")) return false;
-    {   // LN2: dxm = dx + dLN(dh; xm)
-      float* xm = xmid[l]; float* gm = lw.ln2_g;
-      b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(xm, gm, dh, dx, dxm, stats, g_ln2, g_ln2 + D, N, D, 1e-5f, s); });
-    }
-    // ---- out_proj: xm = x + m (ctx Wo^T + bo)
-    if (p_enc > 0.f) {
-      float* d1 = block_grad(dxm, site);
+    // ---- out_proj: xm = x + m (ctx Wo^T + bo)   (post-LN: r1 = x + m (ctx Wo^T + bo), y1 = LN1(r1); dr1 -> dx)
+    if (post) {
+      float* d1 = post_ln_grad(xmid[l], lw.ln1_g, dxm, dh, dx, g_ln1, site);
       if (!wgrad(d1, DT_F32, D, ctx[l].data, act_dt, D, g_out_w, g_out_b, "out_wgrad")) return false;
     } else {
-      if (!wgrad(dxm, DT_F32, D, ctx[l].data, act_dt, D, g_out_w, g_out_b, "out_wgrad")) return false;
-      block_grad(dxm, site);
+      {   // LN2: dxm = dx + dLN(dh; xm)
+        float* xm = xmid[l]; float* gm = lw.ln2_g;
+        b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(xm, gm, dh, dx, dxm, stats, g_ln2, g_ln2 + D, N, D, 1e-5f, s); });
+      }
+      if (p_enc > 0.f) {
+        float* d1 = block_grad(dxm, site);
+        if (!wgrad(d1, DT_F32, D, ctx[l].data, act_dt, D, g_out_w, g_out_b, "out_wgrad")) return false;
+      } else {
+        if (!wgrad(dxm, DT_F32, D, ctx[l].data, act_dt, D, g_out_w, g_out_b, "out_wgrad")) return false;
+        block_grad(dxm, site);
+      }
     }
     if (!dgrad(dxa.op, D, lw.outT, dctx.data, f32, "out_dgrad")) return false;
     {   // attention
@@ -2061,10 +2138,16 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       if (launch_scale(g_qkv_w, (long long)D * D, qscale, s)) return 1;
       return launch_scale(g_qkv_b, D, qscale, s);
     });
-    if (!dgrad(dqkv.op, 3 * D, lw.qkvT, dh, true, "qkv_dgrad")) return false;
-    {   // LN1: dx = dxm + dLN(dh; x)
-      float* xl = xin[l]; float* gm = lw.ln1_g;
-      b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(xl, gm, dh, dxm, dx, stats, g_ln1, g_ln1 + D, N, D, 1e-5f, s); });
+    if (post) {          // dx_l = dr1 + dL/dx_l through the qkv projection: the dgrad accumulates onto dx
+      Epilogue ep = epilogue(dx, D, true);
+      ep.R = dx; ep.ldr = D; ep.r_fp32 = 1;
+      if (!b.linear("qkv_dgrad", dqkv.op, N, 3 * D, lw.qkvT.w, ep)) return false;
+    } else {
+      if (!dgrad(dqkv.op, 3 * D, lw.qkvT, dh, true, "qkv_dgrad")) return false;
+      {   // LN1: dx = dxm + dLN(dh; x)
+        float* xl = xin[l]; float* gm = lw.ln1_g;
+        b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(xl, gm, dh, dxm, dx, stats, g_ln1, g_ln1 + D, N, D, 1e-5f, s); });
+      }
     }
     if (l % 4 == 0) {      // layers l .. l+3 are final: one gradient bucket (Large: 4 x 12.6 M floats)
       b.cur_layer = -1;
@@ -2073,12 +2156,20 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
   }
   b.cur_layer = -1;
   // ---- positional conv block: x1 = m2 (x0 + GELU(c)), c = conv(x0) + bias  (pos-conv weight gradients: see posconv_bwd)
+  //      post-LN: x1 = m2 LN(s), s = x0 + GELU(c)
   {
     float* gpos = grads + (long long)L * LG + 2ll * D;       // bias [D], weight_g [KT], weight_v [D, D/G, KT]
     if (p_enc > 0.f)     // dx = m2 dL/dx1 in place: the gradient of both the residual and the GELU input
       b.push("dropout_bwd", [=](cudaStream_t s) { return launch_dropout_grad(dx, dx, nullptr, 1, N, D, p_enc, seed, 2u, s); });
-    float* dc = dh;                                          // dL/dc = dx * GELU'(c)
-    b.push("gelu_bwd", [=](cudaStream_t s) { return launch_gelu_bwd(cpre, DT_F32, dx, DT_F32, dc, DT_F32, N * D, s); });
+    float* ds = dx;                                          // dL/d(x0 + GELU(c))
+    if (post) {          // encoder.layer_norm: ds = LN^T(m2 dL/dx1; s) into dxm, its gamma / beta into their usual slot
+      float* gfin = grads + (long long)L * LG;
+      float* gm = h->enc_ln_g;
+      b.push("ln_bwd", [=](cudaStream_t s) { return launch_ln_bwd(spre, gm, dx, nullptr, dxm, stats, gfin, gfin + D, N, D, 1e-5f, s); });
+      ds = dxm;
+    }
+    float* dc = dh;                                          // dL/dc = ds * GELU'(c)
+    b.push("gelu_bwd", [=](cudaStream_t s) { return launch_gelu_bwd(cpre, DT_F32, ds, DT_F32, dc, DT_F32, N * D, s); });
     b.push("bias_grad", [=](cudaStream_t s) { return launch_colsum(dc, DT_F32, D, N, D, gpos, 1.0f, s); });
     // dgrad: dx0[t, i] = dx[t, i] + sum_k sum_o dc[t + 64 - k, o] w[o, i, k]: the same shifted-row GEMM over the
     // zero-gapped layout with the taps mirrored and the weights transposed inside every group (pos_wT)
@@ -2088,7 +2179,7 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
     std::vector<Tap> taps;
     for (int k = 0; k < KT; ++k) taps.push_back(Tap{KT / 2 - k, 0, k * win});
     Epilogue ep = epilogue(dxo, D, true);
-    ep.R = dx; ep.ldr = D; ep.r_fp32 = 1;
+    ep.R = ds; ep.ldr = D; ep.r_fp32 = 1;
     ep.row_zero = hm ? plan->mask_dev : nullptr;             // x0 = index_put(features, mask, 0): no gradient into pad rows
     ep.map_mode = MAP_2LEVEL; ep.S2 = Tp; ep.S1 = Tp; ep.H = 1; ep.W = T; ep.O2 = T; ep.O1 = 0; ep.O0 = 0;
     if (!b.gemm("pos_conv_dgrad", dcpad, pad_rows, P * D, h->pos_wT, pad_rows, taps, win / 64, D, ep, 64, h->pos_acol)) return false;

@@ -7,11 +7,14 @@
 // and the kernels below are the element-wise / row-wise / attention parts, fp32 arithmetic, deterministic (no atomics):
 //   gelu_fwd / gelu_bwd        erf GELU and its derivative Phi(u) + u phi(u)      (fairseq/fairseq/modules/gelu.py:95-96)
 //   ln_stats + ln_bwd_dx + ln_bwd_params   LayerNorm backward (fairseq/fairseq/modules/layer_norm.py:51-56 -> F.layer_norm)
+//   ln_post_bwd_dx             the post-LN form: LN^T(residual-path + block-path gradient), with the masked gradient of
+//                               the block that feeds the LayerNorm and its GEMM operand planes in the same pass
 //   attention_bwd_dq / attention_bwd_dkv  softmax attention backward with the probabilities recomputed from the saved
 //                               log-sum-exp of every query row (fairseq/fairseq/modules/multihead_attention.py:170-192)
 #include "attn_tile.cuh"
 #include "common.cuh"
 #include "kernels.h"
+#include "philox.cuh"
 
 #include <cuda_fp16.h>
 
@@ -144,10 +147,77 @@ ln_bwd_dx_kernel(const float* __restrict__ x, const float* __restrict__ gamma, c
   }
   if (lane == 0 && stats != nullptr) stats[row] = make_float2(mean, rstd);
 }
-// dgamma[c] = sum_r dy[r,c] xhat[r,c], dbeta[c] = sum_r dy[r,c]
+// Post-LN LayerNorm backward w.r.t. the input r = res + block output, warp per row, 4 consecutive channels per lane
+// step: dy = dya + (dyb ? dyb : 0) (residual path + block path of the LayerNorm's output), out = dLN/dr(dy).  Also, for
+// the block that feeds r: v = m * out with m the dropout mask of `site` (p = 0: no mask, v = out), written as fp32 to
+// mout (optional) and as GEMM operand planes to op ([rows, planes * C], as split_rows writes them).  Stores (mean, rstd)
+// per row for the parameter-gradient kernel.
+__global__ void __launch_bounds__(256)
+ln_post_bwd_dx_kernel(const float* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ dya,
+                      const float* __restrict__ dyb, float* __restrict__ out, float* __restrict__ mout,
+                      __nv_bfloat16* __restrict__ op, int planes, float2* __restrict__ stats, long long rows, int C, float eps,
+                      float p, const unsigned long long* __restrict__ seed, unsigned int site) {
+  const long long row = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
+  const int lane = threadIdx.x & 31;
+  if (row >= rows) return;
+  const int C4 = C / 4;
+  const float4* xr = reinterpret_cast<const float4*>(x + row * C);
+  const float4* ar = reinterpret_cast<const float4*>(dya + row * C);
+  const float4* br = dyb ? reinterpret_cast<const float4*>(dyb + row * C) : nullptr;
+  const float4* g4 = reinterpret_cast<const float4*>(gamma);
+  float s = 0.f;
+  for (int c = lane; c < C4; c += 32) { const float4 v = xr[c]; s += (v.x + v.y) + (v.z + v.w); }
+  const float mean = wsum(s) / C;
+  float q = 0.f;
+  for (int c = lane; c < C4; c += 32) {
+    const float4 v = xr[c];
+    const float d0 = v.x - mean, d1 = v.y - mean, d2 = v.z - mean, d3 = v.w - mean;
+    q += (d0 * d0 + d1 * d1) + (d2 * d2 + d3 * d3);
+  }
+  const float rstd = rsqrtf(wsum(q) / C + eps);
+  auto grad = [&](int c) {        // dy * gamma
+    float4 d = ar[c];
+    if (br) { const float4 e = br[c]; d.x += e.x; d.y += e.y; d.z += e.z; d.w += e.w; }
+    const float4 g = g4[c];
+    return make_float4(d.x * g.x, d.y * g.y, d.z * g.z, d.w * g.w);
+  };
+  float a = 0.f, b = 0.f;
+  for (int c = lane; c < C4; c += 32) {
+    const float4 g = grad(c), v = xr[c];
+    a += (g.x + g.y) + (g.z + g.w);
+    b += ((g.x * (v.x - mean) + g.y * (v.y - mean)) + (g.z * (v.z - mean) + g.w * (v.w - mean))) * rstd;
+  }
+  a = wsum(a) / C;
+  b = wsum(b) / C;
+  for (int c = lane; c < C4; c += 32) {
+    const float4 g = grad(c), v = xr[c];
+    float4 d;
+    d.x = rstd * (g.x - a - (v.x - mean) * rstd * b);
+    d.y = rstd * (g.y - a - (v.y - mean) * rstd * b);
+    d.z = rstd * (g.z - a - (v.z - mean) * rstd * b);
+    d.w = rstd * (g.w - a - (v.w - mean) * rstd * b);
+    reinterpret_cast<float4*>(out + row * C)[c] = d;
+    if (p > 0.f) {
+      const float4 m = dropout_mask4(*seed, row * C4 + c, site, p);
+      d = make_float4(m.x * d.x, m.y * d.y, m.z * d.z, m.w * d.w);
+    }
+    if (mout) reinterpret_cast<float4*>(mout + row * C)[c] = d;
+    __nv_bfloat16* o = op + row * ((long long)planes * C) + 4 * c;
+    const __nv_bfloat162 h0 = __floats2bfloat162_rn(d.x, d.y), h1 = __floats2bfloat162_rn(d.z, d.w);
+    *reinterpret_cast<uint2*>(o) = make_uint2(*reinterpret_cast<const uint32_t*>(&h0), *reinterpret_cast<const uint32_t*>(&h1));
+    if (planes > 1) {
+      const float2 f0 = __bfloat1622float2(h0), f1 = __bfloat1622float2(h1);
+      *reinterpret_cast<uint2*>(o + C) = make_uint2(pack_bf16(d.x - f0.x, d.y - f0.y), pack_bf16(d.z - f1.x, d.w - f1.y));
+    }
+  }
+  if (lane == 0) stats[row] = make_float2(mean, rstd);
+}
+
+// dgamma[c] = sum_r dy[r,c] xhat[r,c], dbeta[c] = sum_r dy[r,c]; SUM2: dy = dy + dy2 (the post-LN backward's two paths)
+template <bool SUM2>
 __global__ void __launch_bounds__(1024)
-ln_bwd_params_kernel(const float* __restrict__ x, const float* __restrict__ dy, const float2* __restrict__ stats,
-                     long long rows, int C, float* __restrict__ dgamma, float* __restrict__ dbeta) {
+ln_bwd_params_kernel(const float* __restrict__ x, const float* __restrict__ dy, const float* __restrict__ dy2,
+                     const float2* __restrict__ stats, long long rows, int C, float* __restrict__ dgamma, float* __restrict__ dbeta) {
   __shared__ float pg[CS_PH][33], pb[CS_PH][33];
   const int j = threadIdx.x % 32, ph = threadIdx.x / 32;
   const int c = blockIdx.x * 32 + j;
@@ -155,7 +225,7 @@ ln_bwd_params_kernel(const float* __restrict__ x, const float* __restrict__ dy, 
   if (c < C)
     for (long long r = ph; r < rows; r += CS_PH) {
       const float2 st = stats[r];
-      const float d = dy[r * C + c];
+      const float d = SUM2 ? dy[r * C + c] + dy2[r * C + c] : dy[r * C + c];
       sg += d * (x[r * C + c] - st.x) * st.y;
       sb += d;
     }
@@ -468,7 +538,29 @@ int launch_ln_bwd(const float* x, const float* gamma, const float* dy, const flo
   AVH_CHECK(stats != nullptr, "ln_bwd needs the per-row statistics buffer");
   ln_bwd_dx_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, stream>>>(x, gamma, dy, res, dx_out, stats, rows, C, eps);
   AVH_CUDA_OK(cudaGetLastError());
-  ln_bwd_params_kernel<<<(C + 31) / 32, 1024, 0, stream>>>(x, dy, stats, rows, C, dgamma, dbeta);
+  ln_bwd_params_kernel<false><<<(C + 31) / 32, 1024, 0, stream>>>(x, dy, nullptr, stats, rows, C, dgamma, dbeta);
+  AVH_CUDA_OK(cudaGetLastError());
+  count_launch(2);
+  return 0;
+}
+
+int launch_ln_post_bwd(const float* x, const float* gamma, const float* dya, const float* dyb, float* dx_out, float* mout,
+                       void* op, int planes, float2* stats, float* dgamma, float* dbeta, long long rows, int C, float eps,
+                       float p, const unsigned long long* seed, unsigned int site, cudaStream_t stream) {
+  if (rows <= 0) return 0;
+  AVH_CHECK(stats != nullptr && op != nullptr, "ln_post_bwd needs the per-row statistics buffer and the operand output");
+  AVH_CHECK(C % 4 == 0, "ln_post_bwd: row width must be a multiple of 4");
+  AVH_CHECK(p == 0.f || (p > 0.f && p < 1.f && seed != nullptr), "ln_post_bwd: dropout probability in [0, 1), seed for p > 0");
+  AVH_CHECK(dx_out != dya && dx_out != dyb && (mout == nullptr || (mout != dya && mout != dyb)),
+            "ln_post_bwd: the outputs must not alias the incoming gradients (the parameter pass re-reads them)");
+  ln_post_bwd_dx_kernel<<<(unsigned)((rows + 7) / 8), 256, 0, stream>>>(x, gamma, dya, dyb, dx_out, mout,
+                                                                        reinterpret_cast<__nv_bfloat16*>(op), planes, stats,
+                                                                        rows, C, eps, p, seed, site);
+  AVH_CUDA_OK(cudaGetLastError());
+  if (dyb != nullptr)
+    ln_bwd_params_kernel<true><<<(C + 31) / 32, 1024, 0, stream>>>(x, dya, dyb, stats, rows, C, dgamma, dbeta);
+  else
+    ln_bwd_params_kernel<false><<<(C + 31) / 32, 1024, 0, stream>>>(x, dya, nullptr, stats, rows, C, dgamma, dbeta);
   AVH_CUDA_OK(cudaGetLastError());
   count_launch(2);
   return 0;

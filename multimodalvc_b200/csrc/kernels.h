@@ -135,6 +135,12 @@ int launch_gelu_bwd(const void* u, int u_dt, const void* dg, int dg_dt, void* du
 // LayerNorm backward: dx_out = (res ? res : 0) + dLN/dx(dy), dgamma, dbeta; stats = scratch [rows] float2
 int launch_ln_bwd(const float* x, const float* gamma, const float* dy, const float* res, float* dx_out, float2* stats,
                   float* dgamma, float* dbeta, long long rows, int C, float eps, cudaStream_t stream);
+// post-LN LayerNorm backward: dx_out = dLN/dx(dya + dyb) (dyb may be null), dgamma / dbeta of the summed gradient;
+// v = m * dx_out with m the dropout mask of `site` (p = 0: v = dx_out; p > 0: seed is a DEVICE word) into mout (fp32,
+// optional) and op (GEMM operand form, bf16 [rows, planes * C]); C a multiple of 4; outputs must not alias dya / dyb
+int launch_ln_post_bwd(const float* x, const float* gamma, const float* dya, const float* dyb, float* dx_out, float* mout,
+                       void* op, int planes, float2* stats, float* dgamma, float* dbeta, long long rows, int C, float eps,
+                       float p, const unsigned long long* seed, unsigned int site, cudaStream_t stream);
 // attention backward (self-attention over L rows per clip, heads of 64 channels side by side); Dbuf = scratch [B, H, L]
 int launch_attention_bwd(const void* Q, long long ldq, const void* K, long long ldk, const void* V, long long ldv, int dt,
                          const void* dO, const void* O, long long ldo, int o_dt, const float* lse, const unsigned char* key_pad,

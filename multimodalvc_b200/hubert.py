@@ -679,8 +679,6 @@ class AVHubertModel(nn.Module):
         c = self.cfg
         if output_layer is not None:
             raise NotImplementedError("the training step runs the whole encoder (output_layer=None)")
-        if not c.layer_norm_first:
-            raise NotImplementedError("the device backward is built for pre-LN layers (layer_norm_first=True)")
         if c.attention_dropout > 0:
             raise NotImplementedError("attention_dropout > 0 in training mode is not implemented (0.0 in every "
                                       "shipped fine-tune config, avhubert/conf/finetune/*.yaml)")

@@ -11,7 +11,7 @@
 Inference by default (eval mode: LayerDrop and dropout are identity, as in the reference's ``self.training`` gates).
 ``TransformerEncoder(args, trainable=True)`` also differentiates: in ``.train()`` with gradients enabled ``forward`` is a
 ``torch.autograd.Function`` whose backward is the library's (``avh_encoder_train_forward`` / ``avh_encoder_backward``:
-SURVEY row A18, encoder part of BASELINE config 5; pre-LN layers; ``dropout``, ``activation_dropout`` and
+SURVEY row A18, encoder part of BASELINE config 5; pre-LN and post-LN layers; ``dropout``, ``activation_dropout`` and
 ``encoder_layerdrop`` of the args as the reference applies them, ``attention_dropout`` must be 0), so ``loss.backward()``
 fills ``.grad`` of the input and of every encoder parameter (None for the layers LayerDrop dropped).  No CPU path.
 """
@@ -176,8 +176,6 @@ class TransformerEncoder(nn.Module):
             raise RuntimeError("build the module with trainable=True to differentiate through it (or call .eval())")
         if layer is not None:
             raise NotImplementedError("the training-mode forward runs the whole stack (layer=None)")
-        if not self.layer_norm_first:
-            raise NotImplementedError("the device backward is built for pre-LN layers (layer_norm_first=True)")
         dev = self.layer_norm.weight.device
         if x.device != dev or x.dim() != 3 or x.size(2) != self.embedding_dim:
             raise ValueError(f"x must be [B,T,{self.embedding_dim}] on {dev}, got {tuple(x.shape)} on {x.device}")
