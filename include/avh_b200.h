@@ -68,7 +68,8 @@ typedef struct avh_config {
   int32_t conv_pos;                /* hubert.py:213 (128) */
   int32_t conv_pos_groups;         /* hubert.py:217 (16)  */
   int32_t compute_mode;            /* AVH_COMPUTE_* */
-  int32_t frontend_chunk_frames;   /* video frames per lip-frontend pass; 0 = default */
+  int32_t frontend_chunk_frames;   /* video frames per lip-frontend pass; 0 = default.  avh_forward_train runs the whole
+                                      batch in one pass (BatchNorm batch statistics) */
   int32_t capture_stages;          /* non-zero: keep copies of intermediate stages for avh_read_stage (tests) */
   int32_t reserved[4];             /* reserved[0] = 1: the handle holds a bare fairseq TransformerEncoder (state-dict keys
                                       "encoder.*" only; avh_encoder_forward is its one forward entry point);
@@ -309,7 +310,9 @@ AVH_API int avh_forward_host_async(avh_handle* h, const void* video, int video_d
                            void* stream);
 
 /* Intermediate taps for stage-level parity tests; names: "resnet" [B*T,512], "fused" [B*T,E] (before the LayerNorm), "fused_ln" [B*T,E],
- * "enc_in" [B*T,D].  Copies the fp32 value of the last avh_forward into `dst` (device, fp32). */
+ * "enc_in" [B*T,D], and the lip-frontend maps "stem", "layer{L}.{b}.mid" / "layer{L}.{b}.out" (L = 1..4, b = 0, 1) and
+ * "layer{L}.0.ds" (L = 2..4, fp32 mode and training mode only) — layouts in AVHubertModel.read_stage.  Copies the fp32
+ * value of the last avh_forward into `dst` (device, fp32). */
 AVH_API int avh_read_stage(avh_handle* h, const char* name, float* dst, int64_t capacity_elems, void* stream);
 
 /* Audio frontend.  wav: int16 samples of n_clips clips back to back, clip i = [offsets[i], offsets[i+1]).

@@ -1047,6 +1047,16 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     int CB = std::max(1, target / T);
     CB = (B + ((B + CB - 1) / CB) - 1) / ((B + CB - 1) / CB);       // even split over ceil(B/CB) chunks
     if (rg) CB = B;                                                  // ragged: one chunk of Nb packed frames
+    // training mode: one chunk, so that BatchNorm normalises with the statistics of the whole batch and updates the
+    // running statistics once per forward, as nn.BatchNorm does
+    if (train) {
+      if ((long long)B * T > 65535) {      // the stem max-pool runs one grid row per frame
+        set_last_error("training-mode forward: B*T = " + std::to_string((long long)B * T) +
+                       " frames exceed the 65535 frames BatchNorm can take in one frontend pass");
+        return false;
+      }
+      CB = B;
+    }
     const int CF = rg ? (int)N : CB * T;
     FrontendBufs fb;
     if (f32 || train) {     // patch matrix + un-pooled stem maps: only the unfused stem needs them
@@ -1213,7 +1223,8 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
         // rows map 1:1 (TMA-store epilogue); rows of the gap frames hold don't-care values nobody reads
         std::vector<Tap> taps;
         for (int dt = 0; dt < 5; ++dt) taps.push_back(Tap{(dt - 2) * 1936, 0, dt * 64});
-        // batch statistics over the frames of the chunk (gap frames of the clip-padded row space excluded)
+        // batch statistics over all frames of the batch, one chunk in training mode (gap frames of the clip-padded row
+        // space excluded)
         if (!conv_bn(ep, h->stem, rows, (double)nf * 1936.0, (long long)(T + 2) * 1936, (long long)T * 1936, 0, 0,
                      [&](const Epilogue& e) { return b.gemm("stem_gemm", fb.im2col, rows, P * 64, h->stem.w, rows, taps, 1, 64, e); }))
           return false;
@@ -1223,6 +1234,9 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
         Act pv = fb.pooled; pv.rows = (long long)nf * 529;
         b.sync_op(pv);
       }
+      // intermediate maps of this chunk, readable with avh_read_stage (no launch: a later chunk overwrites the entries,
+      // so after a forward they hold the last chunk's frames)
+      b.stage("stem", fb.pooled.data, act_dt, (long long)nf * 529 * 64);
       // ---- trunk
       Act cur = fb.pooled;
       for (int L = 0; L < 4; ++L) {
@@ -1231,6 +1245,13 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
           const BlockW& bw = h->blocks[L][bi];
           Act mid = fb.a[L][bi * 2], out = fb.a[L][bi * 2 + 1];
           mid.rows = out.rows = (long long)nf * S * S;
+          {
+            const long long n = (long long)nf * ((frame_mode && L > 0) ? Hn * Hn : S * S) * Cc;
+            const std::string nm = "layer" + std::to_string(L + 1) + "." + std::to_string(bi);
+            b.stage((nm + ".mid").c_str(), mid.data, act_dt, n);
+            b.stage((nm + ".out").c_str(), out.data, act_dt, n);
+            if (bw.has_ds && !frame_mode) b.stage((nm + ".ds").c_str(), fb.ds[L].data, act_dt, n);
+          }
           const Act* res = &cur;
           Act dsout;
           if (frame_mode && L > 0) {

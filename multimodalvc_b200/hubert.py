@@ -831,7 +831,21 @@ class AVHubertModel(nn.Module):
         return out
 
     def read_stage(self, name, numel):
-        """Intermediate tensor of the last forward (needs cfg.capture_stages=True): 'resnet', 'fused_ln', 'enc_in'."""
+        """Intermediate tensor of the last forward as fp32 (the first `numel` values are written): 'resnet' [N, 512],
+        'fused' / 'fused_ln' [N, E], 'enc_in' [N, D] (needs cfg.capture_stages=True), and the lip ResNet's maps, NHWC
+        over the nf frames of the last frontend chunk (with several chunks the earlier chunks' frames are gone; a packed
+        ragged batch is one chunk of its valid frames back to back, nf = its plan's 128-frame bucket, the frames past the
+        valid ones unspecified):
+
+        - 'stem': the max-pooled stem output, H = 22, C = 64;
+        - 'layer{L}.{b}.mid': conv1 + BN + PReLU of block b (0, 1) of layer L (1..4), H = 22, 11, 6, 3, C = 64 << (L-1);
+        - 'layer{L}.{b}.out': the block output;
+        - 'layer{L}.0.ds' (L = 2..4): the downsample branch's conv + BN, in fp32 mode and in training mode only (the
+          bf16 eval path folds the shortcut into conv2's GEMM and writes no such map).
+
+        Padded maps are [nf, H+1, H+1, C]: pixel (y, x) at y*(H+1) + x, row H and column H a shared zero row and column
+        (the next convolution reads them as padding).  'stem' and layer 1 are padded in every mode, layers 2-4 in fp32
+        mode and in training mode; layers 2-4 of the bf16 eval path are dense [nf, H, H, C]."""
         dev = self.encoder.layer_norm.weight.device
         dst = torch.empty(numel, device=dev, dtype=torch.float32)
         with torch.cuda.device(dev):
