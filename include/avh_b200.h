@@ -125,7 +125,7 @@ AVH_API int avh_forward(avh_handle* h, const void* video, int video_dtype, const
  * Same tensors as avh_forward (float video only).  The updated running statistics are read with avh_read_bn_stats:
  * flat fp32, per BatchNorm (running_mean[C], running_var[C]) in the order frontend3D.1, then for layer1..4, block 0..1:
  * bn1, bn2, downsample.1 (when present).  Eval-mode forwards keep using the statistics folded at the last
- * avh_finalize_weights until the caller re-loads them. */
+ * avh_finalize_weights until the caller re-folds them (avh_refresh_eval_weights_device) or re-loads them. */
 typedef struct avh_train_args {
   float dropout_input, dropout, activation_dropout, attention_dropout;
   float bn_momentum;               /* nn.BatchNorm default 0.1 */
@@ -210,11 +210,23 @@ AVH_API int avh_grad_bucket_count(avh_handle* h, int32_t* count);
  * device-resident parameters: names[i] = state-dict key (the reference's names, as avh_load_tensor), ptrs[i] = device
  * pointer of the contiguous tensor, dtypes[i] = AVH_F32 / AVH_F16 / AVH_BF16, numels[i] = element count.  Plans and
  * captured graphs stay valid (no pointer moves); nothing crosses the host (avh_finalize_weights re-packs through the
- * host: seconds for the Large model).  The eval-only packed forms (BatchNorm folded with the running statistics,
- * LayerNorm folded into the QKV / fc1 weights, the fused stem order) are NOT refreshed: before the next eval-mode
- * forward reload the state dict and call avh_finalize_weights.  Enqueued on `stream`. */
+ * host: seconds for the Large model).  The eval-only packed forms (BatchNorm folded with the running statistics, the
+ * conv2 + shortcut GEMM weights with both BatchNorm scales folded in) are NOT refreshed: before the next eval-mode
+ * forward call avh_refresh_eval_weights_device.  Enqueued on `stream`. */
 AVH_API int avh_refresh_weights_device(avh_handle* h, const char* const* names, const void* const* ptrs, const int32_t* dtypes,
                                        const int64_t* numels, int32_t count, void* stream);
+/* Before an eval-mode forward that follows training on the handle (optimizer steps, or training-mode forwards that moved
+ * the BatchNorm running statistics): on a trainable handle the work of avh_refresh_weights_device, then on every
+ * AV-HuBERT handle the eval-only forms — per BatchNorm scale = gamma / sqrt(running_var + 1e-5) and bias = beta -
+ * running_mean * scale, the fp32 gamma / beta / running statistics the training-mode BatchNorm starts from, and the conv2
+ * + shortcut GEMM weights of layers 2-4 — in place, on the device, bit-identical to what avh_finalize_weights computes
+ * from the same values.  The list holds the parameters AND the BatchNorm buffers ("...running_mean",
+ * "...running_var"), same arguments as avh_refresh_weights_device; plans, arenas and captured graphs stay valid.  The
+ * job list is replayed as its own CUDA graph for the pointer set it was last called with.  Not for Q-Former handles. */
+AVH_API int avh_refresh_eval_weights_device(avh_handle* h, const char* const* names, const void* const* ptrs,
+                                            const int32_t* dtypes, const int64_t* numels, int32_t count, void* stream);
+/* Number of execution plans the handle holds (forward and training plans, all streams); avh_finalize_weights drops them. */
+AVH_API int avh_plan_count(avh_handle* h, int32_t* count);
 AVH_API int avh_grad_bucket_range(avh_handle* h, int k, int64_t* begin, int64_t* end);       /* [begin, end) elements */
 AVH_API int avh_grad_bucket_wait(avh_handle* h, int k, void* stream);
 

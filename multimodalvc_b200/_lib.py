@@ -22,7 +22,7 @@ EXPORTS = [
     "avh_mask_substitute", "avh_compute_logits", "avh_sum_squares", "avh_qformer_forward",
     "avh_encoder_grad_count", "avh_encoder_train_forward", "avh_encoder_backward",
     "avh_encoder_backward_buckets", "avh_grad_bucket_count", "avh_grad_bucket_range", "avh_grad_bucket_wait",
-    "avh_refresh_weights_device",
+    "avh_refresh_weights_device", "avh_refresh_eval_weights_device", "avh_plan_count",
     "avh_tail_grad_count", "avh_tail_train_forward", "avh_full_grad_count", "avh_full_train_forward",
     "avh_set_train_args",
 ]
@@ -101,6 +101,8 @@ def load():
     lib.avh_grad_bucket_wait.argtypes = [vp, i32, vp]
     lib.avh_refresh_weights_device.argtypes = [vp, ctypes.POINTER(ctypes.c_char_p), ctypes.POINTER(vp), ctypes.POINTER(ctypes.c_int32),
                                                ctypes.POINTER(i64), i32, vp]
+    lib.avh_refresh_eval_weights_device.argtypes = lib.avh_refresh_weights_device.argtypes
+    lib.avh_plan_count.argtypes = [vp, ctypes.POINTER(ctypes.c_int32)]
     lib.avh_qformer_forward.argtypes = [vp, vp, i32, vp, ctypes.POINTER(ctypes.c_int32), i32, i32, i32, vp, i32, vp]
     lib.avh_mask_substitute.argtypes = [vp, i32, i32, ctypes.POINTER(i64), i32, i32, i32, vp, vp, i32, vp, vp, i32, vp]
     lib.avh_compute_logits.argtypes = [vp, i32, i64, vp, i32, i64, vp, i64, i32, i32, i32, ctypes.c_float, vp, i64, vp]

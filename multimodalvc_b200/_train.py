@@ -4,6 +4,7 @@ and — when a GradientAllReducer is attached to the module — the all-reduce o
 soon as the library has recorded the bucket's event, so that the collective overlaps the rest of the backward
 (fairseq legacy_distributed_data_parallel.py:76-165 does the reduction after the backward; same result)."""
 import ctypes
+import itertools
 
 import numpy as np
 import torch
@@ -98,9 +99,21 @@ def refresh_weights_device(handle, module, prefix=""):
     """After an optimizer step: rewrite the packed weights the training plans read from `module`'s device-resident
     parameters, in place and on the device (avh_refresh_weights_device) — plans and captured graphs stay valid, nothing
     crosses the host.  `prefix` maps the module's parameter names onto the state-dict keys the handle was loaded with."""
+    _refresh(handle, "avh_refresh_weights_device", module.named_parameters(), prefix)
+
+
+def refresh_eval_weights_device(handle, module, prefix=""):
+    """Before an eval forward that follows training: the same refresh on a trainable handle, then the eval-only packed
+    forms (BatchNorm folded with the running statistics, the conv2 + shortcut GEMM weights) from `module`'s parameters
+    and buffers, in place on the device (avh_refresh_eval_weights_device), bit-identical to a full re-pack."""
+    _refresh(handle, "avh_refresh_eval_weights_device", itertools.chain(module.named_parameters(), module.named_buffers()),
+             prefix)
+
+
+def _refresh(handle, entry, named_tensors, prefix):
     lib = _lib.load()
     names, tensors = [], []
-    for name, p in module.named_parameters():
+    for name, p in named_tensors:
         t = p.detach()
         if not t.is_floating_point():
             continue
@@ -116,4 +129,4 @@ def refresh_weights_device(handle, module, prefix=""):
     dev = tensors[0].device
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(lib.avh_refresh_weights_device(handle, c_names, c_ptrs, c_dts, c_num, n, ctypes.c_void_p(stream)))
+        _lib.check(getattr(lib, entry)(handle, c_names, c_ptrs, c_dts, c_num, n, ctypes.c_void_p(stream)))

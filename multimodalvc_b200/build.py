@@ -18,7 +18,10 @@ LIB = os.path.join(HERE, "libavh_b200.so")
 SOURCES = ["api.cu", "gemm_tcgen05.cu", "conv_window.cu", "conv_frame.cu", "stem_fused.cu", "attention.cu", "attention_tc.cu", "elementwise.cu", "train_ops.cu", "train_dropout.cu", "pretrain_ops.cu", "qformer.cu", "backward_ops.cu", "frontend_train.cu", "refresh.cu", "fbank.cu"]
 NVCC_FLAGS = ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr",
-              "-I", os.path.join(ROOT, "include"), "-I", CSRC]
+              "-I", os.path.join(ROOT, "include"), "-I", CSRC,
+              # host packers round every fp32 operation on its own, as the device refresh kernels do (bit-identical
+              # BatchNorm folds); x86-64 without -march has no FMA anyway, this keeps it so on hosts that do
+              "-Xcompiler", "-ffp-contract=off"]
 NVCC_FLAGS += os.environ.get("AVH_NVCC_EXTRA", "").split()      # e.g. -DAVH_STALL_ACC for tools/gemm_stall.py
 
 

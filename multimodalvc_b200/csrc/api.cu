@@ -350,6 +350,18 @@ struct avh_handle {
   // same tensors in place every step: ~650 small launches become one graph launch)
   std::vector<long long> refresh_key;
   cudaGraphExec_t refresh_exec = nullptr;
+  // every AV-HuBERT handle: how the EVAL-only packed forms derive from BatchNorm parameters and buffers and conv
+  // weights, recorded by the packers; avh_refresh_eval_weights_device replays the list (after the training-form jobs)
+  // with device kernels, captured as its own graph for the pointer set it was last called with
+  struct EvalJob {
+    std::string bn;               // fold: BatchNorm prefix of ".weight", ".bias", ".running_mean", ".running_var"
+    ConvUnit* cu = nullptr;       // fold: writes cu->scale, bias, gamma, beta, rmean, rvar
+    BlockW* bw = nullptr;         // c2ds: writes bw->c2ds and c2ds_bias from the folds of bw->c2 and bw->ds (earlier jobs)
+    std::string w2, wd;           // c2ds: state-dict keys of conv2 and downsample.0 weights
+  };
+  std::vector<EvalJob> eval_jobs;
+  std::vector<long long> eval_refresh_key;
+  cudaGraphExec_t eval_refresh_exec = nullptr;
   std::vector<LayerW> layers;
   // Q-Former handles (cfg.reserved[0] == 2): reserved[1] = encoder_width, reserved[2] = rows of query_tokens
   std::vector<QfLayerW> qf_layers;
@@ -444,6 +456,19 @@ struct Packer {
     h->refresh_jobs.push_back(j);
   }
   void job_vec(const std::string& src, float* dst, long long n, float scale = 1.f) { job(src, RJ_VEC, dst, n, 0, 0, 0, scale); }
+  // eval-only forms (every handle, real pass only)
+  void eval_fold(const std::string& bn, ConvUnit* cu) {
+    if (arena == nullptr) return;
+    avh_handle::EvalJob j;
+    j.bn = bn; j.cu = cu;
+    h->eval_jobs.push_back(j);
+  }
+  void eval_c2ds(const std::string& w2, const std::string& wd, BlockW* bw) {
+    if (arena == nullptr) return;
+    avh_handle::EvalJob j;
+    j.bw = bw; j.w2 = w2; j.wd = wd;
+    h->eval_jobs.push_back(j);
+  }
 };
 
 inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
@@ -485,6 +510,7 @@ bool pack_conv(Packer& pk, const std::string& wkey, const std::string& bnkey, co
   cu->bias = pk.upload_f(bi);
   cu->gamma = pk.upload_f(g->v); cu->beta = pk.upload_f(b->v);
   cu->rmean = pk.upload_f(m->v); cu->rvar = pk.upload_f(v->v);
+  pk.eval_fold(bnkey, cu);
   pk.job_vec(bnkey + ".weight", cu->gamma, cout);
   pk.job_vec(bnkey + ".bias", cu->beta, cout);
   cu->slope = nullptr;
@@ -645,6 +671,7 @@ bool pack_all(Packer& pk) {
       h->stem.slope = pk.upload_f(sl);
       h->stem.gamma = pk.upload_f(g->v); h->stem.beta = pk.upload_f(b->v);
       h->stem.rmean = pk.upload_f(m->v); h->stem.rvar = pk.upload_f(v->v);
+      pk.eval_fold(R + "frontend3D.1", &h->stem);
       pk.job_vec(R + "frontend3D.1.weight", h->stem.gamma, 64);
       pk.job_vec(R + "frontend3D.1.bias", h->stem.beta, 64);
       pk.job_vec(R + "frontend3D.2.weight", h->stem.slope, 64);
@@ -692,6 +719,7 @@ bool pack_all(Packer& pk) {
           bw.c2ds = pk.pack(packed, cout, K, K);
           bw.c2ds_bias = pk.upload_f(bias);
           bw.ones = pk.upload_f(ones);
+          pk.eval_c2ds(pre + "conv2.weight", pre + "downsample.0.weight", &bw);
         } else ok = false;
       }
       const HostTensor* s2 = pk.get(pre + "relu2.weight");
@@ -2726,6 +2754,7 @@ int avh_destroy(avh_handle* h) {
   }
   for (cudaEvent_t e : h->prof_events) cudaEventDestroy(e);
   if (h->refresh_exec) cudaGraphExecDestroy(h->refresh_exec);
+  if (h->eval_refresh_exec) cudaGraphExecDestroy(h->eval_refresh_exec);
   delete h;
   return 0;
 }
@@ -2770,6 +2799,9 @@ int avh_finalize_weights(avh_handle* h) {
   h->refresh_jobs.clear();
   if (h->refresh_exec) { cudaGraphExecDestroy(h->refresh_exec); h->refresh_exec = nullptr; }
   h->refresh_key.clear();
+  h->eval_jobs.clear();
+  if (h->eval_refresh_exec) { cudaGraphExecDestroy(h->eval_refresh_exec); h->eval_refresh_exec = nullptr; }
+  h->eval_refresh_key.clear();
   avh::Packer sizer{h, nullptr, avh::Sizer(), ""};
   const bool ok = avh::pack_all(sizer);
   AVH_CHECK(ok, "missing state-dict key: " + sizer.missing);
@@ -3310,42 +3342,45 @@ int avh_encoder_backward_buckets(avh_handle* h, const void* dout, int dout_dtype
   return encoder_backward(h, dout, dout_dtype, dx, dx_dtype, grads, grads_dtype, grads_capacity, true, stream);
 }
 
-int avh_refresh_weights_device(avh_handle* h, const char* const* names, const void* const* ptrs, const int32_t* dtypes,
-                               const int64_t* numels, int32_t count, void* stream) {
-  AVH_CHECK(h != nullptr && names != nullptr && ptrs != nullptr && dtypes != nullptr && numels != nullptr, "null argument");
-  AVH_CHECK(h->finalized, "weights not finalized (call avh_finalize_weights once; this call refreshes them in place)");
-  AVH_CHECK(h->cfg.reserved[3] != 0, "only trainable handles (avh_config.reserved[3] = 1) record how to refresh their weights");
-  AVH_CUDA_OK(cudaSetDevice(h->device));
-  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+// The caller's tensor list of a device refresh: state-dict key -> index, and the pointer set the captured graph is keyed on
+struct RefreshArgs {
   std::map<std::string, int> idx;
+  const void* const* ptrs = nullptr;
+  const int32_t* dtypes = nullptr;
+  const int64_t* numels = nullptr;
+  std::vector<long long> key;
+};
+
+static int refresh_args(const char* const* names, const void* const* ptrs, const int32_t* dtypes, const int64_t* numels,
+                        int32_t count, RefreshArgs* a) {
+  AVH_CHECK(names != nullptr && ptrs != nullptr && dtypes != nullptr && numels != nullptr, "null argument");
   for (int i = 0; i < count; ++i) {
     AVH_CHECK(names[i] != nullptr && ptrs[i] != nullptr, "null tensor in the parameter list");
     AVH_CHECK(dtypes[i] == AVH_F32 || dtypes[i] == AVH_F16 || dtypes[i] == AVH_BF16, "bad parameter dtype");
-    idx[names[i]] = i;
+    a->idx[names[i]] = i;
   }
-  // same parameter tensors as last time: replay the captured graph
-  std::vector<long long> key;
-  key.reserve(3 * (size_t)count);
+  a->ptrs = ptrs; a->dtypes = dtypes; a->numels = numels;
+  a->key.reserve(3 * (size_t)count);
   for (int i = 0; i < count; ++i) {
-    key.push_back((long long)reinterpret_cast<uintptr_t>(ptrs[i]));
-    key.push_back(dtypes[i]);
-    key.push_back(numels[i]);
+    a->key.push_back((long long)reinterpret_cast<uintptr_t>(ptrs[i]));
+    a->key.push_back(dtypes[i]);
+    a->key.push_back(numels[i]);
   }
-  if (h->refresh_exec != nullptr && key == h->refresh_key) {
-    AVH_CUDA_OK(cudaGraphLaunch(h->refresh_exec, s));
-    return 0;
-  }
-  auto run_jobs = [&]() -> int {
+  return 0;
+}
+
+// the training-form jobs (refresh_jobs; empty on handles that are not trainable)
+static int run_train_refresh(avh_handle* h, const RefreshArgs& a, cudaStream_t s) {
   const int P = h->P;
   const int KT = h->cfg.conv_pos;
   bool ratio_done = false;
   for (const avh_handle::RefreshJob& j : h->refresh_jobs) {
-    auto it = idx.find(j.src);
-    AVH_CHECK(it != idx.end(), "parameter missing from the refresh list: " + j.src);
+    auto it = a.idx.find(j.src);
+    AVH_CHECK(it != a.idx.end(), "parameter missing from the refresh list: " + j.src);
     const int i = it->second;
-    const void* src = ptrs[i];
-    const int dt = dtypes[i];
-    const long long ne = numels[i];
+    const void* src = a.ptrs[i];
+    const int dt = a.dtypes[i];
+    const long long ne = a.numels[i];
     switch (j.form) {
       case avh::RJ_MATRIX:
       case avh::RJ_MATRIX_T:
@@ -3370,9 +3405,9 @@ int avh_refresh_weights_device(avh_handle* h, const char* const* names, const vo
       case avh::RJ_POS_T: {
         AVH_CHECK(ne == j.n * j.k * KT && h->pos_ratio != nullptr, "parameter size changed: " + j.src);
         if (!ratio_done) {
-          auto ig = idx.find("encoder.pos_conv.0.weight_g");
-          AVH_CHECK(ig != idx.end() && numels[ig->second] == KT, "parameter missing from the refresh list: encoder.pos_conv.0.weight_g");
-          if (avh::launch_posconv_ratio(src, dt, ptrs[ig->second], dtypes[ig->second], j.n * j.k, KT, h->pos_ratio, s)) return 1;
+          auto ig = a.idx.find("encoder.pos_conv.0.weight_g");
+          AVH_CHECK(ig != a.idx.end() && a.numels[ig->second] == KT, "parameter missing from the refresh list: encoder.pos_conv.0.weight_g");
+          if (avh::launch_posconv_ratio(src, dt, a.ptrs[ig->second], a.dtypes[ig->second], j.n * j.k, KT, h->pos_ratio, s)) return 1;
           ratio_done = true;
         }
         if (avh::launch_refresh_pos(src, dt, h->pos_ratio, h->pos_acol, (int)j.n, (int)j.k, KT, h->pos_window, j.dst, P,
@@ -3385,31 +3420,104 @@ int avh_refresh_weights_device(avh_handle* h, const char* const* names, const vo
     }
   }
   return 0;
+}
+
+// the eval-only forms (eval_jobs): BatchNorm folds, then the conv2 + shortcut GEMM weights that read them
+static int run_eval_refresh(avh_handle* h, const RefreshArgs& a, cudaStream_t s) {
+  auto find = [&](const std::string& key, long long numel, int* i) -> int {
+    auto it = a.idx.find(key);
+    AVH_CHECK(it != a.idx.end(), "tensor missing from the refresh list: " + key);
+    AVH_CHECK(a.numels[it->second] == numel, "tensor size changed: " + key);
+    *i = it->second;
+    return 0;
   };
-  if (h->refresh_exec) { cudaGraphExecDestroy(h->refresh_exec); h->refresh_exec = nullptr; }
-  h->refresh_key.clear();
+  for (const avh_handle::EvalJob& j : h->eval_jobs) {
+    if (j.bw == nullptr) {
+      ConvUnit* cu = j.cu;
+      const char* part[4] = {".weight", ".bias", ".running_mean", ".running_var"};
+      int i[4];
+      for (int t = 0; t < 4; ++t)
+        if (find(j.bn + part[t], cu->cout, &i[t])) return 1;
+      if (avh::launch_bn_fold(a.ptrs[i[0]], a.dtypes[i[0]], a.ptrs[i[1]], a.dtypes[i[1]], a.ptrs[i[2]], a.dtypes[i[2]], a.ptrs[i[3]],
+                              a.dtypes[i[3]], cu->cout, cu->scale, cu->bias, cu->gamma, cu->beta, cu->rmean, cu->rvar, s))
+        return 1;
+    } else {
+      const BlockW* bw = j.bw;
+      const int cout = bw->c2.cout, cmid = bw->c2.cin, cin = bw->ds.cin;
+      int i2, id;
+      if (find(j.w2, 9LL * cout * cmid, &i2) || find(j.wd, (long long)cout * cin, &id)) return 1;
+      if (avh::launch_refresh_c2ds(a.ptrs[i2], a.dtypes[i2], a.ptrs[id], a.dtypes[id], bw->c2.scale, bw->c2.bias, bw->ds.scale,
+                                   bw->ds.bias, cout, cmid, cin, bw->c2ds.w, h->P, bw->c2ds_bias, s))
+        return 1;
+    }
+  }
+  return 0;
+}
+
+// Runs `jobs` on `s` through a CUDA graph captured for the pointer set `key` (an optimizer updates the same tensors in
+// place every step: hundreds of small launches become one graph launch); `*exec` / `*exec_key` cache the graph.  Directly
+// where the stream cannot be captured (the legacy default stream).
+static int replay_refresh(cudaStream_t s, const std::vector<long long>& key, cudaGraphExec_t* exec, std::vector<long long>* exec_key,
+                          const std::function<int()>& jobs) {
+  if (*exec != nullptr && key == *exec_key) {
+    AVH_CUDA_OK(cudaGraphLaunch(*exec, s));
+    return 0;
+  }
+  if (*exec) { cudaGraphExecDestroy(*exec); *exec = nullptr; }
+  exec_key->clear();
   read_graphs_env();
   cudaStreamCaptureStatus cap_status = cudaStreamCaptureStatusNone;
   const bool real_stream = s != nullptr && s != cudaStreamLegacy && s != cudaStreamPerThread;
   if (real_stream) cudaStreamIsCapturing(s, &cap_status);
   if (graphs_env == 1 && real_stream && cap_status == cudaStreamCaptureStatusNone &&
       cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-    const int rc = run_jobs();
+    const int rc = jobs();
     cudaGraph_t graph = nullptr;
     const cudaError_t e = cudaStreamEndCapture(s, &graph);
-    cudaGraphExec_t exec = nullptr;
-    const bool ok = rc == 0 && e == cudaSuccess && graph != nullptr && cudaGraphInstantiate(&exec, graph, 0) == cudaSuccess;
+    cudaGraphExec_t ex = nullptr;
+    const bool ok = rc == 0 && e == cudaSuccess && graph != nullptr && cudaGraphInstantiate(&ex, graph, 0) == cudaSuccess;
     if (graph != nullptr) cudaGraphDestroy(graph);
     if (rc != 0) return 1;                         // a real error (missing / resized parameter): reported as is
     if (ok) {
-      h->refresh_exec = exec;
-      h->refresh_key = key;
-      AVH_CUDA_OK(cudaGraphLaunch(exec, s));
+      *exec = ex;
+      *exec_key = key;
+      AVH_CUDA_OK(cudaGraphLaunch(ex, s));
       return 0;
     }
   }
   cudaGetLastError();                              // capture not possible on this stream (legacy default stream): direct
-  return run_jobs();
+  return jobs();
+}
+
+int avh_refresh_weights_device(avh_handle* h, const char* const* names, const void* const* ptrs, const int32_t* dtypes,
+                               const int64_t* numels, int32_t count, void* stream) {
+  AVH_CHECK(h != nullptr, "null argument");
+  AVH_CHECK(h->finalized, "weights not finalized (call avh_finalize_weights once; this call refreshes them in place)");
+  AVH_CHECK(h->cfg.reserved[3] != 0, "only trainable handles (avh_config.reserved[3] = 1) record how to refresh their weights");
+  AVH_CUDA_OK(cudaSetDevice(h->device));
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  RefreshArgs a;
+  if (refresh_args(names, ptrs, dtypes, numels, count, &a)) return 1;
+  return replay_refresh(s, a.key, &h->refresh_exec, &h->refresh_key, [&]() { return run_train_refresh(h, a, s); });
+}
+
+int avh_refresh_eval_weights_device(avh_handle* h, const char* const* names, const void* const* ptrs, const int32_t* dtypes,
+                                    const int64_t* numels, int32_t count, void* stream) {
+  AVH_CHECK(h != nullptr, "null argument");
+  AVH_CHECK(h->finalized, "weights not finalized (call avh_finalize_weights once; this call refreshes them in place)");
+  AVH_CHECK(h->cfg.reserved[0] != 2, "Q-Former handles have no device refresh (reload the weights and finalize)");
+  AVH_CUDA_OK(cudaSetDevice(h->device));
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  RefreshArgs a;
+  if (refresh_args(names, ptrs, dtypes, numels, count, &a)) return 1;
+  return replay_refresh(s, a.key, &h->eval_refresh_exec, &h->eval_refresh_key,
+                        [&]() { return run_train_refresh(h, a, s) || run_eval_refresh(h, a, s) ? 1 : 0; });
+}
+
+int avh_plan_count(avh_handle* h, int32_t* count) {
+  AVH_CHECK(h != nullptr && count != nullptr, "null argument");
+  *count = (int32_t)h->plans.size();
+  return 0;
 }
 
 int avh_grad_bucket_count(avh_handle* h, int32_t* count) {

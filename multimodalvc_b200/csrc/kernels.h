@@ -162,6 +162,12 @@ int launch_posconv_ratio(const void* v, int v_dt, const void* g, int g_dt, long 
                          cudaStream_t stream);
 int launch_refresh_pos(const void* v, int dt, const float* ratio, const int* acol, int D, int cg, int KT, int window, void* dst,
                        int planes, int transposed, cudaStream_t stream);
+// eval-only forms: the BatchNorm fold (scale / bias, and the fp32 gamma / beta / running statistics) and the conv2 +
+// shortcut GEMM weights with both BatchNorm scales folded in, bit-identical to the host packers
+int launch_bn_fold(const void* g, int g_dt, const void* b, int b_dt, const void* m, int m_dt, const void* v, int v_dt, int C,
+                   float* scale, float* bias, float* gamma, float* beta, float* rmean, float* rvar, cudaStream_t stream);
+int launch_refresh_c2ds(const void* w2, int w2_dt, const void* wd, int wd_dt, const float* s2, const float* b2, const float* sd,
+                        const float* bd, int cout, int cmid, int cin, void* dst, int planes, float* bias, cudaStream_t stream);
 int launch_im2colT(const void* x, long long n, int H, int C, int ks, int stride, int pad, int Ho, void* colT, long long kp,
                    cudaStream_t stream);          // bf16 x -> bf16 colT [ks*ks*C, kp] (transposed patches)
 int launch_transposeT(const void* in, int dt, long long ld, long long rows, int C, void* out, long long kp, long long out_ld,

@@ -3,7 +3,8 @@
 // convolution and their transposes, fp32 vectors, the weight-normed positional convolution) IN PLACE, so that plans and
 // captured graphs stay valid and no byte crosses the host.  Layouts are the ones pack_all (api.cu) produces on the host:
 // each kernel is the index map of one packer.  (avh_finalize_weights re-packs everything through the host: 6 s for the
-// Large model against a 32 ms training step.)
+// Large model against a 32 ms training step.)  Before the first eval forward after training, the eval-only forms
+// (BatchNorm folds, the conv2 + shortcut GEMM weights) are recomputed here too, bit-identical to the host packers.
 #include "common.cuh"
 #include "kernels.h"
 
@@ -103,6 +104,46 @@ refresh_pos_kernel(const void* __restrict__ v, int dt, const float* __restrict__
   }
 }
 
+// Eval-mode BatchNorm fold per channel, exactly as the host packers compute it (pack_conv, the stem, bn_fold in
+// pack_all): inv = 1 / sqrt(var + 1e-5f), scale = gamma * inv, bias = beta - mean * scale, every operation rounded on
+// its own (the intrinsics keep nvcc from contracting into an FMA, which the host code does not do either).  Also
+// writes the fp32 copies the training-mode BatchNorm starts from.
+__global__ void bn_fold_kernel(const void* __restrict__ g, int g_dt, const void* __restrict__ b, int b_dt,
+                               const void* __restrict__ m, int m_dt, const void* __restrict__ v, int v_dt, int C,
+                               float* __restrict__ scale, float* __restrict__ bias, float* __restrict__ gamma,
+                               float* __restrict__ beta, float* __restrict__ rmean, float* __restrict__ rvar) {
+  const int o = blockIdx.x * blockDim.x + threadIdx.x;
+  if (o >= C) return;
+  const float gv = ldw(g, g_dt, o), bv = ldw(b, b_dt, o), mv = ldw(m, m_dt, o), vv = ldw(v, v_dt, o);
+  const float inv = __fdiv_rn(1.0f, __fsqrt_rn(__fadd_rn(vv, 1e-5f)));
+  const float sc = __fmul_rn(gv, inv);
+  scale[o] = sc;
+  bias[o] = __fsub_rn(bv, __fmul_rn(mv, sc));
+  gamma[o] = gv; beta[o] = bv; rmean[o] = mv; rvar[o] = vv;
+}
+// conv2 + 1x1 shortcut as one GEMM (bf16 frame-row path): [cout, planes*K], K = 9*cmid + cin; column t*cmid + c holds
+// s2[o] * w2[o, c, t], column 9*cmid + c holds sd[o] * wd[o, c]; bias[o] = b2[o] + bd[o] (the folds of bn_fold_kernel)
+__global__ void __launch_bounds__(256)
+refresh_c2ds_kernel(const void* __restrict__ w2, int w2_dt, const void* __restrict__ wd, int wd_dt, const float* __restrict__ s2,
+                    const float* __restrict__ b2, const float* __restrict__ sd, const float* __restrict__ bd, int cout, int cmid,
+                    int cin, __nv_bfloat16* __restrict__ dst, int planes, float* __restrict__ bias) {
+  const long long K = 9LL * cmid + cin;
+  const long long total = (long long)cout * K;
+  for (long long i = (long long)blockIdx.x * 256 + threadIdx.x; i < total; i += (long long)gridDim.x * 256) {
+    const int o = (int)(i / K);
+    const long long kidx = i % K;
+    float val;
+    if (kidx < 9LL * cmid) {
+      const int t = (int)(kidx / cmid), c = (int)(kidx % cmid);
+      val = __fmul_rn(s2[o], ldw(w2, w2_dt, ((long long)o * cmid + c) * 9 + t));
+    } else {
+      val = __fmul_rn(sd[o], ldw(wd, wd_dt, (long long)o * cin + (kidx - 9LL * cmid)));
+    }
+    st_planes(dst, (long long)o * planes * K + kidx, K, planes, val);
+    if (kidx == 0) bias[o] = __fadd_rn(b2[o], bd[o]);
+  }
+}
+
 inline unsigned grid_of(long long n) {
   const long long b = (n + 255) / 256;
   return (unsigned)(b < 148 * 16 ? (b > 0 ? b : 1) : 148 * 16);
@@ -150,6 +191,20 @@ int launch_refresh_pos(const void* v, int dt, const float* ratio, const int* aco
                        int planes, int transposed, cudaStream_t stream) {
   refresh_pos_kernel<<<grid_of((long long)D * cg * KT), 256, 0, stream>>>(v, dt, ratio, acol, D, cg, KT, window,
                                                                          reinterpret_cast<__nv_bfloat16*>(dst), planes, transposed);
+  AVH_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+int launch_bn_fold(const void* g, int g_dt, const void* b, int b_dt, const void* m, int m_dt, const void* v, int v_dt, int C,
+                   float* scale, float* bias, float* gamma, float* beta, float* rmean, float* rvar, cudaStream_t stream) {
+  if (C <= 0) return 0;
+  bn_fold_kernel<<<(C + 255) / 256, 256, 0, stream>>>(g, g_dt, b, b_dt, m, m_dt, v, v_dt, C, scale, bias, gamma, beta, rmean, rvar);
+  AVH_CUDA_OK(cudaGetLastError());
+  return 0;
+}
+int launch_refresh_c2ds(const void* w2, int w2_dt, const void* wd, int wd_dt, const float* s2, const float* b2, const float* sd,
+                        const float* bd, int cout, int cmid, int cin, void* dst, int planes, float* bias, cudaStream_t stream) {
+  refresh_c2ds_kernel<<<grid_of((long long)cout * (9LL * cmid + cin)), 256, 0, stream>>>(
+      w2, w2_dt, wd, wd_dt, s2, b2, sd, bd, cout, cmid, cin, reinterpret_cast<__nv_bfloat16*>(dst), planes, bias);
   AVH_CUDA_OK(cudaGetLastError());
   return 0;
 }

@@ -19,7 +19,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib, masking
-from ._train import StepRegularization, backward_flat, refresh_weights_device
+from ._train import StepRegularization, backward_flat, refresh_eval_weights_device, refresh_weights_device
 
 _DTYPES = {torch.float32: _lib.AVH_F32, torch.float16: _lib.AVH_F16, torch.bfloat16: _lib.AVH_BF16}
 _U8 = _lib.AVH_U8        # raw uint8 video frames (normalised + centre-cropped on the device)
@@ -384,7 +384,8 @@ class AVHubertModel(nn.Module):
     def _sync_trained_weights(self):
         """Training steps: when an optimizer step changed the parameters since the last forward, refresh the packed
         copies the training plans read — on the device, in place (a few ms; the full re-pack through the host takes
-        seconds for Large).  The eval-only packed forms are left stale: the next eval forward re-packs everything."""
+        seconds for Large).  The eval-only packed forms are left stale: the next eval forward refreshes them on the
+        device (_ensure_handle)."""
         versions = [p._version for p in self.parameters()]
         if self._param_versions == versions:
             return
@@ -425,10 +426,17 @@ class AVHubertModel(nn.Module):
                                "device (there is no CPU path)")
         key = (p.device.index if p.device.index is not None else torch.cuda.current_device(),
                self._compute_mode(p.dtype))
+        live = self._handle is not None and key == self._handle_key and not self._dirty
         if not self.training and getattr(self, "_eval_stale", False):
-            # training moved the BatchNorm running statistics / a device-side refresh skipped the eval-only packed forms
-            self._dirty, self._eval_stale = True, False
-        if self._handle is not None and key == self._handle_key and not self._dirty:
+            # training moved the BatchNorm running statistics / a device-side refresh skipped the eval-only packed forms:
+            # refresh them (and, on a trainable handle, every training form) in place on the device from the parameters
+            # and buffers — plans, arenas and captured graphs stay; without a live handle the re-pack below does it
+            self._eval_stale = False
+            if live:
+                refresh_eval_weights_device(self._handle, self)
+                if self.cfg.trainable:
+                    self._param_versions = [p._version for p in self.parameters()]
+        if live:
             return self._handle
         lib = _lib.load()
         if self._handle is None or key != self._handle_key:
@@ -719,9 +727,6 @@ class AVHubertModel(nn.Module):
             src_audio, _ = self.apply_input_mask(source["audio"], padding_mask, None)
             source = {"audio": src_audio, "video": src_video}
         self._check_mode(False, allow_train=True)
-        if not self.training and getattr(self, "_eval_stale", False):
-            # training-mode forwards moved the BatchNorm running statistics: fold the current ones for eval
-            self._dirty, self._eval_stale = True, False
         handle = self._ensure_handle()
         dev = self.encoder.layer_norm.weight.device
         src_video, video_dt, src_audio, pm_u8, padding_mask, B, T = self._check_inputs(

@@ -22,7 +22,7 @@ import torch
 import torch.nn as nn
 
 from . import _lib
-from ._train import StepRegularization, backward_flat, refresh_weights_device
+from ._train import StepRegularization, backward_flat, refresh_eval_weights_device, refresh_weights_device
 from .hubert import _DTYPES, _EncoderParams
 from .hubert_asr import _project
 
@@ -122,9 +122,15 @@ class TransformerEncoder(nn.Module):
             raise RuntimeError("multimodalvc_b200.TransformerEncoder computes on a B200 only (there is no CPU path)")
         mode = _lib.AVH_COMPUTE_FP32 if p.dtype == torch.float32 else _lib.AVH_COMPUTE_BF16
         key = (p.device.index if p.device.index is not None else torch.cuda.current_device(), mode)
+        live = self._handle is not None and key == self._handle_key and not self._dirty
         if not self.training and getattr(self, "_eval_stale", False):
-            self._dirty, self._eval_stale = True, False      # the device-side refresh skipped the eval-only packed forms
-        if self._handle is not None and key == self._handle_key and not self._dirty:
+            # trained since the last eval forward: refresh the packed weights from the parameters in place on the device
+            # (a bare encoder has no eval-only forms; this picks up the optimizer steps since the last training forward)
+            self._eval_stale = False
+            if live:
+                refresh_eval_weights_device(self._handle, self, "encoder.")
+                self._versions = [p._version for p in self.parameters()]
+        if live:
             return self._handle
         lib = _lib.load()
         if self._handle is None or key != self._handle_key:
@@ -192,7 +198,7 @@ class TransformerEncoder(nn.Module):
             self._dirty = True
         elif any(p._version != v for p, v in zip(self.parameters(), self._versions)):
             if self._handle is not None and not self._dirty:     # an optimizer step changed the weights: refresh the packed
-                refresh_weights_device(self._handle, self, "encoder.")   # copies in place on the device (eval forms go stale)
+                refresh_weights_device(self._handle, self, "encoder.")   # copies in place on the device
                 self._eval_stale = True
             else:
                 self._dirty = True
