@@ -162,6 +162,16 @@ AVH_API int avh_compute_logits(const void* feats, int f_dtype, int64_t ldf, cons
                                int64_t ldo, void* stream);
 /* *acc (device double) = sum of x[i]^2 — features_pen = features.float().pow(2).mean() (hubert.py:629) times numel. */
 AVH_API int avh_sum_squares(const void* x, int dtype, int64_t n, double* acc, void* stream);
+/* Backward of avh_compute_logits, same argument conventions: from the forward's feats, emb, logits (fp32 [M,V], read by
+ * sim_type 1 only; may be NULL for 'dot') and dlogits = dL/dlogits (fp32 [M,V]; logits and dlogits share the row stride
+ * ldo), writes dfeats = dL/dfeats (fp32 [M,K], row stride ldd_f), demb = dL/demb (fp32 [V,K], row stride ldd_e) and
+ * dbias = dL/dbias (fp32 [V]); any of the three may be NULL.  Cosine: where |feats_m| |emb_v| < 1e-6 the clamped
+ * denominator is a constant (torch.clamp's gradient).  fp32 arithmetic, every reduction in a fixed order (repeat calls are
+ * bit-identical).  With sim_type 0, logit_temp 1 this is the backward of final_proj. */
+AVH_API int avh_compute_logits_backward(const void* feats, int f_dtype, int64_t ldf, const void* emb, int e_dtype, int64_t lde,
+                                        int64_t M, int V, int K, int sim_type, float logit_temp, const float* logits,
+                                        const float* dlogits, int64_t ldo, float* dfeats, int64_t ldd_f, float* demb,
+                                        int64_t ldd_e, float* dbias, void* stream);
 
 /* Kernel-level entry point of the dropout used above (tests): x[i] = keep(i) ? x[i] / (1 - p) : 0 in place, keep(i) a
  * pure function of (seed, site, i) through Philox4x32-10 — nn.Dropout semantics, this library's own random stream. */
@@ -267,6 +277,23 @@ AVH_API int avh_full_grad_count(avh_handle* h, int has_video, int has_audio, int
 AVH_API int avh_full_train_forward(avh_handle* h, const void* video, int video_dtype, const void* audio, int audio_dtype,
                                    const int64_t* audio_strides, const uint8_t* padding_mask, int B, int T,
                                    float feature_grad_mult, float bn_momentum, void* out, int out_dtype, void* stream);
+
+/* Pretraining step (AVHubertModel.forward in training mode, avhubert/hubert.py:591-674).  avh_set_modality_drop marks the
+ * NEXT avh_forward_train or avh_full_train_forward on the handle, which consumes it, as a pretraining step that drops
+ * `which` modality (0 none, 1 audio, 2 video: the reference's two coins, hubert.py:611-616, drawn by the caller).  Both
+ * modalities must be given.  The dropped arm's projection output is zeros in the fused features, concat or add fusion;
+ * the lip ResNet still runs when video is dropped (its BatchNorm running statistics move).  The backward of a full step
+ * skips the dropped arm and writes zeros into its gradients.  The decision does not select the launch plan (a step
+ * replays its CUDA graphs for any decision); marking a step does.  The frozen-extractor step (avh_tail_train_forward)
+ * takes fused features that already hold the zeros.
+ * avh_train_features_pen: *acc (device double) = sum of squares of the fused features [B,T,E] of the last training
+ * forward on the handle (avh_forward_train, avh_tail_train_forward, avh_full_train_forward); features_pen = *acc / (B T E).
+ * avh_set_features_pen_grad: after a marked avh_full_train_forward and before its backward, dL/dfeatures_pen (a device
+ * float, NULL = 0; 0 unless set) — copied into the plan on `stream`; the backward adds (2 dL/dpen / (B T E)) fused to
+ * dL/dfused before the feature_grad_mult scaling. */
+AVH_API int avh_set_modality_drop(avh_handle* h, int which);
+AVH_API int avh_train_features_pen(avh_handle* h, double* acc, void* stream);
+AVH_API int avh_set_features_pen_grad(avh_handle* h, const float* dpen, void* stream);
 
 /* The Q-Former that compresses the fused AV features into query tokens in MMS-LLaMA (SURVEY 8(f) rank 3):
  * Qformer.bert(query_embeds=query_tokens[:, :Lq], attention_mask, encoder_hidden_states=enc, encoder_attention_mask)

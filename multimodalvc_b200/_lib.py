@@ -24,7 +24,8 @@ EXPORTS = [
     "avh_encoder_backward_buckets", "avh_grad_bucket_count", "avh_grad_bucket_range", "avh_grad_bucket_wait",
     "avh_refresh_weights_device", "avh_refresh_eval_weights_device", "avh_plan_count",
     "avh_tail_grad_count", "avh_tail_train_forward", "avh_full_grad_count", "avh_full_train_forward",
-    "avh_set_train_args",
+    "avh_set_train_args", "avh_compute_logits_backward", "avh_set_modality_drop", "avh_train_features_pen",
+    "avh_set_features_pen_grad",
 ]
 
 
@@ -107,6 +108,11 @@ def load():
     lib.avh_mask_substitute.argtypes = [vp, i32, i32, ctypes.POINTER(i64), i32, i32, i32, vp, vp, i32, vp, vp, i32, vp]
     lib.avh_compute_logits.argtypes = [vp, i32, i64, vp, i32, i64, vp, i64, i32, i32, i32, ctypes.c_float, vp, i64, vp]
     lib.avh_sum_squares.argtypes = [vp, i32, i64, vp, vp]
+    lib.avh_compute_logits_backward.argtypes = [vp, i32, i64, vp, i32, i64, i64, i32, i32, i32, ctypes.c_float, vp, vp, i64,
+                                                vp, i64, vp, i64, vp, vp]
+    lib.avh_set_modality_drop.argtypes = [vp, i32]
+    lib.avh_train_features_pen.argtypes = [vp, vp, vp]
+    lib.avh_set_features_pen_grad.argtypes = [vp, vp, vp]
     lib.avh_dropout.argtypes = [vp, i32, i64, ctypes.c_float, ctypes.c_uint64, ctypes.c_uint32, vp]
     lib.avh_bn_stats_count.argtypes = [vp, ctypes.POINTER(i64)]
     lib.avh_read_bn_stats.argtypes = [vp, vp, i64, vp]

@@ -164,6 +164,8 @@ struct Step {
   int layer = -1;         // encoder layer the step belongs to (LayerDrop skips it in training mode), -1 = none
   bool direct = false;    // reads or writes a CALLER pointer (video, audio, features, output): never part of a CUDA graph
   bool on_drop = false;   // runs only when its layer is dropped (the identity that stands in for the layer)
+  int mod = 0;            // modality dropout: 1 audio / 2 video arm of the step (skipped when that modality is dropped;
+                          // an on_drop step runs only then), 0 = none
 };
 
 struct CallArgs {          // per-call pointers the steps read through the plan
@@ -215,13 +217,17 @@ struct PlanKey {
   // caller draws LayerDrop coins; all 0 / false: the launch list of a step without regularisation
   float p_in = 0.f, p_enc = 0.f, p_act = 0.f;
   bool layerdrop = false;
+  // pretraining steps (avh_set_modality_drop): the plan can drop a modality (TrainForward / FullTrain with both
+  // modalities), and the FullTrain backward adds the features_pen gradient to dL/d(fused); both false: the launch list
+  // of a fine-tuning step
+  bool moddrop = false, pen = false;
   bool training() const { return kind == PlanKind::EncoderTrain || kind == PlanKind::TailTrain || kind == PlanKind::FullTrain; }
   bool dropout() const { return p_in > 0.f || p_enc > 0.f || p_act > 0.f; }
   bool operator<(const PlanKey& o) const {
     return std::tie(kind, B, T, has_video, has_audio, has_mask, output_layer, ragged_rows, Lk, stream, p_in, p_enc, p_act,
-                    layerdrop) <
+                    layerdrop, moddrop, pen) <
            std::tie(o.kind, o.B, o.T, o.has_video, o.has_audio, o.has_mask, o.output_layer, o.ragged_rows, o.Lk, o.stream, o.p_in,
-                    o.p_enc, o.p_act, o.layerdrop);
+                    o.p_enc, o.p_act, o.layerdrop, o.moddrop, o.pen);
   }
 };
 
@@ -230,6 +236,10 @@ struct Plan {
   float p_in = 0.f, p_enc = 0.f, p_act = 0.f, bn_momentum = 0.1f;     // training-mode forward: set per call
   unsigned long long seed = 0;
   std::vector<unsigned char> layer_skip;
+  int mod_drop = 0;                // modality dropped by the current step (key.moddrop plans): 0 none, 1 audio, 2 video
+  float* dpen = nullptr;           // key.pen plans: dL/dfeatures_pen of the current step (device word, avh_set_features_pen_grad)
+  const void* fused_buf = nullptr; // fused features [B*T, E] of the last forward (avh_train_features_pen)
+  int fused_dt = 0;
   size_t fwd_steps = 0;
   float* grads = nullptr;
   long long grad_floats = 0;
@@ -389,6 +399,9 @@ struct avh_handle {
     std::vector<unsigned char> skip;      // LayerDrop coins (1 = dropped); empty = LayerDrop off
   };
   NextTrain next_train;
+  // avh_set_modality_drop: the next training forward is a pretraining step dropping this modality (0 none, 1 audio,
+  // 2 video); -1 = not a pretraining step
+  int next_mod_drop = -1;
 };
 
 namespace avh {
@@ -908,6 +921,7 @@ struct Builder {
   size_t sk_bytes = 0;
   int* sk_flags = nullptr;
   int cur_layer = -1;           // encoder layer of the steps pushed next (LayerDrop skips a dropped layer's steps)
+  int cur_mod = 0;              // modality arm of the steps pushed next (modality dropout skips a dropped arm's steps)
 
   Builder(avh_handle* h_, Plan* plan_, bool sizing_)
       : h(h_), plan(plan_), sizing(sizing_), P(h_->P), f32(h_->cfg.compute_mode == AVH_COMPUTE_FP32) {
@@ -945,15 +959,24 @@ struct Builder {
 
   // `direct`: the step reads or writes caller pointers, so it is launched outside the CUDA graphs
   void push(const std::string& tag, std::function<int(cudaStream_t)> f, double flops = 0.0, bool direct = false) {
-    if (!sizing) plan->steps.push_back(Step{std::move(f), tag, flops, cur_layer, direct});
+    if (!sizing) plan->steps.push_back(Step{std::move(f), tag, flops, cur_layer, direct, false, cur_mod});
   }
   void push_direct(const std::string& tag, std::function<int(cudaStream_t)> f, double flops = 0.0) {
     push(tag, std::move(f), flops, true);
   }
-  // a step of layer cur_layer that runs only when LayerDrop drops that layer (launched directly, between the graphs
-  // of the layers around it)
+  // a step of layer cur_layer (or of modality arm cur_mod) that runs only when LayerDrop drops that layer (modality
+  // dropout that arm), launched directly, between the graphs around it
   void push_on_drop(const std::string& tag, std::function<int(cudaStream_t)> f) {
-    if (!sizing) plan->steps.push_back(Step{std::move(f), tag, 0.0, cur_layer, true, true});
+    if (!sizing) plan->steps.push_back(Step{std::move(f), tag, 0.0, cur_layer, true, true, cur_mod});
+  }
+  // dropped modality arm: zero `cols` columns of fused rows [rows, ld] (elements of es bytes) from column `off`
+  void zero_cols_on_drop(int mod, void* base, long long rows, int ld, int off, int cols, size_t elem) {
+    cur_mod = mod;
+    char* p = reinterpret_cast<char*>(base) + (size_t)off * elem;
+    push_on_drop("modality_drop", [=](cudaStream_t s) {
+      return cudaMemset2DAsync(p, (size_t)ld * elem, 0, (size_t)cols * elem, (size_t)rows, s) == cudaSuccess ? 0 : 1;
+    });
+    cur_mod = 0;
   }
   // fp32 [rows, C] (row stride ld) -> GEMM-operand form (bf16 [rows, P*C])
   void split(const float* src, int ld, void* dst, long long rows, int C) {
@@ -1352,13 +1375,18 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     // ---- SubModel.proj (hubert.py:321,327): Linear 512 -> D into the video columns of the fused buffer
     Epilogue ep = epilogue(reinterpret_cast<char*>(fused.data) + (size_t)v_off * es, E, f32);
     ep.col_bias = h->proj_v.bias;
+    if (key.moddrop) b.cur_mod = 2;
     if (!b.linear("proj_video", pooled_feat.op, N, 512, h->proj_v.w, ep)) return false;
+    // features_video = 0 * features_video (hubert.py:611-616): the ResNet still ran (its running statistics moved); add
+    // fusion: the audio projection adds onto these zeros
+    if (key.moddrop) b.zero_cols_on_drop(2, fused.data, N, E, v_off, D, es);
   }
   // ========================================================================== audio arm
   if (key.has_audio) {
     const int Fa = c.audio_feat_dim, Fp = round_up(Fa, 64);
     Act arows = b.act(N, Fp);       // zero-initialised; only the first Fa columns are ever written
     void* dst = arows.data;
+    if (key.moddrop) b.cur_mod = 1;     // a dropped audio arm: its projection is skipped
     if (rg)
       b.push_direct("audio_rows", [=](cudaStream_t s) {
         return launch_bct_to_rows_ragged(pl->args.audio, pl->args.audio_dt, pl->args.as[0], pl->args.as[1], pl->args.as[2],
@@ -1376,6 +1404,9 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
       ep.R = ep.C; ep.ldr = E; ep.r_fp32 = f32 ? 1 : 0;
     }
     if (!b.linear("proj_audio", arows.op, N, Fp, h->proj_a.w, ep)) return false;
+    b.cur_mod = 0;
+    // features_audio = 0 * features_audio: with add fusion the skipped projection leaves the video features alone
+    if (key.moddrop && c.modality_fuse == AVH_FUSE_CONCAT) b.zero_cols_on_drop(1, fused.data, N, E, a_off, D, es);
   }
   // a missing modality contributes zeros [B,D,T] (hubert.py:703-708): with concat its columns stay at the
   // arena's zero fill (nothing ever writes them for this plan); with add there is nothing to add.
@@ -1389,6 +1420,7 @@ bool build_plan(avh_handle* h, Plan* plan, bool sizing, size_t* bytes_out) {
     });
   } else {
     b.stage("fused", fused.data, act_dt, N * E);     // pre-LayerNorm features (features_pen)
+    if (!sizing) { plan->fused_buf = fused.data; plan->fused_dt = act_dt; }
     Act lnE = b.act(N, E);
     if (h->has_post_proj) {
       b.layernorm("fuse_ln", fused.data, act_dt, h->fuse_ln_g, h->fuse_ln_b, 1e-5f, lnE);
@@ -1868,11 +1900,14 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       }
       Epilogue ep = epilogue(fused + v_off, E, true);
       ep.col_bias = h->proj_v.bias;
+      if (key.moddrop) b.cur_mod = 2;      // modality dropout as in the training-mode forward (build_plan)
       if (!b.linear("proj_video", feat.op, N, 512, h->proj_v.w, ep)) return false;
+      if (key.moddrop) b.zero_cols_on_drop(2, fused, N, E, v_off, D, 4);
     }
     if (key.has_audio) {
       arows = b.act(N, Fp);
       void* dst = arows.data;
+      if (key.moddrop) b.cur_mod = 1;
       b.push_direct("audio_rows", [=](cudaStream_t s) {
         return launch_bct_to_rows(pl->args.audio, pl->args.audio_dt, pl->args.as[0], pl->args.as[1], pl->args.as[2], B, Fa, T, dst,
                                   act_dt, Fp, s);
@@ -1882,6 +1917,8 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       ep.col_bias = h->proj_a.bias;
       if (c.modality_fuse == AVH_FUSE_ADD && key.has_video) { ep.R = ep.C; ep.ldr = E; ep.r_fp32 = 1; }
       if (!b.linear("proj_audio", arows.op, N, Fp, h->proj_a.w, ep)) return false;
+      b.cur_mod = 0;
+      if (key.moddrop && c.modality_fuse == AVH_FUSE_CONCAT) b.zero_cols_on_drop(1, fused, N, E, 0, D, 4);
     }
   }
   if (tail) {
@@ -1894,6 +1931,7 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
         return launch_load_rows(pl->args.xin, pl->args.xin_dt, fused, nullptr, N, E, s);
       });
     }
+    if (!sizing) { plan->fused_buf = fused; plan->fused_dt = DT_F32; }
     if (h->has_post_proj) {
       b.layernorm("fuse_ln", fused, DT_F32, h->fuse_ln_g, h->fuse_ln_b, 1e-5f, fln);
       Epilogue ep = epilogue(x0, D, true);
@@ -2264,6 +2302,13 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
       if (full) {
         // ============================================================ backward of the feature extractors (mode 2)
         float* gf = g_ln + 2ll * E;                         // frontend gradients follow layer_norm.{weight,bias}
+        if (key.pen) {      // features_pen = fused.pow(2).mean() (hubert.py:629) enters the extractors through GradMultiply too
+          float* dp = b.f32buf(4);
+          if (!sizing) plan->dpen = dp;
+          const float* fu = fused;
+          const float sc = 2.0f / (float)(N * E);
+          b.push("pen_grad", [=](cudaStream_t s) { return launch_pen_grad(fu, dfused, N * E, dp, sc, s); });
+        }
         b.push("scale", [=](cudaStream_t s) {               // GradMultiply on the extractor outputs (grad_multiply.py:105-114)
           return pl->fgm != 1.f ? launch_scale(dfused, N * E, pl->fgm, s) : 0;
         });
@@ -2344,12 +2389,25 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
             b.push("bias_grad", [=](cudaStream_t s) { return launch_colsum(dyv, dy_dt, ld_dy, rows, n_out, db, 1.0f, s); });
           return true;
         };
+        // a dropped modality arm (0 * features): its backward is skipped, its gradients are zeros
+        auto zero_grads_on_drop = [&](int mod, float* begin, float* end) {
+          b.cur_mod = mod;
+          b.push_on_drop("modality_drop", [=](cudaStream_t s) {
+            return cudaMemsetAsync(begin, 0, (size_t)(end - begin) * 4, s) == cudaSuccess ? 0 : 1;
+          });
+          b.cur_mod = 0;
+        };
         if (key.has_audio) {
           float* g_w = gf; float* g_b = g_w + (long long)D * Fp;
           gf = g_b + D;
+          if (key.moddrop) b.cur_mod = 1;
           if (!wgrad_rows(dfused, E, D, arows.data, act_dt, Fp, 0, Fp, N, g_w, g_b, "proj_audio_wgrad")) return false;
+          b.cur_mod = 0;
+          if (key.moddrop) zero_grads_on_drop(1, g_w, gf);
         }
         if (key.has_video) {
+          float* g_video = gf;
+          if (key.moddrop) b.cur_mod = 2;
           float* g_w = gf; float* g_b = g_w + (long long)D * 512;
           gf = g_b + D;
           if (!wgrad_rows(dfused + v_off, E, D, feat.data, act_dt, 512, 0, 512, N, g_w, g_b, "proj_video_wgrad")) return false;
@@ -2483,6 +2541,8 @@ bool build_encoder_train_plan(avh_handle* h, Plan* plan, bool sizing, size_t* by
                             graw_dt))
               return false;
           }
+          b.cur_mod = 0;
+          if (key.moddrop) zero_grads_on_drop(2, g_video, gf);
         }
         grad_mark((g_ln + 2ll * E) - grads, GF);         // modality projections + lip ResNet
       }
@@ -2823,23 +2883,28 @@ static void read_graphs_env() {
   graphs_env = ((ev != nullptr && ev[0] == '0') || dbg != nullptr || dbg2 != nullptr) ? 0 : 1;
 }
 
-// LayerDrop: a step of a dropped layer is skipped and an on-drop step of a kept one; steps outside the layers always run
-// (plans without LayerDrop have an empty layer_skip)
+// LayerDrop / modality dropout: a step of a dropped layer or modality arm is skipped and an on-drop step of a kept one;
+// steps outside the layers and arms always run (plans without LayerDrop have an empty layer_skip, plans without modality
+// dropout mod_drop 0)
 static bool step_runs(const avh::Plan* p, const avh::Step& st) {
-  const bool dropped = st.layer >= 0 && st.layer < (int)p->layer_skip.size() && p->layer_skip[st.layer] != 0;
+  const bool dropped = (st.layer >= 0 && st.layer < (int)p->layer_skip.size() && p->layer_skip[st.layer] != 0) ||
+                       (st.mod != 0 && st.mod == p->mod_drop);
   return dropped == st.on_drop;
 }
 
 // capture every maximal run of plan-internal steps (they only enqueue kernels / async copies) into its own graph; in a
-// plan with LayerDrop a run also ends where the layer changes, so that a dropped layer's graphs are skipped whole
+// plan with LayerDrop (modality dropout) a run also ends where the layer (modality arm) changes, so that a dropped
+// layer's (arm's) graphs are skipped whole
 static bool capture_segments(avh::Plan* p, cudaStream_t s) {
   bool ok = true;
   size_t i = 0;
-  const bool by_layer = p->key.layerdrop;
+  const bool by_layer = p->key.layerdrop, by_mod = p->key.moddrop;
   while (ok && i < p->steps.size()) {
     if (p->steps[i].direct) { ++i; continue; }
     size_t j = i;
-    while (j < p->steps.size() && !p->steps[j].direct && (!by_layer || p->steps[j].layer == p->steps[i].layer)) ++j;
+    while (j < p->steps.size() && !p->steps[j].direct && (!by_layer || p->steps[j].layer == p->steps[i].layer) &&
+           (!by_mod || p->steps[j].mod == p->steps[i].mod))
+      ++j;
     const long long before = avh::g_launches.load();
     cudaGraph_t graph = nullptr;
     ok = cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal) == cudaSuccess;
@@ -2873,7 +2938,7 @@ static int replay_range(avh::Plan* p, size_t begin, size_t end, cudaStream_t s) 
   while (sg < p->segments.size() && p->segments[sg].begin < begin) ++sg;
   while (i < end) {
     if (sg < p->segments.size() && p->segments[sg].begin == i && p->segments[sg].end <= end) {
-      if (step_runs(p, p->steps[i])) {      // a segment holds the steps of one layer when LayerDrop is possible
+      if (step_runs(p, p->steps[i])) {      // a segment holds the steps of one layer (arm) when LayerDrop (modality dropout) is possible
         AVH_CUDA_OK(cudaGraphLaunch(p->segments[sg].exec, s));
         avh::count_launch(p->segments[sg].kernels);
         avh::g_graph_launches.fetch_add(1, std::memory_order_relaxed);
@@ -3003,6 +3068,8 @@ int avh_forward(avh_handle* h, const void* video, int video_dtype, const void* a
   return run_steps(h, p, 0, p->steps.size(), reinterpret_cast<cudaStream_t>(stream));
 }
 
+static int take_mod_drop(avh_handle* h, const void* video, const void* audio);
+
 int avh_forward_train(avh_handle* h, const void* video, int video_dtype, const void* audio, int audio_dtype,
                       const int64_t* audio_strides, const uint8_t* padding_mask, int B, int T, int output_layer,
                       const avh_train_args* ta, void* out, int out_dtype, void* stream) {
@@ -3022,15 +3089,19 @@ int avh_forward_train(avh_handle* h, const void* video, int video_dtype, const v
   AVH_CHECK(ta->bn_momentum > 0.f && ta->bn_momentum <= 1.f, "bad BatchNorm momentum");
   AVH_CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const int md = take_mod_drop(h, video, audio);
+  if (md < -1) return 1;
   avh::PlanKey key;
   key.kind = avh::PlanKind::TrainForward;
   key.B = B; key.T = T;
   key.has_video = video != nullptr; key.has_audio = audio != nullptr; key.has_mask = padding_mask != nullptr;
   key.output_layer = output_layer;
   key.stream = s;
+  key.moddrop = md >= 0;
   avh::Plan* p = avh::get_plan(h, key);
   if (p == nullptr) return 1;
   h->last_plan = p;
+  p->mod_drop = md > 0 ? md : 0;
   p->args = avh::CallArgs();
   p->args.video = video; p->args.video_dt = video_dtype;
   p->args.audio = audio; p->args.audio_dt = audio_dtype;
@@ -3094,6 +3165,66 @@ int avh_compute_logits(const void* feats, int f_dtype, int64_t ldf, const void* 
 int avh_sum_squares(const void* x, int dtype, int64_t n, double* acc, void* stream) {
   AVH_CHECK(x != nullptr && acc != nullptr, "null pointer");
   return avh::launch_sumsq(x, dtype, n, acc, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int avh_compute_logits_backward(const void* feats, int f_dtype, int64_t ldf, const void* emb, int e_dtype, int64_t lde, int64_t M,
+                                int V, int K, int sim_type, float logit_temp, const float* logits, const float* dlogits,
+                                int64_t ldo, float* dfeats, int64_t ldd_f, float* demb, int64_t ldd_e, float* dbias, void* stream) {
+  AVH_CHECK(feats != nullptr && emb != nullptr && dlogits != nullptr, "null pointer");
+  AVH_CHECK(sim_type == 0 || sim_type == 1, "sim_type must be 0 (dot) or 1 (cosine)");
+  AVH_CHECK(sim_type == 0 || logits != nullptr, "the cosine backward reads the forward's logits");
+  AVH_CHECK(logit_temp != 0.f, "logit_temp must be non-zero");
+  AVH_CHECK(M >= 0 && V >= 0 && K > 0 && ldf >= K && lde >= K && ldo >= V, "bad leading dimension");
+  AVH_CHECK((dfeats == nullptr || ldd_f >= K) && (demb == nullptr || ldd_e >= K), "bad gradient leading dimension");
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  float* scratch = nullptr;      // norms, row / column sums, split-contraction partials: stream-ordered, freed after use
+  if (M > 0 && V > 0)
+    AVH_CUDA_OK(cudaMallocAsync(reinterpret_cast<void**>(&scratch), (size_t)avh::logits_bwd_scratch_floats(M, V, K) * sizeof(float), s));
+  const int rc = avh::launch_logits_bwd(feats, f_dtype, ldf, emb, e_dtype, lde, M, V, K, sim_type, 1.0f / logit_temp, logits, dlogits,
+                                        ldo, dfeats, ldd_f, demb, ldd_e, dbias, scratch, s);
+  if (scratch != nullptr) AVH_CUDA_OK(cudaFreeAsync(scratch, s));
+  return rc;
+}
+
+int avh_set_modality_drop(avh_handle* h, int which) {
+  AVH_CHECK(h != nullptr && h->cfg.reserved[0] == 0, "modality dropout belongs to an AV-HuBERT handle");
+  AVH_CHECK(which >= 0 && which <= 2, "which must be 0 (none), 1 (audio) or 2 (video)");
+  h->next_mod_drop = which;
+  return 0;
+}
+
+// The pending avh_set_modality_drop decision (consumed): -1 = not a pretraining step
+static int take_mod_drop(avh_handle* h, const void* video, const void* audio) {
+  const int md = h->next_mod_drop;
+  h->next_mod_drop = -1;
+  if (md >= 0 && (video == nullptr || audio == nullptr)) {
+    avh::set_last_error("modality dropout needs both modalities");
+    return -2;
+  }
+  return md;
+}
+
+int avh_train_features_pen(avh_handle* h, double* acc, void* stream) {
+  AVH_CHECK(h != nullptr && acc != nullptr, "null argument");
+  const avh::Plan* p = h->last_plan;
+  AVH_CHECK(p != nullptr && (p->key.kind == avh::PlanKind::TrainForward || p->key.training()) && p->fused_buf != nullptr,
+            "features_pen follows a training-mode forward of an AV-HuBERT handle");
+  AVH_CUDA_OK(cudaSetDevice(h->device));
+  const int E = h->cfg.modality_fuse == AVH_FUSE_CONCAT ? 2 * h->cfg.encoder_embed_dim : h->cfg.encoder_embed_dim;
+  return avh::launch_sumsq(p->fused_buf, p->fused_dt, (long long)p->key.B * p->key.T * E, acc, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int avh_set_features_pen_grad(avh_handle* h, const float* dpen, void* stream) {
+  AVH_CHECK(h != nullptr, "null handle");
+  avh::Plan* p = h->last_plan;
+  AVH_CHECK(p != nullptr && p->dpen != nullptr && p->fwd_done,
+            "the features_pen gradient belongs to a pretraining avh_full_train_forward (avh_set_modality_drop first)");
+  cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  AVH_CHECK(s == p->key.stream, "the features_pen gradient must be set on the stream of its forward");
+  AVH_CUDA_OK(cudaSetDevice(h->device));
+  if (dpen != nullptr) AVH_CUDA_OK(cudaMemcpyAsync(p->dpen, dpen, sizeof(float), cudaMemcpyDeviceToDevice, s));
+  else AVH_CUDA_OK(cudaMemsetAsync(p->dpen, 0, sizeof(float), s));
+  return 0;
 }
 
 int avh_bn_stats_count(avh_handle* h, int64_t* n_floats) {
@@ -3251,14 +3382,19 @@ int avh_full_train_forward(avh_handle* h, const void* video, int video_dtype, co
   AVH_CHECK(B >= 1 && T >= 1 && (long long)B * T < (1ll << 20), "bad batch");
   AVH_CUDA_OK(cudaSetDevice(h->device));
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+  const int md = take_mod_drop(h, video, audio);
+  if (md < -1) return 1;
   avh::PlanKey key;
   key.kind = avh::PlanKind::FullTrain;
   key.B = B; key.T = T;
   key.has_video = video != nullptr; key.has_audio = audio != nullptr; key.has_mask = padding_mask != nullptr;
   key.stream = s;
+  key.moddrop = key.pen = md >= 0;
   avh::Plan* p = training_plan(h, key, true, s);
   if (p == nullptr) return 1;
   h->last_plan = p;
+  p->mod_drop = md > 0 ? md : 0;
+  if (p->dpen != nullptr) AVH_CUDA_OK(cudaMemsetAsync(p->dpen, 0, sizeof(float), s));      // no dL/dpen unless set
   p->args = avh::CallArgs();
   p->args.video = video; p->args.video_dt = video_dtype;
   p->args.audio = audio; p->args.audio_dt = audio_dtype;

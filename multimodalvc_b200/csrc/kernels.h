@@ -105,6 +105,14 @@ int launch_mask_bct(const void* in, int dt, long long sb, long long sc, long lon
 // out[m,v] = (<F_m, E_v> + bias[v]) * inv_temp (mode 0) or / max(|F_m| |E_v|, 1e-6) * inv_temp (mode 1), fp32
 int launch_logits(const void* F, int f_dt, long long ldf, const void* E, int e_dt, long long lde, const float* bias,
                   float* out, long long ldo, long long M, int V, int K, int mode, float inv_temp, cudaStream_t stream);
+// its backward from the forward's logits and dL/dlogits [M,V] (row stride ldo): dF [M,K] (ldd_f), dE [V,K] (ldd_e), dbias [V]
+// (each may be null), fp32; scratch: logits_bwd_scratch_floats(M, V, K) floats
+int launch_logits_bwd(const void* F, int f_dt, long long ldf, const void* E, int e_dt, long long lde, long long M, int V, int K,
+                      int mode, float inv_temp, const float* logits, const float* dlogits, long long ldo, float* dF, long long ldd_f,
+                      float* dE, long long ldd_e, float* dbias, float* scratch, cudaStream_t stream);
+long long logits_bwd_scratch_floats(long long M, int V, int K);
+// dx[i] += dpen[0] * scale * x[i] (dpen: a device word)
+int launch_pen_grad(const float* x, float* dx, long long n, const float* dpen, float scale, cudaStream_t stream);
 // *acc = sum of squares of x (float64; acc is zeroed first)
 int launch_sumsq(const void* x, int dt, long long n, double* acc, cudaStream_t stream);
 

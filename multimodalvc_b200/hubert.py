@@ -242,10 +242,12 @@ class _TailTrainFn(torch.autograd.Function):
 class _FullTrainFn(torch.autograd.Function):
     """The whole fine-tuning step (feature_grad_mult > 0): lip ResNet + projections + fusion + encoder with the library's
     forward (activations saved in the plan) and backward; `spec` = [(buffer shape, to_param)] describes how the flat
-    gradient buffer maps onto the parameters that follow."""
+    gradient buffer maps onto the parameters that follow.  `drop` None: the fine-tuning step, one output; 0 / 1 / 2: a
+    pretraining step dropping no / the audio / the video modality, outputs (y, features_pen) — dL/dfeatures_pen enters
+    the extractors through the library's backward."""
 
     @staticmethod
-    def forward(ctx, model, reg, video, audio, pm_u8, fgm, spec, *params):
+    def forward(ctx, model, reg, video, audio, pm_u8, fgm, spec, drop, *params):
         handle = model._ensure_handle()
         ref = video if video is not None else audio
         dev = ref.device
@@ -256,28 +258,39 @@ class _FullTrainFn(torch.autograd.Function):
         out = torch.empty(B, T, model.encoder_embed_dim, device=dev, dtype=out_dtype)
         strides = (ctypes.c_int64 * 3)(*audio.stride()) if audio is not None else None
         vp = ctypes.c_void_p
+        lib = _lib.load()
         with torch.cuda.device(dev):
             stream = torch.cuda.current_stream(dev).cuda_stream
             reg.set_on(handle)
-            _lib.check(_lib.load().avh_full_train_forward(
+            if drop is not None:
+                _lib.check(lib.avh_set_modality_drop(handle, int(drop)))
+            _lib.check(lib.avh_full_train_forward(
                 handle, vp(video.data_ptr()) if video is not None else None, _DTYPES[video.dtype] if video is not None else 0,
                 vp(audio.data_ptr()) if audio is not None else None, _DTYPES[audio.dtype] if audio is not None else 0, strides,
                 vp(pm_u8.data_ptr()) if pm_u8 is not None else None, B, T, float(fgm), 0.1, vp(out.data_ptr()),
                 _DTYPES[out_dtype], vp(stream)))
         ctx.handle, ctx.stream, ctx.spec, ctx.reg = handle, stream, spec, reg
+        ctx.pretrain = drop is not None
         ctx.model, ctx.params = model, params
         ctx.flags = (int(video is not None), int(audio is not None))
         ctx.keep = (video, audio)                      # the backward re-reads the frames (stem patches are recomputed)
         ctx.dtypes = [p.dtype for p in params]
-        return out
+        if not ctx.pretrain:
+            return out
+        return out, model._train_features_pen(handle, B * T * model.embed)
 
     @staticmethod
-    def backward(ctx, dout):
+    def backward(ctx, dout, dpen=None):
         dev = dout.device
         dout = dout.contiguous()
         if dout.dtype not in _DTYPES:
             dout = dout.float()
         lib = _lib.load()
+        if ctx.pretrain:
+            dp = dpen.detach().float().contiguous() if dpen is not None else None
+            with torch.cuda.device(dev):
+                _lib.check(lib.avh_set_features_pen_grad(ctx.handle, ctypes.c_void_p(dp.data_ptr()) if dp is not None else None,
+                                                         ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
         n = ctypes.c_int64()
         _lib.check(lib.avh_full_grad_count(ctx.handle, ctx.flags[0], ctx.flags[1], ctypes.byref(n)))
         flat = backward_flat(ctx.handle, dout, None, n.value, ctx.dtypes, ctx.stream, ctx.model)
@@ -291,7 +304,53 @@ class _FullTrainFn(torch.autograd.Function):
         assert off == n.value, (off, n.value)
         if flat.reduced:
             ctx.model._grad_sync.mark_reduced(ctx.params)
-        return (None, None, None, None, None, None, None, *ctx.reg.layer_grads(grads, flat.reduced))
+        return (None, None, None, None, None, None, None, None, *ctx.reg.layer_grads(grads, flat.reduced))
+
+
+class _LogitsFn(torch.autograd.Function):
+    """AVHubertModel.compute_logits (hubert.py:576-589) differentiable: avh_compute_logits forward, avh_compute_logits_backward
+    backward.  feats [M,K] (row stride free, unit column stride), emb [V,K], bias [V] or None -> fp32 logits [M,V].  With
+    sim_type 0, logit_temp 1 and a bias this is final_proj (hubert.py:654)."""
+
+    @staticmethod
+    def forward(ctx, feats, emb, bias, sim_type, logit_temp):
+        dev = feats.device
+        f2 = feats if feats.dtype in _DTYPES and feats.stride(-1) == 1 else feats.float().contiguous()
+        e2 = emb.detach()
+        if e2.dtype not in _DTYPES or not e2.is_contiguous():
+            e2 = e2.float().contiguous()
+        b = bias.detach().float().contiguous() if bias is not None else None
+        (M, K), V = f2.shape, e2.size(0)
+        out = torch.empty(M, V, device=dev, dtype=torch.float32)
+        ldf = f2.stride(0) if M > 1 else K
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _lib.check(_lib.load().avh_compute_logits(
+                ctypes.c_void_p(f2.data_ptr()), _DTYPES[f2.dtype], ldf, ctypes.c_void_p(e2.data_ptr()), _DTYPES[e2.dtype], K,
+                ctypes.c_void_p(b.data_ptr()) if b is not None else None, M, V, K, sim_type, float(logit_temp),
+                ctypes.c_void_p(out.data_ptr()), V, ctypes.c_void_p(stream)))
+        ctx.save_for_backward(f2, e2, out)
+        ctx.args = (ldf, sim_type, float(logit_temp), bias is not None, feats.dtype, emb.dtype)
+        return out
+
+    @staticmethod
+    def backward(ctx, dout):
+        f2, e2, out = ctx.saved_tensors
+        ldf, sim_type, temp, has_bias, f_dt, e_dt = ctx.args
+        dev = dout.device
+        dout = dout.float().contiguous()
+        (M, K), V = f2.shape, e2.size(0)
+        df = torch.empty(M, K, device=dev, dtype=torch.float32) if ctx.needs_input_grad[0] else None
+        de = torch.empty(V, K, device=dev, dtype=torch.float32) if ctx.needs_input_grad[1] else None
+        db = torch.empty(V, device=dev, dtype=torch.float32) if has_bias and ctx.needs_input_grad[2] else None
+        vp = lambda t: ctypes.c_void_p(t.data_ptr()) if t is not None else None
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _lib.check(_lib.load().avh_compute_logits_backward(
+                vp(f2), _DTYPES[f2.dtype], ldf, vp(e2), _DTYPES[e2.dtype], K, M, V, K, sim_type, temp, vp(out), vp(dout), V,
+                vp(df), K, vp(de), K, vp(db), ctypes.c_void_p(stream)))
+        return (df.to(f_dt) if df is not None else None, de.to(e_dt) if de is not None else None,
+                db.to(e_dt) if db is not None else None, None, None)
 
 
 class AVHubertModel(nn.Module):
@@ -636,9 +695,10 @@ class AVHubertModel(nn.Module):
                                   activation_dropout=c.activation_dropout, attention_dropout=c.attention_dropout,
                                   layerdrop=c.encoder_layerdrop)
 
-    def _extract_finetune_full(self, source, padding_mask, mask):
+    def _extract_finetune_full(self, source, padding_mask, mask, drop=None):
         """The whole model differentiable (feature_grad_mult > 0, hubert.py:538-547 with GradMultiply): SURVEY row A18 /
-        BASELINE config 5 as stated."""
+        BASELINE config 5 as stated.  Returns (y, padding_mask, features_pen); `drop` (0 / 1 / 2: pretraining step, the
+        modality dropped) makes features_pen differentiable, None (fine-tuning) leaves it None."""
         c = self.cfg
         if mask and c.masking_type == "input":
             with torch.no_grad():
@@ -654,11 +714,12 @@ class AVHubertModel(nn.Module):
             raise NotImplementedError("the training step takes normalised float video")
         params, spec = self.full_parameters(video is not None, audio is not None)
         reg = self._step_regularization()
-        y = _FullTrainFn.apply(self, reg, video, audio, pm_u8, float(c.feature_grad_mult), spec, *params)
+        out = _FullTrainFn.apply(self, reg, video, audio, pm_u8, float(c.feature_grad_mult), spec, drop, *params)
+        y, pen = out if drop is not None else (out, None)
         self._last_train_args = (reg.seed, list(reg.skip))      # what the step used: tests rebuild its masks from it
         if video is not None:
             self._read_back_bn_stats(handle, dev)
-        return y, pm
+        return y, pm, pen
 
     @torch.no_grad()
     def _read_back_bn_stats(self, handle, dev):
@@ -680,10 +741,11 @@ class AVHubertModel(nn.Module):
             off += 2 * C
         self._eval_stale = True
 
-    def _extract_finetune_trainable(self, source, padding_mask, mask, output_layer):
+    def _extract_finetune_trainable(self, source, padding_mask, mask, output_layer, drop=None):
         """Fine-tuning step with frozen feature extractors (feature_grad_mult <= 0: the reference runs them under
         no_grad, hubert.py:538-547).  Extractors + fusion run as in the training-mode forward (batch-statistics
-        BatchNorm), the fused features feed the differentiable tail: layer_norm -> post_extract_proj -> encoder."""
+        BatchNorm), the fused features feed the differentiable tail: layer_norm -> post_extract_proj -> encoder.
+        Returns (y, padding_mask, features_pen) as _extract_finetune_full; here features_pen is a constant."""
         c = self.cfg
         if output_layer is not None:
             raise NotImplementedError("the training step runs the whole encoder (output_layer=None)")
@@ -691,11 +753,13 @@ class AVHubertModel(nn.Module):
             raise NotImplementedError("attention_dropout > 0 in training mode is not implemented (0.0 in every "
                                       "shipped fine-tune config, avhubert/conf/finetune/*.yaml)")
         if c.feature_grad_mult > 0:
-            return self._extract_finetune_full(source, padding_mask, mask)
+            return self._extract_finetune_full(source, padding_mask, mask, drop)
         self._sync_trained_weights()                             # an optimizer step changed the weights: refresh
         with torch.no_grad():
-            # only the "fused" stage is read: no regularisation and no draws, so the step draws its coins once
-            y1, pm = self._extract_finetune_nograd(source, padding_mask, mask=mask, output_layer=1, _regularise=False)
+            # only the "fused" stage is read: no regularisation and no draws, so the step draws its coins once; the
+            # modality dropout happens here (the fused features hold the dropped arm's zeros)
+            y1, pm = self._extract_finetune_nograd(source, padding_mask, mask=mask, output_layer=1, _regularise=False,
+                                                   _drop=drop)
             B, T, _ = y1.shape
             fused = self.read_stage("fused", B * T * self.embed).view(B, T, self.embed)
         self._param_versions = [p._version for p in self.parameters()]
@@ -704,20 +768,31 @@ class AVHubertModel(nn.Module):
         reg = self._step_regularization()
         y = _TailTrainFn.apply(self, reg, fused, pm_u8, *self.tail_parameters())
         self._last_train_args = (reg.seed, list(reg.skip))      # what the step used: tests rebuild its masks from it
-        return y, pm
+        pen = self._train_features_pen(self._handle, B * T * self.embed) if drop is not None else None
+        return y, pm, pen
+
+    def _train_features_pen(self, handle, numel):
+        """features.float().pow(2).mean() (hubert.py:629) over the fused features of the last training forward."""
+        dev = self.encoder.layer_norm.weight.device
+        acc = torch.empty(1, device=dev, dtype=torch.float64)
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _lib.check(_lib.load().avh_train_features_pen(handle, ctypes.c_void_p(acc.data_ptr()), ctypes.c_void_p(stream)))
+        return (acc / numel).float().squeeze(0)
 
     def extract_finetune(self, source, padding_mask=None, mask=False, ret_conv=False, output_layer=None, lengths=None):
         """avhubert/hubert.py:694-745 (see _extract_finetune_nograd).  In .train() with gradients enabled and
         cfg.trainable, the call is differentiable w.r.t. the tail's parameters (fusion LayerNorm, post_extract_proj,
         encoder): SURVEY row A18 with the feature extractors frozen."""
         if self.training and torch.is_grad_enabled() and self.cfg.trainable:
-            return self._extract_finetune_trainable(source, padding_mask, mask, output_layer)
+            y, pm, _ = self._extract_finetune_trainable(source, padding_mask, mask, output_layer)
+            return y, pm
         return self._extract_finetune_nograd(source, padding_mask, mask=mask, ret_conv=ret_conv, output_layer=output_layer,
                                              lengths=lengths)
 
     @torch.no_grad()
     def _extract_finetune_nograd(self, source, padding_mask=None, mask=False, ret_conv=False, output_layer=None, lengths=None,
-                                 _regularise=True):
+                                 _regularise=True, _drop=None):
         """avhubert/hubert.py:694-745.  source = {'audio': [B,F,T] | None, 'video': [B,1,T,88,88] | None};
         padding_mask bool [B,T] (True = padded).  Returns (x [B,T,D], padding_mask).  With cfg.ragged == "packed" (bf16
         mode) ragged batches run packed; `lengths` (valid frames per clip) may be given to skip reading the mask back."""
@@ -747,6 +822,8 @@ class AVHubertModel(nn.Module):
             lib = _lib.load()
             with torch.cuda.device(dev):
                 stream = torch.cuda.current_stream(dev).cuda_stream
+                if _drop is not None:          # pretraining step: the modality dropout decision (forward / _forward_train)
+                    _lib.check(lib.avh_set_modality_drop(handle, int(_drop)))
                 _lib.check(lib.avh_forward_train(
                     handle,
                     ctypes.c_void_p(src_video.data_ptr()) if src_video is not None else None, video_dt,
@@ -1020,18 +1097,92 @@ class AVHubertModel(nn.Module):
                            _want_features=ret_conv)
         return (res["features"] if ret_conv else res["x"]), res["padding_mask"]
 
-    @torch.no_grad()
     def forward(self, source, target_list=None, padding_mask=None, mask=True, features_only=False, output_layer=None,
                 _want_features=True):
-        """The masked-prediction forward, avhubert/hubert.py:591-674, in EVAL mode (what fairseq's validation step and
-        ``extract_features`` run; the training-mode pass needs the backward of SURVEY row A18).  Input span masking
-        (``masking_type='input'``: frames substituted before the frontends) or feature masking (``'feature'``: token
-        rows replaced by ``mask_emb`` after post_extract_proj), the encoder, then — unless ``features_only`` —
-        final_proj, cosine / dot logits against the label embeddings and the masked / unmasked selections.  Returns
-        the reference's dict.  numpy / torch CPU generators are consumed in the reference's order."""
+        """The masked-prediction forward, avhubert/hubert.py:591-674.  Input span masking (``masking_type='input'``:
+        frames substituted before the frontends) or feature masking (``'feature'``: token rows replaced by ``mask_emb``
+        after post_extract_proj), the encoder, then — unless ``features_only`` — final_proj, cosine / dot logits against
+        the label embeddings and the masked / unmasked selections.  Returns the reference's dict.  numpy / torch CPU
+        generators are consumed in the reference's order.
+
+        In .train() with gradients enabled and ``cfg.trainable``: the pretraining step (fairseq's av_hubert_pretraining
+        task), differentiable — modality dropout, ``features_pen`` and the logits carry gradients into final_proj, the
+        label embeddings, the tail and encoder and, with feature_grad_mult > 0, the feature extractors (_forward_train).
+        Otherwise the EVAL-mode pass (fairseq's validation step, ``extract_features``)."""
+        if self.training and torch.is_grad_enabled() and self.cfg.trainable:
+            return self._forward_train(source, target_list, padding_mask, mask, features_only, output_layer)
+        return self._forward_eval(source, target_list, padding_mask, mask, features_only, output_layer, _want_features)
+
+    def _forward_train(self, source, target_list, padding_mask, mask, features_only, output_layer):
+        """hubert.py:591-674 in training mode: span masking (video, then audio), the two modality-dropout coins
+        (hubert.py:611-616: with probability modality_dropout one modality's features become zeros — audio with
+        probability audio_dropout, else video; the dropped extractor still runs, its parameters get zero gradients),
+        features_pen over the fused features, the training step of the tail / whole model (its LayerDrop coins drawn
+        after the modality coins), then final_proj and the logits, both differentiable on the device."""
+        c = self.cfg
+        if features_only or output_layer is not None:
+            raise NotImplementedError("the training-mode pretraining forward computes the whole encoder and the logits "
+                                      "(features_only=False, output_layer=None)")
+        if mask and c.masking_type != "input":
+            raise NotImplementedError("masking_type='feature' in training mode is not implemented (the training plan "
+                                      "would substitute token rows and differentiate mask_emb)")
+        if c.attention_dropout > 0:
+            raise NotImplementedError("attention_dropout > 0 in training mode is not implemented (0.0 in every "
+                                      "shipped fine-tune config, avhubert/conf/finetune/*.yaml)")
+        src_audio, src_video = source["audio"], source["video"]
+        if src_audio is None or src_video is None:
+            raise ValueError("forward / extract_features need both modalities (forward_features fails on None in the "
+                             "reference, hubert.py:609-610); use extract_finetune for single-modality input")
+        if self.final_proj is None or self.num_classes is None:
+            raise RuntimeError("the masked-prediction head was removed (remove_pretraining_modules) or the model was "
+                               "built without dictionaries")
+        if c.sim_type not in ("dot", "cosine"):
+            raise NotImplementedError
+        if padding_mask is None:       # the reference evaluates ~padding_mask (hubert.py:663)
+            raise TypeError("forward(features_only=False) needs a padding_mask (bad operand type for unary ~: 'NoneType')")
+        mask_indices = None
+        if mask:
+            src_video, mi_v = self.apply_input_mask(src_video, padding_mask, target_list)
+            src_audio, mi_a = self.apply_input_mask(src_audio, padding_mask, target_list)
+            mask_indices = torch.logical_or(mi_a, mi_v)      # None here fails as in the reference (prob 0 + mask=True)
+        modality_drop_prob, audio_drop_prob = np.random.random(), np.random.random()
+        drop = 0
+        if modality_drop_prob < c.modality_dropout:
+            drop = 1 if audio_drop_prob < c.audio_dropout else 2
+        if target_list is not None:
+            T = src_video.size(2)
+            if self.feat2tar_ratio * T > min(t.size(1) for t in target_list):
+                raise NotImplementedError("labels shorter than the features (forward_targets would trim the features "
+                                          "mid-forward, hubert.py:553-558): trim the inputs to the labelled frames")
+            idx = (torch.arange(T).float() * self.feat2tar_ratio).long()
+            target_list = [t[:, idx.to(t.device)] for t in target_list]
+        x, pm, pen = self._extract_finetune_trainable({"audio": src_audio, "video": src_video}, padding_mask, False, None,
+                                                      drop)
+        B, T, D = x.shape
+        proj_x = _LogitsFn.apply(x.reshape(B * T, D), self.final_proj.weight, self.final_proj.bias, 0, 1.0)
+        if self.untie_final_proj:
+            proj_x_list = proj_x.chunk(len(self.num_classes), dim=-1)
+        else:
+            proj_x_list = [proj_x for _ in self.num_classes]
+        sim = 1 if c.sim_type == "cosine" else 0
+        label_embs_list = self.label_embs_concat.split(self.num_classes, 0)
+        logit_list = [_LogitsFn.apply(p, e, None, sim, float(c.logit_temp)) for p, e in zip(proj_x_list, label_embs_list)]
+        sel_m = torch.logical_and(mask_indices, ~pm).view(-1)
+        sel_u = torch.logical_and(~mask_indices, ~pm).view(-1)
+        return {
+            "logit_m_list": [lg[sel_m] for lg in logit_list],
+            "logit_u_list": [lg[sel_u] for lg in logit_list],
+            "target_m_list": [t.reshape(-1).to(x.device)[sel_m].long() for t in target_list],
+            "target_u_list": [t.reshape(-1).to(x.device)[sel_u].long() for t in target_list],
+            "padding_mask": pm,
+            "features_pen": pen,
+        }
+
+    @torch.no_grad()
+    def _forward_eval(self, source, target_list, padding_mask, mask, features_only, output_layer, _want_features):
         if self.training:
-            raise NotImplementedError("the pretraining forward runs in eval mode here (modality dropout and the "
-                                      "losses' backward belong to the training configuration, SURVEY row A18)")
+            raise NotImplementedError("the pretraining forward in .train() needs cfg.trainable and gradients enabled "
+                                      "(this is the eval-mode pass)")
         src_audio, src_video = source["audio"], source["video"]
         if src_audio is None or src_video is None:
             raise ValueError("forward / extract_features need both modalities (forward_features fails on None in the "
